@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on host cores
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs (dump_outputs)
 
 A "step" (default workload `ssp`) is one full SSP step of the reference recipe with accumulation_steps=1
 (BASELINE.md §3): zero_grad → 4 backbones forward (2 online with grad, 2 EMA targets) → heads → -mean(cos)/1 →
@@ -58,7 +59,15 @@ def parse():
                          "16-bit patch matrix (u8p, one kernel; default where the step accepts it) or into fp32 views (u8), "
                          "or the reference DataLoader's fp32 views (fp32, 154 MB/step)")
     ap.add_argument("--no-overlap", action="store_true", help="N>1: plain all-reduce after backward instead of the overlapped one")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned, and the model state it left, to DIR/<name>.npy "
+                         "(float32 / float64, at most 64 MB) so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def peaks():
@@ -235,6 +244,35 @@ def eager_gpu_baseline(dev, B):
                     f"batch {B}, same GPU (stock PyTorch kernels)"}
 
 
+DUMP_SAMPLE = 1 << 23     # float32 elements of the parameter sample: 32 MB, within the 64 MB budget of a dump
+
+
+def dump_outputs(dirname, result, model, probs=None):
+    """What the last timed step hands its caller: its return value (`result.npy`), the class probabilities of the
+    forward-only workload (`probs.npy`), and for training workloads the parameters and buffers the step updated, as
+    the L2 norm of every state_dict tensor (`state_norms.npy`, float64, state_dict order) and the values of the
+    concatenated state_dict at DUMP_SAMPLE positions drawn without replacement by numpy's default_rng(0), in
+    ascending order (`state_sample.npy`; every value when the state is smaller than that)."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    out = {"result": result.detach().float().reshape(-1).cpu().numpy()}
+    if probs is not None:
+        out["probs"] = probs.detach().float().cpu().numpy()
+    else:
+        sd = list(model.state_dict().values())
+        out["state_norms"] = np.array([float(v.detach().double().norm()) for v in sd])
+        flat = torch.cat([v.detach().reshape(-1).float() for v in sd])
+        if flat.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_SAMPLE, replace=False))
+        else:
+            idx = np.arange(flat.numel())
+        out["state_sample"] = flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy()
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    for name, a in out.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def main():
     args = parse()
     claim_stdout()
@@ -274,6 +312,7 @@ def main():
     # ---- model / optimizer / step of the chosen workload --------------------------------------------------------
     torch.manual_seed(42)
     sync = None
+    step_out = {}           # what the most recent step returned (and, forward-only, its class probabilities)
     if args.workload in ("ssp", "accum8"):
         model = vit2spn.DualStreamNetwork().to(dev).train()
         model.loss_mode = args.loss
@@ -333,7 +372,8 @@ def main():
 
         def step(a, b):
             with torch.no_grad():
-                return torch.softmax(model(a), dim=1)[:, 0].sum()
+                step_out["probs"] = torch.softmax(model(a), dim=1)
+                return step_out["probs"][:, 0].sum()
         units_per_step, unit, flop_per_unit = B, "images/s", FLOP_PER_IMAGE_FWD
         metric = "forward-only feature extraction images/sec, ViT-Tiny b1024 (BASELINE config 5)"
         workload = "FineTunedModel eval forward (backbone + head + softmax), batch 1024, no_grad (ref:octmnist_ft_vit2spn.py:129-137)"
@@ -363,12 +403,18 @@ def main():
     warm = max(args.warmup, 3)
     for _ in range(warm):
         step(x1, x2)
+
+    def timed_step():
+        step_out["result"] = step(x1, x2)
+
     l0 = _lib.lib.v2s_launch_count() + getattr(model, "graph_replayed_kernels", 0)
     sampler.mark_begin()
-    ms_total = timed(lambda: step(x1, x2), args.steps)
+    ms_total = timed(timed_step, args.steps)
     sampler.mark_end()
     # kernels of this library launched in the timed region (those replayed from a CUDA graph included)
     launches = int(_lib.lib.v2s_launch_count() + getattr(model, "graph_replayed_kernels", 0) - l0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step_out["result"], model, step_out.get("probs"))
     # host-side cost of enqueueing one step (no device wait inside): tells CPU-bound from GPU-bound
     torch.cuda.synchronize()
     h0 = time.perf_counter()

@@ -1,8 +1,8 @@
 """Golden vectors that pin the fine-tune / evaluation path (SURVEY §8f N2) to the REFERENCE.
 
-Run in the build container only (needs /root/reference):   python tests/golden/make_finetune_golden.py
+Needs the original ViT-2SPN:   V2S_REFERENCE_DIR=/path/to/ViT-2SPN python tests/golden/make_finetune_golden.py
 
-`ViTBackbone` and `FineTunedModel` are AST-extracted from /root/reference/octmnist_ft_vit2spn.py:63-87 and executed
+`ViTBackbone` and `FineTunedModel` are AST-extracted from $V2S_REFERENCE_DIR/octmnist_ft_vit2spn.py:63-87 and executed
 unmodified (``from_pretrained`` redirected to the random-init tiny config: no checkpoint offline).  One training step
 as the script does it (ref:95-104,187-192: train mode, weighted CrossEntropyLoss, Adam lr 1e-4 with L2 1e-4) and one
 evaluation forward (ref:129-137: eval mode, softmax) are recorded in tests/golden/finetune_golden.npz.  Dropout(0.5)

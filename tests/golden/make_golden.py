@@ -1,13 +1,13 @@
 """Generate the golden vectors that pin ``oracle/vit2spn_oracle.py`` to the REFERENCE.
 
-Run in the build container only (needs /root/reference, which does not exist on the GPU box):
+Needs a checkout of the original mrsaraei/ViT-2SPN, which the repository does not contain:
 
-    python tests/golden/make_golden.py
+    V2S_REFERENCE_DIR=/path/to/ViT-2SPN python tests/golden/make_golden.py
 
 The reference scripts train at import time, so their class definitions (``ViTBackbone``,
 ``DualStreamNetwork``) are AST-extracted from
-  * /root/reference/ssp_ssl/ssl_vit2spn_scratch.py  (random-init ``ViTModel(ViTConfig(...))``)
-  * /root/reference/ssp_vit2spn_tiny.py             (``from_pretrained`` redirected to the same
+  * $V2S_REFERENCE_DIR/ssp_ssl/ssl_vit2spn_scratch.py  (random-init ``ViTModel(ViTConfig(...))``)
+  * $V2S_REFERENCE_DIR/ssp_vit2spn_tiny.py             (``from_pretrained`` redirected to the same
     random-init tiny config: no checkpoint / network offline)
 and executed, unmodified, against the installed ``transformers`` / ``torch``.  The oracle's
 deterministic state (numpy PCG64) is loaded into them with ``load_state_dict(strict=True)``;
@@ -30,7 +30,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)
 sys.path.insert(0, ROOT)
 from oracle import vit2spn_oracle as orc  # noqa: E402
 
-REF = "/root/reference"
+REF = os.environ.get("V2S_REFERENCE_DIR", "")        # empty: the original is not available
 
 
 def extract_classes(path, names, namespace):

@@ -1,8 +1,8 @@
 """Golden vectors that pin the single-stream variant (SURVEY §8f N3) to the REFERENCE.
 
-Run in the build container only (needs /root/reference):   python tests/golden/make_single_golden.py
+Needs the original ViT-2SPN:   V2S_REFERENCE_DIR=/path/to/ViT-2SPN python tests/golden/make_single_golden.py
 
-`ViTBackbone` and `SingleStreamNetwork` are AST-extracted from /root/reference/dsn_ssn/ssp_single.py:93-138 and
+`ViTBackbone` and `SingleStreamNetwork` are AST-extracted from $V2S_REFERENCE_DIR/dsn_ssn/ssp_single.py:93-138 and
 executed unmodified (``from_pretrained`` redirected to the random-init tiny config).  One micro-step as the script does
 it (ref:195-206: loss = -mean(cos)/accumulation_steps with accumulation_steps = 8, backward, Adam lr 1e-4,
 `update_target_network()` with its default momentum 0.99) is recorded in tests/golden/single_golden.npz; Dropout(0.3)

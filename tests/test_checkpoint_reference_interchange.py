@@ -1,65 +1,55 @@
-"""Checkpoint interchange with the REAL reference code (SURVEY §8f N4).  Needs /root/reference (present in the build
-container only; skipped elsewhere): the reference's own `DualStreamNetwork`, `save_checkpoint` and `load_checkpoint`
-(AST-extracted from ref:ssp_vit2spn_tiny.py:53-72,109-166, executed unmodified) write and read the files."""
+"""Checkpoint interchange with the reference (SURVEY §8f N4): a file in the layout the reference's ``save_checkpoint``
+writes (ref:ssp_vit2spn_tiny.py:53-61, stored in tests/golden/reference_checkpoint_layout.json by
+tests/golden/make_checkpoint_golden.py) loads here bit for bit, and the file this library writes has that same layout
+and loads the way the reference's ``load_checkpoint`` reads it (ref:63-72: ``torch.load``, then ``load_state_dict``
+into the model and into ``torch.optim.Adam``)."""
+import json
 import os
 import sys
 
-import pytest
 import torch
-import torch.nn as nn
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-REF_SCRIPT = "/root/reference/ssp_vit2spn_tiny.py"
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_SCRIPT), reason="the reference is not mounted on this machine")
+import make_checkpoint_golden as mk  # noqa: E402  (helpers only)
+
+with open(mk.GOLDEN) as _f:
+    G = json.load(_f)
 
 
-def _reference():
-    import make_golden as mg
-    ns = mg.reference_namespace("ssp_vit2spn_tiny.py")
-    ns["os"] = os
-    mg.extract_classes(REF_SCRIPT, {"save_checkpoint", "load_checkpoint"}, ns)
-    return ns
+def _same_adam_state(a, b):
+    assert set(a) == set(b) and len(a) == 408                   # Adam state of the 400 + 8 trainable tensors
+    for k in a:
+        for f in ("exp_avg", "exp_avg_sq"):
+            assert torch.equal(a[k][f].cpu(), b[k][f].cpu()), (k, f)
+        assert float(a[k]["step"]) == float(b[k]["step"])
 
 
 def test_reference_checkpoint_loads_here_and_ours_loads_there(tmp_path):
     import vit2spn
-    from oracle import vit2spn_oracle as orc
-    ns = _reference()
-    state = orc.init_state(31, 0.01)
-    ref_model = ns["DualStreamNetwork"]()
-    ref_model.load_state_dict(state, strict=True)
-    ref_opt = torch.optim.Adam(ref_model.parameters(), lr=1e-4)
-    # give the reference optimizer real state: one step on synthetic gradients for every trainable tensor
-    g = torch.Generator().manual_seed(0)
-    for p in ref_model.parameters():
-        if p.requires_grad:
-            p.grad = torch.randn(p.shape, generator=g) * 1e-3
-    ref_opt.step()
+    ref = mk.reference_checkpoint(10, 0.25)
+    assert mk.layout(ref) == G                                  # torch.optim.Adam still writes the stored layout
     path = os.path.join(tmp_path, "ref_ckpt.pth")
-    ns["save_checkpoint"](ref_model, ref_opt, 10, 0.25, path)                 # the reference writes ...
+    torch.save(ref, path)
     ours = vit2spn.DualStreamNetwork()
     ours_opt = vit2spn.FusedAdam(ours.parameters(), lr=1e-4)
-    _, _, epoch, loss = vit2spn.load_checkpoint(ours, ours_opt, path)         # ... this library reads
+    _, _, epoch, loss = vit2spn.load_checkpoint(ours, ours_opt, path)           # a reference file, read here
     assert epoch == 10 and loss == 0.25
-    ref_sd, our_sd = ref_model.state_dict(), ours.state_dict()
+    ref_sd, our_sd = ref["model_state_dict"], ours.state_dict()
     assert list(ref_sd) == list(our_sd)
     assert all(torch.equal(ref_sd[k], our_sd[k]) for k in ref_sd)
-    r_state, o_state = ref_opt.state_dict()["state"], ours_opt.state_dict()["state"]
-    assert set(r_state) == set(o_state) and len(r_state) == 408               # Adam state of the 400 + 8 trainable tensors
-    assert len(ref_opt.state_dict()["param_groups"][0]["params"]) == 808 == len(ours_opt.state_dict()["param_groups"][0]["params"])
-    for k in r_state:
-        for f in ("exp_avg", "exp_avg_sq"):
-            assert torch.equal(r_state[k][f], o_state[k][f].cpu()), (k, f)
-        assert float(r_state[k]["step"]) == float(o_state[k]["step"])
-    # and back: this library writes, the reference's load_checkpoint reads
+    _same_adam_state(ref["optimizer_state_dict"]["state"], ours_opt.state_dict()["state"])
+
+    # and back: this library writes the reference's layout, and the reference's way of reading it restores the state
     back = os.path.join(tmp_path, "our_ckpt.pth")
     vit2spn.save_checkpoint(ours, ours_opt, 11, 0.5, back)
-    ref2 = ns["DualStreamNetwork"]()
-    ref2_opt = torch.optim.Adam(ref2.parameters(), lr=1e-4)
-    ns["device"] = torch.device("cpu")
-    _, _, epoch2, loss2 = ns["load_checkpoint"](ref2, ref2_opt, back)
-    assert epoch2 == 11 and loss2 == 0.5
-    assert all(torch.equal(ref2.state_dict()[k], ref_sd[k]) for k in ref_sd)
-    assert len(ref2_opt.state_dict()["state"]) == 408
+    ck = torch.load(back)
+    assert mk.layout(ck) == G
+    assert ck["epoch"] == 11 and ck["loss"] == 0.5
+    assert all(torch.equal(ck["model_state_dict"][k], ref_sd[k]) for k in ref_sd)
+    params = [torch.nn.Parameter(torch.zeros(shape), requires_grad=not name.startswith(mk.FROZEN))
+              for name, shape, _ in G["model_state_dict"]]
+    torch_opt = torch.optim.Adam(params, lr=1e-4)
+    torch_opt.load_state_dict(ck["optimizer_state_dict"])
+    _same_adam_state(ref["optimizer_state_dict"]["state"], torch_opt.state_dict()["state"])
