@@ -26,7 +26,9 @@
 extern "C" {
 #endif
 
-#define V2S_ABI_VERSION 3 /* 3: v2s_infonce_loss, v2s_preprocess_u8_patches, v2s_group.x_format (was a reserved zero field) */
+#define V2S_ABI_VERSION 3 /* 3: v2s_infonce_loss, v2s_preprocess_u8_patches, v2s_group.x_format (was a reserved zero field);
+                             additive to 3: v2s_group_outputs, v2s_backbone_forward_ex / v2s_backbone_backward_ex,
+                             v2s_test_attention which = 2 */
 
 /* compute modes */
 #define V2S_MODE_FP32 0 /* fp32 activations + fp32 SIMT GEMMs: the "fp32 check mode" of north_star */
@@ -114,6 +116,24 @@ int v2s_backbone_backward(const v2s_group_t* host_groups, int n_groups, int batc
 int v2s_backbone_backward_range(const v2s_group_t* host_groups, int n_groups, int batch, int mode,
                                 void* workspace, int64_t workspace_bytes, int layer_hi, int layer_lo,
                                 void* stream);
+
+/* Per-layer outputs of one group (transformers' output_hidden_states / output_attentions).  Pass an array of n_groups
+ * of these, or NULL for none: with NULL (or every pointer NULL) the calls below launch exactly what the plain entry
+ * points launch.  A saved group's hidden[] must be the same in its forward and its backward call. */
+typedef struct v2s_group_outputs {
+  float* hidden[V2S_LAYERS + 1];        /* out: hidden_states[l] fp32 [batch,197,192]; all 13 or none. When set, the
+                                           group's residual stream lives here; a saved group's backward reads it back */
+  float* attn[V2S_LAYERS];              /* out: softmax(QK^T/8) fp32 [batch,3,197,197]; all 12 or none */
+  const float* dhidden[V2S_LAYERS + 1]; /* backward in: d loss / d hidden_states[l], added; NULL entries skipped.
+                                           dhidden[12] is v2s_group.dhidden (set one of the two).  Without dfeat and
+                                           dhidden[12] the backward starts at the highest l with a gradient: the
+                                           blocks above it are skipped and get no gradient */
+} v2s_group_outputs_t;
+int v2s_backbone_forward_ex(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs /* [n_groups] or NULL */,
+                            int n_groups, int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
+int v2s_backbone_backward_ex(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs, int n_groups,
+                             int batch, int mode, void* workspace, int64_t workspace_bytes, int layer_hi, int layer_lo,
+                             void* stream);
 
 /* projection_head + prediction_head on the concatenated online features and projection_head on
  * the target features (ref:ssp_vit2spn_tiny.py:153-158), fused with the loss
@@ -243,6 +263,8 @@ int v2s_test_gemm(int which, const void* a, const void* b, void* c, int m, int n
 int v2s_test_mlp(int mode, const void* a, const void* w1, const void* w2, const float* b1, const float* b2, void* u,
                  void* h, const float* resid, void* out, void* ln_out, const float* ln_gamma, const float* ln_beta,
                  float* ln_mean, float* ln_rstd, int m, int lp_f16, void* stream);
+/* which 0: forward (qkv -> ctx, lse); 1: backward (qkv, ctx, lse, dctx -> dqkv); 2: attention probabilities
+ * (qkv, lse -> fp32 [batch,3,197,197] written to ctx).  variant bit 0 = SIMT kernels, bit 1 = fp16 instead of bf16 */
 int v2s_test_attention(int which, const void* qkv, void* ctx, float* lse, const void* dctx, void* dqkv,
                        int batch, int variant, void* stream);
 /* reads and clears the device-side pipeline-protocol error flag of the tcgen05 kernels (0 = ok) */

@@ -36,6 +36,11 @@ class Group(C.Structure):
     ]
 
 
+class GroupOutputs(C.Structure):
+    """struct v2s_group_outputs (include/vit2spn.h): per-layer outputs / gradients of one group."""
+    _fields_ = [("hidden", C.c_void_p * 13), ("attn", C.c_void_p * 12), ("dhidden", C.c_void_p * 13)]
+
+
 class Range(C.Structure):
     """struct v2s_range (include/vit2spn.h)."""
     _fields_ = [("params", C.c_void_p), ("grads", C.c_void_p), ("exp_avg", C.c_void_p),
@@ -56,6 +61,9 @@ _SIGS = {
     "v2s_backbone_forward": (C.c_int, [C.POINTER(Group), _i, _i, _i, _vp, _i64, _vp]),
     "v2s_backbone_backward": (C.c_int, [C.POINTER(Group), _i, _i, _i, _vp, _i64, _vp]),
     "v2s_backbone_backward_range": (C.c_int, [C.POINTER(Group), _i, _i, _i, _vp, _i64, _i, _i, _vp]),
+    "v2s_backbone_forward_ex": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), _i, _i, _i, _vp, _i64, _vp]),
+    "v2s_backbone_backward_ex": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), _i, _i, _i, _vp, _i64, _i, _i,
+                                           _vp]),
     "v2s_heads_loss_fwd_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _f, _i,
                                          _vp, _i64, _vp]),
     "v2s_heads_loss_fwd_bwd_amp": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _i,

@@ -969,7 +969,140 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
   }
 }
 
+// ---- attention probabilities (ViTModel output_attentions) -------------------------------------------
+// P = exp(S/8 - lse) as fp32 [B,3,197,197], recomputed from qkv and the forward's log-sum-exp: the hot forward kernel
+// never materialises P in fp32.  S = Q K^T is issued exactly as attn_fwd_persist_kernel issues it (same TMA boxes, same
+// UMMA 128x208x64 order), so S is bit-identical and each row sums to 1 up to fp32 rounding.  One CTA per (query tile,
+// head, image, group), 160 threads: warp 0 loads and issues, warps 1..4 own one query row per thread (TMEM lane quarter
+// warp & 3).  A 197-float row is 788 B, not a multiple of 16, so neither TMA nor 128-bit stores can write the output in
+// place: the tile is staged densely in shared memory (over the dead Q / K tiles) and copied out with coalesced 4-byte
+// stores - the tile's rows are contiguous in the output, so the copy is one linear run of up to 128 x 197 floats.
+constexpr int PR_OFF_Q = 0;
+constexpr int PR_OFF_K = Q_TILE_BYTES;                        // 16384
+constexpr int PR_STG_BYTES = QT * NT * 4;                     // 100864: [128][197] fp32 (odd row stride: no conflicts)
+constexpr int PR_OFF_BAR = PR_STG_BYTES;                      // past both the Q / K tiles and the staging tile
+constexpr int PR_SMEM = PR_OFF_BAR + 64 + 1024;
+constexpr int PR_THREADS = 160;
+static_assert(PR_OFF_K % 1024 == 0 && PR_OFF_K + KV_TILE_BYTES <= PR_STG_BYTES, "attention-probabilities smem map");
+
+struct alignas(64) AttnProbsParams {
+  CUtensorMap tmQ[MAXG], tmKV[MAXG];
+  const float* lse[MAXG];
+  float* probs[MAXG];
+  int* err_flag;
+};
+
+template <typename LP>
+__global__ void __launch_bounds__(PR_THREADS, 2) attn_probs_tc_kernel(const __grid_constant__ AttnProbsParams p) {
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  uint64_t* bar_load = reinterpret_cast<uint64_t*>(smem + PR_OFF_BAR);
+  uint64_t* bar_s = bar_load + 1;
+  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bar_s + 1);
+  float* stg = reinterpret_cast<float*>(smem);
+  const int t = blockIdx.x & 1, h = blockIdx.x >> 1, b = blockIdx.y, g = blockIdx.z;
+  const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;
+  const int nrows = NT - t * QT < QT ? NT - t * QT : QT;
+
+  if (warp == 0) {
+    if (lane == 0) {
+      ptx::mbar_init(bar_load, 1); ptx::mbar_init(bar_s, 1);
+      ptx::fence_barrier_init();
+    }
+    __syncwarp();
+    ptx::tmem_alloc(tmem_ptr, 256);
+    ptx::tmem_relinquish();
+  }
+  ptx::tc_fence_before();
+  __syncthreads();
+  ptx::tc_fence_after();
+  const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_ptr, 0);
+  ptx::pdl_wait();
+  ptx::pdl_launch_dependents();     // after the wait: see the dependent-launch note in gemm_tc.cu
+
+  if (warp == 0) {
+    if (ptx::elect_one()) {
+      ptx::mbar_arrive_expect_tx(bar_load, Q_TILE_BYTES + KV_TILE_BYTES);
+      ptx::tma_load_3d(smem + PR_OFF_Q, &p.tmQ[g], bar_load, h * DH, t * QT, b);
+      ptx::tma_load_3d(smem + PR_OFF_K, &p.tmKV[g], bar_load, D + h * DH, 0, b);
+    }
+    __syncwarp();
+    ptx::mbar_wait(bar_load, 0, p.err_flag, 61);
+    ptx::tc_fence_after();
+    const uint32_t idesc_s = make_idesc_lp(LP::kIdescFmt, QT, KPAD, 0, 0);
+    const uint32_t sq = ptx::smem_u32(smem) + PR_OFF_Q, sk = ptx::smem_u32(smem) + PR_OFF_K;
+    if (ptx::elect_one()) {
+#pragma unroll
+      for (int k = 0; k < DH / 16; ++k) mma(tmem_base, sq + k * 32, 16, sk + k * 32, 16, idesc_s, k > 0);
+      ptx::umma_commit(bar_s);
+    }
+    __syncwarp();
+  } else {
+    const int q = warp & 3;
+    const int row = q * 32 + lane;
+    const int qrow = t * QT + row;
+    const bool valid = row < nrows;
+    const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16);
+    const float lse2 = valid ? __ldg(p.lse[g] + ((int64_t)b * NH + h) * NT + qrow) * LOG2E : 0.f;
+    float* srow = stg + row * NT;
+    uint32_t r[32];
+    ptx::mbar_wait(bar_s, 0, p.err_flag, 62);     // S complete: the Q / K tiles are dead, staging may overwrite them
+    ptx::tc_fence_after();
+#pragma unroll 1
+    for (int c = 0; c < 6; ++c) {
+      ptx::tmem_ld_32x32(taddr + c * 32, r);
+      ptx::tmem_ld_wait();
+      if (valid) {
+#pragma unroll
+        for (int i = 0; i < 32; ++i) srow[c * 32 + i] = ptx::ex2_approx(fmaf(__uint_as_float(r[i]), SCALE_LOG2E, -lse2));
+      }
+    }
+    ptx::tmem_ld_32x16(taddr + 192, r);
+    ptx::tmem_ld_wait();
+    if (valid) {
+#pragma unroll
+      for (int i = 0; i < NT - 192; ++i) srow[192 + i] = ptx::ex2_approx(fmaf(__uint_as_float(r[i]), SCALE_LOG2E, -lse2));
+    }
+  }
+  ptx::tc_fence_before();
+  __syncthreads();
+  {
+    float* dst = p.probs[g] + (((int64_t)b * NH + h) * NT + t * QT) * NT;
+    const int n = nrows * NT;
+    for (int i = threadIdx.x; i < n; i += PR_THREADS) dst[i] = stg[i];
+  }
+  if (warp == 0) {
+    ptx::tc_fence_after();
+    ptx::tmem_dealloc(tmem_base, 256);
+  }
+}
+
 }  // namespace
+
+int launch_attn_probs_tc(const void* const* qkv, const float* const* lse, float* const* probs, int groups, int B,
+                         cudaStream_t s, int lp_f16) {
+  AttnProbsParams p;
+  memset(&p, 0, sizeof(p));
+  p.err_flag = tc_err_flag();
+  for (int g = 0; g < groups; ++g) {
+    if (!lse[g] || !probs[g]) { set_error("attention probabilities: group %d has no lse / output", g); return 1; }
+    V2S_TRY(tmap_get_3d(&p.tmQ[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, QT, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmKV[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, KPAD, true, 128));
+    p.lse[g] = lse[g];
+    p.probs[g] = probs[g];
+  }
+  static bool attr[MAX_DEVICES] = {false};
+  if (!attr[cur_device()]) {
+    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_tc_kernel<LpBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PR_SMEM));
+    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_tc_kernel<LpF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PR_SMEM));
+    attr[cur_device()] = true;
+  }
+  const dim3 grid(NH * 2, B, groups);
+  if (lp_f16) V2S_CUDA_OK(launch_pdl(attn_probs_tc_kernel<LpF16>, grid, dim3(PR_THREADS), (size_t)PR_SMEM, s, p));
+  else V2S_CUDA_OK(launch_pdl(attn_probs_tc_kernel<LpBf16>, grid, dim3(PR_THREADS), (size_t)PR_SMEM, s, p));
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
 
 int launch_attn_fwd_tc(const void* const* qkv, void* const* ctx, float* const* lse, int groups, int B,
                        cudaStream_t s, int lp_f16) {

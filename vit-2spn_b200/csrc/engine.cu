@@ -34,9 +34,9 @@ static int n_recs = 0;
 static int n_events = 0;   // events created so far (recs[i].a/b valid for i < n_events)
 static const char* names[] = {"gemm_patch", "gemm_qkv", "gemm_proj", "gemm_fc1", "gemm_fc2", "gemm_dgrad",
                               "gemm_wgrad", "attn_fwd", "attn_bwd", "ln_fwd", "ln_bwd", "colsum", "misc", "heads", "gemm_mlp_fwd",
-                              "gemm_mlp_bwd"};
+                              "gemm_mlp_bwd", "attn_probs"};
 enum { C_PATCH, C_QKV, C_PROJ, C_FC1, C_FC2, C_DGRAD, C_WGRAD, C_ATTN_F, C_ATTN_B, C_LN_F, C_LN_B, C_COLSUM, C_MISC,
-       C_HEADS, C_MLP_F, C_MLP_B, C_COUNT };
+       C_HEADS, C_MLP_F, C_MLP_B, C_ATTN_P, C_COUNT };
 struct Scope {
   int idx = -1;
   cudaStream_t st;
@@ -206,6 +206,61 @@ int launch_attention_bwd(const void* const* qkv, const void* const* ctx, const f
   return launch_attn_bwd_simt(qkv, ctx, lse, dctx, dqkv, groups, B, at, s);
 }
 
+// fp32 attention probabilities of the groups that asked for them (v2s_group_outputs.attn), recomputed from qkv and lse
+int launch_attention_probs(const void* const* qkv, const float* const* lse, float* const* probs, int groups, int B, int at,
+                           cudaStream_t s) {
+  // algorithmic bytes: Q and K read once, lse, the fp32 probabilities written once
+  prof::Scope scope(prof::C_ATTN_P, 2.0 * B * NH * (double)NT * NT * DH * groups, s,
+                    ((double)B * NT * 2 * D * (at ? 2.0 : 4.0) + (double)B * NH * NT * 4 + (double)B * NH * NT * NT * 4) * groups);
+  if (at != AT_F32 && tc_enabled()) return launch_attn_probs_tc(qkv, lse, probs, groups, B, s, at == AT_F16);
+  return launch_attn_probs_simt(qkv, lse, probs, groups, B, at, s);
+}
+
+// d loss / d hidden_states[k] joins the residual-stream gradient (groups whose dh entry is NULL are skipped); for k > 0 its
+// column sums also go to the fc2 bias gradient of block k - 1, whose output hidden_states[k] is
+int add_hidden_grads(int k, const float* const* dh, float* const* dx, void* const* dxlp, const v2s_group_t* gs, int G, int B,
+                     int at, const Plan& p, cudaStream_t s) {
+  const float* a[MAXG]; float* o[MAXG]; void* lp[MAXG]; float* cs[MAXG]; int n = 0;
+  for (int g = 0; g < G; ++g)
+    if (dh[g]) { a[n] = dh[g]; o[n] = dx[g]; lp[n] = dxlp[g]; cs[n] = k > 0 ? gs[g].grads + layer_off(k - 1) + L_B2 : nullptr; ++n; }
+  if (!n) return 0;
+  prof::Scope sc(prof::C_MISC, (double)p.M * D * (12 + p.es) * n, s);
+  return launch_residual_grad_add(a, o, lp, cs, n, B, at, s);
+}
+
+// v2s_group_outputs checks shared by forward and backward: hidden / attn all or none, 16-byte aligned hidden states
+int check_outputs(const v2s_group_outputs_t* o, int g, const char* what) {
+  if (!o) return 0;
+  int nh = 0, na = 0;
+  for (int l = 0; l <= NL; ++l) {
+    if (!o->hidden[l]) continue;
+    ++nh;
+    if (reinterpret_cast<uintptr_t>(o->hidden[l]) & 15) { set_error("%s: group %d: hidden[%d] is not 16-byte aligned", what, g, l); return 1; }
+  }
+  for (int l = 0; l < NL; ++l) na += o->attn[l] ? 1 : 0;
+  if (nh != 0 && nh != NL + 1) { set_error("%s: group %d: %d of the 13 hidden[] set (all or none)", what, g, nh); return 1; }
+  if (na != 0 && na != NL) { set_error("%s: group %d: %d of the 12 attn[] set (all or none)", what, g, na); return 1; }
+  return 0;
+}
+
+// The residual stream of a saved group that supplied hidden[] lives in the caller's tensors, and its backward reads
+// them back: remember per (workspace, stash slot) which hidden[0] the forward used, so that a backward given other
+// tensors (or none, or some where the forward had none) is an error rather than a silent wrong gradient.
+struct HiddenRec { const void* ws; int slot; const float* h0; };
+static HiddenRec g_hidden_rec[64];
+static int g_n_hidden_rec = 0;
+void record_hidden(const void* ws, int slot, const float* h0) {
+  for (int i = 0; i < g_n_hidden_rec; ++i)
+    if (g_hidden_rec[i].ws == ws && g_hidden_rec[i].slot == slot) { g_hidden_rec[i].h0 = h0; return; }
+  const int i = g_n_hidden_rec < 64 ? g_n_hidden_rec++ : (int)((reinterpret_cast<uintptr_t>(ws) / 1024 + (uintptr_t)slot) % 64);
+  g_hidden_rec[i] = {ws, slot, h0};
+}
+const HiddenRec* find_hidden(const void* ws, int slot) {
+  for (int i = 0; i < g_n_hidden_rec; ++i)
+    if (g_hidden_rec[i].ws == ws && g_hidden_rec[i].slot == slot) return &g_hidden_rec[i];
+  return nullptr;
+}
+
 int wgrad_split(int64_t rows) {
   int64_t s = rows / 1024;
   if (s < 1) s = 1;
@@ -218,8 +273,8 @@ int wgrad_split(int64_t rows) {
 // =============================================================================================
 // backbone forward
 // =============================================================================================
-static int backbone_forward_impl(const v2s_group_t* gs, int G, int B, int mode, void* ws, int64_t ws_bytes,
-                                 cudaStream_t st) {
+static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_t* outs, int G, int B, int mode,
+                                 void* ws, int64_t ws_bytes, cudaStream_t st) {
   if (mode < V2S_MODE_FP32 || mode > V2S_MODE_FP16) { set_error("bad compute mode %d", mode); return 1; }
   if (G < 1 || G > MAXG) { set_error("backbone_forward: 1..4 groups"); return 1; }
   if (B < 1) { set_error("backbone_forward: batch must be >= 1"); return 1; }
@@ -236,8 +291,14 @@ static int backbone_forward_impl(const v2s_group_t* gs, int G, int B, int mode, 
       set_error("backbone_forward: group %d: x_format %d (1 = 16-bit patch rows, 16-bit modes only)", g, gs[g].x_format);
       return 1;
     }
+    V2S_TRY(check_outputs(outs ? &outs[g] : nullptr, g, "backbone_forward"));
   }
   const int64_t M = p.M, MP = p.MP;
+  // hidden_states[0..12] / attention probabilities requested by group g (NULL / false: none)
+  auto hid = [&](int g) -> float* const* { return outs && outs[g].hidden[0] ? outs[g].hidden : nullptr; };
+  auto want_attn = [&](int g) { return outs && outs[g].attn[0]; };
+  for (int g = 0; g < G; ++g)
+    if (gs[g].slot >= 0) record_hidden(ws, gs[g].slot, hid(g) ? hid(g)[0] : nullptr);
 
   // ---- buffer resolution ----
   auto saved = [&](int g) { return gs[g].slot >= 0; };
@@ -270,7 +331,7 @@ static int backbone_forward_impl(const v2s_group_t* gs, int G, int B, int mode, 
     const bool two_pass = at != AT_F32 && tc_enabled();   // tensor-core GEMM into patch rows, then assemble tokens
     d.epi = two_pass ? EPI_STORE : EPI_PATCH;
     for (int g = 0; g < G; ++g) {
-      x_cur[g] = reinterpret_cast<float*>(saved(g) ? sb(g, p.s_x[0]) : fb(g, p.f_xa));
+      x_cur[g] = hid(g) ? hid(g)[0] : reinterpret_cast<float*>(saved(g) ? sb(g, p.s_x[0]) : fb(g, p.f_xa));
       // scratch for the [B*196,192] patch rows: the x_mid buffer of block 0 (written later)
       float* tmp = reinterpret_cast<float*>(saved(g) ? sb(g, p.s_layer[0].x_mid) : fb(g, p.f_xb));
       d.A[g] = patches[g];
@@ -308,10 +369,14 @@ static int backbone_forward_impl(const v2s_group_t* gs, int G, int B, int mode, 
         xout[g] = (float*)sb(g, p.s_x[l + 1]);
       } else {
         xn[g] = fb(g, p.f_xn); qkv[g] = fb(g, p.f_qkv); ctx[g] = fb(g, p.f_ctx);
-        mean[g] = nullptr; rstd[g] = nullptr; lse[g] = nullptr;
+        mean[g] = nullptr; rstd[g] = nullptr;
+        // the probabilities need the log-sum-exp: f_h is dead from the attention forward until fc1 (unfused path) and
+        // never written for these groups by the fused MLP kernel (d.h = NULL), and B*3*197 floats fit in it
+        lse[g] = want_attn(g) ? (float*)fb(g, p.f_h) : nullptr;
         xmid[g] = (float*)fb(g, p.f_xb); u[g] = nullptr; h[g] = fb(g, p.f_h);
         xout[g] = (float*)fb(g, p.f_xa);   // in place: x_in is dead once x_mid exists
       }
+      if (hid(g)) xout[g] = hid(g)[l + 1];
       gam[g] = gs[g].params + lo + L_LN1W; bet[g] = gs[g].params + lo + L_LN1B;
     }
     if (!ln1_done) {
@@ -332,6 +397,10 @@ static int backbone_forward_impl(const v2s_group_t* gs, int G, int B, int mode, 
       const void* cq[MAXG];
       for (int g = 0; g < G; ++g) cq[g] = qkv[g];
       V2S_TRY(launch_attention_fwd(cq, ctx, lse, G, B, at, st));
+      const float* al[MAXG]; float* ap[MAXG]; int na = 0;
+      for (int g = 0; g < G; ++g)
+        if (want_attn(g)) { cq[na] = qkv[g]; al[na] = lse[g]; ap[na] = outs[g].attn[l]; ++na; }
+      if (na) V2S_TRY(launch_attention_probs(cq, al, ap, na, B, at, st));
     }
     {  // attention output projection + residual
       GemmDesc d = make_gemm_desc();
@@ -439,15 +508,40 @@ static int backbone_forward_impl(const v2s_group_t* gs, int G, int B, int mode, 
 // layers [layer_lo, layer_hi) in descending order; layer_hi == NL starts from the feature / hidden-state gradient,
 // layer_lo == 0 finishes with the embedding gradients.  Between two calls the residual-stream gradient lives in the
 // workspace, so a full backward may be issued in several ranges (gradient all-reduce overlapped per range).
-static int backbone_backward_impl(const v2s_group_t* gs_in, int G_in, int B, int mode, void* ws, int64_t ws_bytes,
-                                  cudaStream_t st, int layer_hi = NL, int layer_lo = 0) {
+static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outputs_t* outs_in, int G_in, int B, int mode,
+                                  void* ws, int64_t ws_bytes, cudaStream_t st, int layer_hi = NL, int layer_lo = 0) {
   if (layer_lo < 0 || layer_hi > NL || layer_lo >= layer_hi) { set_error("backbone_backward: bad layer range [%d, %d)", layer_lo, layer_hi); return 1; }
   // keep only the groups that saved activations and want gradients
   v2s_group_t gs[MAXG];
+  const v2s_group_outputs_t* os[MAXG];
   int G = 0;
   for (int i = 0; i < G_in && i < MAXG; ++i)
-    if (gs_in[i].slot >= 0 && gs_in[i].grads) gs[G++] = gs_in[i];
+    if (gs_in[i].slot >= 0 && gs_in[i].grads) { os[G] = outs_in ? &outs_in[i] : nullptr; gs[G++] = gs_in[i]; }
   if (G == 0) { set_error("backbone_backward: no group with slot >= 0 and grads"); return 1; }
+  // per group: its saved hidden states (or NULL), d hidden_states[12], and the highest layer its gradient enters at
+  // (NL: dfeat / dhidden[12]; k < NL: only intermediate hidden-state gradients, the highest being dhidden[k])
+  float* const* hid[MAXG]; const float* dh_top[MAXG]; int top[MAXG];
+  int S = -1;              // where the backward starts: the blocks [S, NL) are skipped
+  for (int g = 0; g < G; ++g) {
+    V2S_TRY(check_outputs(os[g], g, "backbone_backward"));
+    hid[g] = os[g] && os[g]->hidden[0] ? os[g]->hidden : nullptr;
+    const HiddenRec* rec = find_hidden(ws, gs[g].slot);
+    if (rec && rec->h0 != (hid[g] ? hid[g][0] : nullptr)) {
+      set_error("backbone_backward: group %d: hidden[] differs from the forward that filled stash slot %d", g, gs[g].slot);
+      return 1;
+    }
+    const float* dh12 = os[g] ? os[g]->dhidden[NL] : nullptr;
+    if (dh12 && gs[g].dhidden) { set_error("backbone_backward: group %d sets both dhidden and outputs dhidden[12]", g); return 1; }
+    dh_top[g] = dh12 ? dh12 : gs[g].dhidden;
+    top[g] = (gs[g].dfeat || dh_top[g]) ? NL : -1;
+    for (int k = NL - 1; top[g] < 0 && k >= 0 && os[g]; --k)
+      if (os[g]->dhidden[k]) { top[g] = k; dh_top[g] = os[g]->dhidden[k]; }
+    if (top[g] > S) S = top[g];
+  }
+  if (S < 0) {
+    if (layer_hi == NL) { set_error("backbone_backward: group needs dfeat or dhidden"); return 1; }
+    S = NL;                // a later range of a backward whose start the caller already issued
+  }
   const Plan p = make_plan(B, mode);
   const int at = p.at;
   const int n_saved = max_slot(gs_in, G_in) + 1;
@@ -461,11 +555,12 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, int G_in, int B, int
   {
     const float *df[MAXG], *dh[MAXG]; int64_t dfs[MAXG]; void* lp[MAXG];
     for (int g = 0; g < G; ++g) {
-      if (layer_hi == NL && !gs[g].dfeat && !gs[g].dhidden) { set_error("backbone_backward: group needs dfeat or dhidden"); return 1; }
       dx[g] = (float*)bb(g, p.b_dx);
       dxlp[g] = at ? (void*)bb(g, p.b_dxlp) : (void*)dx[g];
       big[g] = bb(g, p.b_big); tmp[g] = bb(g, p.b_tmp);
-      df[g] = gs[g].dfeat; dfs[g] = gs[g].dfeat_stride > 0 ? gs[g].dfeat_stride : D; dh[g] = gs[g].dhidden;
+      // a group whose gradient enters below S starts from zero and gets its dhidden[] added on the way down
+      df[g] = S == NL ? gs[g].dfeat : nullptr; dfs[g] = gs[g].dfeat_stride > 0 ? gs[g].dfeat_stride : D;
+      dh[g] = top[g] == S ? dh_top[g] : nullptr;
       lp[g] = at ? dxlp[g] : nullptr;
     }
     if (layer_hi == NL) V2S_TRY(launch_pool_bwd(df, dfs, dh, dx, lp, G, B, at, st));
@@ -542,9 +637,19 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, int G_in, int B, int
     return launch_colsum(src, dst, G, (int)M, n, at, st);
   };
 
-  for (int l = layer_hi - 1; l >= layer_lo; --l) {
+  // the intermediate hidden-state gradients below the start (dhidden[S] itself started the stream above)
+  auto add_dhidden = [&](int k) -> int {
+    if (k >= S) return 0;
+    const float* a[MAXG];
+    for (int g = 0; g < G; ++g) a[g] = os[g] ? os[g]->dhidden[k] : nullptr;
+    return add_hidden_grads(k, a, dx, dxlp, gs, G, B, at, p, st);
+  };
+  auto x_in = [&](int g, int l) -> const float* { return hid[g] ? hid[g][l] : (const float*)sb(g, p.s_x[l]); };
+
+  for (int l = (layer_hi < S ? layer_hi : S) - 1; l >= layer_lo; --l) {
     const int64_t lo = layer_off(l);
     const LayerStash& s = p.s_layer[l];
+    V2S_TRY(add_dhidden(l + 1));
     void *u[MAXG], *h[MAXG], *xn2[MAXG], *ctx[MAXG], *qkv[MAXG], *xn1[MAXG];
     for (int g = 0; g < G; ++g) {
       u[g] = sb(g, s.u); h[g] = sb(g, s.h); xn2[g] = sb(g, s.xn2);
@@ -556,11 +661,11 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, int G_in, int B, int
     // chain kernels, dWo filling the attention kernel's partial last wave) measured the same or slightly slower.
     // ---- MLP ----
     if (!(merged && mlp_fuse)) V2S_TRY(wgrad(dxlp, D, h, DF, lo + L_W2, false));      // dW2 [192,768]
-    if (l == NL - 1) V2S_TRY(bias_grad(dxlp, D, lo + L_B2));               // lower blocks: fused into LN1-bwd above
+    if (l == S - 1) V2S_TRY(bias_grad(dxlp, D, lo + L_B2));                // lower blocks: fused into LN1-bwd above
     if (mlp_fuse) {
       // du = (dx W2) * gelu'(u) and d xn2 = du W1 chained on chip (du is still written once: dW1 needs it)
       MlpDesc d = make_mlp_desc();
-      d.mode = MLP_BWD; d.M = (int)M; d.groups = G; d.lp_f16 = at == AT_F16 ? 1 : 0; d.late_wait = (!merged && l != NL - 1 && !getenv("V2S_NO_LATE_WAIT")) ? 1 : 0;
+      d.mode = MLP_BWD; d.M = (int)M; d.groups = G; d.lp_f16 = at == AT_F16 ? 1 : 0; d.late_wait = (!merged && l != S - 1 && !getenv("V2S_NO_LATE_WAIT")) ? 1 : 0;
       for (int g = 0; g < G; ++g) {
         d.a[g] = dxlp[g]; d.w1[g] = weight_ptr(gs[g], at, lo + L_W1); d.w2[g] = weight_ptr(gs[g], at, lo + L_W2);
         d.u[g] = u[g]; d.h[g] = big[g]; d.out[g] = tmp[g];
@@ -575,7 +680,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, int G_in, int B, int
       else
         V2S_TRY(wgrad(big, DF, xn2, D, lo + L_W1, false, lo + L_B1));          // dW1 [768,192] and d b1
     } else {
-    V2S_TRY(dgrad(dxlp, D, lo + L_W2, DF, big, EPI_DGELU, u, l != NL - 1));   // du = (dx W2) * gelu'(u)
+    V2S_TRY(dgrad(dxlp, D, lo + L_W2, DF, big, EPI_DGELU, u, l != S - 1));    // du = (dx W2) * gelu'(u)
     V2S_TRY(wgrad(big, DF, xn2, D, lo + L_W1, false, lo + L_B1));          // dW1 [768,192] and d b1
     V2S_TRY(dgrad(big, DF, lo + L_W1, D, tmp, EPI_STORE, nullptr, true));  // d xn2
     }
@@ -608,7 +713,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, int G_in, int B, int
       const void* dy[MAXG]; const float *x[MAXG], *mu[MAXG], *rs[MAXG], *gm[MAXG];
       float *dg[MAXG], *db[MAXG], *cs[MAXG]; void* lp[MAXG];
       for (int g = 0; g < G; ++g) {
-        dy[g] = tmp[g]; x[g] = (const float*)sb(g, p.s_x[l]); mu[g] = (const float*)sb(g, s.mean1);
+        dy[g] = tmp[g]; x[g] = x_in(g, l); mu[g] = (const float*)sb(g, s.mean1);
         rs[g] = (const float*)sb(g, s.rstd1); gm[g] = gs[g].params + lo + L_LN1W;
         dg[g] = gs[g].grads + lo + L_LN1W; db[g] = gs[g].grads + lo + L_LN1B; lp[g] = at ? dxlp[g] : nullptr;
         // d b_2 of the block below = column sums of the gradient w.r.t. this block's input
@@ -620,6 +725,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, int G_in, int B, int
   }
   // ---- embeddings: d pos, d cls, d patch bias, d patch weight ----
   if (layer_lo == 0) {
+    V2S_TRY(add_dhidden(0));
     const float* cdx[MAXG]; float* gr[MAXG]; void* pt[MAXG];
     for (int g = 0; g < G; ++g) {
       cdx[g] = dx[g]; gr[g] = gs[g].grads;
@@ -837,20 +943,33 @@ int64_t v2s_workspace_bytes(int batch, int mode, int n_groups, int n_saved) {
 int v2s_backbone_forward(const v2s_group_t* groups, int n_groups, int batch, int mode, void* workspace,
                          int64_t workspace_bytes, void* stream) {
   if (!groups) { set_error("null groups"); return 1; }
-  return backbone_forward_impl(groups, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
+  return backbone_forward_impl(groups, nullptr, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int v2s_backbone_forward_ex(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, int n_groups, int batch, int mode,
+                            void* workspace, int64_t workspace_bytes, void* stream) {
+  if (!groups) { set_error("null groups"); return 1; }
+  return backbone_forward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int v2s_backbone_backward(const v2s_group_t* groups, int n_groups, int batch, int mode, void* workspace,
                           int64_t workspace_bytes, void* stream) {
   if (!groups) { set_error("null groups"); return 1; }
-  return backbone_backward_impl(groups, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
+  return backbone_backward_impl(groups, nullptr, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int v2s_backbone_backward_range(const v2s_group_t* groups, int n_groups, int batch, int mode, void* workspace,
                                 int64_t workspace_bytes, int layer_hi, int layer_lo, void* stream) {
   if (!groups) { set_error("null groups"); return 1; }
-  return backbone_backward_impl(groups, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream, layer_hi,
-                                layer_lo);
+  return backbone_backward_impl(groups, nullptr, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
+                                layer_hi, layer_lo);
+}
+
+int v2s_backbone_backward_ex(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, int n_groups, int batch,
+                             int mode, void* workspace, int64_t workspace_bytes, int layer_hi, int layer_lo, void* stream) {
+  if (!groups) { set_error("null groups"); return 1; }
+  return backbone_backward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
+                                layer_hi, layer_lo);
 }
 
 int v2s_heads_loss_fwd_bwd(const float* head_params, float* head_grads, const float* feat_online,
@@ -1030,7 +1149,8 @@ int v2s_prof_report(char* host_buf, int64_t buf_bytes) {
   return 0;
 }
 
-// test hook: which = 0 forward (qkv -> ctx, lse), 1 backward (qkv, ctx, lse, dctx -> dqkv);
+// test hook: which = 0 forward (qkv -> ctx, lse), 1 backward (qkv, ctx, lse, dctx -> dqkv), 2 probabilities (qkv, lse ->
+// fp32 [batch,3,197,197] in ctx);
 // variant 0 = tensor-core kernels, 1 = SIMT reference kernels; bf16 tensors, one backbone
 int v2s_test_attention(int which, const void* qkv, void* ctx, float* lse, const void* dctx, void* dqkv, int batch,
                        int variant, void* stream) {
@@ -1047,7 +1167,12 @@ int v2s_test_attention(int which, const void* qkv, void* ctx, float* lse, const 
     if (variant & 1) return launch_attn_bwd_simt(cq, cctx, cls, cd, dq, 1, batch, at, st);
     return launch_attn_bwd_tc(cq, cctx, cls, cd, dq, 1, batch, st, f16);
   }
-  set_error("v2s_test_attention: which must be 0 or 1");
+  if (which == 2) {
+    float* pr[1] = {static_cast<float*>(ctx)};
+    if (variant & 1) return launch_attn_probs_simt(cq, cls, pr, 1, batch, at, st);
+    return launch_attn_probs_tc(cq, cls, pr, 1, batch, st, f16);
+  }
+  set_error("v2s_test_attention: which must be 0, 1 or 2");
   return 1;
 }
 

@@ -487,6 +487,77 @@ __global__ void __launch_bounds__(256) attn_bwd_simt_kernel(G4<const T*> qkv, G4
   }
 }
 
+// attention probabilities P = exp(s / 8 - lse) as fp32 [B,3,197,197] (the SIMT twin of attn_probs_tc_kernel): s is
+// accumulated in the order attn_fwd_simt_kernel uses, so the rows of the check mode sum to 1 up to fp32 rounding.
+template <typename T>
+__global__ void __launch_bounds__(256) attn_probs_simt_kernel(G4<const T*> qkv, G4<const float*> lse, G4<float*> probs) {
+  extern __shared__ float sm[];
+  float* Ks = sm;                    // [197][65]
+  float* Qs = Ks + NT * ASTR;        // [8][64]
+  const int h = blockIdx.x, b = blockIdx.y, g = blockIdx.z;
+  const T* base = qkv.p[g] + (int64_t)b * NT * 3 * D;
+  for (int i = threadIdx.x; i < NT * DH; i += blockDim.x) {
+    const int t = i / DH, d = i % DH;
+    Ks[t * ASTR + d] = to_f<T>(base[(int64_t)t * 3 * D + D + h * DH + d]);
+  }
+  __syncthreads();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  float* Q = Qs + warp * DH;
+  const float scale = 0.125f;
+  for (int i = warp; i < NT; i += 8) {
+    Q[lane] = to_f<T>(base[(int64_t)i * 3 * D + h * DH + lane]);
+    Q[lane + 32] = to_f<T>(base[(int64_t)i * 3 * D + h * DH + lane + 32]);
+    __syncwarp();
+    const float li = lse.p[g][((int64_t)b * NH + h) * NT + i];
+    float* out = probs.p[g] + (((int64_t)b * NH + h) * NT + i) * NT;
+    for (int j = lane; j < NT; j += 32) {
+      float s = 0.f;
+#pragma unroll 16
+      for (int d = 0; d < DH; ++d) s = fmaf(Q[d], Ks[j * ASTR + d], s);
+      s *= scale;
+      out[j] = expf(s - li);
+    }
+    __syncwarp();
+  }
+}
+
+// dx += dh, dx_lp = dx in the activation type: the gradient w.r.t. an intermediate hidden state joins the residual-stream
+// gradient; dcol (optional) += column sums of dh, the part of the producing block's fc2 bias gradient that the fused
+// column sums of LN1-backward (taken before dh is added) do not see.  Launched without the dependent-launch attribute,
+// so it starts after its predecessor has completed.  Threads: 48 float4 columns x 5 row lanes.
+constexpr int RGA_RL = 256 / (D / 4);
+template <typename T>
+__global__ void __launch_bounds__(256) residual_grad_add_kernel(G4<const float*> dh, G4<float*> dx, G4<T*> dx_lp, G4<float*> dcol,
+                                                                int rows) {
+  __shared__ float4 part[RGA_RL][D / 4];
+  const int g = blockIdx.y;
+  const int c4 = threadIdx.x % (D / 4), rl = threadIdx.x / (D / 4);
+  const float4* __restrict__ a = reinterpret_cast<const float4*>(dh.p[g]);
+  float4* __restrict__ o = reinterpret_cast<float4*>(dx.p[g]);
+  T* __restrict__ ol = dx_lp.p[g];
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (rl < RGA_RL)
+    for (int r = blockIdx.x * RGA_RL + rl; r < rows; r += gridDim.x * RGA_RL) {
+      const int64_t i = (int64_t)r * (D / 4) + c4;
+      const float4 x = a[i];
+      float4 v = o[i];
+      v.x += x.x; v.y += x.y; v.z += x.z; v.w += x.w;
+      o[i] = v;
+      if (ol) store4<T>(ol + 4 * i, v.x, v.y, v.z, v.w);
+      acc.x += x.x; acc.y += x.y; acc.z += x.z; acc.w += x.w;
+    }
+  if (dcol.p[g]) {
+    if (rl < RGA_RL) part[rl][c4] = acc;
+    __syncthreads();
+    if (threadIdx.x < D / 4) {
+      float4 s = part[0][c4];
+      for (int k = 1; k < RGA_RL; ++k) { s.x += part[k][c4].x; s.y += part[k][c4].y; s.z += part[k][c4].z; s.w += part[k][c4].w; }
+      float* d = dcol.p[g] + 4 * c4;
+      atomicAdd(d, s.x); atomicAdd(d + 1, s.y); atomicAdd(d + 2, s.z); atomicAdd(d + 3, s.w);
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------
 // loss = -mean_i cos(p_i, z_i) / accum   (torch CosineSimilarity: each norm clamped at 1e-8)
 // dp   = grad_scale * d loss / d p.  Single CTA (B rows x 128), deterministic reduction.
@@ -974,6 +1045,32 @@ int launch_attn_bwd_simt(const void* const* qkv, const void* const* ctx, const f
                                                    pack4<const float*>(lse, groups), pack4<const T*>(dctx, groups),
                                                    pack4<T*>(dqkv, groups));
   });
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_attn_probs_simt(const void* const* qkv, const float* const* lse, float* const* probs, int groups, int B, int at,
+                           cudaStream_t s) {
+  const size_t smem = (size_t)(NT * ASTR + 8 * DH) * sizeof(float);
+  dim3 grid(NH, B, groups);
+  V2S_DISPATCH_AT(at, {
+    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_simt_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attn_probs_simt_kernel<T><<<grid, 256, smem, s>>>(pack4<const T*>(qkv, groups), pack4<const float*>(lse, groups),
+                                                      pack4<float*>(probs, groups));
+  });
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_residual_grad_add(const float* const* dh, float* const* dx, void* const* dx_lp, float* const* dcol, int groups, int B,
+                             int at, cudaStream_t s) {
+  for (int i = 0; i < groups; ++i)
+    if (reinterpret_cast<uintptr_t>(dh[i]) & 15) { set_error("hidden-state gradients must be 16-byte aligned"); return 1; }
+  const int rows = B * NT;
+  dim3 grid(grid_for(rows, RGA_RL, 148 * 2), groups);
+  V2S_DISPATCH_AT(at, residual_grad_add_kernel<T><<<grid, 256, 0, s>>>(pack4<const float*>(dh, groups), pack4<float*>(dx, groups),
+                                                                      pack4<T*>(at ? dx_lp : nullptr, groups),
+                                                                      pack4<float*>(dcol, groups), rows));
   V2S_LAUNCH_CHECK();
   return 0;
 }

@@ -27,6 +27,10 @@ int launch_pool_fwd(const float* const* hidden, float* const* feat, const int64_
 int launch_pool_bwd(const float* const* dfeat, const int64_t* dfeat_stride, const float* const* dhidden,
                     float* const* dx, void* const* dx_lp, int groups, int B, int at, cudaStream_t s);
 int launch_embed_bwd(const float* const* dx, float* const* grads, int groups, int B, cudaStream_t s);
+// dx (fp32, in/out) += dh; dx_lp (activation type, 16-bit modes only) = updated dx; [B,197,192] per group;
+// dcol (optional, per group) += column sums of dh
+int launch_residual_grad_add(const float* const* dh, float* const* dx, void* const* dx_lp, float* const* dcol, int groups, int B,
+                             int at, cudaStream_t s);
 
 // attention over qkv [B,197,576] (q|k|v, head h at columns h*64): ctx [B,197,192], lse [B,3,197]
 int launch_attn_fwd_simt(const void* const* qkv, void* const* ctx, float* const* lse, int groups, int B,
@@ -34,6 +38,9 @@ int launch_attn_fwd_simt(const void* const* qkv, void* const* ctx, float* const*
 int launch_attn_bwd_simt(const void* const* qkv, const void* const* ctx, const float* const* lse,
                          const void* const* dctx, void* const* dqkv, int groups, int B, int at,
                          cudaStream_t s);
+// attention probabilities exp(q k^T / 8 - lse) as fp32 probs [B,3,197,197], from qkv and the forward's lse
+int launch_attn_probs_simt(const void* const* qkv, const float* const* lse, float* const* probs, int groups, int B,
+                           int at, cudaStream_t s);
 
 // tcgen05 versions (bf16, or fp16 with lp_f16 = 1)
 int launch_attn_fwd_tc(const void* const* qkv, void* const* ctx, float* const* lse, int groups, int B,
@@ -41,6 +48,8 @@ int launch_attn_fwd_tc(const void* const* qkv, void* const* ctx, float* const* l
 
 int launch_attn_bwd_tc(const void* const* qkv, const void* const* ctx, const float* const* lse,
                        const void* const* dctx, void* const* dqkv, int groups, int B, cudaStream_t s, int lp_f16 = 0);
+int launch_attn_probs_tc(const void* const* qkv, const float* const* lse, float* const* probs, int groups, int B,
+                         cudaStream_t s, int lp_f16 = 0);
 
 int launch_infonce_loss(const float* p, const float* z_all, float* loss, float* row_loss, float* dp, int B, int n_keys,
                         long long label_offset, float temperature, int accum, float grad_scale, cudaStream_t s,

@@ -28,7 +28,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from ._lib import Group, lib, check, ptr, stream_ptr
+from ._lib import Group, GroupOutputs, lib, check, ptr, stream_ptr
 
 momentum = 0.999            # ref:ssp_vit2spn_tiny.py:38 (module-level constant in the reference)
 
@@ -261,18 +261,25 @@ def preprocess_u8_patches(src_u8, dtype=torch.bfloat16, out=None):
     return out
 
 
-def _run_forward(groups, batch, mode, ws):
-    arr = (Group * len(groups))(*groups)
-    base, nbytes = _aligned(ws)
-    check(lib.v2s_backbone_forward(arr, len(groups), batch, mode, C.c_void_p(base), nbytes, stream_ptr()),
-          "backbone_forward")
+def _outputs_array(outputs, n):
+    """ctypes array of `n` v2s_group_outputs (None entries: nothing requested), or None when nothing is requested."""
+    if outputs is None:
+        return None
+    return (GroupOutputs * n)(*[o if o is not None else GroupOutputs() for o in outputs])
 
 
-def _run_backward(groups, batch, mode, ws):
+def _run_forward(groups, batch, mode, ws, outputs=None):
     arr = (Group * len(groups))(*groups)
     base, nbytes = _aligned(ws)
-    check(lib.v2s_backbone_backward(arr, len(groups), batch, mode, C.c_void_p(base), nbytes, stream_ptr()),
-          "backbone_backward")
+    check(lib.v2s_backbone_forward_ex(arr, _outputs_array(outputs, len(groups)), len(groups), batch, mode,
+                                      C.c_void_p(base), nbytes, stream_ptr()), "backbone_forward")
+
+
+def _run_backward(groups, batch, mode, ws, outputs=None):
+    arr = (Group * len(groups))(*groups)
+    base, nbytes = _aligned(ws)
+    check(lib.v2s_backbone_backward_ex(arr, _outputs_array(outputs, len(groups)), len(groups), batch, mode,
+                                       C.c_void_p(base), nbytes, 12, 0, stream_ptr()), "backbone_backward")
 
 
 def _run_backward_range(groups, batch, mode, ws, layer_hi, layer_lo):
@@ -313,7 +320,7 @@ class ViTConfig:
 
     def __init__(self, hidden_size=192, num_hidden_layers=12, num_attention_heads=3, intermediate_size=768,
                  patch_size=16, image_size=224, output_hidden_states=False, layer_norm_eps=1e-12,
-                 hidden_act="gelu", num_channels=3, qkv_bias=True, initializer_range=0.02, **kw):
+                 hidden_act="gelu", num_channels=3, qkv_bias=True, initializer_range=0.02, output_attentions=False, **kw):
         self.hidden_size = hidden_size
         self.num_hidden_layers = num_hidden_layers
         self.num_attention_heads = num_attention_heads
@@ -321,6 +328,7 @@ class ViTConfig:
         self.patch_size = patch_size
         self.image_size = image_size
         self.output_hidden_states = output_hidden_states
+        self.output_attentions = output_attentions
         self.layer_norm_eps = layer_norm_eps
         self.hidden_act = hidden_act
         self.num_channels = num_channels
@@ -348,7 +356,8 @@ def _linear(i, o):
 
 
 class _HiddenStates:
-    """``output.hidden_states``: the reference reads only ``[-1]`` (ref:ssp_vit2spn_tiny.py:116)."""
+    """``output.hidden_states`` when they were not requested: the reference reads only ``[-1]``
+    (ref:ssp_vit2spn_tiny.py:116), which is the block-12 output the forward produces anyway."""
 
     def __init__(self, last):
         self._last = last
@@ -359,13 +368,18 @@ class _HiddenStates:
     def __getitem__(self, i):
         if i in (-1, 12):
             return self._last
-        raise NotImplementedError("vit2spn keeps only hidden_states[-1] (the only one the reference reads)")
+        raise NotImplementedError("vit2spn keeps only hidden_states[-1] unless the model is called with "
+                                  "output_hidden_states=True (or its config sets it)")
 
 
 class ViTModelOutput:
-    def __init__(self, model, last_hidden):
+    """``hidden_states``: a 13-tuple (embeddings, then every block's output) when requested, else only ``[-1]`` is
+    available; ``attentions``: a 12-tuple of fp32 [B,3,197,197] softmax probabilities when requested, else None."""
+
+    def __init__(self, model, last_hidden, hidden_states=None, attentions=None):
         self._model = model
-        self.hidden_states = _HiddenStates(last_hidden)
+        self.hidden_states = hidden_states if hidden_states is not None else _HiddenStates(last_hidden)
+        self.attentions = attentions
 
     @property
     def last_hidden_state(self):
@@ -381,19 +395,32 @@ class ViTModelOutput:
                                                      m.pooler.dense.bias))
 
 
+def _grad_f32(t):
+    """A gradient as the library reads it: contiguous fp32, 16-byte aligned."""
+    t = t.contiguous().to(torch.float32)
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
 class _BackboneFn(torch.autograd.Function):
-    """x -> (hidden_states[-1] | mean-pooled features) for one backbone, autograd-compatible."""
+    """x -> (hidden_states[-1] | mean-pooled features) for one backbone, autograd-compatible.  With want_hidden /
+    want_attn the outputs are (hidden_states[12], hidden_states[0..11] if want_hidden, attentions[0..11] if
+    want_attn): the residual stream is written straight into the 13 hidden-state tensors, the probabilities by one extra
+    kernel per block.  Gradients w.r.t. any hidden state flow back; the attention probabilities are not differentiable."""
 
     @staticmethod
     @_with_device_of(lambda ctx, x, *a, **k: x)
-    def forward(ctx, x, anchor, model, pooled, need_grad):
+    def forward(ctx, x, anchor, model, pooled, need_grad, want_hidden=False, want_attn=False):
         store = model._store
         store.ensure()
         mode = model._mode()
         B = x.shape[0]
         dev = x.device
+        hidden = [torch.empty(B, 197, 192, dtype=torch.float32, device=dev) for _ in range(13)] if want_hidden else None
+        attn = [torch.empty(B, 3, 197, 197, dtype=torch.float32, device=dev) for _ in range(12)] if want_attn else None
         if pooled:
             out = torch.empty(B, 192, dtype=torch.float32, device=dev)
+        elif want_hidden:
+            out = hidden[12]
         else:
             out = torch.empty(B, 197, 192, dtype=torch.float32, device=dev)
         if need_grad:
@@ -401,27 +428,63 @@ class _BackboneFn(torch.autograd.Function):
         else:
             ws = _scratch_workspace(dev, B, mode, 1, 0)
         g = _group(store, mode, x, 0 if need_grad else -1,
-                   hidden=None if pooled else out, feat=out if pooled else None, feat_stride=192)
-        _run_forward([g], B, mode, ws)
+                   hidden=None if pooled or want_hidden else out, feat=out if pooled else None, feat_stride=192)
+        outs = None
+        if want_hidden or want_attn:
+            o = GroupOutputs()
+            for i, t in enumerate(hidden or ()):
+                o.hidden[i] = t.data_ptr()
+            for i, t in enumerate(attn or ()):
+                o.attn[i] = t.data_ptr()
+            outs = [o]
+        _run_forward([g], B, mode, ws, outs)
+        ctx.set_materialize_grads(False)
         ctx.model, ctx.pooled, ctx.mode, ctx.B = model, pooled, mode, B
+        ctx.want_hidden, ctx.want_attn = want_hidden, want_attn
         ctx.ws = ws if need_grad else None
         ctx.x = x
-        return out
+        if not (want_hidden or want_attn):
+            return out
+        if need_grad and want_hidden:
+            ctx.save_for_backward(*hidden)          # the backward reads the residual stream back from them
+        return (out,) + tuple(hidden[:12] if want_hidden else ()) + tuple(attn or ())
 
     @staticmethod
-    @_with_device_of(lambda ctx, dout: dout)
-    def backward(ctx, dout):
+    @_with_device_of(lambda ctx, dout, *rest: dout if dout is not None else next((t for t in rest if t is not None), None))
+    def backward(ctx, dout, *rest):
         model, store = ctx.model, ctx.model._store
+        n_hidden = 12 if ctx.want_hidden else 0
+        dhid, dattn = rest[:n_hidden], rest[n_hidden:]
+        if any(t is not None for t in dattn):
+            raise RuntimeError("vit2spn: the attention probabilities (output_attentions=True) are not differentiable; "
+                               "detach them before they enter the loss")
         if ctx.ws is None:
             raise RuntimeError("vit2spn: backward through a forward that saved no activations")
-        dout = dout.contiguous().to(torch.float32)
+        nones = (None,) * 7
+        if dout is None and all(t is None for t in dhid):
+            return nones
         grads = store.grads()
-        g = _group(store, ctx.mode, ctx.x, 0, grads=grads,
-                   dfeat=dout if ctx.pooled else None, dfeat_stride=192,
-                   dhidden=None if ctx.pooled else dout)
-        _run_backward([g], ctx.B, ctx.mode, ctx.ws)
+        dout = _grad_f32(dout) if dout is not None else None
+        outs = None
+        keep = []
+        if ctx.want_hidden:
+            o = GroupOutputs()
+            for i, t in enumerate(ctx.saved_tensors):
+                o.hidden[i] = t.data_ptr()
+            for i, t in enumerate(tuple(dhid) + (dout,)):
+                if t is not None:
+                    t = _grad_f32(t)
+                    keep.append(t)
+                    o.dhidden[i] = t.data_ptr()
+            outs = [o]
+            g = _group(store, ctx.mode, ctx.x, 0, grads=grads)
+        else:
+            g = _group(store, ctx.mode, ctx.x, 0, grads=grads,
+                       dfeat=dout if ctx.pooled else None, dfeat_stride=192,
+                       dhidden=None if ctx.pooled else dout)
+        _run_backward([g], ctx.B, ctx.mode, ctx.ws, outs)
         ctx.ws = None
-        return None, None, None, None, None
+        return nones
 
 
 _warned_random_init = False
@@ -529,7 +592,7 @@ class ViTModel(nn.Module):
         weights while the script asked for pretrained ones must not happen silently — unless
         ``V2S_ALLOW_RANDOM_INIT=1`` is set (offline boxes, benchmarks, tests: north_star specifies random init
         there), in which case the HF random initialisation is kept and said so on stderr."""
-        cfg_kw = {k: v for k, v in kw.items() if k in ("output_hidden_states",)}
+        cfg_kw = {k: v for k, v in kw.items() if k in ("output_hidden_states", "output_attentions")}
         model = cls(ViTConfig(**cfg_kw))
         path = _resolve_checkpoint(str(name))
         if path is None:
@@ -572,11 +635,22 @@ class ViTModel(nn.Module):
         a = self.embeddings.cls_token
         return _BackboneFn.apply(x, a, self, True, a.requires_grad and torch.is_grad_enabled())
 
-    def forward(self, pixel_values, **kw):
+    def forward(self, pixel_values, output_hidden_states=None, output_attentions=None, **kw):
+        """As ``transformers.ViTModel``: each flag comes from the keyword, else from the config.  The hidden states
+        cost no extra kernel work (the residual stream is written into them) but keep 13 x [B,197,192] fp32 alive; the
+        attention probabilities are fp32 [B,3,197,197] per block, recomputed by one extra kernel per block."""
         x = _check_images(pixel_values)
         a = self.embeddings.cls_token
-        last = _BackboneFn.apply(x, a, self, False, a.requires_grad and torch.is_grad_enabled())
-        return ViTModelOutput(self, last)
+        want_hidden = bool(self.config.output_hidden_states if output_hidden_states is None else output_hidden_states)
+        want_attn = bool(getattr(self.config, "output_attentions", False) if output_attentions is None else output_attentions)
+        need_grad = a.requires_grad and torch.is_grad_enabled()
+        if not (want_hidden or want_attn):
+            return ViTModelOutput(self, _BackboneFn.apply(x, a, self, False, need_grad))
+        res = _BackboneFn.apply(x, a, self, False, need_grad, want_hidden, want_attn)
+        last = res[0]
+        hidden = tuple(res[1:13]) + (last,) if want_hidden else None
+        attentions = tuple(res[13:] if want_hidden else res[1:]) if want_attn else None
+        return ViTModelOutput(self, last, hidden, attentions)
 
 
 class ViTBackbone(nn.Module):
