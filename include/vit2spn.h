@@ -255,6 +255,8 @@ int v2s_augment_finish_u8(const uint8_t* src, int n, int in_size, const int32_t*
 int v2s_set_sm_limit(int n_sms);
 
 /* test hooks: individual operators, used by tests/ to localise a parity failure */
+/* GEMM, 16-bit operands: which 0 NT (a [m,k], b [n,k] -> c [m,n] 16-bit), 1 NN (b [k,n]), 2 TN (a [k,m], b [k,n],
+ * c [m,n] fp32 +=, split-K), 3 NT with fp32 c.  variant bit 0 = SIMT kernel, bit 1 = fp16 instead of bf16 */
 int v2s_test_gemm(int which, const void* a, const void* b, void* c, int m, int n, int k,
                   int variant, void* stream);
 /* fused MLP half of a block (mlp_tc.cu), one backbone: mode 0 forward (a = LN2 output [m,192]; writes optional u, h

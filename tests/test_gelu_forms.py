@@ -1,7 +1,7 @@
-"""CPU: the one-MUFU GELU forms of the tensor-core epilogues (vit-2spn_b200/csrc/tc_math.cuh) restated in numpy fp32 with
-the coefficients PARSED from the header, against the exact erf GELU of the reference (HF hidden_act="gelu",
-HF:modeling_vit.py:296-299) and its derivative: the approximation error must disappear inside the 16-bit rounding of the
-activations (bf16 2^-9, fp16 2^-11 relative).  tools/fit_gelu.py regenerates the coefficients."""
+"""CPU: the one-MUFU GELU forms of the chained MLP kernel (vit-2spn_b200/csrc/tc_math.cuh, used by mlp_tc.cu) restated
+in numpy fp32 with the coefficients PARSED from the header, against the exact erf GELU of the reference (HF
+hidden_act="gelu", HF:modeling_vit.py:296-299) and its derivative: the approximation error must disappear inside the
+16-bit rounding of the activations (bf16 2^-9, fp16 2^-11 relative).  tools/fit_gelu.py regenerates the coefficients."""
 import os
 import re
 

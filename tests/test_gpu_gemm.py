@@ -48,40 +48,3 @@ def test_tcgen05_gemm_matches_fp32_matmul(which, m, n, k, fmt):
     err = (c.float() - ref).abs().max().item()
     scale = ref.abs().max().item()
     assert err <= (2e-5 if which == 2 else 6e-3 if fmt == 0 else 1e-3) * scale + 1e-3, (err, scale)
-
-
-@pytest.mark.parametrize("m,n,k", [(256, 768, 192), (1576, 768, 192)])
-@pytest.mark.parametrize("fmt", [0, 2])
-def test_gelu_epilogues_match_erf_gelu(m, n, k, fmt):
-    """fc1 epilogue (u = x W^T, h = gelu(u)) and the dgrad epilogue (dy W * gelu'(u)) of the bf16 path against the
-    exact erf form (HF hidden_act="gelu"): the fast erf approximation (|error| < 1.5e-7) must disappear inside the
-    bf16 rounding of the stored value."""
-    from vit2spn import _lib
-    _lib.init_device(0)
-    dev = torch.device("cuda:0")
-    lp = LP[fmt]
-    g = torch.Generator(device=dev).manual_seed(m + n)
-    a = torch.randn(m, k, device=dev, generator=g).to(lp)
-    b = (torch.randn(n, k, device=dev, generator=g) * 0.15).to(lp)          # u ~ N(0, 2): covers both tails
-    out = torch.full((2, m, n), float("nan"), device=dev, dtype=lp)
-    _lib.check(_lib.lib.v2s_test_gemm(5, _lib.ptr(a), _lib.ptr(b), _lib.ptr(out), m, n, k, fmt, _lib.stream_ptr()))
-    torch.cuda.synchronize()
-    assert _lib.lib.v2s_debug_flag() == 0
-    u_ref = a.float() @ b.float().t()
-    h, u = out[0].float(), out[1].float()
-    assert (u - u_ref).abs().max().item() <= 6e-3 * u_ref.abs().max().item() + 1e-3
-    h_ref = torch.nn.functional.gelu(u_ref)                                        # erf form
-    assert ((h - h_ref).abs() <= 4e-3 * h_ref.abs() + 2e-4).all(), (h - h_ref).abs().max().item()
-    # derivative epilogue: dy [m, n2] @ W [n2, n] * gelu'(u)
-    n2 = 192
-    dy = torch.randn(m, n2, device=dev, generator=g).to(lp)
-    w = (torch.randn(n2, n, device=dev, generator=g) * 0.1).to(lp)
-    buf = torch.empty(2, m, n, device=dev, dtype=lp)
-    buf[1] = out[1]
-    _lib.check(_lib.lib.v2s_test_gemm(6, _lib.ptr(dy), _lib.ptr(w), _lib.ptr(buf), m, n, n2, fmt, _lib.stream_ptr()))
-    torch.cuda.synchronize()
-    assert _lib.lib.v2s_debug_flag() == 0
-    uu = out[1].float().requires_grad_(True)
-    torch.nn.functional.gelu(uu).sum().backward()
-    du_ref = (dy.float() @ w.float()) * uu.grad
-    assert ((buf[0].float() - du_ref).abs() <= 6e-3 * du_ref.abs() + 1e-3 * du_ref.abs().max()).all()

@@ -526,8 +526,8 @@ def test_repeatability_under_overlapped_launches(dev):
     atomics, so the loss must be bit-identical over many repetitions; gradients accumulate split-K partial sums
     (and LayerNorm / bias column sums) with fp32 reduce-add in arbitrary order, so they agree only to
     summation-order noise: measured 5-6e-5 rel-L2 (dominated by the patch-embedding and first-block weight
-    gradients, whose partial sums cancel heavily), identical with the overlap switched off (V2S_NO_LATE_WAIT=1) and
-    on the SIMT path (tools/repeat_probe.py).  A missed dependency corrupts whole tiles and lands orders of
+    gradients, whose partial sums cancel heavily), the same spread as measured with the launch overlap switched off
+    and on the SIMT kernels (tools/repeat_probe.py).  A missed dependency corrupts whole tiles and lands orders of
     magnitude above the 5e-4 bound used here."""
     from oracle import vit2spn_oracle as orc
     state = orc.init_state(3, 0.02)

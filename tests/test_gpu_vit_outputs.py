@@ -250,8 +250,8 @@ def test_attentions_are_not_differentiable():
 
 # ---- 8: nothing requested -> the kernels of the previous release --------------------------------------------------
 # v2s_launch_count() of one forward + backward with no per-layer output requested, as the release before the per-layer
-# outputs launched it (bf16, default settings; the wgrad pairing off with V2S_NO_WGRAD_MERGE=1).
-PARENT_LAUNCHES = {("vit", False): 155, ("vit", True): 179, ("dual", False): 363, ("dual", True): 411}
+# outputs launched it (bf16).
+PARENT_LAUNCHES = {"vit": 155, "dual": 363}
 
 
 def _count_launches():
@@ -279,10 +279,9 @@ def _count_launches():
 
 
 def test_launch_count_unchanged_without_outputs():
-    if any(os.environ.get(k) for k in ("V2S_NO_LNFUSE", "V2S_NO_MLPFUSE", "V2S_NO_LATE_WAIT", "V2S_ATTN_FWD", "V2S_GEMM_DEBUG")):
-        pytest.skip("launch counts are pinned for the default kernel selection")
-    nomerge = bool(os.environ.get("V2S_NO_WGRAD_MERGE"))
+    if os.environ.get("V2S_GEMM_DEBUG"):
+        pytest.skip("launch counts are pinned for the uninstrumented kernels")
     vit, dual = _count_launches()
-    _report("launches" + ("_nomerge" if nomerge else ""), {"vit": vit, "dual": dual})
-    assert vit == PARENT_LAUNCHES[("vit", nomerge)], vit
-    assert dual == PARENT_LAUNCHES[("dual", nomerge)], dual
+    _report("launches", {"vit": vit, "dual": dual})
+    assert vit == PARENT_LAUNCHES["vit"], vit
+    assert dual == PARENT_LAUNCHES["dual"], dual

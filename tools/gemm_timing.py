@@ -17,8 +17,6 @@ def run(which, m, n, k, label):
         a = torch.randn(m, k, device=dev).bfloat16(); b = torch.randn(n, k, device=dev).bfloat16(); c = torch.empty(m, n, device=dev, dtype=torch.float32)
     elif which == 0:
         a = torch.randn(m, k, device=dev).bfloat16(); b = torch.randn(n, k, device=dev).bfloat16(); c = torch.empty(m, n, device=dev, dtype=torch.bfloat16)
-    elif which in (4, 5):
-        a = torch.randn(m, k, device=dev).bfloat16(); b = (torch.randn(n, k, device=dev) * 0.1).bfloat16(); c = torch.empty(2, m, n, device=dev, dtype=torch.bfloat16)
     elif which == 1:
         a = torch.randn(m, k, device=dev).bfloat16(); b = torch.randn(k, n, device=dev).bfloat16(); c = torch.empty(m, n, device=dev, dtype=torch.bfloat16)
     else:
@@ -50,8 +48,6 @@ run(3, 8 * 25216, 576, 192, "qkv x8 fp32 out")
 run(0, 25216, 576, 192, "qkv fwd (NT)")
 run(0, 25216, 768, 192, "fc1-like (NT, plain store)")
 run(0, 4 * 25216, 768, 192, "fc1 x4 plain store")
-run(4, 4 * 25216, 768, 192, "fc1 x4 GELU (h)")
-run(5, 4 * 25216, 768, 192, "fc1 x4 GELU (h+u)")
 run(0, 25216, 192, 768, "fc2-like (NT, plain store)")
 run(1, 25216, 192, 576, "dgrad qkv (NN)")
 run(1, 25216, 768, 192, "dgrad W2 (NN)")

@@ -5,8 +5,7 @@
 //   forward:  S = Q K^T (UMMA 128x208x64, both K-major)  ->  P = softmax(S/8) (TMEM -> registers -> bf16
 //             pairs back into TMEM over the consumed scores)  ->  O = P V (UMMA 128x64x208, A = P from
 //             tensor memory, V MN-major)  -> O / rowsum -> bf16 -> TMA store; log-sum-exp saved for the
-//             backward.  attn_fwd_persist_kernel (default): persistent CTAs, two jobs in flight;
-//             attn_fwd_tc_kernel (V2S_ATTN_FWD=v1): one CTA per job, two CTAs per SM.
+//             backward.  attn_fwd_persist_kernel: persistent CTAs, two jobs in flight.
 //   backward: see attn_bwd_tc_kernel.
 #include <string.h>
 
@@ -34,184 +33,11 @@ __device__ __forceinline__ void mma(uint32_t d_tmem, uint32_t a_addr, uint32_t a
                       idesc, accumulate ? 1u : 0u);
 }
 
-// ---- forward --------------------------------------------------------------------------------
-// One CTA per (query tile, head, image, backbone): 160 threads (warp 0 control, warps 1..4 = one softmax
-// thread per query row), 107 KB of smem and 256 TMEM columns, so two CTAs share an SM and the MMA phase
-// of one overlaps the softmax phase of the other.  P (64 KB) is written over K once S = Q K^T has retired.
-constexpr int F_OFF_Q = 0;                                  // 16 KB (later: O staging)
-constexpr int F_OFF_V = Q_TILE_BYTES;                       // 16384
-constexpr int F_OFF_KP = F_OFF_V + KV_TILE_BYTES;           // 43008: K (26 KB), then P (64 KB) in the same place
-constexpr int F_OFF_BAR = F_OFF_KP + P_TILE_BYTES;          // 108544
-constexpr int F_SMEM = F_OFF_BAR + 128 + 1024;
-constexpr int F_THREADS = 160;
-constexpr int F_TM_O = 128;                                 // TMEM: S [0,208) -> P bf16x2 [0,104), O [128,192)
-static_assert(F_OFF_KP % 1024 == 0, "swizzled tiles need 1024-byte alignment");
-
-struct alignas(64) AttnFwdParams {
-  CUtensorMap tmQ[MAXG], tmKV[MAXG], tmCtx[MAXG];
-  float* lse[MAXG];
-  int* err_flag;
-};
-
-__device__ __forceinline__ uint32_t pack2(float a, float b) {
-  __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&v);
-}
-
 // writes 8 consecutive bf16 (one 16-byte chunk) of row r, key group c8 (keys 8*c8..8*c8+7) into a
 // K-major SWIZZLE_128B operand tile made of 64-key column blocks of [128 rows x 128 B]
 __device__ __forceinline__ void store_p_chunk(uint8_t* tile, int r, int c8, uint4 v) {
   const int block = c8 >> 3, chunk = c8 & 7;
   *reinterpret_cast<uint4*>(tile + block * (QT * 128) + r * 128 + ((chunk ^ (r & 7)) << 4)) = v;
-}
-
-__global__ void __launch_bounds__(F_THREADS, 2) attn_fwd_tc_kernel(const __grid_constant__ AttnFwdParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint64_t* bar_load = reinterpret_cast<uint64_t*>(smem + F_OFF_BAR);
-  uint64_t* bar_s = bar_load + 1;
-  uint64_t* bar_p = bar_s + 1;
-  uint64_t* bar_o = bar_p + 1;
-  uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bar_o + 1);
-  const int t = blockIdx.x & 1, h = blockIdx.x >> 1, b = blockIdx.y, g = blockIdx.z;
-  const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;   // warp-uniform for the compiler
-
-  if (warp == 0) {
-    if (lane == 0) {
-      ptx::mbar_init(bar_load, 1); ptx::mbar_init(bar_s, 1); ptx::mbar_init(bar_p, 128); ptx::mbar_init(bar_o, 1);
-      ptx::fence_barrier_init();
-    }
-    __syncwarp();
-    ptx::tmem_alloc(tmem_ptr, 256);
-    ptx::tmem_relinquish();
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_ptr, 0);
-  ptx::pdl_wait();                  // prologue above overlapped the predecessor's tail
-  ptx::pdl_launch_dependents();     // after the wait: see the dependent-launch note in gemm_tc.cu
-
-  if (warp == 0) {
-    // control warp: every lane walks the same path and waits on the barriers; one elected lane issues
-    if (ptx::elect_one()) {
-      ptx::mbar_arrive_expect_tx(bar_load, Q_TILE_BYTES + 2 * KV_TILE_BYTES);
-      ptx::tma_load_3d(smem + F_OFF_Q, &p.tmQ[g], bar_load, h * DH, t * QT, b);
-      ptx::tma_load_3d(smem + F_OFF_KP, &p.tmKV[g], bar_load, D + h * DH, 0, b);
-      ptx::tma_load_3d(smem + F_OFF_V, &p.tmKV[g], bar_load, 2 * D + h * DH, 0, b);
-    }
-    __syncwarp();
-    ptx::mbar_wait(bar_load, 0, p.err_flag, 11);
-    ptx::tc_fence_after();
-    const uint32_t idesc_s = ptx::make_idesc_bf16(QT, KPAD, 0, 0);
-    const uint32_t idesc_o = ptx::make_idesc_bf16(QT, DH, 0, 1);
-    const uint32_t sbase = ptx::smem_u32(smem);
-    const uint32_t sq = sbase + F_OFF_Q, skp = sbase + F_OFF_KP, sv = sbase + F_OFF_V;
-    if (ptx::elect_one()) {
-#pragma unroll
-      for (int k = 0; k < DH / 16; ++k) mma(tmem_base, sq + k * 32, 16, skp + k * 32, 16, idesc_s, k > 0);
-      ptx::umma_commit(bar_s);
-    }
-    __syncwarp();
-    ptx::mbar_wait(bar_p, 0, p.err_flag, 12);
-    ptx::tc_fence_after();
-    if (ptx::elect_one()) {
-#pragma unroll
-      for (int j = 0; j < KPAD / 16; ++j)     // O (columns [128,192)) = P (tensor memory, 8 columns per K-step) x V
-        ptx::umma_bf16_ts(tmem_base + F_TM_O, tmem_base + j * 8, ptx::desc_lo(sv + j * 2048, 8192),
-                          ptx::DESC_HI_SW128_SBO1024, idesc_o, j > 0 ? 1u : 0u);
-      ptx::umma_commit(bar_o);
-    }
-    __syncwarp();
-  } else {
-    const int q = warp & 3;                     // TMEM lane quarter this warp may access
-    const int row = q * 32 + lane;
-    const int qrow = t * QT + row;
-    const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16);
-    uint8_t* ptile = smem + F_OFF_KP;
-    ptx::mbar_wait(bar_s, 0, p.err_flag, 13);   // S complete: K is dead, its smem becomes P
-    ptx::tc_fence_after();
-    // pass 1: row maximum over the 197 real keys
-    float mx = -INFINITY;
-    uint32_t r[32];
-#pragma unroll 1
-    for (int c = 0; c < 6; ++c) {
-      ptx::tmem_ld_32x32(taddr + c * 32, r);
-      ptx::tmem_ld_wait();
-#pragma unroll
-      for (int i = 0; i < 32; ++i) mx = fmaxf(mx, __uint_as_float(r[i]));
-    }
-    ptx::tmem_ld_32x16(taddr + 192, r);
-    ptx::tmem_ld_wait();
-#pragma unroll
-    for (int i = 0; i < NT - 192; ++i) mx = fmaxf(mx, __uint_as_float(r[i]));
-    // pass 2: p = exp2((s - max) * scale * log2e), row sum; bf16 P goes back into tensor memory over the
-    // scores already consumed (two keys per 32-bit column, the A-operand layout of the P V UMMA)
-    const float moff = mx * SCALE_LOG2E;
-    float sum = 0.f;
-#pragma unroll 1
-    for (int c = 0; c < 6; ++c) {
-      ptx::tmem_ld_32x32(taddr + c * 32, r);
-      ptx::tmem_ld_wait();
-      uint32_t pw[16];
-#pragma unroll
-      for (int i = 0; i < 16; ++i) {
-        const float e0 = ptx::ex2_approx(fmaf(__uint_as_float(r[2 * i]), SCALE_LOG2E, -moff));
-        const float e1 = ptx::ex2_approx(fmaf(__uint_as_float(r[2 * i + 1]), SCALE_LOG2E, -moff));
-        sum += e0 + e1;
-        pw[i] = pack2(e0, e1);
-      }
-      ptx::tmem_st_32x16(taddr + c * 16, pw);
-    }
-    {
-      ptx::tmem_ld_32x16(taddr + 192, r);
-      ptx::tmem_ld_wait();
-      uint32_t pw[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const float e0 = (192 + 2 * i < NT) ? ptx::ex2_approx(fmaf(__uint_as_float(r[2 * i]), SCALE_LOG2E, -moff)) : 0.f;
-        const float e1 = (193 + 2 * i < NT) ? ptx::ex2_approx(fmaf(__uint_as_float(r[2 * i + 1]), SCALE_LOG2E, -moff)) : 0.f;
-        sum += e0 + e1;
-        pw[i] = pack2(e0, e1);
-      }
-      ptx::tmem_st_32x8(taddr + 96, pw);
-    }
-    ptx::tmem_st_wait();
-    ptx::tc_fence_before();
-    ptx::mbar_arrive(bar_p);
-    if (qrow < NT && p.lse[g]) p.lse[g][((int64_t)b * NH + h) * NT + qrow] = mx * SCALE + __logf(sum);
-    const float inv = 1.0f / sum;
-    ptx::mbar_wait(bar_o, 0, p.err_flag, 14);
-    ptx::tc_fence_after();
-    uint8_t* stg = smem + F_OFF_Q;              // the Q tile is dead once S is complete
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      ptx::tmem_ld_32x32(taddr + F_TM_O + c * 32, r);
-      ptx::tmem_ld_wait();
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        uint4 v;
-        v.x = pack2(__uint_as_float(r[8 * j]) * inv, __uint_as_float(r[8 * j + 1]) * inv);
-        v.y = pack2(__uint_as_float(r[8 * j + 2]) * inv, __uint_as_float(r[8 * j + 3]) * inv);
-        v.z = pack2(__uint_as_float(r[8 * j + 4]) * inv, __uint_as_float(r[8 * j + 5]) * inv);
-        v.w = pack2(__uint_as_float(r[8 * j + 6]) * inv, __uint_as_float(r[8 * j + 7]) * inv);
-        *reinterpret_cast<uint4*>(stg + row * 128 + (((c * 4 + j) ^ (row & 7)) << 4)) = v;
-      }
-    }
-    ptx::fence_proxy_async();
-    ptx::bar_sync(1, 128);
-    if (threadIdx.x == 32) {
-      ptx::tma_store_3d(&p.tmCtx[g], stg, h * DH, t * QT, b);   // rows >= 197 are clipped by TMA
-      ptx::tma_commit_group();
-      ptx::tma_wait_group<0>();
-    }
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    ptx::tc_fence_after();
-    ptx::tmem_dealloc(tmem_base, 256);
-  }
 }
 
 // ---- forward, persistent ----------------------------------------------------------------------
@@ -1106,31 +932,15 @@ int launch_attn_probs_tc(const void* const* qkv, const float* const* lse, float*
 
 int launch_attn_fwd_tc(const void* const* qkv, void* const* ctx, float* const* lse, int groups, int B,
                        cudaStream_t s, int lp_f16) {
-  AttnFwdParams p;
+  AttnFwdPParams p;
   memset(&p, 0, sizeof(p));
-  p.err_flag = tc_err_flag();
   for (int g = 0; g < groups; ++g) {
     V2S_TRY(tmap_get_3d(&p.tmQ[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, QT, true, 128));
     V2S_TRY(tmap_get_3d(&p.tmKV[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, KPAD, true, 128));
     V2S_TRY(tmap_get_3d(&p.tmCtx[g], ctx[g], D, NT, B, D * 2, (uint64_t)NT * D * 2, DH, QT, true, 128));
     p.lse[g] = lse ? lse[g] : nullptr;
   }
-  static const bool legacy = getenv("V2S_ATTN_FWD") && strcmp(getenv("V2S_ATTN_FWD"), "v1") == 0;
-  if (legacy && !lp_f16) {      // one CTA per job, two CTAs per SM (kept for A/B measurements; bf16 only)
-    static bool attr[MAX_DEVICES] = {false};
-    if (!attr[cur_device()]) {
-      V2S_CUDA_OK(cudaFuncSetAttribute(attn_fwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, F_SMEM));
-      attr[cur_device()] = true;
-    }
-    V2S_CUDA_OK(launch_pdl(attn_fwd_tc_kernel, dim3(NH * 2, B, groups), dim3(F_THREADS), (size_t)F_SMEM, s, p));
-    V2S_LAUNCH_CHECK();
-    return 0;
-  }
-  AttnFwdPParams pp;
-  memset(&pp, 0, sizeof(pp));
-  memcpy(pp.tmQ, p.tmQ, sizeof(p.tmQ)); memcpy(pp.tmKV, p.tmKV, sizeof(p.tmKV)); memcpy(pp.tmCtx, p.tmCtx, sizeof(p.tmCtx));
-  for (int g = 0; g < groups; ++g) pp.lse[g] = p.lse[g];
-  pp.B = B; pp.total_jobs = 2 * NH * B * groups; pp.err_flag = p.err_flag; pp.dbg = tc_dbg_counters();
+  p.B = B; p.total_jobs = 2 * NH * B * groups; p.err_flag = tc_err_flag(); p.dbg = tc_dbg_counters();
   static bool pattr[MAX_DEVICES] = {false};
   if (!pattr[cur_device()]) {
     V2S_CUDA_OK(cudaFuncSetAttribute(attn_fwd_persist_kernel<false, LpBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PF_SMEM));
@@ -1140,13 +950,13 @@ int launch_attn_fwd_tc(const void* const* qkv, void* const* ctx, float* const* l
     pattr[cur_device()] = true;
   }
   const int num_sms = tc_num_sms();
-  const int grid = pp.total_jobs < num_sms ? pp.total_jobs : num_sms;
+  const int grid = p.total_jobs < num_sms ? p.total_jobs : num_sms;
   if (lp_f16) {
-    if (pp.dbg) V2S_CUDA_OK(launch_pdl(attn_fwd_persist_kernel<true, LpF16>, dim3(grid), dim3(PF_THREADS), (size_t)PF_SMEM, s, pp));
-    else V2S_CUDA_OK(launch_pdl(attn_fwd_persist_kernel<false, LpF16>, dim3(grid), dim3(PF_THREADS), (size_t)PF_SMEM, s, pp));
+    if (p.dbg) V2S_CUDA_OK(launch_pdl(attn_fwd_persist_kernel<true, LpF16>, dim3(grid), dim3(PF_THREADS), (size_t)PF_SMEM, s, p));
+    else V2S_CUDA_OK(launch_pdl(attn_fwd_persist_kernel<false, LpF16>, dim3(grid), dim3(PF_THREADS), (size_t)PF_SMEM, s, p));
   } else {
-    if (pp.dbg) V2S_CUDA_OK(launch_pdl(attn_fwd_persist_kernel<true, LpBf16>, dim3(grid), dim3(PF_THREADS), (size_t)PF_SMEM, s, pp));
-    else V2S_CUDA_OK(launch_pdl(attn_fwd_persist_kernel<false, LpBf16>, dim3(grid), dim3(PF_THREADS), (size_t)PF_SMEM, s, pp));
+    if (p.dbg) V2S_CUDA_OK(launch_pdl(attn_fwd_persist_kernel<true, LpBf16>, dim3(grid), dim3(PF_THREADS), (size_t)PF_SMEM, s, p));
+    else V2S_CUDA_OK(launch_pdl(attn_fwd_persist_kernel<false, LpBf16>, dim3(grid), dim3(PF_THREADS), (size_t)PF_SMEM, s, p));
   }
   V2S_LAUNCH_CHECK();
   return 0;

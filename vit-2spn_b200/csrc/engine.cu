@@ -196,13 +196,13 @@ inline const void* weight_ptr(const v2s_group_t& g, int at, int64_t off) {
 int launch_attention_fwd(const void* const* qkv, void* const* ctx, float* const* lse, int groups, int B, int at,
                          cudaStream_t s) {
   prof::Scope scope(prof::C_ATTN_F, 4.0 * B * NH * (double)NT * NT * DH * groups, s, (double)B * NT * 4 * D * 2.0 * groups);
-  if (at != AT_F32 && tc_enabled()) return launch_attn_fwd_tc(qkv, ctx, lse, groups, B, s, at == AT_F16);
+  if (at != AT_F32) return launch_attn_fwd_tc(qkv, ctx, lse, groups, B, s, at == AT_F16);
   return launch_attn_fwd_simt(qkv, ctx, lse, groups, B, at, s);
 }
 int launch_attention_bwd(const void* const* qkv, const void* const* ctx, const float* const* lse,
                          const void* const* dctx, void* const* dqkv, int groups, int B, int at, cudaStream_t s) {
   prof::Scope scope(prof::C_ATTN_B, 10.0 * B * NH * (double)NT * NT * DH * groups, s, (double)B * NT * 8 * D * 2.0 * groups);
-  if (at != AT_F32 && tc_enabled()) return launch_attn_bwd_tc(qkv, ctx, lse, dctx, dqkv, groups, B, s, at == AT_F16);
+  if (at != AT_F32) return launch_attn_bwd_tc(qkv, ctx, lse, dctx, dqkv, groups, B, s, at == AT_F16);
   return launch_attn_bwd_simt(qkv, ctx, lse, dctx, dqkv, groups, B, at, s);
 }
 
@@ -212,7 +212,7 @@ int launch_attention_probs(const void* const* qkv, const float* const* lse, floa
   // algorithmic bytes: Q and K read once, lse, the fp32 probabilities written once
   prof::Scope scope(prof::C_ATTN_P, 2.0 * B * NH * (double)NT * NT * DH * groups, s,
                     ((double)B * NT * 2 * D * (at ? 2.0 : 4.0) + (double)B * NH * NT * 4 + (double)B * NH * NT * NT * 4) * groups);
-  if (at != AT_F32 && tc_enabled()) return launch_attn_probs_tc(qkv, lse, probs, groups, B, s, at == AT_F16);
+  if (at != AT_F32) return launch_attn_probs_tc(qkv, lse, probs, groups, B, s, at == AT_F16);
   return launch_attn_probs_simt(qkv, lse, probs, groups, B, at, s);
 }
 
@@ -328,7 +328,7 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
     d.a_rs = KPE; d.a_cs = 1; d.b_rs = 1; d.b_cs = KPE;
     d.ldc = D;
     const float* pp[MAXG]; const float* tok[MAXG];
-    const bool two_pass = at != AT_F32 && tc_enabled();   // tensor-core GEMM into patch rows, then assemble tokens
+    const bool two_pass = at != AT_F32;   // tensor-core GEMM into patch rows, then assemble tokens
     d.epi = two_pass ? EPI_STORE : EPI_PATCH;
     for (int g = 0; g < G; ++g) {
       x_cur[g] = hid(g) ? hid(g)[0] : reinterpret_cast<float*>(saved(g) ? sb(g, p.s_x[0]) : fb(g, p.f_xa));
@@ -347,13 +347,11 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
   }
 
   // ---- 12 pre-LN blocks ----
-  // On the tensor-core path every LayerNorm except the first is fused into the epilogue of the GEMM that
-  // produces its input row (attention projection → LN2, fc2 → LN1 of the next block): V2S_NO_LNFUSE=1 disables.
-  const bool ln_fuse = at != AT_F32 && tc_enabled() && !getenv("V2S_NO_LNFUSE");
-  // fc1 -> GELU -> fc2 chained on chip (mlp_tc.cu): V2S_NO_MLPFUSE=1 falls back to the two separate GEMMs
-  const bool mlp_fuse = ln_fuse && !getenv("V2S_NO_MLPFUSE");
+  // In the 16-bit modes every LayerNorm except the first is fused into the epilogue of the kernel that produces its
+  // input row (attention projection → LN2, the chained MLP → LN1 of the next block), and fc1 -> GELU -> fc2 runs as
+  // one chained kernel (mlp_tc.cu).  The fp32 check mode runs the separate LayerNorm and GEMM kernels.
+  const bool tc = at != AT_F32;
   const int lp_f16 = at == AT_F16 ? 1 : 0;
-  bool ln1_done = false;
   for (int l = 0; l < NL; ++l) {
     const int64_t lo = layer_off(l);
     const float *xin[MAXG], *gam[MAXG], *bet[MAXG];
@@ -370,8 +368,9 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
       } else {
         xn[g] = fb(g, p.f_xn); qkv[g] = fb(g, p.f_qkv); ctx[g] = fb(g, p.f_ctx);
         mean[g] = nullptr; rstd[g] = nullptr;
-        // the probabilities need the log-sum-exp: f_h is dead from the attention forward until fc1 (unfused path) and
-        // never written for these groups by the fused MLP kernel (d.h = NULL), and B*3*197 floats fit in it
+        // the probabilities need the log-sum-exp, and B*3*197 floats fit in f_h: in the 16-bit modes these groups use
+        // f_h for nothing else (the chained MLP kernel gets d.h = NULL); in the fp32 mode fc1 writes h there only after
+        // the probabilities have been computed
         lse[g] = want_attn(g) ? (float*)fb(g, p.f_h) : nullptr;
         xmid[g] = (float*)fb(g, p.f_xb); u[g] = nullptr; h[g] = fb(g, p.f_h);
         xout[g] = (float*)fb(g, p.f_xa);   // in place: x_in is dead once x_mid exists
@@ -379,7 +378,7 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
       if (hid(g)) xout[g] = hid(g)[l + 1];
       gam[g] = gs[g].params + lo + L_LN1W; bet[g] = gs[g].params + lo + L_LN1B;
     }
-    if (!ln1_done) {
+    if (l == 0 || !tc) {
       prof::Scope sc(prof::C_LN_F, (double)M * D * (4 + p.es) * G, st);
       V2S_TRY(launch_ln_fwd(xin, gam, bet, xn, mean, rstd, G, (int)M, at, st));
     }
@@ -409,7 +408,7 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
       for (int g = 0; g < G; ++g) {
         d.A[g] = ctx[g]; d.B[g] = weight_ptr(gs[g], at, lo + L_WO);
         d.bias[g] = gs[g].params + lo + L_BO; d.resid[g] = xin[g]; d.out[g] = xmid[g];
-        if (ln_fuse) {     // LN2 of this block, fused
+        if (tc) {     // LN2 of this block, fused
           d.ln_out[g] = saved(g) ? (void*)sb(g, p.s_layer[l].xn2) : (void*)fb(g, p.f_xn);
           d.ln_gamma[g] = gs[g].params + lo + L_LN2W; d.ln_beta[g] = gs[g].params + lo + L_LN2B;
           d.ln_mean[g] = saved(g) ? (float*)sb(g, p.s_layer[l].mean2) : nullptr;
@@ -427,11 +426,7 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
         if (saved(g)) { xn2[g] = sb(g, p.s_layer[l].xn2); m2[g] = (float*)sb(g, p.s_layer[l].mean2); r2[g] = (float*)sb(g, p.s_layer[l].rstd2); }
         else { xn2[g] = fb(g, p.f_xn); m2[g] = nullptr; r2[g] = nullptr; }
       }
-      if (!ln_fuse) {
-        prof::Scope sc(prof::C_LN_F, (double)M * D * (4 + p.es) * G, st);
-        V2S_TRY(launch_ln_fwd(xm, gam, bet, xn2, m2, r2, G, (int)M, at, st));
-      }
-      if (mlp_fuse) {
+      if (tc) {
         // fc1 -> GELU -> fc2 + residual (+ LN1 of the next block) as ONE chained kernel: h never leaves the chip for
         // the EMA-target groups; the online groups still write u and h for the backward pass
         MlpDesc d = make_mlp_desc();
@@ -455,9 +450,12 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
         }
         prof::Scope scope(prof::C_MLP_F, 4.0 * M * D * (double)DF * G, st, bytes);
         V2S_TRY(launch_mlp_tc(d, st));
-        ln1_done = l + 1 < NL;
         for (int g = 0; g < G; ++g) x_cur[g] = xout[g];
         continue;
+      }
+      {
+        prof::Scope sc(prof::C_LN_F, (double)M * D * (4 + p.es) * G, st);
+        V2S_TRY(launch_ln_fwd(xm, gam, bet, xn2, m2, r2, G, (int)M, at, st));
       }
       GemmDesc d = make_gemm_desc();   // fc1 + GELU
       d.M = (int)M; d.N = DF; d.K = D; d.groups = G;
@@ -475,16 +473,8 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
       for (int g = 0; g < G; ++g) {
         d.A[g] = h[g]; d.B[g] = weight_ptr(gs[g], at, lo + L_W2);
         d.bias[g] = gs[g].params + lo + L_B2; d.resid[g] = xmid[g]; d.out[g] = xout[g];
-        if (ln_fuse && l + 1 < NL) {     // LN1 of the next block, fused
-          const int64_t ln = layer_off(l + 1);
-          d.ln_out[g] = saved(g) ? (void*)sb(g, p.s_layer[l + 1].xn1) : (void*)fb(g, p.f_xn);
-          d.ln_gamma[g] = gs[g].params + ln + L_LN1W; d.ln_beta[g] = gs[g].params + ln + L_LN1B;
-          d.ln_mean[g] = saved(g) ? (float*)sb(g, p.s_layer[l + 1].mean1) : nullptr;
-          d.ln_rstd[g] = saved(g) ? (float*)sb(g, p.s_layer[l + 1].rstd1) : nullptr;
-        }
       }
       V2S_TRY(run_gemm(d, at, at, 0, st, prof::C_FC2));
-      ln1_done = ln_fuse && l + 1 < NL;
     }
     for (int g = 0; g < G; ++g) x_cur[g] = xout[g];
   }
@@ -570,8 +560,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
   // dW[N_out, K_in] += dY[M, N_out]^T * X[M, K_in]   (token dimension is the reduction)
   // bias_goff >= 0: also accumulate the bias gradient (column sums of dY) — inside the tensor-core wgrad
   // kernel (extra N=16 MMA against a ones tile), or with the column-sum kernel on the SIMT path
-  const bool tc = at != AT_F32 && tc_enabled();
-  const bool mlp_fuse = tc && !getenv("V2S_NO_MLPFUSE") && !getenv("V2S_NO_LNFUSE");
+  const bool tc = at != AT_F32;
   auto wgrad = [&](void* const* dy, int n_out, void* const* x, int k_in, int64_t goff, bool remap,
                    int64_t bias_goff = -1) -> int {
     if (bias_goff >= 0 && !tc) {
@@ -591,16 +580,12 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     }
     return run_gemm(d, at, at, 0, st, prof::C_WGRAD);
   };
-  // two weight gradients of one block in ONE split-K launch (tensor-core path): the groups of the second problem
-  // follow those of the first (GemmDesc::M2 / N2).  Four ~20 us launches per block become two: one ramp / one tail,
-  // longer K ranges per CTA and a third less reduce-add traffic.
-  static const bool merge_wgrads = !getenv("V2S_NO_WGRAD_MERGE");
+  // two weight gradients of one block in ONE split-K launch (tensor-core path, at most two groups): the groups of the
+  // second problem follow those of the first (GemmDesc::M2 / N2).  Four ~20 us launches per block become two: one
+  // ramp / one tail, longer K ranges per CTA and a third less reduce-add traffic.
+  const bool merged = tc && 2 * G <= MAXG;
   auto wgrad2 = [&](void* const* dy1, int n_out1, void* const* x1, int k_in1, int64_t goff1, int64_t bias1,
                     void* const* dy2, int n_out2, void* const* x2, int k_in2, int64_t goff2, int64_t bias2) -> int {
-    if (!tc || !merge_wgrads || 2 * G > MAXG) {
-      V2S_TRY(wgrad(dy1, n_out1, x1, k_in1, goff1, false, bias1));
-      return wgrad(dy2, n_out2, x2, k_in2, goff2, false, bias2);
-    }
     GemmDesc d = make_gemm_desc();
     d.M = n_out1; d.N = k_in1; d.K = (int)M; d.groups = 2 * G;
     d.a_rs = 1; d.a_cs = n_out1; d.b_rs = k_in1; d.b_cs = 1;
@@ -614,7 +599,6 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     }
     return run_gemm(d, at, at, 0, st, prof::C_WGRAD);
   };
-  const bool merged = tc && merge_wgrads && 2 * G <= MAXG;
   // dX[M, K_in] = dY[M, N_out] * W[N_out, K_in]
   // late: the kernel launched just before this one is a wgrad whose inputs this GEMM shares, and nothing the wgrad
   // touches is written here (GemmDesc::late_wait)
@@ -660,12 +644,12 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     // runs "late" (GemmDesc::late_wait): it does not drain that wgrad.  The mirrored order (wgrads late after the
     // chain kernels, dWo filling the attention kernel's partial last wave) measured the same or slightly slower.
     // ---- MLP ----
-    if (!(merged && mlp_fuse)) V2S_TRY(wgrad(dxlp, D, h, DF, lo + L_W2, false));      // dW2 [192,768]
+    if (!merged) V2S_TRY(wgrad(dxlp, D, h, DF, lo + L_W2, false));      // dW2 [192,768]
     if (l == S - 1) V2S_TRY(bias_grad(dxlp, D, lo + L_B2));                // lower blocks: fused into LN1-bwd above
-    if (mlp_fuse) {
+    if (tc) {
       // du = (dx W2) * gelu'(u) and d xn2 = du W1 chained on chip (du is still written once: dW1 needs it)
       MlpDesc d = make_mlp_desc();
-      d.mode = MLP_BWD; d.M = (int)M; d.groups = G; d.lp_f16 = at == AT_F16 ? 1 : 0; d.late_wait = (!merged && l != S - 1 && !getenv("V2S_NO_LATE_WAIT")) ? 1 : 0;
+      d.mode = MLP_BWD; d.M = (int)M; d.groups = G; d.lp_f16 = at == AT_F16 ? 1 : 0; d.late_wait = (!merged && l != S - 1) ? 1 : 0;
       for (int g = 0; g < G; ++g) {
         d.a[g] = dxlp[g]; d.w1[g] = weight_ptr(gs[g], at, lo + L_W1); d.w2[g] = weight_ptr(gs[g], at, lo + L_W2);
         d.u[g] = u[g]; d.h[g] = big[g]; d.out[g] = tmp[g];
@@ -680,9 +664,9 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       else
         V2S_TRY(wgrad(big, DF, xn2, D, lo + L_W1, false, lo + L_B1));          // dW1 [768,192] and d b1
     } else {
-    V2S_TRY(dgrad(dxlp, D, lo + L_W2, DF, big, EPI_DGELU, u, l != S - 1));    // du = (dx W2) * gelu'(u)
-    V2S_TRY(wgrad(big, DF, xn2, D, lo + L_W1, false, lo + L_B1));          // dW1 [768,192] and d b1
-    V2S_TRY(dgrad(big, DF, lo + L_W1, D, tmp, EPI_STORE, nullptr, true));  // d xn2
+      V2S_TRY(dgrad(dxlp, D, lo + L_W2, DF, big, EPI_DGELU, u, l != S - 1));    // du = (dx W2) * gelu'(u)
+      V2S_TRY(wgrad(big, DF, xn2, D, lo + L_W1, false, lo + L_B1));          // dW1 [768,192] and d b1
+      V2S_TRY(dgrad(big, DF, lo + L_W1, D, tmp, EPI_STORE, nullptr, true));  // d xn2
     }
     {
       const void* dy[MAXG]; const float *x[MAXG], *mu[MAXG], *rs[MAXG], *gm[MAXG];

@@ -11,13 +11,13 @@
 //               TMEM (2 x 192 of 512 columns) so the epilogue of tile i overlaps the MMAs of tile i+1;
 //               wgrad adds an N=16 MMA against a constant ones tile: bias gradient in columns [192,208)
 //   warps 2,3   store warps of the two epilogue groups: own every TMA store / reduce-add and the prefetch of the
-//               auxiliary operand (residual, pre-GELU activation) into the staging ring (warp 2 also owns TMEM)
+//               auxiliary operand (the residual) into the staging ring (warp 2 also owns TMEM)
 //   warps 4-19  epilogue: two groups of eight warps; group g drains accumulator stage g (the CTA's even / odd
 //               tiles).  Warps w, w+4 of a group read TMEM lane quarter w%4 (tcgen05.ld 32x32b) and take the
 //               two 16-column halves of each 32-column chunk: thread = one row x 16 columns.  Epilogues: bias,
 //               bias + residual (fp32 stream, updated in place in the staging buffer) with optional fused
-//               LayerNorm (row parked in TMEM, second pass writes the normalised bf16 row), bias + erf-GELU
-//               (writes u and gelu(u)), x gelu'(u), fp32 reduce-add (split-K wgrad).
+//               LayerNorm (row parked in TMEM, second pass writes the normalised bf16 row), fp32 reduce-add
+//               (split-K wgrad).
 // Staging ring protocol: see the epilogue.  Every mbarrier wait is bounded (ptx::mbar_wait).
 #include <string.h>
 
@@ -47,17 +47,15 @@ constexpr int N_THREADS = 640;                    // 4 control/idle warps + 16 e
 enum TcEpi : int {
   T_STORE = 0,   // out = acc (+bias)            OutT = bf16 | fp32
   T_RESID = 1,   // out(fp32) = acc + bias + aux(fp32)
-  T_GELU = 2,    // u = acc + bias -> out2 (optional), gelu(u) -> out   (bf16)
-  T_DGELU = 3,   // out(bf16) = acc * gelu'(aux(bf16))
   T_ACCUM = 4,   // global(fp32) += acc          (TMA reduce-add; split-K)
 };
 
-// per-variant epilogue staging: a ring of NSTG buffers of STG bytes per epilogue group.  Variants with an
-// auxiliary operand (prefetched two chunks ahead into the ring) and the plain bf16 store use 3 buffers;
-// bf16 chunks are 8 KB (SWIZZLE_64B), fp32 chunks and the GELU pair (u | h) 16 KB.
+// per-variant epilogue staging: a ring of NSTG buffers of STG bytes per epilogue group.  The residual variant
+// (auxiliary operand prefetched two chunks ahead into the ring) and the plain bf16 store use 3 buffers;
+// bf16 chunks are 8 KB (SWIZZLE_64B), fp32 chunks 16 KB.
 template <int EPI, bool OUT_BF16> struct Cfg {
   static constexpr int NSTG = (EPI == T_ACCUM || (EPI == T_STORE && !OUT_BF16)) ? 2 : 3;
-  static constexpr int STG = (OUT_BF16 && EPI != T_GELU) ? 8192 : 16384;
+  static constexpr int STG = OUT_BF16 ? 8192 : 16384;
   static constexpr int STAGING_BYTES = 2 * NSTG * STG;
 };
 
@@ -73,7 +71,7 @@ struct alignas(64) TcParams {
   // hetero (split-K wgrad only): the second half of the groups has its own shape (GemmDesc::M2 / N2)
   int hetero, M2, N2, tiles_m2, tiles_n2, base2;      // base2 = first tile index of the second half
   int a_mn, b_mn;
-  int out2_mask;      // bit g: group g writes the secondary output (pre-GELU u)
+  int dbg_flags;      // experiments (V2S_GEMM_DEBUG=<n>): 2 skip TMEM loads, 4 skip epilogue math + stores, 16 skip TMA stores only
   int b_stationary;   // K <= 192: the CTA keeps its [192 x K] B tile in smem and walks m-tiles only
   int ctas_per_combo; // b_stationary: CTAs sharing one (group, n_tile)
   int stages;         // smem ring depth: [A|B] slots when streaming, A-only slots when B-stationary
@@ -83,7 +81,6 @@ struct alignas(64) TcParams {
   int late_wait;      // see GemmDesc::late_wait
   int* err_flag;
   long long* dbg;     // optional per-role cycle counters of CTA 0 (V2S_GEMM_DEBUG=1)
-  int dbg_flags;      // experiments (V2S_GEMM_DEBUG=<n>): 2 skip TMEM loads, 4 skip epilogue math + stores, 8 skip the u store, 16 skip TMA stores only
 };
 
 
@@ -300,8 +297,8 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
     uint64_t* abar = aux_bar + ge * 3;
     uint64_t* sfull = sfull_bar + ge * 3;
     uint64_t* sfree = sfree_bar + ge * 3;
-    constexpr bool HAS_AUX = (EPI == T_RESID || EPI == T_DGELU);
-    constexpr int AUX_BYTES = (EPI == T_RESID) ? BM * CHUNK * 4 : BM * CHUNK * 2;
+    constexpr bool HAS_AUX = EPI == T_RESID;
+    constexpr int AUX_BYTES = BM * CHUNK * 4;
     const bool LN = (EPI == T_RESID) && p.ln != 0;
     const int RPT = LN ? 2 * N_CHUNKS : N_CHUNKS;
     // slot n becomes reusable: prefetch the auxiliary operand of its next user into the buffer, or release it
@@ -325,7 +322,6 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
     int g, m_tile, split, n_tile;
     for (int i = ge; tile_at(i, g, m_tile, split, n_tile); i += 2) {
       const int m0 = m_tile * BM, n0 = n_tile * BN;
-      const bool write_u = (EPI == T_GELU) && ((p.out2_mask >> g) & 1) && !(DBG && (p.dbg_flags & 8));
 #pragma unroll 1
       for (int c = 0; c < RPT; ++c, ++n) {
         const int b = n % N_STG;
@@ -339,7 +335,6 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
               if (col0 < cols_of(g)) {
                 if (EPI == T_ACCUM) ptx::tma_reduce_add_2d(&p.tmOut[g], stg, col0, m0);
                 else ptx::tma_store_2d(&p.tmOut[g], stg, col0, m0);
-                if (write_u) ptx::tma_store_2d(&p.tmOut2[g], stg + 8192, col0, m0);
               }
             } else {
               ptx::tma_store_2d(&p.tmOut2[g], stg, (c - N_CHUNKS) * CHUNK, m0);   // normalised row chunk
@@ -371,7 +366,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
     uint64_t* sfull = sfull_bar + ge * 3;
     uint64_t* sfree = sfree_bar + ge * 3;
     const int bar_id = 1 + ge;
-    constexpr bool HAS_AUX = (EPI == T_RESID || EPI == T_DGELU);
+    constexpr bool HAS_AUX = EPI == T_RESID;
     // With the fused LayerNorm every tile takes 12 ring slots: 6 residual chunks (pass 1) + 6 normalised chunks.
     const bool LN = (EPI == T_RESID) && p.ln != 0;
     const int RPT = LN ? 2 * N_CHUNKS : N_CHUNKS;      // ring slots per tile
@@ -410,8 +405,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
       if (DBG) e_tfull += clock64() - w0;
       acc_phase ^= 1;
       ptx::tc_fence_after();
-      const bool write_u = (EPI == T_GELU) && ((p.out2_mask >> g) & 1) && !(DBG && (p.dbg_flags & 8));
-      const float* bias = (EPI != T_ACCUM && EPI != T_DGELU) ? p.bias[g] : nullptr;
+      const float* bias = EPI != T_ACCUM ? p.bias[g] : nullptr;
       const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16) + ge * ACC_STRIDE;
       float ln_s1 = 0.f, ln_s2 = 0.f;
 #pragma unroll 1
@@ -470,49 +464,20 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
         if (DBG) e_aux += clock64() - w0;
         if (DBG && (p.dbg_flags & 4)) { publish_slot(cnt); continue; }
         if (HAS_AUX) {
-          if (EPI == T_RESID) {
 #pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const uint32_t slot = stg_s + row * 128 + (((hf * 4 + j) ^ (row & 7)) << 4);
-              const float4 a = ptx::lds128f(slot);
-              v[4 * j] += a.x; v[4 * j + 1] += a.y; v[4 * j + 2] += a.z; v[4 * j + 3] += a.w;
-              ptx::sts128f(slot, v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-            }
-            if (LN) {     // row statistics, and the finished row back into TMEM for the normalisation pass
-              uint32_t xr[16];
+          for (int j = 0; j < 4; ++j) {
+            const uint32_t slot = stg_s + row * 128 + (((hf * 4 + j) ^ (row & 7)) << 4);
+            const float4 a = ptx::lds128f(slot);
+            v[4 * j] += a.x; v[4 * j + 1] += a.y; v[4 * j + 2] += a.z; v[4 * j + 3] += a.w;
+            ptx::sts128f(slot, v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+          }
+          if (LN) {     // row statistics, and the finished row back into TMEM for the normalisation pass
+            uint32_t xr[16];
 #pragma unroll
-              for (int k = 0; k < 16; ++k) { ln_s1 += v[k]; ln_s2 = fmaf(v[k], v[k], ln_s2); xr[k] = __float_as_uint(v[k]); }
-              ptx::tmem_st_32x16(tlane + c * CHUNK + hf * 16, xr);
-            }
-          } else {
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-              const uint32_t slot = stg_s + row * 64 + (((hf * 2 + j) ^ ((row >> 1) & 3)) << 4);
-              const uint4 a = ptx::lds128(slot);
-              const uint32_t w[4] = {a.x, a.y, a.z, a.w};
-              uint32_t o[4];
-#pragma unroll
-              for (int e = 0; e < 4; ++e) {
-                o[e] = LP::pack(v[8 * j + 2 * e] * gelu_grad_fast(LP::lo(w[e])),
-                                v[8 * j + 2 * e + 1] * gelu_grad_fast(LP::hi(w[e])));
-              }
-              ptx::sts128(slot, o[0], o[1], o[2], o[3]);
-            }
+            for (int k = 0; k < 16; ++k) { ln_s1 += v[k]; ln_s2 = fmaf(v[k], v[k], ln_s2); xr[k] = __float_as_uint(v[k]); }
+            ptx::tmem_st_32x16(tlane + c * CHUNK + hf * 16, xr);
           }
         } else if (OUT_BF16) {
-          if (EPI == T_GELU) {
-            if (write_u) {
-#pragma unroll
-              for (int j = 0; j < 2; ++j) {
-                uint4 o;
-                o.x = LP::pack(v[8 * j], v[8 * j + 1]); o.y = LP::pack(v[8 * j + 2], v[8 * j + 3]);
-                o.z = LP::pack(v[8 * j + 4], v[8 * j + 5]); o.w = LP::pack(v[8 * j + 6], v[8 * j + 7]);
-                ptx::sts128(stg_s + 8192 + row * 64 + (((hf * 2 + j) ^ ((row >> 1) & 3)) << 4), o.x, o.y, o.z, o.w);
-              }
-            }
-#pragma unroll
-            for (int k = 0; k < 16; ++k) v[k] = gelu_fast(v[k]);
-          }
 #pragma unroll
           for (int j = 0; j < 2; ++j) {
             uint4 o;
@@ -604,7 +569,6 @@ long long* g_dbg[MAX_DEVICES] = {nullptr};     // 32 counters, only with V2S_GEM
 int g_num_sms_dev[MAX_DEVICES] = {0};
 int g_sm_limit = 0;             // v2s_set_sm_limit: persistent grids leave SMs to a concurrent collective
 int g_dbg_flags = 0;
-bool g_disabled = false;
 
 struct MapKey {
   const void* ptr; uint64_t d0, d1, stride1; uint32_t b0, b1, dtype, swz;
@@ -700,7 +664,6 @@ int tc_num_sms() {
 void tc_set_sm_limit(int n) { g_sm_limit = n > 0 ? n : 0; }
 int* tc_err_flag() { return g_err_flag[cur_device()]; }
 long long* tc_dbg_counters() { return g_dbg[cur_device()]; }
-bool tc_enabled() { return g_encode != nullptr && !g_disabled; }
 
 namespace {
 
@@ -768,8 +731,6 @@ int gemm_tc_init() {
       return 1;
     }
     g_encode = reinterpret_cast<EncodeTiledFn>(fn);
-    const char* env = getenv("V2S_GEMM");
-    g_disabled = env && strcmp(env, "simt") == 0;   // debugging: route every GEMM through the SIMT kernel
     if (getenv("V2S_GEMM_DEBUG")) g_dbg_flags = atoi(getenv("V2S_GEMM_DEBUG"));
   }
   // per-device state of the CURRENT device
@@ -804,24 +765,21 @@ int gemm_tc_error_flag() {
 
 int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t stream, int* handled) {
   *handled = 0;
-  if (g_disabled || !g_encode) return 0;
   if (ta == 0 || ta != tb) return 0;                      // fp32 check mode stays on the SIMT kernel
   if (to != 0 && to != ta) return 0;
+  if (!g_encode) { set_error("tensor maps not initialised (v2s_init)"); return 1; }
   const int lp_f16 = (ta == AT_F16) ? 1 : 0;
   if (d.a_remap || d.b_remap) return 0;
   int epi;
   switch (d.epi) {
     case EPI_STORE: epi = T_STORE; break;
     case EPI_BIAS_RESID: epi = T_RESID; break;
-    case EPI_BIAS_GELU: epi = T_GELU; break;
-    case EPI_DGELU: epi = T_DGELU; break;
     case EPI_ACCUM: epi = T_ACCUM; break;
     default: return 0;
   }
   if (d.alpha != 1.0f) return 0;
   const bool out_bf16 = (to != 0);                        // 16-bit output (bf16 or fp16, as the operands)
   if ((epi == T_RESID || epi == T_ACCUM) && out_bf16) return 0;
-  if ((epi == T_GELU || epi == T_DGELU) && !out_bf16) return 0;
   int a_mn, b_mn;
   int64_t a_ld, b_ld;
   if (d.a_cs == 1) { a_mn = 0; a_ld = d.a_rs; } else if (d.a_rs == 1) { a_mn = 1; a_ld = d.a_cs; } else return 0;
@@ -862,13 +820,13 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
   }
   p.a_mn = a_mn; p.b_mn = b_mn;
   const int combos = d.groups * p.tiles_n;
-  if (epi != T_ACCUM && p.kb_total <= 3 && combos <= g_num_sms && !getenv("V2S_NO_BSTAT")) {
+  if (epi != T_ACCUM && p.kb_total <= 3 && combos <= g_num_sms) {
     int cpc = g_num_sms / combos;
     if (cpc > p.tiles_m) cpc = p.tiles_m;
     p.b_stationary = 1;
     p.ctas_per_combo = cpc;
   }
-  p.late_wait = (d.late_wait && !getenv("V2S_NO_LATE_WAIT")) ? 1 : 0;
+  p.late_wait = d.late_wait ? 1 : 0;
   p.err_flag = tc_err_flag();
   p.dbg = tc_dbg_counters();
   p.dbg_flags = g_dbg_flags;
@@ -886,15 +844,9 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
     else V2S_TRY(get_map(&p.tmA[g], d.A[g], d.M, d.K, a_ld, 64, BK, true, CU_TENSOR_MAP_SWIZZLE_128B));
     if (!b_mn) V2S_TRY(get_map(&p.tmB[g], d.B[g], d.K, d.N, b_ld, BK, BN, true, CU_TENSOR_MAP_SWIZZLE_128B));
     else V2S_TRY(get_map(&p.tmB[g], d.B[g], d.N, d.K, b_ld, 64, BK, true, CU_TENSOR_MAP_SWIZZLE_128B));
-    void* outp = (epi == T_GELU) ? d.out2[g] : d.out[g];      // GELU: primary = h (GemmDesc.out2), secondary = u
-    V2S_TRY(get_map(&p.tmOut[g], outp, d.N, d.M, d.ldc, CHUNK, BM, out_bf16, out_swz));
-    if (epi == T_GELU && d.out[g]) {
-      V2S_TRY(get_map(&p.tmOut2[g], d.out[g], d.N, d.M, d.ldc, CHUNK, BM, true, CU_TENSOR_MAP_SWIZZLE_64B));
-      p.out2_mask |= 1 << g;
-    }
+    V2S_TRY(get_map(&p.tmOut[g], d.out[g], d.N, d.M, d.ldc, CHUNK, BM, out_bf16, out_swz));
     if (epi == T_RESID) V2S_TRY(get_map(&p.tmAux[g], d.resid[g], d.N, d.M, d.ldc, CHUNK, BM, false, CU_TENSOR_MAP_SWIZZLE_128B));
-    if (epi == T_DGELU) V2S_TRY(get_map(&p.tmAux[g], d.aux[g], d.N, d.M, d.ldc, CHUNK, BM, true, CU_TENSOR_MAP_SWIZZLE_64B));
-    p.bias[g] = (epi == T_ACCUM || epi == T_DGELU) ? nullptr : d.bias[g];
+    p.bias[g] = (epi == T_ACCUM) ? nullptr : d.bias[g];
     p.rowsum[g] = (epi == T_ACCUM) ? d.rowsum_out[g] : nullptr;
     if (epi == T_RESID && d.ln_out[g] != nullptr) {
       if (d.N != BN || d.ldc != BN) { set_error("gemm_tc: fused LayerNorm needs N == 192"); return 1; }
@@ -907,8 +859,6 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
   switch (epi) {
     case T_STORE: rc = out_bf16 ? launch_kernel<T_STORE, true>(p, lp_f16, stream) : launch_kernel<T_STORE, false>(p, lp_f16, stream); break;
     case T_RESID: rc = launch_kernel<T_RESID, false>(p, lp_f16, stream); break;
-    case T_GELU: rc = launch_kernel<T_GELU, true>(p, lp_f16, stream); break;
-    case T_DGELU: rc = launch_kernel<T_DGELU, true>(p, lp_f16, stream); break;
     default: rc = launch_kernel<T_ACCUM, false>(p, lp_f16, stream); break;
   }
   if (rc) return rc;
@@ -917,7 +867,7 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
 }
 
 // test hook (v2s_test_gemm): which = 0 NT (A[M,K], B[N,K]), 1 NN/dgrad (A[M,K], B[K,N]),
-// 2 TN/wgrad (A[K,M], B[K,N], out fp32 +=); variant: 0 = tensor-core path, 1 = SIMT reference.
+// 2 TN/wgrad (A[K,M], B[K,N], out fp32 +=), 3 NT with fp32 out; variant: 0 = tensor-core path, 1 = SIMT reference.
 // bf16 operands; out bf16 for which 0/1, fp32 accumulate-into for which 2.
 int gemm_tc_test(int which, const void* a, const void* b, void* c, int m, int n, int k, int variant,
                  cudaStream_t stream) {
@@ -928,15 +878,7 @@ int gemm_tc_test(int which, const void* a, const void* b, void* c, int m, int n,
   else if (which == 1) { d.a_rs = k; d.a_cs = 1; d.b_rs = n; d.b_cs = 1; d.epi = EPI_STORE; }
   else if (which == 2) { d.a_rs = 1; d.a_cs = m; d.b_rs = n; d.b_cs = 1; d.epi = EPI_ACCUM; to = 0; d.split_k = 1; }
   else if (which == 3) { d.a_rs = k; d.a_cs = 1; d.b_rs = 1; d.b_cs = k; d.epi = EPI_STORE; to = 0; }   // NT, fp32 out
-  else if (which == 4 || which == 5) {   // NT with the erf-GELU epilogue: h -> c, and (which 5) pre-activation u -> c + m*n
-    d.a_rs = k; d.a_cs = 1; d.b_rs = 1; d.b_cs = k; d.epi = EPI_BIAS_GELU;
-    d.out2[0] = c; d.out[0] = (which == 5) ? static_cast<bf16*>(c) + (size_t)m * n : nullptr;
-  }
-  else if (which == 6) {   // NN (dgrad) with the GELU' epilogue: c = (A B) * gelu'(u), u (bf16 [m,n]) read from c + m*n
-    d.a_rs = k; d.a_cs = 1; d.b_rs = n; d.b_cs = 1; d.epi = EPI_DGELU;
-    d.aux[0] = static_cast<const bf16*>(c) + (size_t)m * n;
-  }
-  else { set_error("gemm_tc_test: which must be 0..6"); return 1; }
+  else { set_error("gemm_tc_test: which must be 0..3"); return 1; }
   // variant: bit 0 = SIMT reference instead of the tensor-core path, bit 1 = fp16 instead of bf16 tensors
   const int t16 = (variant & 2) ? AT_F16 : AT_BF16;
   if (to) to = t16;

@@ -627,7 +627,6 @@ int launch_impl(const MlpParams& p, int grid, cudaStream_t stream) {
 }  // namespace
 
 int launch_mlp_tc(const MlpDesc& d, cudaStream_t stream) {
-  if (!tc_enabled()) { set_error("mlp_tc: tensor-core path not initialised"); return 1; }
   if (d.groups < 1 || d.groups > MAXG || d.M < 1) { set_error("mlp_tc: bad shape"); return 1; }
   MlpParams p;
   memset(&p, 0, sizeof(p));

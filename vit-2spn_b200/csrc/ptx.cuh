@@ -293,16 +293,5 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr, uint32_t 
   d |= (uint64_t)2 << 61;                                 // bits [61,64) layout type: SWIZZLE_128B
   return d;
 }
-// instruction descriptor for kind::f16: bf16 x bf16 -> fp32, M x N tile, per-operand major-ness
-__host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N, int a_mn_major, int b_mn_major) {
-  return (1u << 4)                         // c_format = F32
-         | (1u << 7)                       // a_format = BF16
-         | (1u << 10)                      // b_format = BF16
-         | ((uint32_t)a_mn_major << 15)    // a_major: 0 = K-major, 1 = MN-major
-         | ((uint32_t)b_mn_major << 16)    // b_major
-         | ((uint32_t)(N >> 3) << 17)      // n_dim
-         | ((uint32_t)(M >> 4) << 24);     // m_dim
-}
-
 }  // namespace ptx
 }  // namespace v2s

@@ -1,5 +1,5 @@
 // Shared device helpers of the tensor-core kernels: the 16-bit operand formats (bf16 / fp16) and the fast erf-GELU
-// used by the GELU-type epilogues.
+// used by the chained MLP kernel.
 #pragma once
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -39,8 +39,13 @@ struct LpF16 {
 
 // instruction descriptor for kind::f16 with a given operand format: 16-bit x 16-bit -> fp32, M x N tile
 __host__ __device__ constexpr uint32_t make_idesc_lp(uint32_t fmt, int M, int N, int a_mn_major, int b_mn_major) {
-  return (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
-         ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+  return (1u << 4)                         // c_format = F32
+         | (fmt << 7)                      // a_format: 0 = F16, 1 = BF16
+         | (fmt << 10)                     // b_format
+         | ((uint32_t)a_mn_major << 15)    // a_major: 0 = K-major, 1 = MN-major
+         | ((uint32_t)b_mn_major << 16)    // b_major
+         | ((uint32_t)(N >> 3) << 17)      // n_dim
+         | ((uint32_t)(M >> 4) << 24);     // m_dim
 }
 
 // ---- fast erf-GELU ------------------------------------------------------------------------------
