@@ -254,9 +254,23 @@ int v2s_augment_finish_u8(const uint8_t* src, int n, int in_size, const int32_t*
  * SMs to a collective that runs concurrently with the backward pass (gradient all-reduce overlap, SURVEY 8e). */
 int v2s_set_sm_limit(int n_sms);
 
+/* Deterministic mode (on != 0; off by default), read when work is enqueued and covering every entry point: the backward
+ * passes (backbone and heads) sum every cross-CTA reduction in a fixed order -- split-K weight gradients, bias and
+ * LayerNorm parameter gradients, embedding gradients -- so their results are bit-identical from run to run on the same
+ * device model, batch, compute mode and inputs.  The split-K split count then follows the device's SM count, not
+ * v2s_set_sm_limit.  The partials and arrival counters live at the tail of the workspace: while the switch is on,
+ * v2s_workspace_bytes includes them (for n_saved > 0).  A backward fails when the workspace has no room for them beyond
+ * the stash and backward regions it uses; they may then overlay the forward-only regions, which a backward does not
+ * read, so size the workspace while the switch is on.  With the
+ * switch off nothing changes, v2s_workspace_bytes included.  Python sets it from torch.are_deterministic_algorithms_enabled(). */
+int v2s_set_deterministic(int on);
+
 /* test hooks: individual operators, used by tests/ to localise a parity failure */
 /* GEMM, 16-bit operands: which 0 NT (a [m,k], b [n,k] -> c [m,n] 16-bit), 1 NN (b [k,n]), 2 TN (a [k,m], b [k,n],
- * c [m,n] fp32 +=, split-K), 3 NT with fp32 c.  variant bit 0 = SIMT kernel, bit 1 = fp16 instead of bf16 */
+ * c [m,n] fp32 +=, split-K), 3 NT with fp32 c, 4 = 2 plus the bias row sums of a (+=) in c[m*n .. m*n + m).
+ * variant bit 0 = SIMT kernel, bit 1 = fp16 instead of bf16.  In deterministic mode (v2s_set_deterministic), which 2 / 4
+ * take their scratch from the caller: c continues after its outputs with 1024 + n_sms * (128 * 192 + 128) floats
+ * (n_sms = the device's SM count; m a multiple of 8). */
 int v2s_test_gemm(int which, const void* a, const void* b, void* c, int m, int n, int k,
                   int variant, void* stream);
 /* fused MLP half of a block (mlp_tc.cu), one backbone: mode 0 forward (a = LN2 output [m,192]; writes optional u, h

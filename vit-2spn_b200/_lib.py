@@ -58,6 +58,7 @@ _SIGS = {
     "v2s_backbone_layout": (C.c_int, [C.POINTER(_i64)]),
     "v2s_heads_layout": (C.c_int, [C.POINTER(_i64)]),
     "v2s_workspace_bytes": (_i64, [_i, _i, _i, _i]),
+    "v2s_set_deterministic": (C.c_int, [_i]),
     "v2s_backbone_forward": (C.c_int, [C.POINTER(Group), _i, _i, _i, _vp, _i64, _vp]),
     "v2s_backbone_backward": (C.c_int, [C.POINTER(Group), _i, _i, _i, _vp, _i64, _vp]),
     "v2s_backbone_backward_range": (C.c_int, [C.POINTER(Group), _i, _i, _i, _vp, _i64, _i, _i, _vp]),

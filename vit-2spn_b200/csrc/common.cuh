@@ -84,6 +84,17 @@ inline int cur_device() {
 void set_error(const char* fmt, ...);
 extern int64_t g_launch_count;
 
+// ---- deterministic mode (v2s_set_deterministic) ------------------------------------------------
+// Scratch the fixed-order reductions of a backward call take from the tail of the caller's workspace.  `counters`
+// are arrival counters: zero before every launch that uses them (cleared once per backward call, then reset by each
+// launch's last arriver).  `part` holds per-CTA partial rows / split-K partial tiles of one launch at a time.
+constexpr int DET_COUNTERS = 1024;
+struct DetScratch {
+  unsigned* counters;
+  float* part;
+  int64_t part_floats;
+};
+
 #define V2S_CUDA_OK(expr)                                                                     \
   do {                                                                                        \
     cudaError_t _e = (expr);                                                                  \

@@ -123,6 +123,34 @@ int64_t plan_total(const Plan& p, int n_groups, int n_saved) {
   return p.heads_bytes + (int64_t)n_groups * p.f_bytes + (int64_t)n_saved * (p.s_bytes + p.b_bytes);
 }
 
+int wgrad_split(int64_t rows);
+
+// deterministic mode: scratch of a backward call at the tail of the workspace (DetScratch): the arrival counters, then
+// one region for the partials of one launch at a time -- the per-CTA rows of the column reductions (at most 296 rows of at
+// most 768 columns per group), the tensor-core split-K slab (one wave of fp32 tiles), or the fp32 check mode's split-K
+// slabs (one per group)
+int64_t det_scratch_bytes(const Plan& p, int n_saved) {
+  if (n_saved <= 0) return 0;
+  int64_t part = (int64_t)MAXG * 296 * DF;
+  const int64_t wg = p.at ? gemm_tc_det_part_floats() : (int64_t)n_saved * wgrad_split(p.M) * DF * D;
+  if (wg > part) part = wg;
+  return align_up(DET_COUNTERS * sizeof(unsigned)) + align_up(part * 4);
+}
+
+int resolve_det(const Plan& p, void* ws, int64_t ws_bytes, int n_saved, DetScratch* det) {
+  const int64_t bytes = det_scratch_bytes(p, n_saved);
+  if (ws_bytes < plan_total(p, 0, n_saved) + bytes) {
+    set_error("deterministic mode: workspace too small (%lld bytes; size it with v2s_workspace_bytes while the switch is on)",
+              (long long)ws_bytes);
+    return 1;
+  }
+  char* tail = static_cast<char*>(ws) + ((ws_bytes - bytes) & ~int64_t(1023));
+  det->counters = reinterpret_cast<unsigned*>(tail);
+  det->part = reinterpret_cast<float*>(tail + align_up(DET_COUNTERS * sizeof(unsigned)));
+  det->part_floats = (bytes - align_up(DET_COUNTERS * sizeof(unsigned))) / 4;
+  return 0;
+}
+
 // base addresses inside the workspace; regions are laid out for the maximum MAXG groups so that
 // forward and backward calls agree regardless of how many groups each call carries
 struct Regions {
@@ -185,6 +213,11 @@ int run_gemm(const GemmDesc& d, int ta, int tb, int to, cudaStream_t s, int cls 
   int handled = 0;
   V2S_TRY(launch_gemm_tc(d, ta, tb, to, s, &handled));
   if (handled) return 0;
+  if (d.det && ta != AT_F32 && d.epi == EPI_ACCUM && d.split_k > 1) {
+    // the SIMT kernel's split-K adds with atomics: in deterministic mode that is an error, not a fall-back
+    set_error("deterministic mode: a 16-bit split-K weight gradient the tensor-core kernel declined (M %d N %d K %d)", d.M, d.N, d.K);
+    return 1;
+  }
   return launch_gemm_simt(d, ta, tb, to, s);
 }
 
@@ -219,13 +252,13 @@ int launch_attention_probs(const void* const* qkv, const float* const* lse, floa
 // d loss / d hidden_states[k] joins the residual-stream gradient (groups whose dh entry is NULL are skipped); for k > 0 its
 // column sums also go to the fc2 bias gradient of block k - 1, whose output hidden_states[k] is
 int add_hidden_grads(int k, const float* const* dh, float* const* dx, void* const* dxlp, const v2s_group_t* gs, int G, int B,
-                     int at, const Plan& p, cudaStream_t s) {
+                     int at, const Plan& p, cudaStream_t s, const DetScratch* det) {
   const float* a[MAXG]; float* o[MAXG]; void* lp[MAXG]; float* cs[MAXG]; int n = 0;
   for (int g = 0; g < G; ++g)
     if (dh[g]) { a[n] = dh[g]; o[n] = dx[g]; lp[n] = dxlp[g]; cs[n] = k > 0 ? gs[g].grads + layer_off(k - 1) + L_B2 : nullptr; ++n; }
   if (!n) return 0;
   prof::Scope sc(prof::C_MISC, (double)p.M * D * (12 + p.es) * n, s);
-  return launch_residual_grad_add(a, o, lp, cs, n, B, at, s);
+  return launch_residual_grad_add(a, o, lp, cs, n, B, at, s, det);
 }
 
 // v2s_group_outputs checks shared by forward and backward: hidden / attn all or none, 16-byte aligned hidden states
@@ -540,6 +573,14 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
   const int64_t M = p.M, MP = p.MP;
   auto sb = [&](int g, int64_t off) -> char* { return R.stash[gs[g].slot] + off; };
   auto bb = [&](int g, int64_t off) -> char* { return R.bwd[gs[g].slot] + off; };
+  // deterministic mode (v2s_set_deterministic): every cross-CTA sum below runs in a fixed order through `det`
+  DetScratch det_s;
+  const DetScratch* det = nullptr;
+  if (tc_deterministic()) {
+    V2S_TRY(resolve_det(p, ws, ws_bytes, n_saved, &det_s));
+    V2S_CUDA_OK(cudaMemsetAsync(det_s.counters, 0, DET_COUNTERS * sizeof(unsigned), st));
+    det = &det_s;
+  }
 
   float* dx[MAXG]; void* dxlp[MAXG]; void* big[MAXG]; void* tmp[MAXG];
   {
@@ -567,16 +608,27 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       const void* src[MAXG]; float* dst[MAXG];
       for (int g = 0; g < G; ++g) { src[g] = dy[g]; dst[g] = gs[g].grads + bias_goff; }
       prof::Scope sc(prof::C_COLSUM, (double)M * n_out * p.es * G, st);
-      V2S_TRY(launch_colsum(src, dst, G, (int)M, n_out, at, st));
+      V2S_TRY(launch_colsum(src, dst, G, (int)M, n_out, at, st, det));
     }
     GemmDesc d = make_gemm_desc();
     d.M = n_out; d.N = k_in; d.K = remap ? (int)MP : (int)M; d.groups = G;
     d.a_rs = 1; d.a_cs = n_out; d.b_rs = k_in; d.b_cs = 1;
     d.a_remap = remap ? 2 : 0;
-    d.epi = EPI_ACCUM; d.ldc = k_in; d.split_k = split;
+    d.epi = EPI_ACCUM; d.ldc = k_in; d.split_k = split; d.det = det;
     for (int g = 0; g < G; ++g) {
       d.A[g] = dy[g]; d.B[g] = x[g]; d.out[g] = gs[g].grads + goff;
       d.rowsum_out[g] = (bias_goff >= 0 && tc) ? gs[g].grads + bias_goff : nullptr;
+    }
+    if (det && !tc && split > 1) {
+      // fp32 check mode: the splits write partial slabs, then a fixed-order sum adds them into each gradient
+      const int64_t mn = (int64_t)n_out * k_in;
+      if ((int64_t)G * split * mn > det->part_floats) { set_error("wgrad: deterministic scratch too small"); return 1; }
+      d.epi = EPI_STORE; d.split_stride = mn;
+      for (int g = 0; g < G; ++g) d.out[g] = det->part + g * split * mn;
+      V2S_TRY(run_gemm(d, at, at, 0, st, prof::C_WGRAD));
+      for (int g = 0; g < G; ++g)
+        V2S_TRY(launch_splitk_reduce(gs[g].grads + goff, det->part + g * split * mn, nullptr, n_out, k_in, split, st, true));
+      return 0;
     }
     return run_gemm(d, at, at, 0, st, prof::C_WGRAD);
   };
@@ -590,7 +642,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     d.M = n_out1; d.N = k_in1; d.K = (int)M; d.groups = 2 * G;
     d.a_rs = 1; d.a_cs = n_out1; d.b_rs = k_in1; d.b_cs = 1;
     d.M2 = n_out2; d.N2 = k_in2;
-    d.epi = EPI_ACCUM; d.ldc = k_in1; d.split_k = split;
+    d.epi = EPI_ACCUM; d.ldc = k_in1; d.split_k = split; d.det = det;
     for (int g = 0; g < G; ++g) {
       d.A[g] = dy1[g]; d.B[g] = x1[g]; d.out[g] = gs[g].grads + goff1;
       d.rowsum_out[g] = bias1 >= 0 ? gs[g].grads + bias1 : nullptr;
@@ -618,7 +670,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     const void* src[MAXG]; float* dst[MAXG];
     for (int g = 0; g < G; ++g) { src[g] = dy[g]; dst[g] = gs[g].grads + goff; }
     prof::Scope sc(prof::C_COLSUM, (double)M * n * p.es * G, st);
-    return launch_colsum(src, dst, G, (int)M, n, at, st);
+    return launch_colsum(src, dst, G, (int)M, n, at, st, det);
   };
 
   // the intermediate hidden-state gradients below the start (dhidden[S] itself started the stream above)
@@ -626,7 +678,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     if (k >= S) return 0;
     const float* a[MAXG];
     for (int g = 0; g < G; ++g) a[g] = os[g] ? os[g]->dhidden[k] : nullptr;
-    return add_hidden_grads(k, a, dx, dxlp, gs, G, B, at, p, st);
+    return add_hidden_grads(k, a, dx, dxlp, gs, G, B, at, p, st, det);
   };
   auto x_in = [&](int g, int l) -> const float* { return hid[g] ? hid[g][l] : (const float*)sb(g, p.s_x[l]); };
 
@@ -678,7 +730,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
         cs[g] = gs[g].grads + lo + L_BO;          // d b_o = column sums of the gradient w.r.t. x_mid
       }
       { prof::Scope sc(prof::C_LN_B, (double)M * D * (12 + 2 * p.es) * G, st);
-        V2S_TRY(launch_ln_bwd(dy, x, mu, rs, gm, dx, lp, dg, db, cs, G, (int)M, at, st)); }
+        V2S_TRY(launch_ln_bwd(dy, x, mu, rs, gm, dx, lp, dg, db, cs, G, (int)M, at, st, det)); }
     }
     // ---- attention ----
     if (!merged) V2S_TRY(wgrad(dxlp, D, ctx, D, lo + L_WO, false));        // dWo (d b_o: fused into LN2-bwd)
@@ -704,7 +756,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
         cs[g] = l > 0 ? gs[g].grads + layer_off(l - 1) + L_B2 : nullptr;
       }
       { prof::Scope sc(prof::C_LN_B, (double)M * D * (12 + 2 * p.es) * G, st);
-        V2S_TRY(launch_ln_bwd(dy, x, mu, rs, gm, dx, lp, dg, db, cs, G, (int)M, at, st)); }
+        V2S_TRY(launch_ln_bwd(dy, x, mu, rs, gm, dx, lp, dg, db, cs, G, (int)M, at, st, det)); }
     }
   }
   // ---- embeddings: d pos, d cls, d patch bias, d patch weight ----
@@ -715,14 +767,14 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       cdx[g] = dx[g]; gr[g] = gs[g].grads;
       pt[g] = gs[g].x_format == 1 ? const_cast<void*>(gs[g].x) : static_cast<void*>(sb(g, p.s_patches));
     }
-    V2S_TRY(launch_embed_bwd(cdx, gr, G, B, st));
+    V2S_TRY(launch_embed_bwd(cdx, gr, G, B, st, det));
     if (tc) {          // compact the patch rows, then the ordinary tensor-core wgrad
       const void* src[MAXG];
       for (int g = 0; g < G; ++g) src[g] = dxlp[g];
       V2S_TRY(launch_gather_patch_rows(src, tmp, G, B, at, st));
       GemmDesc d = make_gemm_desc();
       d.M = D; d.N = KPE; d.K = (int)MP; d.groups = G;
-      d.a_rs = 1; d.a_cs = D; d.b_rs = KPE; d.b_cs = 1; d.epi = EPI_ACCUM; d.ldc = KPE; d.split_k = split;
+      d.a_rs = 1; d.a_cs = D; d.b_rs = KPE; d.b_cs = 1; d.epi = EPI_ACCUM; d.ldc = KPE; d.split_k = split; d.det = det;
       for (int g = 0; g < G; ++g) { d.A[g] = tmp[g]; d.B[g] = pt[g]; d.out[g] = gs[g].grads + OFF_WPE; }
       V2S_TRY(run_gemm(d, at, at, 0, st, prof::C_WGRAD));
     } else {
@@ -809,6 +861,10 @@ static int heads_backward_impl(const float* hp, float* hg, const float* fo, cons
   V2S_TRY(heads_bufs(ws, ws_bytes, B, &hb));
   const float* dp = dpred ? dpred : hb.dp;
   const int PH = V2S_PROJ_HID, PO = V2S_PROJ_OUT, PI = V2S_PROJ_IN;
+  // deterministic mode: the weight gradients below and dfeat run without a K split (one add per element), the bias
+  // gradients sum their B rows in one CTA
+  const DetScratch det_rows = {nullptr, nullptr, 0};
+  const DetScratch* det = tc_deterministic() ? &det_rows : nullptr;
   auto wgrad = [&](const float* dy, int n, const float* x, int k, int64_t woff) -> int {
     GemmDesc d = make_gemm_desc();
     d.M = n; d.N = k; d.K = B; d.a_rs = 1; d.a_cs = n; d.b_rs = k; d.b_cs = 1; d.epi = EPI_ACCUM; d.ldc = k;
@@ -817,7 +873,7 @@ static int heads_backward_impl(const float* hp, float* hg, const float* fo, cons
   };
   auto bgrad = [&](const float* dy, int n, int64_t boff) -> int {
     const void* s[1] = {dy}; float* o[1] = {hg + boff};
-    return launch_colsum(s, o, 1, B, n, 0, st);
+    return launch_colsum(s, o, 1, B, n, 0, st, det);
   };
   auto dgrad = [&](const float* dy, int n, int64_t woff, int k, float* out, int epi, const float* relu_src,
                    const float* mask) -> int {
@@ -840,7 +896,8 @@ static int heads_backward_impl(const float* hp, float* hg, const float* fo, cons
   {   // d feat = dy1 W1: K = 1024 → split-K accumulate into the zeroed [B,384] output
     V2S_CUDA_OK(cudaMemsetAsync(dfo, 0, (size_t)B * PI * sizeof(float), st));
     GemmDesc d = make_gemm_desc();
-    d.M = B; d.N = PI; d.K = PH; d.a_rs = PH; d.a_cs = 1; d.b_rs = PI; d.b_cs = 1; d.epi = EPI_ACCUM; d.ldc = PI; d.split_k = 8;
+    d.M = B; d.N = PI; d.K = PH; d.a_rs = PH; d.a_cs = 1; d.b_rs = PI; d.b_cs = 1; d.epi = EPI_ACCUM; d.ldc = PI;
+    d.split_k = det ? 1 : 8;
     d.A[0] = hb.dy1; d.B[0] = hp + H_W1; d.out[0] = dfo;
     V2S_TRY(launch_gemm_simt(d, 0, 0, 0, st));
   }
@@ -921,7 +978,8 @@ int v2s_heads_layout(int64_t* o) {
 
 int64_t v2s_workspace_bytes(int batch, int mode, int n_groups, int n_saved) {
   if (batch < 1 || n_groups < 0 || n_groups > MAXG || n_saved < 0 || n_saved > MAXG) return -1;
-  return plan_total(make_plan(batch, mode), n_groups, n_saved);
+  const Plan p = make_plan(batch, mode);
+  return plan_total(p, n_groups, n_saved) + (tc_deterministic() ? det_scratch_bytes(p, n_saved) : 0);
 }
 
 int v2s_backbone_forward(const v2s_group_t* groups, int n_groups, int batch, int mode, void* workspace,
@@ -1099,6 +1157,11 @@ int64_t v2s_launch_count(void) { return g_launch_count; }
 
 int v2s_set_sm_limit(int n_sms) {
   tc_set_sm_limit(n_sms);
+  return 0;
+}
+
+int v2s_set_deterministic(int on) {
+  tc_set_deterministic(on);
   return 0;
 }
 

@@ -52,6 +52,9 @@ struct GemmDesc {
   // [0, groups / 2) use M, N and the strides above, groups [groups / 2, groups) use M2, N2 (a_cs = M2, b_rs = N2,
   // ldc = N2: both operands token-major).  One launch ramp and one balanced wave instead of two.
   int M2, N2;
+  // deterministic mode, tensor-core split-K wgrad (EPI_ACCUM) only: scratch for the partial tiles and the per-output-tile
+  // arrival counters; the split count then ignores v2s_set_sm_limit and the partials are summed in split order
+  const DetScratch* det;
 };
 
 inline GemmDesc make_gemm_desc() {

@@ -48,13 +48,14 @@ enum TcEpi : int {
   T_STORE = 0,   // out = acc (+bias)            OutT = bf16 | fp32
   T_RESID = 1,   // out(fp32) = acc + bias + aux(fp32)
   T_ACCUM = 4,   // global(fp32) += acc          (TMA reduce-add; split-K)
+  T_ACCUM_DET = 5,   // deterministic T_ACCUM: partial tiles to a slab, summed in split order by the last CTA to arrive
 };
 
 // per-variant epilogue staging: a ring of NSTG buffers of STG bytes per epilogue group.  The residual variant
 // (auxiliary operand prefetched two chunks ahead into the ring) and the plain bf16 store use 3 buffers;
 // bf16 chunks are 8 KB (SWIZZLE_64B), fp32 chunks 16 KB.
 template <int EPI, bool OUT_BF16> struct Cfg {
-  static constexpr int NSTG = (EPI == T_ACCUM || (EPI == T_STORE && !OUT_BF16)) ? 2 : 3;
+  static constexpr int NSTG = (EPI == T_ACCUM || EPI == T_ACCUM_DET || (EPI == T_STORE && !OUT_BF16)) ? 2 : 3;
   static constexpr int STG = OUT_BF16 ? 8192 : 16384;
   static constexpr int STAGING_BYTES = 2 * NSTG * STG;
 };
@@ -81,6 +82,13 @@ struct alignas(64) TcParams {
   int late_wait;      // see GemmDesc::late_wait
   int* err_flag;
   long long* dbg;     // optional per-role cycle counters of CTA 0 (V2S_GEMM_DEBUG=1)
+  // T_ACCUM_DET: the gradients (+ row stride), the slab of partial tiles (tmOut2[0] maps it: tile slot s = rows
+  // [128 s, 128 s + 128)), the partial row sums [slot][128] and one arrival counter per output tile
+  float* det_out[MAXG];
+  int64_t det_ldc[MAXG];
+  float* det_slab;
+  float* det_rowpart;
+  unsigned* det_counters;
 };
 
 
@@ -107,6 +115,9 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
   // warp index through a shuffle: tells the compiler it is warp-uniform, so that the single-thread
   // roles below compile to straight uniform-datapath code (no per-lane convergence loops around TMA / MMA)
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;
+  constexpr bool ACC = EPI == T_ACCUM || EPI == T_ACCUM_DET, DET = EPI == T_ACCUM_DET;
+  // T_ACCUM_DET: output tiles whose last split this CTA stored ([0] = count; the LayerNorm scratch is unused here)
+  int* fix_list = reinterpret_cast<int*>(ln_part);
 
   if (warp == 0 && lane == 0) {
     for (int g = 0; g < p.groups; ++g) {
@@ -126,10 +137,11 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
     ptx::tmem_alloc(tmem_ptr, TMEM_COLS);
     ptx::tmem_relinquish();
   }
-  if (EPI == T_ACCUM && warp == 3) {
+  if (ACC && warp == 3) {
     // a row of 16-bit 1.0 values; the swizzle only permutes 16-byte chunks inside a row, so a constant row is layout-proof
     for (int i = lane; i < 2048 / 4; i += 32)
       reinterpret_cast<uint32_t*>(ones_tile)[i] = (i < 32) ? LP::kOnePair : 0u;
+    if (DET && lane == 0) fix_list[0] = 0;
     ptx::fence_proxy_async();
   }
   // Programmatic dependent launch.  Every kernel of this library waits for its predecessor and only THEN
@@ -179,6 +191,13 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
   };
   auto rows_of = [&](int g) { return (p.hetero && g >= p.groups / 2) ? p.M2 : p.M; };
   auto cols_of = [&](int g) { return (p.hetero && g >= p.groups / 2) ? p.N2 : p.N; };
+  // T_ACCUM_DET: index of an output tile (all splits of it share one arrival counter); its split s has slab slot
+  // out_tile * splits + s
+  auto out_tile = [&](int g, int m_tile, int n_tile) {
+    if (p.hetero && g >= p.groups / 2)
+      return p.base2 / p.splits + ((g - p.groups / 2) * p.tiles_m2 + m_tile) * p.tiles_n2 + n_tile;
+    return (g * p.tiles_m + m_tile) * p.tiles_n + n_tile;
+  };
   // smem map of the operand region: streaming mode = 3 stages of [A 16 KB | B 24 KB];
   // B-stationary mode = [B tile: kb_total (<= 3) k-blocks x 24 KB] followed by a ring of A slots (16 KB)
   uint8_t* bres = smem;
@@ -274,7 +293,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
           ptx::umma_bf16_lohi(d_tmem, a_lo + a_step, b_lo + b_step, ptx::DESC_HI_SW128_SBO1024, idesc, 1u);
           ptx::umma_bf16_lohi(d_tmem, a_lo + 2 * a_step, b_lo + 2 * b_step, ptx::DESC_HI_SW128_SBO1024, idesc, 1u);
           ptx::umma_bf16_lohi(d_tmem, a_lo + 3 * a_step, b_lo + 3 * b_step, ptx::DESC_HI_SW128_SBO1024, idesc, 1u);
-          if (EPI == T_ACCUM && n_tile == 0 && p.rowsum[g] != nullptr && !(DBG && (p.dbg_flags & 32))) {
+          if (ACC && n_tile == 0 && p.rowsum[g] != nullptr && !(DBG && (p.dbg_flags & 32))) {
             // row sums of A (= bias gradient in a wgrad) into accumulator columns [192,208): A x ones
 #pragma unroll
             for (int k = 0; k < 4; ++k)
@@ -333,7 +352,8 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
             if (c < N_CHUNKS) {
               const int col0 = n0 + c * CHUNK;
               if (col0 < cols_of(g)) {
-                if (EPI == T_ACCUM) ptx::tma_reduce_add_2d(&p.tmOut[g], stg, col0, m0);
+                if (DET) ptx::tma_store_2d(&p.tmOut2[0], stg, c * CHUNK, (out_tile(g, m_tile, n_tile) * p.splits + split) * BM);
+                else if (EPI == T_ACCUM) ptx::tma_reduce_add_2d(&p.tmOut[g], stg, col0, m0);
                 else ptx::tma_store_2d(&p.tmOut[g], stg, col0, m0);
               }
             } else {
@@ -344,6 +364,15 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
           if (n >= 1) {
             ptx::tma_wait_group_read<1>();             // the store of slot n-1 has left its buffer
             recycle(n - 1);
+          }
+          if (DET && c == RPT - 1) {
+            // the tile's partial (and, through sfull, its row sums) is in global memory: count this split in.  The
+            // split that completes the count owns the fix-up; nobody waits for anybody.
+            ptx::tma_wait_group<0>();
+            ptx::fence_proxy_async_global();
+            const int o = out_tile(g, m_tile, n_tile);
+            if (ptx::atom_add_acq_rel_gpu(&p.det_counters[o], 1u) == (unsigned)(p.splits - 1))
+              fix_list[1 + atomicAdd(&fix_list[0], 1)] = (g << 24) | (m_tile << 12) | n_tile;
           }
         }
         __syncwarp();
@@ -405,7 +434,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
       if (DBG) e_tfull += clock64() - w0;
       acc_phase ^= 1;
       ptx::tc_fence_after();
-      const float* bias = EPI != T_ACCUM ? p.bias[g] : nullptr;
+      const float* bias = !ACC ? p.bias[g] : nullptr;
       const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16) + ge * ACC_STRIDE;
       float ln_s1 = 0.f, ln_s2 = 0.f;
 #pragma unroll 1
@@ -438,11 +467,16 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
         }
         if (DBG) e_ld += clock64() - w0;
         if (c == N_CHUNKS - 1 && !LN) {             // accumulator fully read: hand the stage back to the MMA warp
-          if (EPI == T_ACCUM && hf == 0 && n_tile == 0 && p.rowsum[g] != nullptr) {
+          if (ACC && hf == 0 && n_tile == 0 && p.rowsum[g] != nullptr) {
             uint32_t rs[16];
             ptx::tmem_ld_32x16(tlane + BN, rs);
             ptx::tmem_ld_wait();
-            if (m0 + row < rows_of(g)) atomicAdd(p.rowsum[g] + m0 + row, __uint_as_float(rs[0]));
+            if (DET) {
+              p.det_rowpart[(out_tile(g, m_tile, n_tile) * p.splits + split) * BM + row] = __uint_as_float(rs[0]);
+              __threadfence();
+            } else if (m0 + row < rows_of(g)) {
+              atomicAdd(p.rowsum[g] + m0 + row, __uint_as_float(rs[0]));
+            }
           }
           ptx::tc_fence_before();
           if (lane == 0) ptx::mbar_arrive(&tempty_bar[ge]);
@@ -551,6 +585,31 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
   if (p.late_wait) { ptx::pdl_wait(); ptx::pdl_launch_dependents(); }
   ptx::tc_fence_before();
   __syncthreads();
+  if (DET) {
+    // fix-up of the output tiles this CTA completed, by all its threads: gradient += partial 0 + ... + partial S-1
+    for (int e = 0; e < fix_list[0]; ++e) {
+      const int code = fix_list[1 + e], g = code >> 24, m_tile = (code >> 12) & 4095, n_tile = code & 4095;
+      const int o = out_tile(g, m_tile, n_tile), m0 = m_tile * BM, n0 = n_tile * BN;
+      const int rows = min(BM, rows_of(g) - m0), c4s = min(BN, cols_of(g) - n0) / 4;
+      const float* slab = p.det_slab + (int64_t)o * p.splits * BM * BN;
+      for (int i = threadIdx.x; i < rows * c4s; i += N_THREADS) {
+        const int r = i / c4s, c4 = i - r * c4s;
+        float4* dst = reinterpret_cast<float4*>(p.det_out[g] + (int64_t)(m0 + r) * p.det_ldc[g] + n0) + c4;
+        float4 v = *dst;
+        for (int s = 0; s < p.splits; ++s) {
+          const float4 a = __ldcg(reinterpret_cast<const float4*>(slab + ((int64_t)s * BM + r) * BN) + c4);
+          v.x += a.x; v.y += a.y; v.z += a.z; v.w += a.w;
+        }
+        *dst = v;
+      }
+      if (n_tile == 0 && p.rowsum[g] != nullptr && threadIdx.x < rows) {
+        float v = p.rowsum[g][m0 + threadIdx.x];
+        for (int s = 0; s < p.splits; ++s) v += __ldcg(p.det_rowpart + (o * p.splits + s) * BM + threadIdx.x);
+        p.rowsum[g][m0 + threadIdx.x] = v;
+      }
+      if (threadIdx.x == 0) p.det_counters[o] = 0;     // zero again for the next launch
+    }
+  }
   if (warp == 2) {
     ptx::tc_fence_after();
     ptx::tmem_dealloc(tmem_base, TMEM_COLS);
@@ -568,6 +627,7 @@ int* g_err_flag[MAX_DEVICES] = {nullptr};      // device int per GPU, allocated 
 long long* g_dbg[MAX_DEVICES] = {nullptr};     // 32 counters, only with V2S_GEMM_DEBUG=1
 int g_num_sms_dev[MAX_DEVICES] = {0};
 int g_sm_limit = 0;             // v2s_set_sm_limit: persistent grids leave SMs to a concurrent collective
+int g_deterministic = 0;        // v2s_set_deterministic
 int g_dbg_flags = 0;
 
 struct MapKey {
@@ -662,6 +722,11 @@ int tc_num_sms() {
   return (g_sm_limit > 0 && g_sm_limit < n) ? g_sm_limit : n;
 }
 void tc_set_sm_limit(int n) { g_sm_limit = n > 0 ? n : 0; }
+void tc_set_deterministic(int on) { g_deterministic = on ? 1 : 0; }
+int tc_deterministic() { return g_deterministic; }
+static int tc_device_sms() { return g_num_sms_dev[cur_device()] > 0 ? g_num_sms_dev[cur_device()] : 148; }
+// a deterministic split-K launch has at most one tile per SM of the device (see launch_gemm_tc)
+int64_t gemm_tc_det_part_floats() { return (int64_t)tc_device_sms() * (BM * BN + BM); }
 int* tc_err_flag() { return g_err_flag[cur_device()]; }
 long long* tc_dbg_counters() { return g_dbg[cur_device()]; }
 
@@ -691,7 +756,7 @@ int launch_kernel_impl(TcParams& p, cudaStream_t stream) {
   }
   p.stg_off = p.op_bytes;
   p.bar_off = p.op_bytes + Cfg<EPI, OUT_BF16>::STAGING_BYTES;
-  if (EPI == T_ACCUM && !p.b_stationary && p.total_tiles <= g_num_sms) {
+  if ((EPI == T_ACCUM || EPI == T_ACCUM_DET) && !p.b_stationary && p.total_tiles <= g_num_sms) {
     // one tile per CTA (the one-wave split-K wgrad): its epilogue starts after the last MMA has retired, when
     // the operand ring is dead, so the staging buffers overlay the ring and the ring gets their 64 KB
     int st = (SMEM_LIMIT - 1024 - SMEM_BAR_BYTES) / STAGE_BYTES;
@@ -802,10 +867,11 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
   }
   if (epi == T_ACCUM) {
     // split-K so that the launch is ONE balanced wave: base * splits <= #SMs (a second, partial wave of a few
-    // tiles would double the makespan of these long-K tiles)
+    // tiles would double the makespan of these long-K tiles).  Deterministic mode sizes it for the whole device, so
+    // that the summation order does not depend on v2s_set_sm_limit; a limited grid walks several tiles per CTA.
     const int base = hetero ? (d.groups / 2) * (p.tiles_m * p.tiles_n + p.tiles_m2 * p.tiles_n2)
                             : d.groups * p.tiles_m * p.tiles_n;
-    int s = g_num_sms / base;
+    int s = (d.det ? tc_device_sms() : g_num_sms) / base;
     const int max_s = p.kb_total / 4 > 0 ? p.kb_total / 4 : 1;
     if (s > max_s) s = max_s;
     if (s < 1) s = 1;
@@ -855,10 +921,29 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
       p.ln = 1;
     }
   }
+  // deterministic mode: with one split every element already receives exactly one reduce-add (and every row sum one
+  // atomic add), so only a split launch needs the slab and the in-kernel fix-up
+  if (epi == T_ACCUM && d.det && p.splits > 1) {
+    const int64_t slots = p.total_tiles;      // <= SMs of the device: splits > 1 implies base * splits <= SMs
+    if (slots * (BM * BN + BM) > d.det->part_floats || slots / p.splits > DET_COUNTERS || slots >= 1024 || !d.det->counters) {
+      set_error("gemm_tc: deterministic scratch too small for %lld partial tiles", (long long)slots);
+      return 1;
+    }
+    p.det_slab = d.det->part;
+    p.det_rowpart = d.det->part + slots * BM * BN;
+    p.det_counters = d.det->counters;
+    V2S_TRY(get_map(&p.tmOut2[0], p.det_slab, BN, (uint64_t)slots * BM, BN, CHUNK, BM, false, CU_TENSOR_MAP_SWIZZLE_128B));
+    for (int g = 0; g < d.groups; ++g) {
+      p.det_out[g] = static_cast<float*>(d.out[g]);
+      p.det_ldc[g] = (hetero && g >= d.groups / 2) ? d.N2 : d.ldc;
+    }
+    epi = T_ACCUM_DET;
+  }
   int rc;
   switch (epi) {
     case T_STORE: rc = out_bf16 ? launch_kernel<T_STORE, true>(p, lp_f16, stream) : launch_kernel<T_STORE, false>(p, lp_f16, stream); break;
     case T_RESID: rc = launch_kernel<T_RESID, false>(p, lp_f16, stream); break;
+    case T_ACCUM_DET: rc = launch_kernel<T_ACCUM_DET, false>(p, lp_f16, stream); break;
     default: rc = launch_kernel<T_ACCUM, false>(p, lp_f16, stream); break;
   }
   if (rc) return rc;
@@ -867,8 +952,10 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
 }
 
 // test hook (v2s_test_gemm): which = 0 NT (A[M,K], B[N,K]), 1 NN/dgrad (A[M,K], B[K,N]),
-// 2 TN/wgrad (A[K,M], B[K,N], out fp32 +=), 3 NT with fp32 out; variant: 0 = tensor-core path, 1 = SIMT reference.
-// bf16 operands; out bf16 for which 0/1, fp32 accumulate-into for which 2.
+// 2 TN/wgrad (A[K,M], B[K,N], out fp32 +=), 3 NT with fp32 out, 4 = 2 plus the bias row sums (+=) at c + M*N;
+// variant: 0 = tensor-core path, 1 = SIMT reference.  bf16 operands; out bf16 for which 0/1, fp32 accumulate-into for
+// which 2/4.  Deterministic mode, which 2/4: the caller's c buffer continues with the scratch a backward call takes
+// from its workspace (DetScratch: DET_COUNTERS counters, then gemm_tc_det_part_floats() floats)
 int gemm_tc_test(int which, const void* a, const void* b, void* c, int m, int n, int k, int variant,
                  cudaStream_t stream) {
   GemmDesc d = make_gemm_desc();
@@ -878,11 +965,24 @@ int gemm_tc_test(int which, const void* a, const void* b, void* c, int m, int n,
   else if (which == 1) { d.a_rs = k; d.a_cs = 1; d.b_rs = n; d.b_cs = 1; d.epi = EPI_STORE; }
   else if (which == 2) { d.a_rs = 1; d.a_cs = m; d.b_rs = n; d.b_cs = 1; d.epi = EPI_ACCUM; to = 0; d.split_k = 1; }
   else if (which == 3) { d.a_rs = k; d.a_cs = 1; d.b_rs = 1; d.b_cs = k; d.epi = EPI_STORE; to = 0; }   // NT, fp32 out
-  else { set_error("gemm_tc_test: which must be 0..3"); return 1; }
+  else if (which == 4) {
+    d.a_rs = 1; d.a_cs = m; d.b_rs = n; d.b_cs = 1; d.epi = EPI_ACCUM; to = 0; d.split_k = 1;
+    d.rowsum_out[0] = static_cast<float*>(c) + (int64_t)m * n;
+  }
+  else { set_error("gemm_tc_test: which must be 0..4"); return 1; }
   // variant: bit 0 = SIMT reference instead of the tensor-core path, bit 1 = fp16 instead of bf16 tensors
   const int t16 = (variant & 2) ? AT_F16 : AT_BF16;
   if (to) to = t16;
   if (variant & 1) return launch_gemm_simt(d, t16, t16, to, stream);
+  DetScratch det = {nullptr, nullptr, 0};
+  if ((which == 2 || which == 4) && tc_deterministic()) {
+    if (m % 8) { set_error("gemm_tc_test: deterministic scratch needs M %% 8 == 0"); return 1; }
+    det.counters = reinterpret_cast<unsigned*>(static_cast<float*>(c) + (int64_t)m * n + (which == 4 ? m : 0));
+    det.part = reinterpret_cast<float*>(det.counters + DET_COUNTERS);
+    det.part_floats = gemm_tc_det_part_floats();
+    V2S_CUDA_OK(cudaMemsetAsync(det.counters, 0, DET_COUNTERS * sizeof(unsigned), stream));
+    d.det = &det;
+  }
   int handled = 0;
   V2S_TRY(launch_gemm_tc(d, t16, t16, to, stream, &handled));
   if (!handled) { set_error("gemm_tc_test: shape not handled by the tensor-core path"); return 1; }

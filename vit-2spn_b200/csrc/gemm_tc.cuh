@@ -21,6 +21,10 @@ int tmap_get_2d(CUtensorMap* out, const void* ptr, uint64_t d0, uint64_t d1, uin
                 uint32_t b1, bool is_lp, int swizzle_bytes);
 int tc_num_sms();              // SMs persistent grids may use on the current device (see v2s_set_sm_limit)
 void tc_set_sm_limit(int n);
+void tc_set_deterministic(int on);   // v2s_set_deterministic
+int tc_deterministic();
+// floats of DetScratch::part the deterministic split-K wgrad needs on the current device (one wave of fp32 tiles)
+int64_t gemm_tc_det_part_floats();
 int* tc_err_flag();
 long long* tc_dbg_counters();   // 32 device counters when V2S_GEMM_DEBUG is set, else NULL
 int gemm_tc_debug_counters(long long* host32);

@@ -179,6 +179,49 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const __grid_constant__ LnF
   }
 }
 
+// Deterministic mode: fixed-order column reduction across the CTAs of one launch.  Each CTA has written its partial row
+// (n floats) to part[blk]; the CTA whose arrival completes the counter sums rows 0..nblk-1 and calls add(c, total) per
+// column.  Rows are summed in R contiguous ranges (R threads per float4 column, partials through `red`, capacity
+// `red_floats`), then the R range sums in order: the order depends on nblk, n and the block size only, never on which CTA
+// came last.  No CTA waits for another.  Called by every thread of the CTA; n a multiple of 4.
+template <typename Add>
+__device__ __forceinline__ void det_reduce_rows(const float* part, int n, int nblk, unsigned* counter, float* red, int red_floats, Add add) {
+  __shared__ unsigned s_last;
+  __threadfence();                   // this CTA's partial row is visible device-wide before it is counted
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    unsigned old;
+    asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], 1;" : "=r"(old) : "l"(counter) : "memory");
+    s_last = old == (unsigned)(nblk - 1);
+  }
+  __syncthreads();
+  if (!s_last) return;
+  const int n4 = n / 4;
+  int R = red_floats / n;
+  if (R > 8) R = 8;
+  if (R > nblk) R = nblk;
+  const int per = (nblk + R - 1) / R;
+  for (int it = threadIdx.x; it < R * n4; it += blockDim.x) {
+    const int r = it / n4, c4 = it - r * n4;
+    const int b1 = min(nblk, (r + 1) * per);
+    float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll 4
+    for (int b = r * per; b < b1; ++b) {
+      const float4 v = __ldcg(reinterpret_cast<const float4*>(part + (int64_t)b * n) + c4);
+      s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+    }
+    float* rr = red + r * n + 4 * c4;          // `red` may be only 4-byte aligned
+    rr[0] = s.x; rr[1] = s.y; rr[2] = s.z; rr[3] = s.w;
+  }
+  __syncthreads();
+  for (int c = threadIdx.x; c < n; c += blockDim.x) {
+    float s = red[c];
+    for (int r = 1; r < R; ++r) s += red[r * n + c];
+    add(c, s);
+  }
+  if (threadIdx.x == 0) *counter = 0;      // zero again for the next launch
+}
+
 // dres (fp32, in/out) += LN-backward(dy);  dres_lp = updated dres in the activation type;
 // dgamma / dbeta / (optional) dcolsum[n] += sum over rows of the UPDATED dres (= bias gradient of the
 // linear layer that consumes this residual-stream gradient).
@@ -187,11 +230,13 @@ struct LnBwdP {
   const float* gamma[MAXG]; float* dres[MAXG]; void* dres_lp[MAXG]; float* dgamma[MAXG]; float* dbeta[MAXG];
   float* dcolsum[MAXG];
   int M;
+  float* det_part;             // DET: [group][CTA][3 * 192] partial rows
+  unsigned* det_counters;      // DET: one per group
 };
 
-template <typename T>
+template <typename T, bool DET>
 __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnBwdP p) {
-  __shared__ float red[16][3 * D];          // 36 KB
+  __shared__ __align__(16) float red[16][3 * D];          // 36 KB; float4 accesses
   // wait for the predecessor, THEN release the successor: a successor flagged "late wait" (gemm_tc.cu) relies on
   // everything before its predecessor being complete when it starts
   asm volatile("griddepcontrol.wait;" ::: "memory");
@@ -245,13 +290,25 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnB
     *reinterpret_cast<float4*>(&red[hw][2 * D + c]) = ac[i];
   }
   __syncthreads();
+  float* part = DET ? p.det_part + ((int64_t)g * gridDim.x + blockIdx.x) * 3 * D : nullptr;
   for (int c = threadIdx.x; c < 3 * D; c += blockDim.x) {
     float s = 0.f;
 #pragma unroll
     for (int w = 0; w < 16; ++w) s += red[w][c];
-    if (c < D) atomicAdd(p.dgamma[g] + c, s);
+    if (DET) part[c] = s;
+    else if (c < D) atomicAdd(p.dgamma[g] + c, s);
     else if (c < 2 * D) atomicAdd(p.dbeta[g] + (c - D), s);
     else if (p.dcolsum[g]) atomicAdd(p.dcolsum[g] + (c - 2 * D), s);
+  }
+  if constexpr (DET) {
+    __syncthreads();                 // red is reused by the reduction
+    float* dgm = p.dgamma[g]; float* dbt = p.dbeta[g]; float* dcs = p.dcolsum[g];
+    det_reduce_rows(p.det_part + (int64_t)g * gridDim.x * 3 * D, 3 * D, gridDim.x, p.det_counters + g, &red[0][0], 16 * 3 * D,
+                    [&](int c, float s) {
+                      if (c < D) dgm[c] += s;
+                      else if (c < 2 * D) dbt[c - D] += s;
+                      else if (dcs) dcs[c - 2 * D] += s;
+                    });
   }
 }
 
@@ -259,9 +316,11 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnB
 struct ColsumP {
   const void* dy[MAXG]; float* db[MAXG];
   int M, N, rows_per_block;
+  float* det_part;             // DET with more than one CTA per group: [group][CTA][N] partial rows
+  unsigned* det_counters;
 };
 
-template <typename T>
+template <typename T, bool DET>
 __global__ void __launch_bounds__(256) colsum_kernel(const __grid_constant__ ColsumP p) {
   __shared__ float red[2048];
   const int g = blockIdx.y;
@@ -286,10 +345,20 @@ __global__ void __launch_bounds__(256) colsum_kernel(const __grid_constant__ Col
     for (int i = 0; i < 8; ++i) red[rt * p.N + ct * 8 + i] = acc[i];
   }
   __syncthreads();
+  float* part = (DET && gridDim.x > 1) ? p.det_part + ((int64_t)g * gridDim.x + blockIdx.x) * p.N : nullptr;
   for (int n = threadIdx.x; n < p.N; n += blockDim.x) {
     float s = 0.f;
     for (int w = 0; w < rows_t; ++w) s += red[w * p.N + n];
-    atomicAdd(p.db[g] + n, s);
+    if (!DET) atomicAdd(p.db[g] + n, s);
+    else if (part) part[n] = s;
+    else p.db[g][n] += s;            // one CTA per group: the only writer
+  }
+  if constexpr (DET) {
+    if (gridDim.x == 1) return;
+    __syncthreads();
+    float* db = p.db[g];
+    det_reduce_rows(p.det_part + (int64_t)g * gridDim.x * p.N, p.N, gridDim.x, p.det_counters + g, red, 2048,
+                    [db](int c, float s) { db[c] += s; });
   }
 }
 
@@ -328,7 +397,9 @@ __global__ void __launch_bounds__(256) pool_bwd_kernel(G4<const float*> dfeat, G
 }
 
 // d pos / d cls / d patch-bias from the gradient of the embedding output
-__global__ void embed_bwd_kernel(G4<const float*> dx, G4<float*> grads, int B) {
+// DET: the patch-bias sum over the 196 patch tokens goes through det_part [group][196][192] in token order
+template <bool DET>
+__global__ void embed_bwd_kernel(G4<const float*> dx, G4<float*> grads, int B, float* det_part, unsigned* det_counters) {
   const int g = blockIdx.y, t = blockIdx.x, n = threadIdx.x;
   const float* d = dx.p[g] + (int64_t)t * D + n;
   float s = 0.f;
@@ -336,7 +407,14 @@ __global__ void embed_bwd_kernel(G4<const float*> dx, G4<float*> grads, int B) {
   float* gr = grads.p[g];
   gr[OFF_POS + (int64_t)t * D + n] += s;
   if (t == 0) gr[OFF_CLS + n] += s;
-  else atomicAdd(gr + OFF_BPE + n, s);
+  else if (!DET) atomicAdd(gr + OFF_BPE + n, s);
+  if constexpr (DET) {
+    if (t == 0) return;
+    __shared__ __align__(16) float red[8 * D];
+    float* part = det_part + (int64_t)g * NP * D;
+    part[(int64_t)(t - 1) * D + n] = s;
+    det_reduce_rows(part, D, NP, det_counters + g, red, 8 * D, [gr](int c, float v) { gr[OFF_BPE + c] += v; });
+  }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -526,9 +604,9 @@ __global__ void __launch_bounds__(256) attn_probs_simt_kernel(G4<const T*> qkv, 
 // column sums of LN1-backward (taken before dh is added) do not see.  Launched without the dependent-launch attribute,
 // so it starts after its predecessor has completed.  Threads: 48 float4 columns x 5 row lanes.
 constexpr int RGA_RL = 256 / (D / 4);
-template <typename T>
+template <typename T, bool DET>
 __global__ void __launch_bounds__(256) residual_grad_add_kernel(G4<const float*> dh, G4<float*> dx, G4<T*> dx_lp, G4<float*> dcol,
-                                                                int rows) {
+                                                                int rows, float* det_part, unsigned* det_counters) {
   __shared__ float4 part[RGA_RL][D / 4];
   const int g = blockIdx.y;
   const int c4 = threadIdx.x % (D / 4), rl = threadIdx.x / (D / 4);
@@ -552,8 +630,18 @@ __global__ void __launch_bounds__(256) residual_grad_add_kernel(G4<const float*>
     if (threadIdx.x < D / 4) {
       float4 s = part[0][c4];
       for (int k = 1; k < RGA_RL; ++k) { s.x += part[k][c4].x; s.y += part[k][c4].y; s.z += part[k][c4].z; s.w += part[k][c4].w; }
-      float* d = dcol.p[g] + 4 * c4;
-      atomicAdd(d, s.x); atomicAdd(d + 1, s.y); atomicAdd(d + 2, s.z); atomicAdd(d + 3, s.w);
+      if (DET) {
+        reinterpret_cast<float4*>(det_part + ((int64_t)g * gridDim.x + blockIdx.x) * D)[c4] = s;
+      } else {
+        float* d = dcol.p[g] + 4 * c4;
+        atomicAdd(d, s.x); atomicAdd(d + 1, s.y); atomicAdd(d + 2, s.z); atomicAdd(d + 3, s.w);
+      }
+    }
+    if constexpr (DET) {
+      __syncthreads();
+      float* dc = dcol.p[g];
+      det_reduce_rows(det_part + (int64_t)g * gridDim.x * D, D, gridDim.x, det_counters + g, &part[0][0].x, RGA_RL * D,
+                      [dc](int c, float v) { dc[c] += v; });
     }
   }
 }
@@ -955,7 +1043,8 @@ int launch_ln_fwd(const float* const* x, const float* const* gamma, const float*
 
 int launch_ln_bwd(const void* const* dy, const float* const* x, const float* const* mean, const float* const* rstd,
                   const float* const* gamma, float* const* dres, void* const* dres_lp, float* const* dgamma,
-                  float* const* dbeta, float* const* dcolsum, int groups, int M, int at, cudaStream_t s) {
+                  float* const* dbeta, float* const* dcolsum, int groups, int M, int at, cudaStream_t s,
+                  const DetScratch* det) {
   LnBwdP p;
   memset(&p, 0, sizeof(p));
   for (int g = 0; g < groups; ++g) {
@@ -966,13 +1055,20 @@ int launch_ln_bwd(const void* const* dy, const float* const* x, const float* con
   p.M = M;
   int bx = (M + 15) / 16;
   if (bx > 148 * 4) bx = 148 * 4;
+  if (det) {         // a fixed number of row ranges bounds the partial rows the last CTA sums
+    if (bx > 148) bx = 148;
+    if ((int64_t)groups * bx * 3 * D > det->part_floats) { set_error("ln_bwd: deterministic scratch too small"); return 1; }
+    p.det_part = det->part; p.det_counters = det->counters;
+  }
   dim3 grid(bx, groups);
-  V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<T>, grid, dim3(256), 0, s, p)));
+  if (det) { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<T, true>, grid, dim3(256), 0, s, p))); }
+  else { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<T, false>, grid, dim3(256), 0, s, p))); }
   V2S_LAUNCH_CHECK();
   return 0;
 }
 
-int launch_colsum(const void* const* dy, float* const* db, int groups, int M, int N, int t, cudaStream_t s) {
+int launch_colsum(const void* const* dy, float* const* db, int groups, int M, int N, int t, cudaStream_t s,
+                  const DetScratch* det) {
   if (N % 8 || N > 2048) { set_error("colsum: N must be a multiple of 8 and <= 2048 (got %d)", N); return 1; }
   ColsumP p;
   memset(&p, 0, sizeof(p));
@@ -983,9 +1079,16 @@ int launch_colsum(const void* const* dy, float* const* db, int groups, int M, in
   int bx = (M + rows_t * 16 - 1) / (rows_t * 16);     // >= 16 rows per row-lane
   if (bx > 148 * 4) bx = 148 * 4;
   if (bx < 1) bx = 1;
+  if (det) {         // partial rows through the scratch; without scratch (the heads' few rows) one CTA per group
+    if (bx > 148) bx = 148;
+    if (!det->part) bx = 1;
+    if (bx > 1 && (int64_t)groups * bx * N > det->part_floats) { set_error("colsum: deterministic scratch too small"); return 1; }
+    p.det_part = det->part; p.det_counters = det->counters;
+  }
   p.rows_per_block = (M + bx - 1) / bx;
   dim3 grid(bx, groups);
-  V2S_DISPATCH_AT(t, colsum_kernel<T><<<grid, 256, 0, s>>>(p));
+  if (det) { V2S_DISPATCH_AT(t, (colsum_kernel<T, true><<<grid, 256, 0, s>>>(p))); }
+  else { V2S_DISPATCH_AT(t, (colsum_kernel<T, false><<<grid, 256, 0, s>>>(p))); }
   V2S_LAUNCH_CHECK();
   return 0;
 }
@@ -1017,8 +1120,15 @@ int launch_pool_bwd(const float* const* dfeat, const int64_t* dfeat_stride, cons
   return 0;
 }
 
-int launch_embed_bwd(const float* const* dx, float* const* grads, int groups, int B, cudaStream_t s) {
-  embed_bwd_kernel<<<dim3(NT, groups), D, 0, s>>>(pack4<const float*>(dx, groups), pack4<float*>(grads, groups), B);
+int launch_embed_bwd(const float* const* dx, float* const* grads, int groups, int B, cudaStream_t s, const DetScratch* det) {
+  if (det) {
+    if ((int64_t)groups * NP * D > det->part_floats) { set_error("embed_bwd: deterministic scratch too small"); return 1; }
+    embed_bwd_kernel<true><<<dim3(NT, groups), D, 0, s>>>(pack4<const float*>(dx, groups), pack4<float*>(grads, groups), B,
+                                                          det->part, det->counters);
+  } else {
+    embed_bwd_kernel<false><<<dim3(NT, groups), D, 0, s>>>(pack4<const float*>(dx, groups), pack4<float*>(grads, groups), B,
+                                                           nullptr, nullptr);
+  }
   V2S_LAUNCH_CHECK();
   return 0;
 }
@@ -1063,14 +1173,21 @@ int launch_attn_probs_simt(const void* const* qkv, const float* const* lse, floa
 }
 
 int launch_residual_grad_add(const float* const* dh, float* const* dx, void* const* dx_lp, float* const* dcol, int groups, int B,
-                             int at, cudaStream_t s) {
+                             int at, cudaStream_t s, const DetScratch* det) {
   for (int i = 0; i < groups; ++i)
     if (reinterpret_cast<uintptr_t>(dh[i]) & 15) { set_error("hidden-state gradients must be 16-byte aligned"); return 1; }
   const int rows = B * NT;
   dim3 grid(grid_for(rows, RGA_RL, 148 * 2), groups);
-  V2S_DISPATCH_AT(at, residual_grad_add_kernel<T><<<grid, 256, 0, s>>>(pack4<const float*>(dh, groups), pack4<float*>(dx, groups),
-                                                                      pack4<T*>(at ? dx_lp : nullptr, groups),
-                                                                      pack4<float*>(dcol, groups), rows));
+  if (det && (int64_t)groups * grid.x * D > det->part_floats) { set_error("residual_grad_add: deterministic scratch too small"); return 1; }
+  if (det) {
+    V2S_DISPATCH_AT(at, (residual_grad_add_kernel<T, true><<<grid, 256, 0, s>>>(
+                            pack4<const float*>(dh, groups), pack4<float*>(dx, groups), pack4<T*>(at ? dx_lp : nullptr, groups),
+                            pack4<float*>(dcol, groups), rows, det->part, det->counters)));
+  } else {
+    V2S_DISPATCH_AT(at, (residual_grad_add_kernel<T, false><<<grid, 256, 0, s>>>(
+                            pack4<const float*>(dh, groups), pack4<float*>(dx, groups), pack4<T*>(at ? dx_lp : nullptr, groups),
+                            pack4<float*>(dcol, groups), rows, nullptr, nullptr)));
+  }
   V2S_LAUNCH_CHECK();
   return 0;
 }
@@ -1190,18 +1307,20 @@ int launch_preprocess_u8(const uint8_t* src, float* dst, int B, cudaStream_t s) 
   return 0;
 }
 
+template <bool ADD>
 __global__ void splitk_reduce_kernel(float* __restrict__ out, const float* __restrict__ part,
                                      const float* __restrict__ bias, int MN, int N, int splits) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < MN; i += gridDim.x * blockDim.x) {
-    float v = bias ? bias[i % N] : 0.f;
+    float v = ADD ? out[i] : bias ? bias[i % N] : 0.f;
     for (int s = 0; s < splits; ++s) v += part[(int64_t)s * MN + i];      // fixed order: deterministic
     out[i] = v;
   }
 }
 
-// out[m,n] = bias[n] + sum_s part[s][m][n]: deterministic second pass of a split-K GEMM
-int launch_splitk_reduce(float* out, const float* part, const float* bias, int M, int N, int splits, cudaStream_t s) {
-  splitk_reduce_kernel<<<grid_for((int64_t)M * N, 256, 148), 256, 0, s>>>(out, part, bias, M * N, N, splits);
+// out[m,n] = bias[n] + sum_s part[s][m][n] (add: out[m,n] += sum_s part[s][m][n]): deterministic second pass of a split-K GEMM
+int launch_splitk_reduce(float* out, const float* part, const float* bias, int M, int N, int splits, cudaStream_t s, bool add) {
+  if (add) splitk_reduce_kernel<true><<<grid_for((int64_t)M * N, 256, 148), 256, 0, s>>>(out, part, nullptr, M * N, N, splits);
+  else splitk_reduce_kernel<false><<<grid_for((int64_t)M * N, 256, 148), 256, 0, s>>>(out, part, bias, M * N, N, splits);
   V2S_LAUNCH_CHECK();
   return 0;
 }

@@ -19,18 +19,21 @@ int launch_ln_fwd(const float* const* x, const float* const* gamma, const float*
 int launch_ln_bwd(const void* const* dy, const float* const* x, const float* const* mean,
                   const float* const* rstd, const float* const* gamma, float* const* dres,
                   void* const* dres_lp, float* const* dgamma, float* const* dbeta, float* const* dcolsum,
-                  int groups, int M, int at, cudaStream_t s);
-// db[n] += sum_m dy[m,n]; src type tag `t`
-int launch_colsum(const void* const* dy, float* const* db, int groups, int M, int N, int t, cudaStream_t s);
+                  int groups, int M, int at, cudaStream_t s, const DetScratch* det = nullptr);
+// db[n] += sum_m dy[m,n]; src type tag `t`.  With `det` (deterministic mode) the sum has a fixed order: partial rows in
+// det->part, or, when det->part is NULL, one CTA per group
+int launch_colsum(const void* const* dy, float* const* db, int groups, int M, int N, int t, cudaStream_t s,
+                  const DetScratch* det = nullptr);
 int launch_pool_fwd(const float* const* hidden, float* const* feat, const int64_t* feat_stride,
                     int groups, int B, cudaStream_t s);
 int launch_pool_bwd(const float* const* dfeat, const int64_t* dfeat_stride, const float* const* dhidden,
                     float* const* dx, void* const* dx_lp, int groups, int B, int at, cudaStream_t s);
-int launch_embed_bwd(const float* const* dx, float* const* grads, int groups, int B, cudaStream_t s);
+int launch_embed_bwd(const float* const* dx, float* const* grads, int groups, int B, cudaStream_t s,
+                     const DetScratch* det = nullptr);
 // dx (fp32, in/out) += dh; dx_lp (activation type, 16-bit modes only) = updated dx; [B,197,192] per group;
 // dcol (optional, per group) += column sums of dh
 int launch_residual_grad_add(const float* const* dh, float* const* dx, void* const* dx_lp, float* const* dcol, int groups, int B,
-                             int at, cudaStream_t s);
+                             int at, cudaStream_t s, const DetScratch* det = nullptr);
 
 // attention over qkv [B,197,576] (q|k|v, head h at columns h*64): ctx [B,197,192], lse [B,3,197]
 int launch_attn_fwd_simt(const void* const* qkv, void* const* ctx, float* const* lse, int groups, int B,
@@ -72,6 +75,7 @@ int launch_augment_finish(const uint8_t* src, int n, int in_size, const int32_t*
                           const float* k1d, const int32_t* erase, const float* mean3, const float* std3, float* dst,
                           cudaStream_t s);
 int launch_zero(void* p, int64_t bytes, cudaStream_t s);
-int launch_splitk_reduce(float* out, const float* part, const float* bias, int M, int N, int splits, cudaStream_t s);
+int launch_splitk_reduce(float* out, const float* part, const float* bias, int M, int N, int splits, cudaStream_t s,
+                         bool add = false);
 
 }  // namespace v2s

@@ -210,9 +210,18 @@ _STORES = weakref.WeakSet()
 _workspaces = {}
 
 
+def _deterministic():
+    """Pass ``torch.are_deterministic_algorithms_enabled()`` on to the library (``v2s_set_deterministic``): called before
+    every call that sizes a workspace or enqueues a backward pass, so that the library's fixed-order reductions follow
+    torch's flag.  Returns the flag."""
+    on = bool(torch.are_deterministic_algorithms_enabled())
+    check(lib.v2s_set_deterministic(int(on)), "set_deterministic")
+    return on
+
+
 def _scratch_workspace(device, batch, mode, n_groups, n_saved):
     """Persistent scratch for calls that keep nothing across calls (no-grad forwards)."""
-    key = (device, batch, mode, n_groups, n_saved)
+    key = (device, batch, mode, n_groups, n_saved, _deterministic())
     ws = _workspaces.get(key)
     if ws is None:
         nbytes = lib.v2s_workspace_bytes(batch, mode, n_groups, n_saved)
@@ -229,6 +238,7 @@ def _aligned(ws):
 
 
 def _new_workspace(device, batch, mode, n_groups, n_saved):
+    _deterministic()                # the deterministic mode's scratch is part of the size
     nbytes = lib.v2s_workspace_bytes(batch, mode, n_groups, n_saved)
     if nbytes < 0:
         raise RuntimeError("v2s_workspace_bytes: bad arguments")
@@ -463,6 +473,7 @@ class _BackboneFn(torch.autograd.Function):
         nones = (None,) * 7
         if dout is None and all(t is None for t in dhid):
             return nones
+        _deterministic()
         grads = store.grads()
         dout = _grad_f32(dout) if dout is not None else None
         outs = None
@@ -715,6 +726,7 @@ class _DualStreamFn(torch.autograd.Function):
         B, mode, ws = ctx.B, ctx.mode, ctx.ws
         dpred = dpred.contiguous().to(torch.float32)
         dfeat = torch.empty(B, 384, dtype=torch.float32, device=dpred.device)
+        _deterministic()
         base, nbytes = _aligned(ws)
         check(lib.v2s_heads_backward(ptr(hs.flat), ptr(hs.grads()), ptr(feat_o), ptr(mask_o), ptr(dpred), ptr(dfeat),
                                      B, C.c_void_p(base), nbytes, stream_ptr()), "heads_backward")
@@ -815,7 +827,7 @@ class DualStreamNetwork(nn.Module):
                 self.target_network_1.vit._store, self.target_network_2.vit._store]
 
     def _take_workspace(self, dev, B, mode):
-        key = (dev, B, mode)
+        key = (dev, B, mode, _deterministic())
         ws = self._ws.get(key)
         if ws is None:
             ws = _new_workspace(dev, B, mode, 4, 2)
@@ -976,7 +988,7 @@ class DualStreamNetwork(nn.Module):
             s_.ensure()                     # host-side state the eager step maintains: flat buffers, attached .grad views
         ptrs = tuple(s_.flat.data_ptr() for s_ in st + [hs]) + tuple(s_.grads().data_ptr() for s_ in (st[0], st[1], hs))
         key = (tuple(x1.shape), x1.device, self._mode(), int(accumulation_steps), self.loss_mode, float(self.temperature),
-               dropout_on, float(drop.p), self._fixed_masks is not None, ptrs)
+               dropout_on, float(drop.p), self._fixed_masks is not None, ptrs, torch.are_deterministic_algorithms_enabled())
         graphs = self.__dict__.setdefault("_graphs", {})
         if len(graphs) > 8:                 # parameters moved (.to(), re-flattening): stale graphs
             graphs.clear()
