@@ -26,15 +26,18 @@
 extern "C" {
 #endif
 
-#define V2S_ABI_VERSION 3 /* 3: v2s_infonce_loss, v2s_preprocess_u8_patches, v2s_group.x_format (was a reserved zero field);
-                             additive to 3: v2s_group_outputs, v2s_backbone_forward_ex / v2s_backbone_backward_ex,
-                             v2s_test_attention which = 2 */
+#define V2S_ABI_VERSION 4 /* 4: one entry point per operation: v2s_backbone_forward / _backward take the per-group outputs
+                             and (backward) the layer range, v2s_heads_loss_fwd_bwd the device loss scale, v2s_adam_step
+                             and v2s_ema_update the lp_format; their narrower variants and the bf16-only cast are
+                             removed.  3: v2s_infonce_loss, v2s_preprocess_u8_patches, v2s_group.x_format (was a
+                             reserved zero field); additive to 3: v2s_group_outputs, v2s_test_attention which = 2 */
 
 /* compute modes */
 #define V2S_MODE_FP32 0 /* fp32 activations + fp32 SIMT GEMMs: the "fp32 check mode" of north_star */
 #define V2S_MODE_BF16 1 /* bf16 GEMM operands (tcgen05), fp32 accumulate / residual / LN / softmax */
 #define V2S_MODE_FP16 2 /* fp16 GEMM operands: the reference's own CUDA precision (torch.autocast default dtype +
-                           GradScaler, ref:ssp_vit2spn_tiny.py:175,209-217); needs loss scaling (v2s_*_amp) */
+                           GradScaler, ref:ssp_vit2spn_tiny.py:175,209-217); needs loss scaling (grad_scale_dev of
+                           v2s_heads_loss_fwd_bwd / v2s_infonce_loss, v2s_adam_step_amp) */
 
 /* format of the 16-bit shadow copy of a flat parameter buffer (params_lp) */
 #define V2S_LP_BF16 0
@@ -102,24 +105,10 @@ typedef struct v2s_group {
   int32_t x_format;       /* 0 or 1, see x (1: bf16 / fp16 modes only) */
 } v2s_group_t;
 
-/* ViTBackbone.forward for up to 4 backbones (ref:ssp_vit2spn_tiny.py:114-118; HF
- * modeling_vit.py:100-128,328-346): patch-embed, 12 pre-LN blocks, mean over 197 tokens. */
-int v2s_backbone_forward(const v2s_group_t* host_groups, int n_groups, int batch, int mode,
-                         void* workspace, int64_t workspace_bytes, void* stream);
-/* autograd backward of the above for the groups with slot >= 0 (ref:213 loss.backward()) */
-int v2s_backbone_backward(const v2s_group_t* host_groups, int n_groups, int batch, int mode,
-                          void* workspace, int64_t workspace_bytes, void* stream);
-/* The same for blocks [layer_lo, layer_hi) only, highest block first.  layer_hi == V2S_LAYERS starts from dfeat /
- * dhidden; layer_lo == 0 ends with the embedding gradients; the residual-stream gradient is carried between calls in
- * the workspace.  The flat gradient layout is block-contiguous, so after the call for [lo, hi) the gradients of those
- * blocks are final: a data-parallel host can all-reduce that slice while the next range computes (SURVEY 8e). */
-int v2s_backbone_backward_range(const v2s_group_t* host_groups, int n_groups, int batch, int mode,
-                                void* workspace, int64_t workspace_bytes, int layer_hi, int layer_lo,
-                                void* stream);
-
-/* Per-layer outputs of one group (transformers' output_hidden_states / output_attentions).  Pass an array of n_groups
- * of these, or NULL for none: with NULL (or every pointer NULL) the calls below launch exactly what the plain entry
- * points launch.  A saved group's hidden[] must be the same in its forward and its backward call. */
+/* Per-layer outputs of one group (transformers' output_hidden_states / output_attentions).  The two calls below take an
+ * array of n_groups of these, or NULL for none.  NULL (or every pointer NULL) requests nothing and costs nothing: the
+ * call then launches exactly the kernels of a backbone pass without per-layer outputs.  A saved group's hidden[] must
+ * be the same in its forward and its backward call. */
 typedef struct v2s_group_outputs {
   float* hidden[V2S_LAYERS + 1];        /* out: hidden_states[l] fp32 [batch,197,192]; all 13 or none. When set, the
                                            group's residual stream lives here; a saved group's backward reads it back */
@@ -129,11 +118,19 @@ typedef struct v2s_group_outputs {
                                            dhidden[12] the backward starts at the highest l with a gradient: the
                                            blocks above it are skipped and get no gradient */
 } v2s_group_outputs_t;
-int v2s_backbone_forward_ex(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs /* [n_groups] or NULL */,
-                            int n_groups, int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
-int v2s_backbone_backward_ex(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs, int n_groups,
-                             int batch, int mode, void* workspace, int64_t workspace_bytes, int layer_hi, int layer_lo,
-                             void* stream);
+
+/* ViTBackbone.forward for up to 4 backbones (ref:ssp_vit2spn_tiny.py:114-118; HF
+ * modeling_vit.py:100-128,328-346): patch-embed, 12 pre-LN blocks, mean over 197 tokens. */
+int v2s_backbone_forward(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs /* [n_groups] or NULL */,
+                         int n_groups, int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
+/* Autograd backward of the above for the groups with slot >= 0 (ref:213 loss.backward()), over blocks
+ * [layer_lo, layer_hi) only, highest block first: [0, V2S_LAYERS) is the whole backward.  layer_hi == V2S_LAYERS starts
+ * from dfeat / dhidden; layer_lo == 0 ends with the embedding gradients; the residual-stream gradient is carried between
+ * calls in the workspace.  The flat gradient layout is block-contiguous, so after the call for [lo, hi) the gradients of
+ * those blocks are final: a data-parallel host can all-reduce that slice while the next range computes (SURVEY 8e). */
+int v2s_backbone_backward(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs /* [n_groups] or NULL */,
+                          int n_groups, int batch, int mode, void* workspace, int64_t workspace_bytes, int layer_hi,
+                          int layer_lo, void* stream);
 
 /* projection_head + prediction_head on the concatenated online features and projection_head on
  * the target features (ref:ssp_vit2spn_tiny.py:153-158), fused with the loss
@@ -143,20 +140,15 @@ int v2s_backbone_backward_ex(const v2s_group_t* host_groups, const v2s_group_out
  *   feat_online / feat_target: [batch,384] fp32;  dfeat_online: out [batch,384]
  *   mask_online / mask_target: dropout multipliers [batch,1024] (0 or 1/(1-p)); NULL = no dropout
  *   pred / target_proj: optional outs [batch,128];  loss: out, 1 float (already / accum)
- *   grad_scale: upstream gradient of the loss (1.0, or GradScaler's scale; ref:213) */
+ *   upstream gradient of the loss = grad_scale * *grad_scale_dev; grad_scale_dev may be NULL (= 1).  grad_scale is a
+ *   host value (1.0, or a fixed loss scale); grad_scale_dev is read on the device (torch.amp.GradScaler's scale tensor:
+ *   scaler.scale(loss).backward() of ref:213 without a host synchronisation) */
 int v2s_heads_loss_fwd_bwd(const float* head_params, float* head_grads, const float* feat_online,
                            const float* feat_target, const float* mask_online,
                            const float* mask_target, float* dfeat_online, float* pred,
                            float* target_proj, float* loss, int batch, int accumulation_steps,
-                           float grad_scale, int with_backward, void* workspace,
+                           float grad_scale, const float* grad_scale_dev, int with_backward, void* workspace,
                            int64_t workspace_bytes, void* stream);
-/* same with the loss scale read from device memory (*grad_scale_dev, e.g. torch.amp.GradScaler's scale tensor):
- * scaler.scale(loss).backward() of ref:ssp_vit2spn_tiny.py:213 without a host synchronisation */
-int v2s_heads_loss_fwd_bwd_amp(const float* head_params, float* head_grads, const float* feat_online,
-                               const float* feat_target, const float* mask_online, const float* mask_target,
-                               float* dfeat_online, float* pred, float* target_proj, float* loss, int batch,
-                               int accumulation_steps, const float* grad_scale_dev, int with_backward,
-                               void* workspace, int64_t workspace_bytes, void* stream);
 
 /* The same three stages as separate calls, for the autograd-compatible path where the script's
  * own criterion computes the loss between forward and backward (ref:210-213).  The heads'
@@ -190,7 +182,8 @@ int v2s_dropout_mask(float* mask, int64_t n, float p, uint64_t seed, uint64_t of
  * eps 1e-8, no weight decay unless weight_decay != 0 (L2, as the fine-tune scripts use).
  * Hyper-parameters are doubles, converted exactly as torch converts its Python floats.
  * `step` is the 1-based step count; grads are multiplied by grad_scale first (1/world, 1/scale).
- * If params_lp != NULL the bf16 shadow copy is refreshed in the same pass. */
+ * If params_lp != NULL its 16-bit shadow copy, in format lp_format (V2S_LP_BF16 / V2S_LP_FP16), is refreshed in the
+ * same pass. */
 typedef struct v2s_range {
   float* params;
   const float* grads;
@@ -200,10 +193,7 @@ typedef struct v2s_range {
   int64_t numel;
 } v2s_range_t;
 int v2s_adam_step(const v2s_range_t* host_ranges, int n_ranges, int64_t step, double lr, double beta1,
-                  double beta2, double eps, double weight_decay, double grad_scale, void* stream);
-/* same, with the format of params_lp given (V2S_LP_BF16 / V2S_LP_FP16) */
-int v2s_adam_step_lp(const v2s_range_t* host_ranges, int n_ranges, int64_t step, double lr, double beta1,
-                     double beta2, double eps, double weight_decay, double grad_scale, int lp_format, void* stream);
+                  double beta2, double eps, double weight_decay, double grad_scale, int lp_format, void* stream);
 /* The optimizer step under torch.amp.GradScaler (ref:ssp_vit2spn_tiny.py:175,216-217: scaler.step(optimizer) /
  * scaler.update()), without a host synchronisation: the step count lives on the device and the call is a no-op when
  * the scaler found an inf / nan.  state8 = 8 caller-owned device floats, state8[0] = optimizer steps taken so far
@@ -218,18 +208,13 @@ int v2s_adam_step_amp(const v2s_range_t* host_ranges, int n_ranges, float* state
                       const float* grad_scale_dev, const float* found_inf_dev, int lp_format, int advance_step,
                       void* stream);
 
-/* update_target_network (ref:162-166): target = m*target + (1-m)*online over flat buffers */
+/* update_target_network (ref:162-166): target = m*target + (1-m)*online over flat buffers; host_targets_lp (may be
+ * NULL): the targets' 16-bit shadow copies, refreshed in the same pass in format lp_format (V2S_LP_BF16 / V2S_LP_FP16) */
 int v2s_ema_update(float* const* host_targets, const float* const* host_onlines,
-                   void* const* host_targets_lp, int n_pairs, int64_t numel, double momentum,
+                   void* const* host_targets_lp, int n_pairs, int64_t numel, double momentum, int lp_format,
                    void* stream);
 
-int v2s_ema_update_lp(float* const* host_targets, const float* const* host_onlines,
-                      void* const* host_targets_lp, int n_pairs, int64_t numel, double momentum, int lp_format,
-                      void* stream);
-
-/* fp32 → bf16 shadow copy of a flat buffer */
-int v2s_cast_bf16(const float* src, void* dst, int64_t numel, void* stream);
-/* fp32 → 16-bit shadow copy in the given format (V2S_LP_BF16 / V2S_LP_FP16) */
+/* fp32 → 16-bit shadow copy of a flat buffer in the given format (V2S_LP_BF16 / V2S_LP_FP16) */
 int v2s_cast_lp(const float* src, void* dst, int64_t numel, int lp_format, void* stream);
 
 /* synthetic OCTMNIST-shaped input pipeline (ref:ssp_vit2spn_tiny.py:84-96, deterministic part):

@@ -3,7 +3,7 @@
 * ``vit_outputs_oracle.backbone_outputs`` (stated with the oracle's functions) is pinned to ``transformers.ViTModel``
   with eager attention on the same weights;
 * the host API resolves the two flags as transformers does and keeps the old hidden-state accessor's contract;
-* the C entry points reject malformed ``v2s_group_outputs`` before touching the device.
+* the C entry points reject malformed ``v2s_group_outputs`` and layer ranges before touching the device.
 """
 import ctypes as C
 import os
@@ -53,8 +53,9 @@ def test_output_flags_and_accessors():
     assert modules.ViTModelOutput(m, torch.zeros(1, 197, 192)).attentions is None
 
 
-def _call(fn, outputs, *, slot=0, dhidden=None, dfeat=None):
-    """Calls a backbone _ex entry point with fake (never dereferenced) device pointers: the argument checks run first."""
+def _call(fn, outputs, *, slot=0, dhidden=None, dfeat=None, layer_hi=12, layer_lo=0):
+    """Calls a backbone entry point with fake (never dereferenced) device pointers: the argument checks run first.
+    ``outputs=None`` passes NULL for the per-group outputs."""
     from vit2spn import _lib
     B, mode = 2, _lib.MODE_FP32
     nbytes = _lib.lib.v2s_workspace_bytes(B, mode, 1, 1)
@@ -62,15 +63,15 @@ def _call(fn, outputs, *, slot=0, dhidden=None, dfeat=None):
     g.params, g.x, g.grads, g.slot = 0x10000, 0x20000, 0x30000, slot
     g.dhidden, g.dfeat = dhidden, dfeat
     arr = (_lib.Group * 1)(g)
-    outs = (_lib.GroupOutputs * 1)(outputs)
+    outs = (_lib.GroupOutputs * 1)(outputs) if outputs is not None else None
     if fn == "forward":
-        rc = _lib.lib.v2s_backbone_forward_ex(arr, outs, 1, B, mode, C.c_void_p(1 << 20), nbytes, None)
+        rc = _lib.lib.v2s_backbone_forward(arr, outs, 1, B, mode, C.c_void_p(1 << 20), nbytes, None)
     else:
-        rc = _lib.lib.v2s_backbone_backward_ex(arr, outs, 1, B, mode, C.c_void_p(1 << 20), nbytes, 12, 0, None)
+        rc = _lib.lib.v2s_backbone_backward(arr, outs, 1, B, mode, C.c_void_p(1 << 20), nbytes, layer_hi, layer_lo, None)
     return rc, _lib.lib.v2s_last_error().decode()
 
 
-def test_ex_entry_points_reject_malformed_outputs():
+def test_backbone_entry_points_reject_malformed_outputs_and_ranges():
     from vit2spn import _lib
     assert C.sizeof(_lib.GroupOutputs) == (13 + 12 + 13) * 8
     o = _lib.GroupOutputs()
@@ -93,3 +94,5 @@ def test_ex_entry_points_reject_malformed_outputs():
     assert rc != 0 and "both" in err, err
     rc, err = _call("backward", _lib.GroupOutputs())      # no gradient at all
     assert rc != 0 and "needs dfeat or dhidden" in err, err
+    rc, err = _call("backward", None, dfeat=0x40000, layer_hi=4, layer_lo=8)    # empty layer range, no outputs
+    assert rc != 0 and "bad layer range" in err, err

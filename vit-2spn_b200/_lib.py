@@ -17,6 +17,7 @@ MODE_FP16 = 2
 LP_BF16 = 0
 LP_FP16 = 1
 MAX_GROUPS = 4
+ABI_VERSION = 4      # V2S_ABI_VERSION of include/vit2spn.h that the signatures below bind
 
 if not os.path.exists(LIB_PATH):
     raise ImportError(
@@ -24,6 +25,11 @@ if not os.path.exists(LIB_PATH):
         "vit2spn has no CPU fallback; the sm_100a CUDA library is required.")
 
 lib = C.CDLL(LIB_PATH)
+# Entry points keep their names across ABI versions while their signatures change, so a stale library would bind and
+# then be called with the wrong arguments: refuse it here instead (ctypes' default return type is int).
+if lib.v2s_abi_version() != ABI_VERSION:
+    raise ImportError(f"{LIB_PATH} has C ABI version {lib.v2s_abi_version()}, this package binds version "
+                      f"{ABI_VERSION}: rebuild with ./build.sh")
 
 
 class Group(C.Structure):
@@ -59,28 +65,20 @@ _SIGS = {
     "v2s_heads_layout": (C.c_int, [C.POINTER(_i64)]),
     "v2s_workspace_bytes": (_i64, [_i, _i, _i, _i]),
     "v2s_set_deterministic": (C.c_int, [_i]),
-    "v2s_backbone_forward": (C.c_int, [C.POINTER(Group), _i, _i, _i, _vp, _i64, _vp]),
-    "v2s_backbone_backward": (C.c_int, [C.POINTER(Group), _i, _i, _i, _vp, _i64, _vp]),
-    "v2s_backbone_backward_range": (C.c_int, [C.POINTER(Group), _i, _i, _i, _vp, _i64, _i, _i, _vp]),
-    "v2s_backbone_forward_ex": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), _i, _i, _i, _vp, _i64, _vp]),
-    "v2s_backbone_backward_ex": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), _i, _i, _i, _vp, _i64, _i, _i,
-                                           _vp]),
-    "v2s_heads_loss_fwd_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _f, _i,
+    "v2s_backbone_forward": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), _i, _i, _i, _vp, _i64, _vp]),
+    "v2s_backbone_backward": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), _i, _i, _i, _vp, _i64, _i, _i,
+                                        _vp]),
+    "v2s_heads_loss_fwd_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _f, _vp, _i,
                                          _vp, _i64, _vp]),
-    "v2s_heads_loss_fwd_bwd_amp": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _i,
-                                             _vp, _i64, _vp]),
     "v2s_heads_forward": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _vp]),
     "v2s_heads_backward": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _vp]),
     "v2s_cosine_loss": (C.c_int, [_vp, _vp, _vp, _vp, _i, _i, _f, _vp]),
     "v2s_infonce_loss": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i64, _f, _i, _f, _vp, _vp]),
     "v2s_dropout_mask": (C.c_int, [_vp, _i64, _f, C.c_uint64, C.c_uint64, _vp]),
-    "v2s_adam_step": (C.c_int, [C.POINTER(Range), _i, _i64, _d, _d, _d, _d, _d, _d, _vp]),
-    "v2s_adam_step_lp": (C.c_int, [C.POINTER(Range), _i, _i64, _d, _d, _d, _d, _d, _d, _i, _vp]),
+    "v2s_adam_step": (C.c_int, [C.POINTER(Range), _i, _i64, _d, _d, _d, _d, _d, _d, _i, _vp]),
     "v2s_adam_step_amp": (C.c_int, [C.POINTER(Range), _i, _vp, _d, _d, _d, _d, _d, _d, _vp, _vp, _i, _i, _vp]),
-    "v2s_ema_update_lp": (C.c_int, [C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), _i, _i64, _d, _i, _vp]),
+    "v2s_ema_update": (C.c_int, [C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), _i, _i64, _d, _i, _vp]),
     "v2s_cast_lp": (C.c_int, [_vp, _vp, _i64, _i, _vp]),
-    "v2s_ema_update": (C.c_int, [C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp), _i, _i64, _d, _vp]),
-    "v2s_cast_bf16": (C.c_int, [_vp, _vp, _i64, _vp]),
     "v2s_preprocess_u8": (C.c_int, [_vp, _vp, _i, _vp]),
     "v2s_preprocess_u8_patches": (C.c_int, [_vp, _vp, _i, _i, _vp]),
     "v2s_augment_finish_u8": (C.c_int, [_vp, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp]),

@@ -532,7 +532,7 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
 // layer_lo == 0 finishes with the embedding gradients.  Between two calls the residual-stream gradient lives in the
 // workspace, so a full backward may be issued in several ranges (gradient all-reduce overlapped per range).
 static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outputs_t* outs_in, int G_in, int B, int mode,
-                                  void* ws, int64_t ws_bytes, cudaStream_t st, int layer_hi = NL, int layer_lo = 0) {
+                                  void* ws, int64_t ws_bytes, cudaStream_t st, int layer_hi, int layer_lo) {
   if (layer_lo < 0 || layer_hi > NL || layer_lo >= layer_hi) { set_error("backbone_backward: bad layer range [%d, %d)", layer_lo, layer_hi); return 1; }
   // keep only the groups that saved activations and want gradients
   v2s_group_t gs[MAXG];
@@ -904,18 +904,6 @@ static int heads_backward_impl(const float* hp, float* hg, const float* fo, cons
   return 0;
 }
 
-static int heads_impl(const float* hp, float* hg, const float* fo, const float* ft, const float* mo, const float* mt,
-                      float* dfo, float* pred_out, float* tgt_out, float* loss, int B, int accum, float grad_scale,
-                      int with_backward, void* ws, int64_t ws_bytes, cudaStream_t st, const float* grad_scale_dev = nullptr) {
-  if (!loss) { set_error("heads: null loss"); return 1; }
-  V2S_TRY(heads_forward_impl(hp, fo, ft, mo, mt, pred_out, tgt_out, B, ws, ws_bytes, st));
-  HeadsBufs hb;
-  V2S_TRY(heads_bufs(ws, ws_bytes, B, &hb));
-  V2S_TRY(launch_cosine_loss(hb.pr, hb.zt, loss, with_backward ? hb.dp : nullptr, B, accum, grad_scale, st, grad_scale_dev));
-  if (!with_backward) return 0;
-  return heads_backward_impl(hp, hg, fo, mo, nullptr, dfo, B, ws, ws_bytes, st);
-}
-
 }  // namespace v2s
 
 // =============================================================================================
@@ -982,33 +970,14 @@ int64_t v2s_workspace_bytes(int batch, int mode, int n_groups, int n_saved) {
   return plan_total(p, n_groups, n_saved) + (tc_deterministic() ? det_scratch_bytes(p, n_saved) : 0);
 }
 
-int v2s_backbone_forward(const v2s_group_t* groups, int n_groups, int batch, int mode, void* workspace,
-                         int64_t workspace_bytes, void* stream) {
-  if (!groups) { set_error("null groups"); return 1; }
-  return backbone_forward_impl(groups, nullptr, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
-}
-
-int v2s_backbone_forward_ex(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, int n_groups, int batch, int mode,
-                            void* workspace, int64_t workspace_bytes, void* stream) {
+int v2s_backbone_forward(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, int n_groups, int batch, int mode,
+                         void* workspace, int64_t workspace_bytes, void* stream) {
   if (!groups) { set_error("null groups"); return 1; }
   return backbone_forward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
-int v2s_backbone_backward(const v2s_group_t* groups, int n_groups, int batch, int mode, void* workspace,
-                          int64_t workspace_bytes, void* stream) {
-  if (!groups) { set_error("null groups"); return 1; }
-  return backbone_backward_impl(groups, nullptr, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
-}
-
-int v2s_backbone_backward_range(const v2s_group_t* groups, int n_groups, int batch, int mode, void* workspace,
-                                int64_t workspace_bytes, int layer_hi, int layer_lo, void* stream) {
-  if (!groups) { set_error("null groups"); return 1; }
-  return backbone_backward_impl(groups, nullptr, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
-                                layer_hi, layer_lo);
-}
-
-int v2s_backbone_backward_ex(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, int n_groups, int batch,
-                             int mode, void* workspace, int64_t workspace_bytes, int layer_hi, int layer_lo, void* stream) {
+int v2s_backbone_backward(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, int n_groups, int batch,
+                          int mode, void* workspace, int64_t workspace_bytes, int layer_hi, int layer_lo, void* stream) {
   if (!groups) { set_error("null groups"); return 1; }
   return backbone_backward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
                                 layer_hi, layer_lo);
@@ -1017,23 +986,20 @@ int v2s_backbone_backward_ex(const v2s_group_t* groups, const v2s_group_outputs_
 int v2s_heads_loss_fwd_bwd(const float* head_params, float* head_grads, const float* feat_online,
                            const float* feat_target, const float* mask_online, const float* mask_target,
                            float* dfeat_online, float* pred, float* target_proj, float* loss, int batch,
-                           int accumulation_steps, float grad_scale, int with_backward, void* workspace,
-                           int64_t workspace_bytes, void* stream) {
+                           int accumulation_steps, float grad_scale, const float* grad_scale_dev, int with_backward,
+                           void* workspace, int64_t workspace_bytes, void* stream) {
   if (batch < 1 || accumulation_steps < 1) { set_error("heads: bad batch/accumulation_steps"); return 1; }
-  return heads_impl(head_params, head_grads, feat_online, feat_target, mask_online, mask_target, dfeat_online, pred,
-                    target_proj, loss, batch, accumulation_steps, grad_scale, with_backward, workspace,
-                    workspace_bytes, (cudaStream_t)stream);
-}
-
-int v2s_heads_loss_fwd_bwd_amp(const float* head_params, float* head_grads, const float* feat_online,
-                               const float* feat_target, const float* mask_online, const float* mask_target,
-                               float* dfeat_online, float* pred, float* target_proj, float* loss, int batch,
-                               int accumulation_steps, const float* grad_scale_dev, int with_backward, void* workspace,
-                               int64_t workspace_bytes, void* stream) {
-  if (batch < 1 || accumulation_steps < 1) { set_error("heads: bad batch/accumulation_steps"); return 1; }
-  return heads_impl(head_params, head_grads, feat_online, feat_target, mask_online, mask_target, dfeat_online, pred,
-                    target_proj, loss, batch, accumulation_steps, 1.0f, with_backward, workspace, workspace_bytes,
-                    (cudaStream_t)stream, grad_scale_dev);
+  if (!loss) { set_error("heads: null loss"); return 1; }
+  const cudaStream_t st = (cudaStream_t)stream;
+  V2S_TRY(heads_forward_impl(head_params, feat_online, feat_target, mask_online, mask_target, pred, target_proj, batch,
+                             workspace, workspace_bytes, st));
+  HeadsBufs hb;
+  V2S_TRY(heads_bufs(workspace, workspace_bytes, batch, &hb));
+  V2S_TRY(launch_cosine_loss(hb.pr, hb.zt, loss, with_backward ? hb.dp : nullptr, batch, accumulation_steps, grad_scale,
+                             st, grad_scale_dev));
+  if (!with_backward) return 0;
+  return heads_backward_impl(head_params, head_grads, feat_online, mask_online, nullptr, dfeat_online, batch, workspace,
+                             workspace_bytes, st);
 }
 
 int v2s_heads_forward(const float* head_params, const float* feat_online, const float* feat_target,
@@ -1072,18 +1038,6 @@ int v2s_dropout_mask(float* mask, int64_t n, float p, uint64_t seed, uint64_t of
   return launch_dropout_mask(mask, n, p, seed, offset, (cudaStream_t)stream);
 }
 
-int v2s_adam_step(const v2s_range_t* ranges, int n_ranges, int64_t step, double lr, double beta1, double beta2,
-                  double eps, double weight_decay, double grad_scale, void* stream) {
-  if (!ranges || step < 1) { set_error("adam: bad argument"); return 1; }
-  for (int i = 0; i < n_ranges; ++i)
-    if ((reinterpret_cast<uintptr_t>(ranges[i].params) | reinterpret_cast<uintptr_t>(ranges[i].grads) |
-         reinterpret_cast<uintptr_t>(ranges[i].exp_avg) | reinterpret_cast<uintptr_t>(ranges[i].exp_avg_sq)) & 15) {
-      set_error("adam: range %d is not 16-byte aligned", i);
-      return 1;
-    }
-  return launch_adam(ranges, n_ranges, step, lr, beta1, beta2, eps, weight_decay, grad_scale, (cudaStream_t)stream);
-}
-
 static int check_ranges(const v2s_range_t* ranges, int n_ranges) {
   for (int i = 0; i < n_ranges; ++i)
     if ((reinterpret_cast<uintptr_t>(ranges[i].params) | reinterpret_cast<uintptr_t>(ranges[i].grads) |
@@ -1094,8 +1048,8 @@ static int check_ranges(const v2s_range_t* ranges, int n_ranges) {
   return 0;
 }
 
-int v2s_adam_step_lp(const v2s_range_t* ranges, int n_ranges, int64_t step, double lr, double beta1, double beta2,
-                     double eps, double weight_decay, double grad_scale, int lp_format, void* stream) {
+int v2s_adam_step(const v2s_range_t* ranges, int n_ranges, int64_t step, double lr, double beta1, double beta2,
+                  double eps, double weight_decay, double grad_scale, int lp_format, void* stream) {
   if (!ranges || step < 1) { set_error("adam: bad argument"); return 1; }
   V2S_TRY(check_ranges(ranges, n_ranges));
   return launch_adam(ranges, n_ranges, step, lr, beta1, beta2, eps, weight_decay, grad_scale, (cudaStream_t)stream,
@@ -1112,13 +1066,7 @@ int v2s_adam_step_amp(const v2s_range_t* ranges, int n_ranges, float* state8, do
 }
 
 int v2s_ema_update(float* const* targets, const float* const* onlines, void* const* targets_lp, int n_pairs,
-                   int64_t numel, double momentum, void* stream) {
-  if (!targets || !onlines) { set_error("ema: null"); return 1; }
-  return launch_ema(targets, onlines, targets_lp, n_pairs, numel, momentum, (cudaStream_t)stream);
-}
-
-int v2s_ema_update_lp(float* const* targets, const float* const* onlines, void* const* targets_lp, int n_pairs,
-                      int64_t numel, double momentum, int lp_format, void* stream) {
+                   int64_t numel, double momentum, int lp_format, void* stream) {
   if (!targets || !onlines) { set_error("ema: null"); return 1; }
   return launch_ema(targets, onlines, targets_lp, n_pairs, numel, momentum, (cudaStream_t)stream, lp_format == V2S_LP_FP16);
 }
@@ -1126,13 +1074,7 @@ int v2s_ema_update_lp(float* const* targets, const float* const* onlines, void* 
 int v2s_cast_lp(const float* src, void* dst, int64_t numel, int lp_format, void* stream) {
   if (!src || !dst || numel < 0) { set_error("cast: bad argument"); return 1; }
   if (numel == 0) return 0;
-  return launch_cast_bf16(src, dst, numel, (cudaStream_t)stream, lp_format == V2S_LP_FP16);
-}
-
-int v2s_cast_bf16(const float* src, void* dst, int64_t numel, void* stream) {
-  if (!src || !dst || numel < 0) { set_error("cast: bad argument"); return 1; }
-  if (numel == 0) return 0;
-  return launch_cast_bf16(src, dst, numel, (cudaStream_t)stream);
+  return launch_cast_lp(src, dst, numel, (cudaStream_t)stream, lp_format == V2S_LP_FP16);
 }
 
 int v2s_preprocess_u8_patches(const uint8_t* src, void* patch_rows, int n_images, int lp_format, void* stream) {

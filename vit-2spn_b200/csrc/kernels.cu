@@ -1281,7 +1281,7 @@ int launch_ema(float* const* tgt, const float* const* onl, void* const* tgt_lp, 
   return 0;
 }
 
-int launch_cast_bf16(const float* src, void* dst, int64_t n, cudaStream_t s, int lp_f16) {
+int launch_cast_lp(const float* src, void* dst, int64_t n, cudaStream_t s, int lp_f16) {
   cast_lp_kernel<<<grid_for(n / 4 + 1, 256, 148 * 8), 256, 0, s>>>(src, static_cast<uint16_t*>(dst), n, lp_f16);
   V2S_LAUNCH_CHECK();
   return 0;

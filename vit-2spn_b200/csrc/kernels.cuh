@@ -60,14 +60,14 @@ int launch_infonce_loss(const float* p, const float* z_all, float* loss, float* 
 int launch_cosine_loss(const float* p, const float* z, float* loss, float* dp, int B, int accum,
                        float grad_scale, cudaStream_t s, const float* grad_scale_dev = nullptr);
 int launch_adam(const v2s_range_t* ranges, int n, int64_t step, double lr, double b1, double b2, double eps,
-                double wd, double grad_scale, cudaStream_t s, int lp_f16 = 0);
+                double wd, double grad_scale, cudaStream_t s, int lp_f16);
 // device-resident step state (GradScaler-style skipping, CUDA-graph capturable): see v2s_adam_step_amp
 int launch_adam_amp(const v2s_range_t* ranges, int n, float* state8, double lr, double b1, double b2, double eps, double wd,
                     double grad_multiplier, const float* grad_scale_dev, const float* found_inf_dev, int lp_f16, int advance,
                     cudaStream_t s);
 int launch_ema(float* const* tgt, const float* const* onl, void* const* tgt_lp, int n_pairs,
-               int64_t numel, double momentum, cudaStream_t s, int lp_f16 = 0);
-int launch_cast_bf16(const float* src, void* dst, int64_t n, cudaStream_t s, int lp_f16 = 0);
+               int64_t numel, double momentum, cudaStream_t s, int lp_f16);
+int launch_cast_lp(const float* src, void* dst, int64_t n, cudaStream_t s, int lp_f16);
 int launch_dropout_mask(float* mask, int64_t n, float p, uint64_t seed, uint64_t offset, cudaStream_t s);
 int launch_preprocess_u8(const uint8_t* src, float* dst, int B, cudaStream_t s);
 int launch_preprocess_u8_patches(const uint8_t* src, void* out, int B, int lp_f16, cudaStream_t s);

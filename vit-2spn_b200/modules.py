@@ -281,22 +281,17 @@ def _outputs_array(outputs, n):
 def _run_forward(groups, batch, mode, ws, outputs=None):
     arr = (Group * len(groups))(*groups)
     base, nbytes = _aligned(ws)
-    check(lib.v2s_backbone_forward_ex(arr, _outputs_array(outputs, len(groups)), len(groups), batch, mode,
-                                      C.c_void_p(base), nbytes, stream_ptr()), "backbone_forward")
+    check(lib.v2s_backbone_forward(arr, _outputs_array(outputs, len(groups)), len(groups), batch, mode,
+                                   C.c_void_p(base), nbytes, stream_ptr()), "backbone_forward")
 
 
-def _run_backward(groups, batch, mode, ws, outputs=None):
+def _run_backward(groups, batch, mode, ws, outputs=None, layer_hi=12, layer_lo=0):
+    """Backward over blocks [layer_lo, layer_hi), highest first; the default range is the whole backward."""
     arr = (Group * len(groups))(*groups)
     base, nbytes = _aligned(ws)
-    check(lib.v2s_backbone_backward_ex(arr, _outputs_array(outputs, len(groups)), len(groups), batch, mode,
-                                       C.c_void_p(base), nbytes, 12, 0, stream_ptr()), "backbone_backward")
-
-
-def _run_backward_range(groups, batch, mode, ws, layer_hi, layer_lo):
-    arr = (Group * len(groups))(*groups)
-    base, nbytes = _aligned(ws)
-    check(lib.v2s_backbone_backward_range(arr, len(groups), batch, mode, C.c_void_p(base), nbytes, int(layer_hi),
-                                          int(layer_lo), stream_ptr()), "backbone_backward_range")
+    check(lib.v2s_backbone_backward(arr, _outputs_array(outputs, len(groups)), len(groups), batch, mode,
+                                    C.c_void_p(base), nbytes, int(layer_hi), int(layer_lo), stream_ptr()),
+          "backbone_backward")
 
 
 def _group(store, mode, x, slot, grads=None, hidden=None, feat=None, feat_stride=0, dfeat=None,
@@ -873,7 +868,7 @@ class DualStreamNetwork(nn.Module):
         fmt = st[2].lp_fmt if fmt is None else fmt
         lp = (C.c_void_p * 2)(st[2].lp(refresh=False, fmt=fmt).data_ptr(), st[3].lp(refresh=False, fmt=fmt).data_ptr())
         m = globals().get("momentum", 0.999) if self.momentum is None else self.momentum
-        check(lib.v2s_ema_update_lp(tg, on, lp, 2, n, float(m), fmt, stream_ptr()), "ema_update")
+        check(lib.v2s_ema_update(tg, on, lp, 2, n, float(m), fmt, stream_ptr()), "ema_update")
         st[2].mark_lp_fresh()
         st[3].mark_lp_fresh()
 
@@ -937,16 +932,11 @@ class DualStreamNetwork(nn.Module):
                                                  C.c_void_p(base), nbytes, stream_ptr()), "heads_backward")
             elif self.loss_mode != "cosine":
                 raise ValueError(f"loss_mode {self.loss_mode!r}: 'cosine' (reference) or 'infonce'")
-            elif scale_t is not None:
-                check(lib.v2s_heads_loss_fwd_bwd_amp(ptr(hs.flat), ptr(hg), ptr(feat_o), ptr(feat_t), ptr(mask_o),
-                                                     ptr(mask_t), ptr(dfeat), None, None, ptr(loss), B,
-                                                     int(accumulation_steps), ptr(scale_t), 1 if with_backward else 0,
-                                                     C.c_void_p(base), nbytes, stream_ptr()), "heads_loss_fwd_bwd_amp")
             else:
                 check(lib.v2s_heads_loss_fwd_bwd(ptr(hs.flat), ptr(hg), ptr(feat_o), ptr(feat_t), ptr(mask_o), ptr(mask_t),
                                                  ptr(dfeat), None, None, ptr(loss), B, int(accumulation_steps),
-                                                 float(grad_scale), 1 if with_backward else 0, C.c_void_p(base), nbytes,
-                                                 stream_ptr()), "heads_loss_fwd_bwd")
+                                                 float(grad_scale), ptr(scale_t), 1 if with_backward else 0,
+                                                 C.c_void_p(base), nbytes, stream_ptr()), "heads_loss_fwd_bwd")
             if with_backward:
                 bw = [
                     _group(st[0], mode, x1, 0, grads=st[0].grads(), dfeat=dfeat, dfeat_stride=384),
@@ -958,7 +948,7 @@ class DualStreamNetwork(nn.Module):
                     grad_sync.begin()
                     grad_sync.heads_ready()                      # the head gradients are final before the backbones start
                     for hi, lo in grad_sync.ranges:
-                        _run_backward_range(bw, B, mode, ws, hi, lo)
+                        _run_backward(bw, B, mode, ws, layer_hi=hi, layer_lo=lo)
                         grad_sync.range_ready(hi, lo)
         finally:
             self._release_workspace(ws)
@@ -1054,7 +1044,7 @@ class SingleStreamNetwork(nn.Module):
         tg = (C.c_void_p * 1)(st.flat.data_ptr())
         on = (C.c_void_p * 1)(so.flat.data_ptr())
         lp = (C.c_void_p * 1)(st.lp(refresh=False).data_ptr())
-        check(lib.v2s_ema_update_lp(tg, on, lp, 1, so.numel, float(momentum), st.lp_fmt, stream_ptr()), "ema_update")
+        check(lib.v2s_ema_update(tg, on, lp, 1, so.numel, float(momentum), st.lp_fmt, stream_ptr()), "ema_update")
         st.mark_lp_fresh()
 
 

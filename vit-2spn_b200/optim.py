@@ -253,8 +253,8 @@ class FusedAdam(torch.optim.Optimizer):
                     chunk = rs[i:i + 4]
                     arr = (Range * len(chunk))(*chunk)
                     with torch.cuda.device(dev_of[chunk[0].params]):
-                        check(lib.v2s_adam_step_lp(arr, len(chunk), int(step), float(lr), float(b1), float(b2), float(eps),
-                                                   float(wd), float(self.grad_multiplier), int(fmt), stream_ptr()), "adam_step")
+                        check(lib.v2s_adam_step(arr, len(chunk), int(step), float(lr), float(b1), float(b2), float(eps),
+                                                float(wd), float(self.grad_multiplier), int(fmt), stream_ptr()), "adam_step")
             advanced = set()
             for (sid, fmt), (state8, rs) in dev_launches.items():
                 dev = state8.device
