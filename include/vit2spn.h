@@ -30,7 +30,8 @@ extern "C" {
                              and (backward) the layer range, v2s_heads_loss_fwd_bwd the device loss scale, v2s_adam_step
                              and v2s_ema_update the lp_format; their narrower variants and the bf16-only cast are
                              removed.  3: v2s_infonce_loss, v2s_preprocess_u8_patches, v2s_group.x_format (was a
-                             reserved zero field); additive to 3: v2s_group_outputs, v2s_test_attention which = 2 */
+                             reserved zero field); additive to 3: v2s_group_outputs, v2s_test_attention which = 2.  Additive to 4:
+                             v2s_backbone_input_backward, v2s_test_gemm which = 5 */
 
 /* compute modes */
 #define V2S_MODE_FP32 0 /* fp32 activations + fp32 SIMT GEMMs: the "fp32 check mode" of north_star */
@@ -131,6 +132,14 @@ int v2s_backbone_forward(const v2s_group_t* host_groups, const v2s_group_outputs
 int v2s_backbone_backward(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs /* [n_groups] or NULL */,
                           int n_groups, int batch, int mode, void* workspace, int64_t workspace_bytes, int layer_hi,
                           int layer_lo, void* stream);
+/* d loss / d pixel_values (transformers' input gradient): the backward of v2s_backbone_backward over all blocks that also
+ * writes, for each group with host_dpixels[g] != NULL, the fp32 image gradient [batch,3,224,224] (overwritten, 16-byte
+ * aligned; not for x_format 1 groups).  host_dpixels has n_groups entries.
+ * weight_grads = 1: weight gradients accumulated exactly as v2s_backbone_backward does (same kernels, same bits);
+ * 0: no parameter gradient is computed and grads may be NULL (frozen backbones; no deterministic scratch is used). */
+int v2s_backbone_input_backward(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs,
+                                float* const* host_dpixels, int weight_grads, int n_groups, int batch, int mode,
+                                void* workspace, int64_t workspace_bytes, void* stream);
 
 /* projection_head + prediction_head on the concatenated online features and projection_head on
  * the target features (ref:ssp_vit2spn_tiny.py:153-158), fused with the loss
@@ -252,7 +261,9 @@ int v2s_set_deterministic(int on);
 
 /* test hooks: individual operators, used by tests/ to localise a parity failure */
 /* GEMM, 16-bit operands: which 0 NT (a [m,k], b [n,k] -> c [m,n] 16-bit), 1 NN (b [k,n]), 2 TN (a [k,m], b [k,n],
- * c [m,n] fp32 +=, split-K), 3 NT with fp32 c, 4 = 2 plus the bias row sums of a (+=) in c[m*n .. m*n + m).
+ * c [m,n] fp32 +=, split-K), 3 NT with fp32 c, 4 = 2 plus the bias row sums of a (+=) in c[m*n .. m*n + m),
+ * 5 the image gradient of the patch embedding (a = patch-row gradient [m = batch*196, 192], b = W_pe [192, 768], c = fp32
+ * [batch,3,224,224] written; n = 768, k = 192, tensor-core kernel only).
  * variant bit 0 = SIMT kernel, bit 1 = fp16 instead of bf16.  In deterministic mode (v2s_set_deterministic), which 2 / 4
  * take their scratch from the caller: c continues after its outputs with 1024 + n_sms * (128 * 192 + 128) floats
  * (n_sms = the device's SM count; m a multiple of 8). */

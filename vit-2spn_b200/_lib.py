@@ -68,6 +68,8 @@ _SIGS = {
     "v2s_backbone_forward": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), _i, _i, _i, _vp, _i64, _vp]),
     "v2s_backbone_backward": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), _i, _i, _i, _vp, _i64, _i, _i,
                                         _vp]),
+    "v2s_backbone_input_backward": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), C.POINTER(_vp), _i, _i, _i, _i,
+                                              _vp, _i64, _vp]),
     "v2s_heads_loss_fwd_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _f, _vp, _i,
                                          _vp, _i64, _vp]),
     "v2s_heads_forward": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _vp]),

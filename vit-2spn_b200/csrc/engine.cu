@@ -34,9 +34,9 @@ static int n_recs = 0;
 static int n_events = 0;   // events created so far (recs[i].a/b valid for i < n_events)
 static const char* names[] = {"gemm_patch", "gemm_qkv", "gemm_proj", "gemm_fc1", "gemm_fc2", "gemm_dgrad",
                               "gemm_wgrad", "attn_fwd", "attn_bwd", "ln_fwd", "ln_bwd", "colsum", "misc", "heads", "gemm_mlp_fwd",
-                              "gemm_mlp_bwd", "attn_probs"};
+                              "gemm_mlp_bwd", "attn_probs", "gemm_pixels"};
 enum { C_PATCH, C_QKV, C_PROJ, C_FC1, C_FC2, C_DGRAD, C_WGRAD, C_ATTN_F, C_ATTN_B, C_LN_F, C_LN_B, C_COLSUM, C_MISC,
-       C_HEADS, C_MLP_F, C_MLP_B, C_ATTN_P, C_COUNT };
+       C_HEADS, C_MLP_F, C_MLP_B, C_ATTN_P, C_PIX, C_COUNT };
 struct Scope {
   int idx = -1;
   cudaStream_t st;
@@ -249,13 +249,17 @@ int launch_attention_probs(const void* const* qkv, const float* const* lse, floa
   return launch_attn_probs_simt(qkv, lse, probs, groups, B, at, s);
 }
 
-// d loss / d hidden_states[k] joins the residual-stream gradient (groups whose dh entry is NULL are skipped); for k > 0 its
-// column sums also go to the fc2 bias gradient of block k - 1, whose output hidden_states[k] is
+// d loss / d hidden_states[k] joins the residual-stream gradient (groups whose dh entry is NULL are skipped); for k > 0 and
+// with weight gradients its column sums also go to the fc2 bias gradient of block k - 1, whose output hidden_states[k] is
 int add_hidden_grads(int k, const float* const* dh, float* const* dx, void* const* dxlp, const v2s_group_t* gs, int G, int B,
-                     int at, const Plan& p, cudaStream_t s, const DetScratch* det) {
+                     int at, const Plan& p, cudaStream_t s, const DetScratch* det, int weight_grads) {
   const float* a[MAXG]; float* o[MAXG]; void* lp[MAXG]; float* cs[MAXG]; int n = 0;
   for (int g = 0; g < G; ++g)
-    if (dh[g]) { a[n] = dh[g]; o[n] = dx[g]; lp[n] = dxlp[g]; cs[n] = k > 0 ? gs[g].grads + layer_off(k - 1) + L_B2 : nullptr; ++n; }
+    if (dh[g]) {
+      a[n] = dh[g]; o[n] = dx[g]; lp[n] = dxlp[g];
+      cs[n] = (k > 0 && weight_grads) ? gs[g].grads + layer_off(k - 1) + L_B2 : nullptr;
+      ++n;
+    }
   if (!n) return 0;
   prof::Scope sc(prof::C_MISC, (double)p.M * D * (12 + p.es) * n, s);
   return launch_residual_grad_add(a, o, lp, cs, n, B, at, s, det);
@@ -531,15 +535,28 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
 // layers [layer_lo, layer_hi) in descending order; layer_hi == NL starts from the feature / hidden-state gradient,
 // layer_lo == 0 finishes with the embedding gradients.  Between two calls the residual-stream gradient lives in the
 // workspace, so a full backward may be issued in several ranges (gradient all-reduce overlapped per range).
+// dpix_in (whole backward only; NULL or one entry per input group): the groups with dpix_in[g] != NULL also get the fp32
+// image gradient [B,3,224,224] (overwritten).  weight_grads = 0: no parameter gradient at all -- no weight-gradient GEMM,
+// no bias / LayerNorm-parameter / embedding column sum -- and grads may be NULL.
 static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outputs_t* outs_in, int G_in, int B, int mode,
-                                  void* ws, int64_t ws_bytes, cudaStream_t st, int layer_hi, int layer_lo) {
+                                  void* ws, int64_t ws_bytes, cudaStream_t st, int layer_hi, int layer_lo,
+                                  float* const* dpix_in, int weight_grads) {
   if (layer_lo < 0 || layer_hi > NL || layer_lo >= layer_hi) { set_error("backbone_backward: bad layer range [%d, %d)", layer_lo, layer_hi); return 1; }
   // keep only the groups that saved activations and want gradients
   v2s_group_t gs[MAXG];
   const v2s_group_outputs_t* os[MAXG];
+  float* dpix[MAXG];
   int G = 0;
   for (int i = 0; i < G_in && i < MAXG; ++i)
-    if (gs_in[i].slot >= 0 && gs_in[i].grads) { os[G] = outs_in ? &outs_in[i] : nullptr; gs[G++] = gs_in[i]; }
+    if (gs_in[i].slot >= 0 && (gs_in[i].grads || !weight_grads)) {
+      os[G] = outs_in ? &outs_in[i] : nullptr;
+      dpix[G] = dpix_in ? dpix_in[i] : nullptr;
+      if (dpix[G] && gs_in[i].x_format != 0) {
+        set_error("backbone_input_backward: group %d: no image gradient for 16-bit patch-row inputs (x_format 1)", i);
+        return 1;
+      }
+      gs[G++] = gs_in[i];
+    }
   if (G == 0) { set_error("backbone_backward: no group with slot >= 0 and grads"); return 1; }
   // per group: its saved hidden states (or NULL), d hidden_states[12], and the highest layer its gradient enters at
   // (NL: dfeat / dhidden[12]; k < NL: only intermediate hidden-state gradients, the highest being dhidden[k])
@@ -576,7 +593,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
   // deterministic mode (v2s_set_deterministic): every cross-CTA sum below runs in a fixed order through `det`
   DetScratch det_s;
   const DetScratch* det = nullptr;
-  if (tc_deterministic()) {
+  if (tc_deterministic() && weight_grads) {     // a weight-free backward has no cross-CTA sum
     V2S_TRY(resolve_det(p, ws, ws_bytes, n_saved, &det_s));
     V2S_CUDA_OK(cudaMemsetAsync(det_s.counters, 0, DET_COUNTERS * sizeof(unsigned), st));
     det = &det_s;
@@ -604,6 +621,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
   const bool tc = at != AT_F32;
   auto wgrad = [&](void* const* dy, int n_out, void* const* x, int k_in, int64_t goff, bool remap,
                    int64_t bias_goff = -1) -> int {
+    if (!weight_grads) return 0;
     if (bias_goff >= 0 && !tc) {
       const void* src[MAXG]; float* dst[MAXG];
       for (int g = 0; g < G; ++g) { src[g] = dy[g]; dst[g] = gs[g].grads + bias_goff; }
@@ -638,6 +656,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
   const bool merged = tc && 2 * G <= MAXG;
   auto wgrad2 = [&](void* const* dy1, int n_out1, void* const* x1, int k_in1, int64_t goff1, int64_t bias1,
                     void* const* dy2, int n_out2, void* const* x2, int k_in2, int64_t goff2, int64_t bias2) -> int {
+    if (!weight_grads) return 0;
     GemmDesc d = make_gemm_desc();
     d.M = n_out1; d.N = k_in1; d.K = (int)M; d.groups = 2 * G;
     d.a_rs = 1; d.a_cs = n_out1; d.b_rs = k_in1; d.b_cs = 1;
@@ -653,13 +672,14 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
   };
   // dX[M, K_in] = dY[M, N_out] * W[N_out, K_in]
   // late: the kernel launched just before this one is a wgrad whose inputs this GEMM shares, and nothing the wgrad
-  // touches is written here (GemmDesc::late_wait)
+  // touches is written here (GemmDesc::late_wait).  Without weight gradients the kernel before is the producer of dy:
+  // every launch waits.
   auto dgrad = [&](void* const* dy, int n_out, int64_t woff, int k_in, void* const* out, int epi,
                    void* const* aux, bool late = false) -> int {
     GemmDesc d = make_gemm_desc();
     d.M = (int)M; d.N = k_in; d.K = n_out; d.groups = G;
     d.a_rs = n_out; d.a_cs = 1; d.b_rs = k_in; d.b_cs = 1;
-    d.epi = epi; d.ldc = k_in; d.late_wait = late ? 1 : 0;
+    d.epi = epi; d.ldc = k_in; d.late_wait = (late && weight_grads) ? 1 : 0;
     for (int g = 0; g < G; ++g) {
       d.A[g] = dy[g]; d.B[g] = weight_ptr(gs[g], at, woff); d.out[g] = out[g];
       d.aux[g] = aux ? aux[g] : nullptr;
@@ -667,6 +687,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     return run_gemm(d, at, at, at, st, prof::C_DGRAD);
   };
   auto bias_grad = [&](void* const* dy, int n, int64_t goff) -> int {
+    if (!weight_grads) return 0;
     const void* src[MAXG]; float* dst[MAXG];
     for (int g = 0; g < G; ++g) { src[g] = dy[g]; dst[g] = gs[g].grads + goff; }
     prof::Scope sc(prof::C_COLSUM, (double)M * n * p.es * G, st);
@@ -678,7 +699,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     if (k >= S) return 0;
     const float* a[MAXG];
     for (int g = 0; g < G; ++g) a[g] = os[g] ? os[g]->dhidden[k] : nullptr;
-    return add_hidden_grads(k, a, dx, dxlp, gs, G, B, at, p, st, det);
+    return add_hidden_grads(k, a, dx, dxlp, gs, G, B, at, p, st, det, weight_grads);
   };
   auto x_in = [&](int g, int l) -> const float* { return hid[g] ? hid[g][l] : (const float*)sb(g, p.s_x[l]); };
 
@@ -701,7 +722,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     if (tc) {
       // du = (dx W2) * gelu'(u) and d xn2 = du W1 chained on chip (du is still written once: dW1 needs it)
       MlpDesc d = make_mlp_desc();
-      d.mode = MLP_BWD; d.M = (int)M; d.groups = G; d.lp_f16 = at == AT_F16 ? 1 : 0; d.late_wait = (!merged && l != S - 1) ? 1 : 0;
+      d.mode = MLP_BWD; d.M = (int)M; d.groups = G; d.lp_f16 = at == AT_F16 ? 1 : 0; d.late_wait = (!merged && l != S - 1 && weight_grads) ? 1 : 0;
       for (int g = 0; g < G; ++g) {
         d.a[g] = dxlp[g]; d.w1[g] = weight_ptr(gs[g], at, lo + L_W1); d.w2[g] = weight_ptr(gs[g], at, lo + L_W2);
         d.u[g] = u[g]; d.h[g] = big[g]; d.out[g] = tmp[g];
@@ -726,11 +747,13 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       for (int g = 0; g < G; ++g) {
         dy[g] = tmp[g]; x[g] = (const float*)sb(g, s.x_mid); mu[g] = (const float*)sb(g, s.mean2);
         rs[g] = (const float*)sb(g, s.rstd2); gm[g] = gs[g].params + lo + L_LN2W;
-        dg[g] = gs[g].grads + lo + L_LN2W; db[g] = gs[g].grads + lo + L_LN2B; lp[g] = at ? dxlp[g] : nullptr;
+        lp[g] = at ? dxlp[g] : nullptr;
+        if (!weight_grads) continue;
+        dg[g] = gs[g].grads + lo + L_LN2W; db[g] = gs[g].grads + lo + L_LN2B;
         cs[g] = gs[g].grads + lo + L_BO;          // d b_o = column sums of the gradient w.r.t. x_mid
       }
       { prof::Scope sc(prof::C_LN_B, (double)M * D * (12 + 2 * p.es) * G, st);
-        V2S_TRY(launch_ln_bwd(dy, x, mu, rs, gm, dx, lp, dg, db, cs, G, (int)M, at, st, det)); }
+        V2S_TRY(launch_ln_bwd(dy, x, mu, rs, gm, dx, lp, weight_grads ? dg : nullptr, weight_grads ? db : nullptr, weight_grads ? cs : nullptr, G, (int)M, at, st, det)); }
     }
     // ---- attention ----
     if (!merged) V2S_TRY(wgrad(dxlp, D, ctx, D, lo + L_WO, false));        // dWo (d b_o: fused into LN2-bwd)
@@ -751,34 +774,60 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       for (int g = 0; g < G; ++g) {
         dy[g] = tmp[g]; x[g] = x_in(g, l); mu[g] = (const float*)sb(g, s.mean1);
         rs[g] = (const float*)sb(g, s.rstd1); gm[g] = gs[g].params + lo + L_LN1W;
-        dg[g] = gs[g].grads + lo + L_LN1W; db[g] = gs[g].grads + lo + L_LN1B; lp[g] = at ? dxlp[g] : nullptr;
+        lp[g] = at ? dxlp[g] : nullptr;
+        if (!weight_grads) continue;
+        dg[g] = gs[g].grads + lo + L_LN1W; db[g] = gs[g].grads + lo + L_LN1B;
         // d b_2 of the block below = column sums of the gradient w.r.t. this block's input
         cs[g] = l > 0 ? gs[g].grads + layer_off(l - 1) + L_B2 : nullptr;
       }
       { prof::Scope sc(prof::C_LN_B, (double)M * D * (12 + 2 * p.es) * G, st);
-        V2S_TRY(launch_ln_bwd(dy, x, mu, rs, gm, dx, lp, dg, db, cs, G, (int)M, at, st, det)); }
+        V2S_TRY(launch_ln_bwd(dy, x, mu, rs, gm, dx, lp, weight_grads ? dg : nullptr, weight_grads ? db : nullptr, weight_grads ? cs : nullptr, G, (int)M, at, st, det)); }
     }
   }
-  // ---- embeddings: d pos, d cls, d patch bias, d patch weight ----
+  // ---- embeddings: d pos, d cls, d patch bias, d patch weight; the image gradient ----
   if (layer_lo == 0) {
     V2S_TRY(add_dhidden(0));
     const float* cdx[MAXG]; float* gr[MAXG]; void* pt[MAXG];
+    // the groups that want the image gradient, compacted: dX_patches [B*196, 768] = dE [B*196, 192] W_pe [192, 768]
+    int px[MAXG], npx = 0;
     for (int g = 0; g < G; ++g) {
       cdx[g] = dx[g]; gr[g] = gs[g].grads;
       pt[g] = gs[g].x_format == 1 ? const_cast<void*>(gs[g].x) : static_cast<void*>(sb(g, p.s_patches));
+      if (dpix[g]) px[npx++] = g;
     }
-    V2S_TRY(launch_embed_bwd(cdx, gr, G, B, st, det));
+    if (weight_grads) V2S_TRY(launch_embed_bwd(cdx, gr, G, B, st, det));
+    GemmDesc dp = make_gemm_desc();
+    dp.M = (int)MP; dp.N = KPE; dp.K = D; dp.groups = npx;
+    dp.a_rs = D; dp.a_cs = 1; dp.b_rs = KPE; dp.b_cs = 1; dp.ldc = KPE;
     if (tc) {          // compact the patch rows, then the ordinary tensor-core wgrad
       const void* src[MAXG];
       for (int g = 0; g < G; ++g) src[g] = dxlp[g];
       V2S_TRY(launch_gather_patch_rows(src, tmp, G, B, at, st));
-      GemmDesc d = make_gemm_desc();
-      d.M = D; d.N = KPE; d.K = (int)MP; d.groups = G;
-      d.a_rs = 1; d.a_cs = D; d.b_rs = KPE; d.b_cs = 1; d.epi = EPI_ACCUM; d.ldc = KPE; d.split_k = split; d.det = det;
-      for (int g = 0; g < G; ++g) { d.A[g] = tmp[g]; d.B[g] = pt[g]; d.out[g] = gs[g].grads + OFF_WPE; }
-      V2S_TRY(run_gemm(d, at, at, 0, st, prof::C_WGRAD));
+      if (weight_grads) {
+        GemmDesc d = make_gemm_desc();
+        d.M = D; d.N = KPE; d.K = (int)MP; d.groups = G;
+        d.a_rs = 1; d.a_cs = D; d.b_rs = KPE; d.b_cs = 1; d.epi = EPI_ACCUM; d.ldc = KPE; d.split_k = split; d.det = det;
+        for (int g = 0; g < G; ++g) { d.A[g] = tmp[g]; d.B[g] = pt[g]; d.out[g] = gs[g].grads + OFF_WPE; }
+        V2S_TRY(run_gemm(d, at, at, 0, st, prof::C_WGRAD));
+      }
+      if (npx) {       // the image gradient straight from the epilogue; after the patch wgrad it shares its input rows
+        dp.epi = EPI_PIXELS; dp.late_wait = weight_grads;
+        for (int i = 0; i < npx; ++i) { dp.A[i] = tmp[px[i]]; dp.B[i] = weight_ptr(gs[px[i]], at, OFF_WPE); dp.out[i] = dpix[px[i]]; }
+        V2S_TRY(run_gemm(dp, at, at, 0, st, prof::C_PIX));
+      }
     } else {
       V2S_TRY(wgrad(dxlp, D, pt, KPE, OFF_WPE, true));
+      if (npx) {       // fp32 check mode: the patch rows of the token-row gradient into `big`, then col2im
+        const float* rows[MAXG]; float* img[MAXG];
+        dp.epi = EPI_STORE; dp.a_remap = 1;
+        for (int i = 0; i < npx; ++i) {
+          dp.A[i] = dx[px[i]]; dp.B[i] = gs[px[i]].params + OFF_WPE; dp.out[i] = big[px[i]];
+          rows[i] = static_cast<const float*>(big[px[i]]); img[i] = dpix[px[i]];
+        }
+        V2S_TRY(run_gemm(dp, at, at, 0, st, prof::C_PIX));
+        prof::Scope sc(prof::C_MISC, (double)MP * KPE * 8 * npx, st);
+        V2S_TRY(launch_col2im(rows, img, npx, B, st));
+      }
     }
   }
   return 0;
@@ -980,7 +1029,20 @@ int v2s_backbone_backward(const v2s_group_t* groups, const v2s_group_outputs_t* 
                           int mode, void* workspace, int64_t workspace_bytes, int layer_hi, int layer_lo, void* stream) {
   if (!groups) { set_error("null groups"); return 1; }
   return backbone_backward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
-                                layer_hi, layer_lo);
+                                layer_hi, layer_lo, nullptr, 1);
+}
+
+int v2s_backbone_input_backward(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, float* const* dpixels,
+                                int weight_grads, int n_groups, int batch, int mode, void* workspace, int64_t workspace_bytes,
+                                void* stream) {
+  if (!groups || !dpixels) { set_error("backbone_input_backward: null groups / dpixels"); return 1; }
+  for (int g = 0; g < n_groups && g < MAXG; ++g)
+    if (dpixels[g] && (reinterpret_cast<uintptr_t>(dpixels[g]) & 15)) {
+      set_error("backbone_input_backward: dpixels[%d] is not 16-byte aligned", g);
+      return 1;
+    }
+  return backbone_backward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
+                                NL, 0, dpixels, weight_grads ? 1 : 0);
 }
 
 int v2s_heads_loss_fwd_bwd(const float* head_params, float* head_grads, const float* feat_online,

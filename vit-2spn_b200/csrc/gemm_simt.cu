@@ -177,6 +177,7 @@ int launch_t(const GemmDesc& d, cudaStream_t stream) {
 
 int launch_gemm_simt(const GemmDesc& d, int ta, int tb, int to, cudaStream_t stream) {
   if (d.M <= 0 || d.N <= 0 || d.K <= 0) return 0;
+  if (d.epi == EPI_PIXELS) { set_error("gemm_simt: EPI_PIXELS is a tensor-core epilogue"); return 1; }
   if (d.split_k > 1 && d.epi != EPI_ACCUM && !(d.epi == EPI_STORE && d.split_stride > 0)) {
     set_error("gemm_simt: split_k requires EPI_ACCUM, or EPI_STORE with a split_stride");
     return 1;

@@ -14,6 +14,9 @@ enum GemmEpi : int {
   EPI_ACCUM = 5,        // atomicAdd(out(fp32), alpha*acc)  (wgrad, split-K)
   EPI_BIAS_RELU_MASK = 6,  // a = relu(acc+bias) -> out ; a*mask -> out2
   EPI_DRELU_MASK = 7,      // out = acc * (aux > 0) * mask
+  // tensor-core path only (the SIMT kernel refuses it): acc [B*196, 768] of the patch-embedding dgrad is stored fp32
+  // straight into the NCHW image gradient out [B,3,224,224]: row (b, py, px), column c*256 + ky*16 + kx
+  EPI_PIXELS = 8,
 };
 
 struct GemmDesc {

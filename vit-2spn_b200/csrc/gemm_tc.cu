@@ -49,15 +49,16 @@ enum TcEpi : int {
   T_RESID = 1,   // out(fp32) = acc + bias + aux(fp32)
   T_ACCUM = 4,   // global(fp32) += acc          (TMA reduce-add; split-K)
   T_ACCUM_DET = 5,   // deterministic T_ACCUM: partial tiles to a slab, summed in split order by the last CTA to arrive
+  T_PIXELS = 6,  // fp32 image gradient (EPI_PIXELS): the epilogue threads store their rows straight to global memory
 };
 
 // per-variant epilogue staging: a ring of NSTG buffers of STG bytes per epilogue group.  The residual variant
 // (auxiliary operand prefetched two chunks ahead into the ring) and the plain bf16 store use 3 buffers;
-// bf16 chunks are 8 KB (SWIZZLE_64B), fp32 chunks 16 KB.
+// bf16 chunks are 8 KB (SWIZZLE_64B), fp32 chunks 16 KB.  T_PIXELS stages nothing.
 template <int EPI, bool OUT_BF16> struct Cfg {
   static constexpr int NSTG = (EPI == T_ACCUM || EPI == T_ACCUM_DET || (EPI == T_STORE && !OUT_BF16)) ? 2 : 3;
   static constexpr int STG = OUT_BF16 ? 8192 : 16384;
-  static constexpr int STAGING_BYTES = 2 * NSTG * STG;
+  static constexpr int STAGING_BYTES = EPI == T_PIXELS ? 0 : 2 * NSTG * STG;
 };
 
 struct alignas(64) TcParams {
@@ -89,6 +90,7 @@ struct alignas(64) TcParams {
   float* det_slab;
   float* det_rowpart;
   unsigned* det_counters;
+  float* pixels[MAXG];   // T_PIXELS: the fp32 image gradients [M / 196, 3, 224, 224] (no tensor map)
 };
 
 
@@ -123,7 +125,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
     for (int g = 0; g < p.groups; ++g) {
       ptx::prefetch_tmap(&p.tmA[g]);
       ptx::prefetch_tmap(&p.tmB[g]);
-      ptx::prefetch_tmap(&p.tmOut[g]);
+      if constexpr (EPI != T_PIXELS) ptx::prefetch_tmap(&p.tmOut[g]);
     }
   }
   if (warp == 1 && lane == 0) {
@@ -309,7 +311,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
     }
     if (DBG && blockIdx.x == 0 && lane == 0) { p.dbg[2] = w_full; p.dbg[3] = w_tempty; p.dbg[4] = clock64() - mma_t0; p.dbg[5] = ntiles; }
-  } else if (warp == 2 || warp == 3) {
+  } else if (EPI != T_PIXELS && (warp == 2 || warp == 3)) {
     // ================= store warp of epilogue group ge (whole warp walks the loop; one elected lane issues) ====
     const int ge = warp - 2;
     uint8_t* stg_base = smem + p.stg_off + ge * N_STG * STG_BYTES;
@@ -380,7 +382,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
     }
     if (ptx::elect_one()) ptx::tma_wait_group<0>();
     __syncwarp();
-  } else if (warp >= 4) {
+  } else if (EPI != T_PIXELS && warp >= 4) {
     // ================= epilogue =================
     // 16 warps = 2 groups of 8.  Group ge drains accumulator stage ge.  Inside a group, warps w and w+4 share
     // TMEM lane quarter w%4 and split every 32-column chunk into two 16-column halves (thread = one row x 16 cols).
@@ -579,6 +581,43 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
     if (DBG && blockIdx.x == 0 && (threadIdx.x == 128 || threadIdx.x == 384 + 37)) {
       long long* d = p.dbg + 8 + (threadIdx.x == 128 ? 0 : 8);
       d[0] = e_tfull; d[1] = e_aux; d[2] = e_pub; d[3] = e_ld; d[4] = clock64() - epi_t0; d[5] = cnt;
+    }
+  } else if (warp >= 4) {
+    // ================= image-gradient epilogue (EPI_PIXELS) =================
+    // The TMEM drain of the epilogue above (group ge = accumulator stage, warps w and w+4 = lane quarter w%4 and the two
+    // 16-column halves of each chunk) without staging: row m = (b, py, px), columns [colh, colh + 16) = (c, ky, kx 0..15)
+    // are 64 contiguous bytes of image row py*16 + ky, stored straight from registers.  The 32 lanes of a warp are
+    // consecutive rows, i.e. mostly consecutive px, so the warp's four 16-byte stores fill one 2 KB run of 64-byte
+    // segments (the stride-16 patch convolution's col2im is a pure permutation).
+    const int ge = (warp - 4) >> 3, q = warp & 3, hf = ((warp - 4) >> 2) & 1, row = q * 32 + lane;
+    uint32_t acc_phase = 0;
+    int g, m_tile, split, n_tile;
+    for (int i = ge; tile_at(i, g, m_tile, split, n_tile); i += 2) {
+      const int m = m_tile * BM + row;
+      const int b = m / NP, t = m - b * NP, py = t / 14, px = t - py * 14;
+      float* img = p.pixels[g] + (int64_t)b * 3 * V2S_IMG * V2S_IMG + py * 16 * V2S_IMG + px * 16;
+      ptx::mbar_wait(&tfull_bar[ge], acc_phase, p.err_flag, 4);
+      acc_phase ^= 1;
+      ptx::tc_fence_after();
+      const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16) + ge * ACC_STRIDE;
+#pragma unroll 1
+      for (int c = 0; c < N_CHUNKS; ++c) {
+        const int colh = n_tile * BN + c * CHUNK + hf * 16;
+        uint32_t r[16];
+        ptx::tmem_ld_32x16(tlane + c * CHUNK + hf * 16, r);
+        ptx::tmem_ld_wait();
+        if (c == N_CHUNKS - 1) {                    // accumulator fully read: hand the stage back to the MMA warp
+          ptx::tc_fence_before();
+          if (lane == 0) ptx::mbar_arrive(&tempty_bar[ge]);
+        }
+        if (m < p.M) {
+          float4* dst = reinterpret_cast<float4*>(img + (colh >> 8) * V2S_IMG * V2S_IMG + ((colh >> 4) & 15) * V2S_IMG);
+#pragma unroll
+          for (int j = 0; j < 4; ++j)
+            dst[j] = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]),
+                                 __uint_as_float(r[4 * j + 3]));
+        }
+      }
     }
   }
 
@@ -840,10 +879,15 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
     case EPI_STORE: epi = T_STORE; break;
     case EPI_BIAS_RESID: epi = T_RESID; break;
     case EPI_ACCUM: epi = T_ACCUM; break;
+    case EPI_PIXELS: epi = T_PIXELS; break;
     default: return 0;
   }
   if (d.alpha != 1.0f) return 0;
   const bool out_bf16 = (to != 0);                        // 16-bit output (bf16 or fp16, as the operands)
+  if (epi == T_PIXELS && (out_bf16 || d.M % NP || d.N != KPE || d.ldc != KPE || d.a_remap || d.b_remap)) {
+    set_error("gemm_tc: the image-gradient epilogue needs [B*196, 768] fp32 output (M %d N %d)", d.M, d.N);
+    return 1;
+  }
   if ((epi == T_RESID || epi == T_ACCUM) && out_bf16) return 0;
   int a_mn, b_mn;
   int64_t a_ld, b_ld;
@@ -910,6 +954,11 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
     else V2S_TRY(get_map(&p.tmA[g], d.A[g], d.M, d.K, a_ld, 64, BK, true, CU_TENSOR_MAP_SWIZZLE_128B));
     if (!b_mn) V2S_TRY(get_map(&p.tmB[g], d.B[g], d.K, d.N, b_ld, BK, BN, true, CU_TENSOR_MAP_SWIZZLE_128B));
     else V2S_TRY(get_map(&p.tmB[g], d.B[g], d.N, d.K, b_ld, 64, BK, true, CU_TENSOR_MAP_SWIZZLE_128B));
+    if (epi == T_PIXELS) {
+      if (reinterpret_cast<uintptr_t>(d.out[g]) & 15) { set_error("gemm_tc: image gradient not 16-byte aligned"); return 1; }
+      p.pixels[g] = static_cast<float*>(d.out[g]);
+      continue;
+    }
     V2S_TRY(get_map(&p.tmOut[g], d.out[g], d.N, d.M, d.ldc, CHUNK, BM, out_bf16, out_swz));
     if (epi == T_RESID) V2S_TRY(get_map(&p.tmAux[g], d.resid[g], d.N, d.M, d.ldc, CHUNK, BM, false, CU_TENSOR_MAP_SWIZZLE_128B));
     p.bias[g] = (epi == T_ACCUM) ? nullptr : d.bias[g];
@@ -944,6 +993,7 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
     case T_STORE: rc = out_bf16 ? launch_kernel<T_STORE, true>(p, lp_f16, stream) : launch_kernel<T_STORE, false>(p, lp_f16, stream); break;
     case T_RESID: rc = launch_kernel<T_RESID, false>(p, lp_f16, stream); break;
     case T_ACCUM_DET: rc = launch_kernel<T_ACCUM_DET, false>(p, lp_f16, stream); break;
+    case T_PIXELS: rc = launch_kernel<T_PIXELS, false>(p, lp_f16, stream); break;
     default: rc = launch_kernel<T_ACCUM, false>(p, lp_f16, stream); break;
   }
   if (rc) return rc;
@@ -952,8 +1002,9 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
 }
 
 // test hook (v2s_test_gemm): which = 0 NT (A[M,K], B[N,K]), 1 NN/dgrad (A[M,K], B[K,N]),
-// 2 TN/wgrad (A[K,M], B[K,N], out fp32 +=), 3 NT with fp32 out, 4 = 2 plus the bias row sums (+=) at c + M*N;
-// variant: 0 = tensor-core path, 1 = SIMT reference.  bf16 operands; out bf16 for which 0/1, fp32 accumulate-into for
+// 2 TN/wgrad (A[K,M], B[K,N], out fp32 +=), 3 NT with fp32 out, 4 = 2 plus the bias row sums (+=) at c + M*N,
+// 5 the image gradient (A = patch-row gradient [M = B*196, 192], B = W_pe [192, 768], c fp32 [B,3,224,224] written;
+// tensor-core path only); variant: 0 = tensor-core path, 1 = SIMT reference.  bf16 operands; out bf16 for which 0/1, fp32 accumulate-into for
 // which 2/4.  Deterministic mode, which 2/4: the caller's c buffer continues with the scratch a backward call takes
 // from its workspace (DetScratch: DET_COUNTERS counters, then gemm_tc_det_part_floats() floats)
 int gemm_tc_test(int which, const void* a, const void* b, void* c, int m, int n, int k, int variant,
@@ -969,7 +1020,11 @@ int gemm_tc_test(int which, const void* a, const void* b, void* c, int m, int n,
     d.a_rs = 1; d.a_cs = m; d.b_rs = n; d.b_cs = 1; d.epi = EPI_ACCUM; to = 0; d.split_k = 1;
     d.rowsum_out[0] = static_cast<float*>(c) + (int64_t)m * n;
   }
-  else { set_error("gemm_tc_test: which must be 0..4"); return 1; }
+  else if (which == 5) {
+    if (n != KPE || k != D || (variant & 1)) { set_error("gemm_tc_test: which 5 is n = 768, k = 192, tensor-core path"); return 1; }
+    d.a_rs = k; d.a_cs = 1; d.b_rs = n; d.b_cs = 1; d.epi = EPI_PIXELS; to = 0;
+  }
+  else { set_error("gemm_tc_test: which must be 0..5"); return 1; }
   // variant: bit 0 = SIMT reference instead of the tensor-core path, bit 1 = fp16 instead of bf16 tensors
   const int t16 = (variant & 2) ? AT_F16 : AT_BF16;
   if (to) to = t16;

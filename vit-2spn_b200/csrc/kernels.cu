@@ -76,6 +76,23 @@ __global__ void __launch_bounds__(256) gather_patch_rows_kernel(G4<const T*> src
     reinterpret_cast<uint2*>(d)[i] = reinterpret_cast<const uint2*>(s)[i];
 }
 
+// the inverse permutation of im2col (stride = kernel, no overlap-add): patch rows [B*196, 768] fp32 -> NCHW fp32
+// [B,3,224,224]; one float4 of the image per thread, so the stores are contiguous (fp32 check mode's image gradient)
+__global__ void __launch_bounds__(256) col2im_kernel(G4<const float*> rows, G4<float*> img, int B) {
+  const int g = blockIdx.y;
+  const float* __restrict__ src = rows.p[g];
+  float* __restrict__ dst = img.p[g];
+  const int64_t total = (int64_t)B * 3 * V2S_IMG * (V2S_IMG / 4);
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int x4 = i % (V2S_IMG / 4), y = (i / (V2S_IMG / 4)) % V2S_IMG;
+    const int c = (i / (V2S_IMG * V2S_IMG / 4)) % 3;
+    const int64_t b = i / (3 * V2S_IMG * V2S_IMG / 4);
+    const int px = x4 / 4, py = y / 16;
+    reinterpret_cast<float4*>(dst)[i] = *reinterpret_cast<const float4*>(
+        src + (b * NP + py * 14 + px) * KPE + c * 256 + (y % 16) * 16 + (x4 % 4) * 4);
+  }
+}
+
 // ------------------------------------------------------------------------------------------
 // LayerNorm over D=192 (eps 1e-12).  Half a warp per row: 16 lanes x 3 float4 = 192 floats, so a
 // warp keeps two rows (6 x 128-bit loads per lane) in flight; reductions are 4 shuffle steps.
@@ -223,8 +240,9 @@ __device__ __forceinline__ void det_reduce_rows(const float* part, int n, int nb
 }
 
 // dres (fp32, in/out) += LN-backward(dy);  dres_lp = updated dres in the activation type;
-// dgamma / dbeta / (optional) dcolsum[n] += sum over rows of the UPDATED dres (= bias gradient of the
-// linear layer that consumes this residual-stream gradient).
+// PARAMS: dgamma / dbeta / (optional) dcolsum[n] += sum over rows of the UPDATED dres (= bias gradient of the
+// linear layer that consumes this residual-stream gradient).  !PARAMS (input-gradient backward of a frozen backbone): the
+// row-wise part only, no column sums.
 struct LnBwdP {
   const void* dy[MAXG]; const float* x[MAXG]; const float* mean[MAXG]; const float* rstd[MAXG];
   const float* gamma[MAXG]; float* dres[MAXG]; void* dres_lp[MAXG]; float* dgamma[MAXG]; float* dbeta[MAXG];
@@ -234,7 +252,7 @@ struct LnBwdP {
   unsigned* det_counters;      // DET: one per group
 };
 
-template <typename T, bool DET>
+template <typename T, bool DET, bool PARAMS>
 __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnBwdP p) {
   __shared__ __align__(16) float red[16][3 * D];          // 36 KB; float4 accesses
   // wait for the predecessor, THEN release the successor: a successor flagged "late wait" (gemm_tc.cu) relies on
@@ -268,8 +286,10 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnB
       gd[i] = make_float4(d[i].x * gm[i].x, d[i].y * gm[i].y, d[i].z * gm[i].z, d[i].w * gm[i].w);
       c1 += (gd[i].x + gd[i].y) + (gd[i].z + gd[i].w);
       c2 += (gd[i].x * xh[i].x + gd[i].y * xh[i].y) + (gd[i].z * xh[i].z + gd[i].w * xh[i].w);
-      ag[i].x += d[i].x * xh[i].x; ag[i].y += d[i].y * xh[i].y; ag[i].z += d[i].z * xh[i].z; ag[i].w += d[i].w * xh[i].w;
-      ab[i].x += d[i].x; ab[i].y += d[i].y; ab[i].z += d[i].z; ab[i].w += d[i].w;
+      if constexpr (PARAMS) {
+        ag[i].x += d[i].x * xh[i].x; ag[i].y += d[i].y * xh[i].y; ag[i].z += d[i].z * xh[i].z; ag[i].w += d[i].w * xh[i].w;
+        ab[i].x += d[i].x; ab[i].y += d[i].y; ab[i].z += d[i].z; ab[i].w += d[i].w;
+      }
     }
     c1 = hw_sum(c1, hmask) * (1.0f / D);
     c2 = hw_sum(c2, hmask) * (1.0f / D);
@@ -279,9 +299,10 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnB
       o[i].z += rs * (gd[i].z - c1 - xh[i].z * c2); o[i].w += rs * (gd[i].w - c1 - xh[i].w * c2);
       reinterpret_cast<float4*>(dres + (int64_t)row * D)[l + 16 * i] = o[i];
       if (dlp) store4<T>(dlp + (int64_t)row * D + 4 * (l + 16 * i), o[i].x, o[i].y, o[i].z, o[i].w);
-      ac[i].x += o[i].x; ac[i].y += o[i].y; ac[i].z += o[i].z; ac[i].w += o[i].w;
+      if constexpr (PARAMS) { ac[i].x += o[i].x; ac[i].y += o[i].y; ac[i].z += o[i].z; ac[i].w += o[i].w; }
     }
   }
+  if constexpr (!PARAMS) return;
 #pragma unroll
   for (int i = 0; i < 3; ++i) {
     const int c = 4 * (l + 16 * i);
@@ -1024,6 +1045,13 @@ int launch_gather_patch_rows(const void* const* src, void* const* dst, int group
   return 0;
 }
 
+int launch_col2im(const float* const* rows, float* const* img, int groups, int B, cudaStream_t s) {
+  dim3 grid(grid_for((int64_t)B * 3 * V2S_IMG * (V2S_IMG / 4), 256, 148 * 16), groups);
+  col2im_kernel<<<grid, 256, 0, s>>>(pack4<const float*>(rows, groups), pack4<float*>(img, groups), B);
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
 int launch_ln_fwd(const float* const* x, const float* const* gamma, const float* const* beta, void* const* y,
                   float* const* mean, float* const* rstd, int groups, int M, int at, cudaStream_t s) {
   LnFwdP p;
@@ -1049,20 +1077,22 @@ int launch_ln_bwd(const void* const* dy, const float* const* x, const float* con
   memset(&p, 0, sizeof(p));
   for (int g = 0; g < groups; ++g) {
     p.dy[g] = dy[g]; p.x[g] = x[g]; p.mean[g] = mean[g]; p.rstd[g] = rstd[g]; p.gamma[g] = gamma[g];
-    p.dres[g] = dres[g]; p.dres_lp[g] = dres_lp ? dres_lp[g] : nullptr; p.dgamma[g] = dgamma[g]; p.dbeta[g] = dbeta[g];
+    p.dres[g] = dres[g]; p.dres_lp[g] = dres_lp ? dres_lp[g] : nullptr;
+    p.dgamma[g] = dgamma ? dgamma[g] : nullptr; p.dbeta[g] = dbeta ? dbeta[g] : nullptr;
     p.dcolsum[g] = dcolsum ? dcolsum[g] : nullptr;
   }
   p.M = M;
   int bx = (M + 15) / 16;
   if (bx > 148 * 4) bx = 148 * 4;
-  if (det) {         // a fixed number of row ranges bounds the partial rows the last CTA sums
+  if (det && dgamma) {         // a fixed number of row ranges bounds the partial rows the last CTA sums
     if (bx > 148) bx = 148;
     if ((int64_t)groups * bx * 3 * D > det->part_floats) { set_error("ln_bwd: deterministic scratch too small"); return 1; }
     p.det_part = det->part; p.det_counters = det->counters;
   }
   dim3 grid(bx, groups);
-  if (det) { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<T, true>, grid, dim3(256), 0, s, p))); }
-  else { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<T, false>, grid, dim3(256), 0, s, p))); }
+  if (!dgamma) { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<T, false, false>, grid, dim3(256), 0, s, p))); }
+  else if (det) { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<T, true, true>, grid, dim3(256), 0, s, p))); }
+  else { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<T, false, true>, grid, dim3(256), 0, s, p))); }
   V2S_LAUNCH_CHECK();
   return 0;
 }

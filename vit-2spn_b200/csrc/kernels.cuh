@@ -11,11 +11,14 @@ int launch_cls_rows(const float* const* params, float* const* hidden, int groups
 int launch_assemble_tokens(const float* const* params, const float* const* tok, float* const* hidden, int groups,
                            int B, cudaStream_t s);
 int launch_gather_patch_rows(const void* const* src, void* const* dst, int groups, int B, int at, cudaStream_t s);
+// inverse of launch_im2col for fp32: patch rows [B*196, 768] -> NCHW [B,3,224,224] (overwritten)
+int launch_col2im(const float* const* rows, float* const* img, int groups, int B, cudaStream_t s);
 int launch_ln_fwd(const float* const* x, const float* const* gamma, const float* const* beta,
                   void* const* y, float* const* mean, float* const* rstd, int groups, int M, int at,
                   cudaStream_t s);
 // dres (fp32, in/out) += LN-backward(dy); dres_lp (optional, activation type) = updated dres;
-// dcolsum (optional) += column sums of the updated dres (bias gradient of the next linear layer)
+// dcolsum (optional) += column sums of the updated dres (bias gradient of the next linear layer);
+// dgamma == NULL: no parameter gradient at all (dbeta, dcolsum and det ignored)
 int launch_ln_bwd(const void* const* dy, const float* const* x, const float* const* mean,
                   const float* const* rstd, const float* const* gamma, float* const* dres,
                   void* const* dres_lp, float* const* dgamma, float* const* dbeta, float* const* dcolsum,

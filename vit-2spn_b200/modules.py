@@ -248,6 +248,9 @@ def _new_workspace(device, batch, mode, n_groups, n_saved):
 def _check_images(x, allow_patches=False):
     if allow_patches and x.dim() == 3 and tuple(x.shape[1:]) == (196, 768) and x.dtype in (torch.bfloat16, torch.float16):
         _require_cuda(x, "patch rows")          # the 16-bit patch matrix of preprocess_u8_patches (v2s_group.x_format 1)
+        if x.requires_grad and torch.is_grad_enabled():
+            raise ValueError("vit2spn: no gradient w.r.t. 16-bit patch rows; pass fp32 pixel_values [B,3,224,224] to get "
+                             "d loss / d pixel_values")
         return x.contiguous()
     if x.dim() != 4 or tuple(x.shape[1:]) != (3, 224, 224):
         raise ValueError(f"expected pixel_values of shape [B,3,224,224], got {tuple(x.shape)}")
@@ -292,6 +295,16 @@ def _run_backward(groups, batch, mode, ws, outputs=None, layer_hi=12, layer_lo=0
     check(lib.v2s_backbone_backward(arr, _outputs_array(outputs, len(groups)), len(groups), batch, mode,
                                     C.c_void_p(base), nbytes, int(layer_hi), int(layer_lo), stream_ptr()),
           "backbone_backward")
+
+
+def _run_input_backward(groups, batch, mode, ws, dpixels, weight_grads, outputs=None):
+    """The whole backward, plus the fp32 image gradient of each group whose ``dpixels`` entry is a tensor (None: none);
+    weight_grads False computes no parameter gradient at all (the groups' grads may be None)."""
+    arr = (Group * len(groups))(*groups)
+    dp = (C.c_void_p * len(groups))(*[t.data_ptr() if t is not None else None for t in dpixels])
+    base, nbytes = _aligned(ws)
+    check(lib.v2s_backbone_input_backward(arr, _outputs_array(outputs, len(groups)), dp, int(bool(weight_grads)), len(groups),
+                                          batch, mode, C.c_void_p(base), nbytes, stream_ptr()), "backbone_input_backward")
 
 
 def _group(store, mode, x, slot, grads=None, hidden=None, feat=None, feat_stride=0, dfeat=None,
@@ -410,7 +423,9 @@ class _BackboneFn(torch.autograd.Function):
     """x -> (hidden_states[-1] | mean-pooled features) for one backbone, autograd-compatible.  With want_hidden /
     want_attn the outputs are (hidden_states[12], hidden_states[0..11] if want_hidden, attentions[0..11] if
     want_attn): the residual stream is written straight into the 13 hidden-state tensors, the probabilities by one extra
-    kernel per block.  Gradients w.r.t. any hidden state flow back; the attention probabilities are not differentiable."""
+    kernel per block.  Gradients w.r.t. any hidden state flow back, to the parameters that require them and, when x requires
+    grad, to the pixels (v2s_backbone_input_backward; a frozen backbone then computes no weight gradient at all); the
+    attention probabilities are not differentiable."""
 
     @staticmethod
     @_with_device_of(lambda ctx, x, *a, **k: x)
@@ -469,7 +484,8 @@ class _BackboneFn(torch.autograd.Function):
         if dout is None and all(t is None for t in dhid):
             return nones
         _deterministic()
-        grads = store.grads()
+        want_x, want_w = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        grads = store.grads() if want_w else None
         dout = _grad_f32(dout) if dout is not None else None
         outs = None
         keep = []
@@ -488,9 +504,14 @@ class _BackboneFn(torch.autograd.Function):
             g = _group(store, ctx.mode, ctx.x, 0, grads=grads,
                        dfeat=dout if ctx.pooled else None, dfeat_stride=192,
                        dhidden=None if ctx.pooled else dout)
-        _run_backward([g], ctx.B, ctx.mode, ctx.ws, outs)
+        if not want_x:
+            _run_backward([g], ctx.B, ctx.mode, ctx.ws, outs)
+            ctx.ws = None
+            return nones
+        dx = torch.empty(ctx.B, 3, 224, 224, dtype=torch.float32, device=ctx.x.device)
+        _run_input_backward([g], ctx.B, ctx.mode, ctx.ws, [dx], want_w, outs)
         ctx.ws = None
-        return nones
+        return (dx,) + nones[1:]
 
 
 _warned_random_init = False
@@ -639,7 +660,7 @@ class ViTModel(nn.Module):
         """Mean over the 197 tokens of ``hidden_states[-1]`` (fused pooling)."""
         x = _check_images(pixel_values)
         a = self.embeddings.cls_token
-        return _BackboneFn.apply(x, a, self, True, a.requires_grad and torch.is_grad_enabled())
+        return _BackboneFn.apply(x, a, self, True, torch.is_grad_enabled() and (a.requires_grad or x.requires_grad))
 
     def forward(self, pixel_values, output_hidden_states=None, output_attentions=None, **kw):
         """As ``transformers.ViTModel``: each flag comes from the keyword, else from the config.  The hidden states
@@ -649,7 +670,7 @@ class ViTModel(nn.Module):
         a = self.embeddings.cls_token
         want_hidden = bool(self.config.output_hidden_states if output_hidden_states is None else output_hidden_states)
         want_attn = bool(getattr(self.config, "output_attentions", False) if output_attentions is None else output_attentions)
-        need_grad = a.requires_grad and torch.is_grad_enabled()
+        need_grad = torch.is_grad_enabled() and (a.requires_grad or x.requires_grad)
         if not (want_hidden or want_attn):
             return ViTModelOutput(self, _BackboneFn.apply(x, a, self, False, need_grad))
         res = _BackboneFn.apply(x, a, self, False, need_grad, want_hidden, want_attn)
@@ -719,20 +740,29 @@ class _DualStreamFn(torch.autograd.Function):
         x1, x2, feat_o, mask_o = ctx.keep
         st, hs = model._stores(), model._head_store
         B, mode, ws = ctx.B, ctx.mode, ctx.ws
+        want_x1, want_x2, want_w = ctx.needs_input_grad[:3]
         dpred = dpred.contiguous().to(torch.float32)
         dfeat = torch.empty(B, 384, dtype=torch.float32, device=dpred.device)
         _deterministic()
         base, nbytes = _aligned(ws)
-        check(lib.v2s_heads_backward(ptr(hs.flat), ptr(hs.grads()), ptr(feat_o), ptr(mask_o), ptr(dpred), ptr(dfeat),
+        # a frozen model (pixel gradients only) still runs the heads' backward for dfeat: its head gradients go to scratch
+        hg = hs.grads() if want_w else torch.zeros(hs.numel, dtype=torch.float32, device=dpred.device)
+        check(lib.v2s_heads_backward(ptr(hs.flat), ptr(hg), ptr(feat_o), ptr(mask_o), ptr(dpred), ptr(dfeat),
                                      B, C.c_void_p(base), nbytes, stream_ptr()), "heads_backward")
         groups = [
-            _group(st[0], mode, x1, 0, grads=st[0].grads(), dfeat=dfeat, dfeat_stride=384),
-            _group(st[1], mode, x2, 1, grads=st[1].grads(), dfeat=dfeat[:, 192:], dfeat_stride=384),
+            _group(st[0], mode, x1, 0, grads=st[0].grads() if want_w else None, dfeat=dfeat, dfeat_stride=384),
+            _group(st[1], mode, x2, 1, grads=st[1].grads() if want_w else None, dfeat=dfeat[:, 192:], dfeat_stride=384),
         ]
-        _run_backward(groups, B, mode, ws)
+        if not (want_x1 or want_x2):
+            _run_backward(groups, B, mode, ws)
+            dx1 = dx2 = None
+        else:
+            dx1 = torch.empty(B, 3, 224, 224, dtype=torch.float32, device=dpred.device) if want_x1 else None
+            dx2 = torch.empty(B, 3, 224, 224, dtype=torch.float32, device=dpred.device) if want_x2 else None
+            _run_input_backward(groups, B, mode, ws, [dx1, dx2], want_w)
         model._release_workspace(ws)
         ctx.ws = None
-        return None, None, None, None, None
+        return dx1, dx2, None, None, None
 
 
 def gather_keys(target_proj, group=None):
@@ -852,7 +882,8 @@ class DualStreamNetwork(nn.Module):
         if x1.shape != x2.shape:
             raise ValueError("x1 and x2 must have the same shape")
         anchor = self.online_network_1.vit.embeddings.cls_token
-        return _DualStreamFn.apply(x1, x2, anchor, self, anchor.requires_grad and torch.is_grad_enabled())
+        need_grad = torch.is_grad_enabled() and (anchor.requires_grad or x1.requires_grad or x2.requires_grad)
+        return _DualStreamFn.apply(x1, x2, anchor, self, need_grad)
 
     @_with_device_of(lambda self: self.online_network_1.vit._store.flat)
     def update_target_network(self):
