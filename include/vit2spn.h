@@ -31,7 +31,8 @@ extern "C" {
                              and v2s_ema_update the lp_format; their narrower variants and the bf16-only cast are
                              removed.  3: v2s_infonce_loss, v2s_preprocess_u8_patches, v2s_group.x_format (was a
                              reserved zero field); additive to 3: v2s_group_outputs, v2s_test_attention which = 2.  Additive to 4:
-                             v2s_backbone_input_backward, v2s_test_gemm which = 5 */
+                             v2s_backbone_input_backward, v2s_test_gemm which = 5; v2s_backbone_backward_attn_grads,
+                             v2s_test_attention which = 3 */
 
 /* compute modes */
 #define V2S_MODE_FP32 0 /* fp32 activations + fp32 SIMT GEMMs: the "fp32 check mode" of north_star */
@@ -140,6 +141,13 @@ int v2s_backbone_backward(const v2s_group_t* host_groups, const v2s_group_output
 int v2s_backbone_input_backward(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs,
                                 float* const* host_dpixels, int weight_grads, int n_groups, int batch, int mode,
                                 void* workspace, int64_t workspace_bytes, void* stream);
+/* v2s_backbone_input_backward, plus: for every group g and block l with host_dattn[g*12+l] != NULL, the gradient of the
+ * loss w.r.t. that block's attention probabilities, fp32 [batch,3,197,197] (overwritten, 4-byte aligned): d ctx V^T,
+ * what retain_grad() gives on transformers' attentions.  Blocks at or above the highest layer the loss reaches (see
+ * v2s_group_outputs.dhidden) get nothing written.  host_dattn has n_groups*12 entries; host_dpixels may be NULL. */
+int v2s_backbone_backward_attn_grads(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs,
+                                     float* const* host_dattn, float* const* host_dpixels, int weight_grads, int n_groups,
+                                     int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* projection_head + prediction_head on the concatenated online features and projection_head on
  * the target features (ref:ssp_vit2spn_tiny.py:153-158), fused with the loss
@@ -276,7 +284,8 @@ int v2s_test_mlp(int mode, const void* a, const void* w1, const void* w2, const 
                  void* h, const float* resid, void* out, void* ln_out, const float* ln_gamma, const float* ln_beta,
                  float* ln_mean, float* ln_rstd, int m, int lp_f16, void* stream);
 /* which 0: forward (qkv -> ctx, lse); 1: backward (qkv, ctx, lse, dctx -> dqkv); 2: attention probabilities
- * (qkv, lse -> fp32 [batch,3,197,197] written to ctx).  variant bit 0 = SIMT kernels, bit 1 = fp16 instead of bf16 */
+ * (qkv, lse -> fp32 [batch,3,197,197] written to ctx); 3: their gradient dctx V^T (qkv, dctx -> fp32 [batch,3,197,197]
+ * written to ctx).  variant bit 0 = SIMT kernels, bit 1 = fp16 instead of bf16 */
 int v2s_test_attention(int which, const void* qkv, void* ctx, float* lse, const void* dctx, void* dqkv,
                        int batch, int variant, void* stream);
 /* reads and clears the device-side pipeline-protocol error flag of the tcgen05 kernels (0 = ok) */

@@ -8,6 +8,6 @@ from ._lib import LIB_PATH, EXPORTED, MODE_BF16, MODE_FP32  # noqa: F401  (raise
 from .modules import (DualStreamNetwork, FineTunedModel, InfoNCELoss, SingleStreamNetwork, ViTBackbone, ViTConfig, ViTModel,  # noqa: F401
                       get_compute_mode, momentum, preprocess_u8_patches, set_compute_mode)
 from .optim import FusedAdam  # noqa: F401
-from . import augment, parallel  # noqa: F401
+from . import augment, explain, parallel  # noqa: F401
 from .train import (accumulation_steps, batch_size, epochs, learning_rate, load_checkpoint,  # noqa: F401
                     save_checkpoint, train_self_supervised)

@@ -803,6 +803,9 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
 // warp & 3).  A 197-float row is 788 B, not a multiple of 16, so neither TMA nor 128-bit stores can write the output in
 // place: the tile is staged densely in shared memory (over the dead Q / K tiles) and copied out with coalesced 4-byte
 // stores - the tile's rows are contiguous in the output, so the copy is one linear run of up to 128 x 197 floats.
+// DP = true: the same tile of dP = dO V^T, the gradient w.r.t. the probabilities (ViTModel attentions' retain_grad): A is
+// the backward's d ctx tile (row stride 192, the box of tmDO in launch_attn_bwd_tc), B is V, and the epilogue is the
+// identity (the 1/8 scale sits before the softmax, so dP has none).
 constexpr int PR_OFF_Q = 0;
 constexpr int PR_OFF_K = Q_TILE_BYTES;                        // 16384
 constexpr int PR_STG_BYTES = QT * NT * 4;                     // 100864: [128][197] fp32 (odd row stride: no conflicts)
@@ -812,13 +815,13 @@ constexpr int PR_THREADS = 160;
 static_assert(PR_OFF_K % 1024 == 0 && PR_OFF_K + KV_TILE_BYTES <= PR_STG_BYTES, "attention-probabilities smem map");
 
 struct alignas(64) AttnProbsParams {
-  CUtensorMap tmQ[MAXG], tmKV[MAXG];
-  const float* lse[MAXG];
+  CUtensorMap tmQ[MAXG], tmKV[MAXG];   // tmQ: the A operand, Q (probabilities) or d ctx (DP)
+  const float* lse[MAXG];              // unused by DP
   float* probs[MAXG];
   int* err_flag;
 };
 
-template <typename LP>
+template <typename LP, bool DP>
 __global__ void __launch_bounds__(PR_THREADS, 2) attn_probs_tc_kernel(const __grid_constant__ AttnProbsParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -850,7 +853,7 @@ __global__ void __launch_bounds__(PR_THREADS, 2) attn_probs_tc_kernel(const __gr
     if (ptx::elect_one()) {
       ptx::mbar_arrive_expect_tx(bar_load, Q_TILE_BYTES + KV_TILE_BYTES);
       ptx::tma_load_3d(smem + PR_OFF_Q, &p.tmQ[g], bar_load, h * DH, t * QT, b);
-      ptx::tma_load_3d(smem + PR_OFF_K, &p.tmKV[g], bar_load, D + h * DH, 0, b);
+      ptx::tma_load_3d(smem + PR_OFF_K, &p.tmKV[g], bar_load, (DP ? 2 * D : D) + h * DH, 0, b);   // V or K
     }
     __syncwarp();
     ptx::mbar_wait(bar_load, 0, p.err_flag, 61);
@@ -869,7 +872,8 @@ __global__ void __launch_bounds__(PR_THREADS, 2) attn_probs_tc_kernel(const __gr
     const int qrow = t * QT + row;
     const bool valid = row < nrows;
     const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16);
-    const float lse2 = valid ? __ldg(p.lse[g] + ((int64_t)b * NH + h) * NT + qrow) * LOG2E : 0.f;
+    const float lse2 = !DP && valid ? __ldg(p.lse[g] + ((int64_t)b * NH + h) * NT + qrow) * LOG2E : 0.f;
+    auto epi = [&](uint32_t v) { return DP ? __uint_as_float(v) : ptx::ex2_approx(fmaf(__uint_as_float(v), SCALE_LOG2E, -lse2)); };
     float* srow = stg + row * NT;
     uint32_t r[32];
     ptx::mbar_wait(bar_s, 0, p.err_flag, 62);     // S complete: the Q / K tiles are dead, staging may overwrite them
@@ -880,14 +884,14 @@ __global__ void __launch_bounds__(PR_THREADS, 2) attn_probs_tc_kernel(const __gr
       ptx::tmem_ld_wait();
       if (valid) {
 #pragma unroll
-        for (int i = 0; i < 32; ++i) srow[c * 32 + i] = ptx::ex2_approx(fmaf(__uint_as_float(r[i]), SCALE_LOG2E, -lse2));
+        for (int i = 0; i < 32; ++i) srow[c * 32 + i] = epi(r[i]);
       }
     }
     ptx::tmem_ld_32x16(taddr + 192, r);
     ptx::tmem_ld_wait();
     if (valid) {
 #pragma unroll
-      for (int i = 0; i < NT - 192; ++i) srow[192 + i] = ptx::ex2_approx(fmaf(__uint_as_float(r[i]), SCALE_LOG2E, -lse2));
+      for (int i = 0; i < NT - 192; ++i) srow[192 + i] = epi(r[i]);
     }
   }
   ptx::tc_fence_before();
@@ -901,6 +905,22 @@ __global__ void __launch_bounds__(PR_THREADS, 2) attn_probs_tc_kernel(const __gr
     ptx::tc_fence_after();
     ptx::tmem_dealloc(tmem_base, 256);
   }
+}
+
+// launches attn_probs_tc_kernel<LP, DP> over (2 query tiles x 3 heads, B images, groups)
+template <bool DP>
+int launch_probs_kernel(const AttnProbsParams& p, int groups, int B, cudaStream_t s, int lp_f16) {
+  static bool attr[MAX_DEVICES] = {false};
+  if (!attr[cur_device()]) {
+    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_tc_kernel<LpBf16, DP>, cudaFuncAttributeMaxDynamicSharedMemorySize, PR_SMEM));
+    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_tc_kernel<LpF16, DP>, cudaFuncAttributeMaxDynamicSharedMemorySize, PR_SMEM));
+    attr[cur_device()] = true;
+  }
+  const dim3 grid(NH * 2, B, groups);
+  if (lp_f16) V2S_CUDA_OK(launch_pdl(attn_probs_tc_kernel<LpF16, DP>, grid, dim3(PR_THREADS), (size_t)PR_SMEM, s, p));
+  else V2S_CUDA_OK(launch_pdl(attn_probs_tc_kernel<LpBf16, DP>, grid, dim3(PR_THREADS), (size_t)PR_SMEM, s, p));
+  V2S_LAUNCH_CHECK();
+  return 0;
 }
 
 }  // namespace
@@ -917,17 +937,21 @@ int launch_attn_probs_tc(const void* const* qkv, const float* const* lse, float*
     p.lse[g] = lse[g];
     p.probs[g] = probs[g];
   }
-  static bool attr[MAX_DEVICES] = {false};
-  if (!attr[cur_device()]) {
-    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_tc_kernel<LpBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PR_SMEM));
-    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_tc_kernel<LpF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PR_SMEM));
-    attr[cur_device()] = true;
+  return launch_probs_kernel<false>(p, groups, B, s, lp_f16);
+}
+
+int launch_attn_dprobs_tc(const void* const* qkv, const void* const* dctx, float* const* dprobs, int groups, int B,
+                          cudaStream_t s, int lp_f16) {
+  AttnProbsParams p;
+  memset(&p, 0, sizeof(p));
+  p.err_flag = tc_err_flag();
+  for (int g = 0; g < groups; ++g) {
+    if (!dctx[g] || !dprobs[g]) { set_error("attention-probability gradient: group %d has no d ctx / output", g); return 1; }
+    V2S_TRY(tmap_get_3d(&p.tmQ[g], dctx[g], D, NT, B, D * 2, (uint64_t)NT * D * 2, DH, QT, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmKV[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, KPAD, true, 128));
+    p.probs[g] = dprobs[g];
   }
-  const dim3 grid(NH * 2, B, groups);
-  if (lp_f16) V2S_CUDA_OK(launch_pdl(attn_probs_tc_kernel<LpF16>, grid, dim3(PR_THREADS), (size_t)PR_SMEM, s, p));
-  else V2S_CUDA_OK(launch_pdl(attn_probs_tc_kernel<LpBf16>, grid, dim3(PR_THREADS), (size_t)PR_SMEM, s, p));
-  V2S_LAUNCH_CHECK();
-  return 0;
+  return launch_probs_kernel<true>(p, groups, B, s, lp_f16);
 }
 
 int launch_attn_fwd_tc(const void* const* qkv, void* const* ctx, float* const* lse, int groups, int B,

@@ -34,9 +34,9 @@ static int n_recs = 0;
 static int n_events = 0;   // events created so far (recs[i].a/b valid for i < n_events)
 static const char* names[] = {"gemm_patch", "gemm_qkv", "gemm_proj", "gemm_fc1", "gemm_fc2", "gemm_dgrad",
                               "gemm_wgrad", "attn_fwd", "attn_bwd", "ln_fwd", "ln_bwd", "colsum", "misc", "heads", "gemm_mlp_fwd",
-                              "gemm_mlp_bwd", "attn_probs", "gemm_pixels"};
+                              "gemm_mlp_bwd", "attn_probs", "gemm_pixels", "attn_dprobs"};
 enum { C_PATCH, C_QKV, C_PROJ, C_FC1, C_FC2, C_DGRAD, C_WGRAD, C_ATTN_F, C_ATTN_B, C_LN_F, C_LN_B, C_COLSUM, C_MISC,
-       C_HEADS, C_MLP_F, C_MLP_B, C_ATTN_P, C_PIX, C_COUNT };
+       C_HEADS, C_MLP_F, C_MLP_B, C_ATTN_P, C_PIX, C_ATTN_DP, C_COUNT };
 struct Scope {
   int idx = -1;
   cudaStream_t st;
@@ -247,6 +247,16 @@ int launch_attention_probs(const void* const* qkv, const float* const* lse, floa
                     ((double)B * NT * 2 * D * (at ? 2.0 : 4.0) + (double)B * NH * NT * 4 + (double)B * NH * NT * NT * 4) * groups);
   if (at != AT_F32) return launch_attn_probs_tc(qkv, lse, probs, groups, B, s, at == AT_F16);
   return launch_attn_probs_simt(qkv, lse, probs, groups, B, at, s);
+}
+
+// fp32 gradient w.r.t. the attention probabilities of the groups that asked for it, dP = d ctx V^T
+int launch_attention_dprobs(const void* const* qkv, const void* const* dctx, float* const* dprobs, int groups, int B, int at,
+                            cudaStream_t s) {
+  // algorithmic bytes: d ctx and V read once, the fp32 gradient written once
+  prof::Scope scope(prof::C_ATTN_DP, 2.0 * B * NH * (double)NT * NT * DH * groups, s,
+                    ((double)B * NT * 2 * D * (at ? 2.0 : 4.0) + (double)B * NH * NT * NT * 4) * groups);
+  if (at != AT_F32) return launch_attn_dprobs_tc(qkv, dctx, dprobs, groups, B, s, at == AT_F16);
+  return launch_attn_dprobs_simt(qkv, dctx, dprobs, groups, B, at, s);
 }
 
 // d loss / d hidden_states[k] joins the residual-stream gradient (groups whose dh entry is NULL are skipped); for k > 0 and
@@ -540,17 +550,19 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
 // no bias / LayerNorm-parameter / embedding column sum -- and grads may be NULL.
 static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outputs_t* outs_in, int G_in, int B, int mode,
                                   void* ws, int64_t ws_bytes, cudaStream_t st, int layer_hi, int layer_lo,
-                                  float* const* dpix_in, int weight_grads) {
+                                  float* const* dpix_in, int weight_grads, float* const* dattn_in = nullptr) {
   if (layer_lo < 0 || layer_hi > NL || layer_lo >= layer_hi) { set_error("backbone_backward: bad layer range [%d, %d)", layer_lo, layer_hi); return 1; }
   // keep only the groups that saved activations and want gradients
   v2s_group_t gs[MAXG];
   const v2s_group_outputs_t* os[MAXG];
   float* dpix[MAXG];
+  float* const* dattn[MAXG];   // per group: NL gradients w.r.t. the attention probabilities (NULL entries skipped), or NULL
   int G = 0;
   for (int i = 0; i < G_in && i < MAXG; ++i)
     if (gs_in[i].slot >= 0 && (gs_in[i].grads || !weight_grads)) {
       os[G] = outs_in ? &outs_in[i] : nullptr;
       dpix[G] = dpix_in ? dpix_in[i] : nullptr;
+      dattn[G] = dattn_in ? dattn_in + (int64_t)i * NL : nullptr;
       if (dpix[G] && gs_in[i].x_format != 0) {
         set_error("backbone_input_backward: group %d: no image gradient for 16-bit patch-row inputs (x_format 1)", i);
         return 1;
@@ -762,6 +774,11 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       const void *cq[MAXG], *cc[MAXG], *cd[MAXG]; const float* ls[MAXG];
       for (int g = 0; g < G; ++g) { cq[g] = qkv[g]; cc[g] = ctx[g]; cd[g] = tmp[g]; ls[g] = (const float*)sb(g, s.lse); }
       V2S_TRY(launch_attention_bwd(cq, cc, ls, cd, big, G, B, at, st));    // d qkv in `big` [M,576]
+      // d loss / d probabilities = d ctx V^T, while `tmp` still holds d ctx; before the wgrad and its late-wait partner
+      const void *aq[MAXG], *ad[MAXG]; float* dp[MAXG]; int n = 0;
+      for (int g = 0; g < G; ++g)
+        if (dattn[g] && dattn[g][l]) { aq[n] = qkv[g]; ad[n] = tmp[g]; dp[n] = dattn[g][l]; ++n; }
+      if (n) V2S_TRY(launch_attention_dprobs(aq, ad, dp, n, B, at, st));
     }
     if (merged)        // dWo [192,192] (its gradient dxlp is only overwritten by LN1-bwd below) with dWqkv [576,192], d b_qkv
       V2S_TRY(wgrad2(dxlp, D, ctx, D, lo + L_WO, -1, big, 3 * D, xn1, D, lo + L_WQKV, lo + L_BQKV));
@@ -1045,6 +1062,25 @@ int v2s_backbone_input_backward(const v2s_group_t* groups, const v2s_group_outpu
                                 NL, 0, dpixels, weight_grads ? 1 : 0);
 }
 
+int v2s_backbone_backward_attn_grads(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, float* const* dattn,
+                                     float* const* dpixels, int weight_grads, int n_groups, int batch, int mode,
+                                     void* workspace, int64_t workspace_bytes, void* stream) {
+  if (!groups || !dattn) { set_error("backbone_backward_attn_grads: null groups / dattn"); return 1; }
+  for (int g = 0; g < n_groups && g < MAXG; ++g) {
+    for (int l = 0; l < NL; ++l)
+      if (reinterpret_cast<uintptr_t>(dattn[g * NL + l]) & 3) {
+        set_error("backbone_backward_attn_grads: dattn[%d] (group %d, block %d) is not 4-byte aligned", g * NL + l, g, l);
+        return 1;
+      }
+    if (dpixels && (reinterpret_cast<uintptr_t>(dpixels[g]) & 15)) {
+      set_error("backbone_backward_attn_grads: dpixels[%d] is not 16-byte aligned", g);
+      return 1;
+    }
+  }
+  return backbone_backward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
+                                NL, 0, dpixels, weight_grads ? 1 : 0, dattn);
+}
+
 int v2s_heads_loss_fwd_bwd(const float* head_params, float* head_grads, const float* feat_online,
                            const float* feat_target, const float* mask_online, const float* mask_target,
                            float* dfeat_online, float* pred, float* target_proj, float* loss, int batch,
@@ -1201,7 +1237,7 @@ int v2s_prof_report(char* host_buf, int64_t buf_bytes) {
 }
 
 // test hook: which = 0 forward (qkv -> ctx, lse), 1 backward (qkv, ctx, lse, dctx -> dqkv), 2 probabilities (qkv, lse ->
-// fp32 [batch,3,197,197] in ctx);
+// fp32 [batch,3,197,197] in ctx), 3 their gradient (qkv, dctx -> fp32 [batch,3,197,197] in ctx);
 // variant 0 = tensor-core kernels, 1 = SIMT reference kernels; bf16 tensors, one backbone
 int v2s_test_attention(int which, const void* qkv, void* ctx, float* lse, const void* dctx, void* dqkv, int batch,
                        int variant, void* stream) {
@@ -1223,7 +1259,12 @@ int v2s_test_attention(int which, const void* qkv, void* ctx, float* lse, const 
     if (variant & 1) return launch_attn_probs_simt(cq, cls, pr, 1, batch, at, st);
     return launch_attn_probs_tc(cq, cls, pr, 1, batch, st, f16);
   }
-  set_error("v2s_test_attention: which must be 0, 1 or 2");
+  if (which == 3) {
+    float* dp[1] = {static_cast<float*>(ctx)};
+    if (variant & 1) return launch_attn_dprobs_simt(cq, cd, dp, 1, batch, at, st);
+    return launch_attn_dprobs_tc(cq, cd, dp, 1, batch, st, f16);
+  }
+  set_error("v2s_test_attention: which must be 0, 1, 2 or 3");
   return 1;
 }
 

@@ -588,33 +588,41 @@ __global__ void __launch_bounds__(256) attn_bwd_simt_kernel(G4<const T*> qkv, G4
 
 // attention probabilities P = exp(s / 8 - lse) as fp32 [B,3,197,197] (the SIMT twin of attn_probs_tc_kernel): s is
 // accumulated in the order attn_fwd_simt_kernel uses, so the rows of the check mode sum to 1 up to fp32 rounding.
-template <typename T>
-__global__ void __launch_bounds__(256) attn_probs_simt_kernel(G4<const T*> qkv, G4<const float*> lse, G4<float*> probs) {
+// DP = true: dP = dO V^T, the gradient w.r.t. the probabilities, with a = d ctx [B,197,192] (else a = qkv).
+template <typename T, bool DP>
+__global__ void __launch_bounds__(256) attn_probs_simt_kernel(G4<const T*> qkv, G4<const T*> a, G4<const float*> lse,
+                                                              G4<float*> probs) {
   extern __shared__ float sm[];
-  float* Ks = sm;                    // [197][65]
-  float* Qs = Ks + NT * ASTR;        // [8][64]
+  float* Ks = sm;                    // [197][65]: K, or V (DP)
+  float* Qs = Ks + NT * ASTR;        // [8][64]: rows of Q, or of d ctx (DP)
   const int h = blockIdx.x, b = blockIdx.y, g = blockIdx.z;
+  constexpr int A_LD = DP ? D : 3 * D;
   const T* base = qkv.p[g] + (int64_t)b * NT * 3 * D;
+  const T* abase = a.p[g] + (int64_t)b * NT * A_LD;
   for (int i = threadIdx.x; i < NT * DH; i += blockDim.x) {
     const int t = i / DH, d = i % DH;
-    Ks[t * ASTR + d] = to_f<T>(base[(int64_t)t * 3 * D + D + h * DH + d]);
+    Ks[t * ASTR + d] = to_f<T>(base[(int64_t)t * 3 * D + (DP ? 2 * D : D) + h * DH + d]);
   }
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* Q = Qs + warp * DH;
   const float scale = 0.125f;
   for (int i = warp; i < NT; i += 8) {
-    Q[lane] = to_f<T>(base[(int64_t)i * 3 * D + h * DH + lane]);
-    Q[lane + 32] = to_f<T>(base[(int64_t)i * 3 * D + h * DH + lane + 32]);
+    Q[lane] = to_f<T>(abase[(int64_t)i * A_LD + h * DH + lane]);
+    Q[lane + 32] = to_f<T>(abase[(int64_t)i * A_LD + h * DH + lane + 32]);
     __syncwarp();
-    const float li = lse.p[g][((int64_t)b * NH + h) * NT + i];
+    const float li = DP ? 0.f : lse.p[g][((int64_t)b * NH + h) * NT + i];
     float* out = probs.p[g] + (((int64_t)b * NH + h) * NT + i) * NT;
     for (int j = lane; j < NT; j += 32) {
       float s = 0.f;
 #pragma unroll 16
       for (int d = 0; d < DH; ++d) s = fmaf(Q[d], Ks[j * ASTR + d], s);
-      s *= scale;
-      out[j] = expf(s - li);
+      if (DP) {
+        out[j] = s;
+      } else {
+        s *= scale;
+        out[j] = expf(s - li);
+      }
     }
     __syncwarp();
   }
@@ -1194,9 +1202,22 @@ int launch_attn_probs_simt(const void* const* qkv, const float* const* lse, floa
   const size_t smem = (size_t)(NT * ASTR + 8 * DH) * sizeof(float);
   dim3 grid(NH, B, groups);
   V2S_DISPATCH_AT(at, {
-    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_simt_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attn_probs_simt_kernel<T><<<grid, 256, smem, s>>>(pack4<const T*>(qkv, groups), pack4<const float*>(lse, groups),
-                                                      pack4<float*>(probs, groups));
+    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_simt_kernel<T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attn_probs_simt_kernel<T, false><<<grid, 256, smem, s>>>(pack4<const T*>(qkv, groups), pack4<const T*>(qkv, groups),
+                                                             pack4<const float*>(lse, groups), pack4<float*>(probs, groups));
+  });
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_attn_dprobs_simt(const void* const* qkv, const void* const* dctx, float* const* dprobs, int groups, int B, int at,
+                            cudaStream_t s) {
+  const size_t smem = (size_t)(NT * ASTR + 8 * DH) * sizeof(float);
+  dim3 grid(NH, B, groups);
+  V2S_DISPATCH_AT(at, {
+    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_simt_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    attn_probs_simt_kernel<T, true><<<grid, 256, smem, s>>>(pack4<const T*>(qkv, groups), pack4<const T*>(dctx, groups),
+                                                            G4<const float*>{}, pack4<float*>(dprobs, groups));
   });
   V2S_LAUNCH_CHECK();
   return 0;

@@ -47,6 +47,9 @@ int launch_attn_bwd_simt(const void* const* qkv, const void* const* ctx, const f
 // attention probabilities exp(q k^T / 8 - lse) as fp32 probs [B,3,197,197], from qkv and the forward's lse
 int launch_attn_probs_simt(const void* const* qkv, const float* const* lse, float* const* probs, int groups, int B,
                            int at, cudaStream_t s);
+// the gradient w.r.t. those probabilities, dP = dctx V^T as fp32 dprobs [B,3,197,197], from qkv and dctx [B,197,192]
+int launch_attn_dprobs_simt(const void* const* qkv, const void* const* dctx, float* const* dprobs, int groups, int B,
+                            int at, cudaStream_t s);
 
 // tcgen05 versions (bf16, or fp16 with lp_f16 = 1)
 int launch_attn_fwd_tc(const void* const* qkv, void* const* ctx, float* const* lse, int groups, int B,
@@ -56,6 +59,8 @@ int launch_attn_bwd_tc(const void* const* qkv, const void* const* ctx, const flo
                        const void* const* dctx, void* const* dqkv, int groups, int B, cudaStream_t s, int lp_f16 = 0);
 int launch_attn_probs_tc(const void* const* qkv, const float* const* lse, float* const* probs, int groups, int B,
                          cudaStream_t s, int lp_f16 = 0);
+int launch_attn_dprobs_tc(const void* const* qkv, const void* const* dctx, float* const* dprobs, int groups, int B,
+                          cudaStream_t s, int lp_f16 = 0);
 
 int launch_infonce_loss(const float* p, const float* z_all, float* loss, float* row_loss, float* dp, int B, int n_keys,
                         long long label_offset, float temperature, int accum, float grad_scale, cudaStream_t s,

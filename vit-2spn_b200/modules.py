@@ -297,14 +297,23 @@ def _run_backward(groups, batch, mode, ws, outputs=None, layer_hi=12, layer_lo=0
           "backbone_backward")
 
 
-def _run_input_backward(groups, batch, mode, ws, dpixels, weight_grads, outputs=None):
+def _run_input_backward(groups, batch, mode, ws, dpixels, weight_grads, outputs=None, attn_grads=None):
     """The whole backward, plus the fp32 image gradient of each group whose ``dpixels`` entry is a tensor (None: none);
-    weight_grads False computes no parameter gradient at all (the groups' grads may be None)."""
+    weight_grads False computes no parameter gradient at all (the groups' grads may be None).  ``attn_grads``: per group
+    12 fp32 [B,3,197,197] tensors (or None entries) that receive the gradients w.r.t. the attention probabilities;
+    ``dpixels`` may then be None."""
     arr = (Group * len(groups))(*groups)
-    dp = (C.c_void_p * len(groups))(*[t.data_ptr() if t is not None else None for t in dpixels])
+    dp = (C.c_void_p * len(groups))(*[t.data_ptr() if t is not None else None for t in dpixels]) if dpixels else None
     base, nbytes = _aligned(ws)
-    check(lib.v2s_backbone_input_backward(arr, _outputs_array(outputs, len(groups)), dp, int(bool(weight_grads)), len(groups),
-                                          batch, mode, C.c_void_p(base), nbytes, stream_ptr()), "backbone_input_backward")
+    if attn_grads is None:
+        check(lib.v2s_backbone_input_backward(arr, _outputs_array(outputs, len(groups)), dp, int(bool(weight_grads)),
+                                              len(groups), batch, mode, C.c_void_p(base), nbytes, stream_ptr()),
+              "backbone_input_backward")
+        return
+    da = (C.c_void_p * (12 * len(groups)))(*[t.data_ptr() if t is not None else None for ts in attn_grads for t in ts])
+    check(lib.v2s_backbone_backward_attn_grads(arr, _outputs_array(outputs, len(groups)), da, dp, int(bool(weight_grads)),
+                                               len(groups), batch, mode, C.c_void_p(base), nbytes, stream_ptr()),
+          "backbone_backward_attn_grads")
 
 
 def _group(store, mode, x, slot, grads=None, hidden=None, feat=None, feat_stride=0, dfeat=None,
@@ -424,8 +433,10 @@ class _BackboneFn(torch.autograd.Function):
     want_attn the outputs are (hidden_states[12], hidden_states[0..11] if want_hidden, attentions[0..11] if
     want_attn): the residual stream is written straight into the 13 hidden-state tensors, the probabilities by one extra
     kernel per block.  Gradients w.r.t. any hidden state flow back, to the parameters that require them and, when x requires
-    grad, to the pixels (v2s_backbone_input_backward; a frozen backbone then computes no weight gradient at all); the
-    attention probabilities are not differentiable."""
+    grad, to the pixels (v2s_backbone_input_backward; a frozen backbone then computes no weight gradient at all).  The
+    attention probabilities are not differentiable: a loss must not use them.  But a returned attention on which
+    retain_grad() was called receives d loss / d probabilities in .grad, as in transformers (one extra kernel per such
+    block in the same backward call; blocks at or above the highest layer the loss reaches keep .grad None)."""
 
     @staticmethod
     @_with_device_of(lambda ctx, x, *a, **k: x)
@@ -463,6 +474,8 @@ class _BackboneFn(torch.autograd.Function):
         ctx.want_hidden, ctx.want_attn = want_hidden, want_attn
         ctx.ws = ws if need_grad else None
         ctx.x = x
+        # weak: the outputs hold this node through grad_fn; backward fills .grad of those that retain_grad()
+        ctx.attn_refs = [weakref.ref(t) for t in attn] if want_attn and need_grad else None
         if not (want_hidden or want_attn):
             return out
         if need_grad and want_hidden:
@@ -504,13 +517,23 @@ class _BackboneFn(torch.autograd.Function):
             g = _group(store, ctx.mode, ctx.x, 0, grads=grads,
                        dfeat=dout if ctx.pooled else None, dfeat_stride=192,
                        dhidden=None if ctx.pooled else dout)
-        if not want_x:
+        # the retained attentions below the start of the backward (the highest hidden state with a gradient)
+        start = 12 if dout is not None else max(i for i, t in enumerate(dhid) if t is not None)
+        retained = [(l, t) for l, t in enumerate(r() for r in ctx.attn_refs or ())
+                    if l < start and t is not None and t.retains_grad]
+        if not want_x and not retained:
             _run_backward([g], ctx.B, ctx.mode, ctx.ws, outs)
             ctx.ws = None
             return nones
-        dx = torch.empty(ctx.B, 3, 224, 224, dtype=torch.float32, device=ctx.x.device)
-        _run_input_backward([g], ctx.B, ctx.mode, ctx.ws, [dx], want_w, outs)
+        dx = torch.empty(ctx.B, 3, 224, 224, dtype=torch.float32, device=ctx.x.device) if want_x else None
+        attn_grads = [None] * 12
+        for l, _ in retained:
+            attn_grads[l] = torch.empty(ctx.B, 3, 197, 197, dtype=torch.float32, device=ctx.x.device)
+        _run_input_backward([g], ctx.B, ctx.mode, ctx.ws, [dx] if want_x else None, want_w, outs,
+                            [attn_grads] if retained else None)
         ctx.ws = None
+        for l, t in retained:          # as the retain_grad hook: set, or accumulate out of place
+            t.grad = attn_grads[l] if t.grad is None else t.grad + attn_grads[l]
         return (dx,) + nones[1:]
 
 
