@@ -32,7 +32,7 @@ extern "C" {
                              removed.  3: v2s_infonce_loss, v2s_preprocess_u8_patches, v2s_group.x_format (was a
                              reserved zero field); additive to 3: v2s_group_outputs, v2s_test_attention which = 2.  Additive to 4:
                              v2s_backbone_input_backward, v2s_test_gemm which = 5; v2s_backbone_backward_attn_grads,
-                             v2s_test_attention which = 3 */
+                             v2s_test_attention which = 3; v2s_backbone_forward_masked, v2s_backbone_backward_masked */
 
 /* compute modes */
 #define V2S_MODE_FP32 0 /* fp32 activations + fp32 SIMT GEMMs: the "fp32 check mode" of north_star */
@@ -148,6 +148,26 @@ int v2s_backbone_input_backward(const v2s_group_t* host_groups, const v2s_group_
 int v2s_backbone_backward_attn_grads(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs,
                                      float* const* host_dattn, float* const* host_dpixels, int weight_grads, int n_groups,
                                      int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
+/* Masked patch tokens (transformers' ViTModel(use_mask_token=True) with bool_masked_pos, the input of SimMIM-style masked
+ * image modelling): v2s_backbone_forward, where each group g with host_masks[g] != NULL replaces the embedding of every
+ * patch p of image b with host_masks[g][b*196 + p] != 0 by the mask token, after the patch projection and its bias and
+ * before the position embedding is added.  host_masks[g]: uint8 [batch,196] (device); host_mask_tokens[g]: fp32 [192]
+ * (device, 16-byte aligned), required where a mask is set.  host_masks may be NULL (no group masked), as may
+ * host_mask_tokens when no group is masked.  A saved group's backward must pass the same mask array. */
+int v2s_backbone_forward_masked(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs,
+                                const uint8_t* const* host_masks, const float* const* host_mask_tokens, int n_groups,
+                                int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
+/* The whole backward (blocks [0, 12)) of a forward that may have been masked: v2s_backbone_backward_attn_grads plus, per
+ * group, host_masks[g] (the forward's mask array, or NULL) and host_dmask_tokens[g] (fp32 [192], 4-byte aligned, +=;
+ * with weight_grads = 1 only: weight_grads = 0 computes no mask-token gradient).  d mask_token sums the residual-stream
+ * gradient of the masked (image, patch) tokens; the patch weight and bias gradients and the image gradient come from
+ * the unmasked patches only (the image gradient is exactly 0 on masked patches).  Every array may be NULL (n_groups
+ * entries each, host_dattn n_groups*12); with all of them NULL this is v2s_backbone_backward_attn_grads.  A masked
+ * group's backward over a partial layer range (v2s_backbone_backward) is refused. */
+int v2s_backbone_backward_masked(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs,
+                                 const uint8_t* const* host_masks, float* const* host_dmask_tokens,
+                                 float* const* host_dattn, float* const* host_dpixels, int weight_grads, int n_groups,
+                                 int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* projection_head + prediction_head on the concatenated online features and projection_head on
  * the target features (ref:ssp_vit2spn_tiny.py:153-158), fused with the loss

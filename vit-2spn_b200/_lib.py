@@ -72,6 +72,10 @@ _SIGS = {
                                               _vp, _i64, _vp]),
     "v2s_backbone_backward_attn_grads": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), C.POINTER(_vp),
                                                    C.POINTER(_vp), _i, _i, _i, _i, _vp, _i64, _vp]),
+    "v2s_backbone_forward_masked": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), C.POINTER(_vp), C.POINTER(_vp),
+                                              _i, _i, _i, _vp, _i64, _vp]),
+    "v2s_backbone_backward_masked": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), C.POINTER(_vp), C.POINTER(_vp),
+                                               C.POINTER(_vp), C.POINTER(_vp), _i, _i, _i, _i, _vp, _i64, _vp]),
     "v2s_heads_loss_fwd_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _f, _vp, _i,
                                          _vp, _i64, _vp]),
     "v2s_heads_forward": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _vp]),

@@ -292,15 +292,16 @@ int check_outputs(const v2s_group_outputs_t* o, int g, const char* what) {
 
 // The residual stream of a saved group that supplied hidden[] lives in the caller's tensors, and its backward reads
 // them back: remember per (workspace, stash slot) which hidden[0] the forward used, so that a backward given other
-// tensors (or none, or some where the forward had none) is an error rather than a silent wrong gradient.
-struct HiddenRec { const void* ws; int slot; const float* h0; };
+// tensors (or none, or some where the forward had none) is an error rather than a silent wrong gradient.  The same
+// holds for the patch mask: the backward must be given the mask array its forward used (or none for none).
+struct HiddenRec { const void* ws; int slot; const float* h0; const uint8_t* mask; };
 static HiddenRec g_hidden_rec[64];
 static int g_n_hidden_rec = 0;
-void record_hidden(const void* ws, int slot, const float* h0) {
+void record_hidden(const void* ws, int slot, const float* h0, const uint8_t* mask) {
   for (int i = 0; i < g_n_hidden_rec; ++i)
-    if (g_hidden_rec[i].ws == ws && g_hidden_rec[i].slot == slot) { g_hidden_rec[i].h0 = h0; return; }
+    if (g_hidden_rec[i].ws == ws && g_hidden_rec[i].slot == slot) { g_hidden_rec[i].h0 = h0; g_hidden_rec[i].mask = mask; return; }
   const int i = g_n_hidden_rec < 64 ? g_n_hidden_rec++ : (int)((reinterpret_cast<uintptr_t>(ws) / 1024 + (uintptr_t)slot) % 64);
-  g_hidden_rec[i] = {ws, slot, h0};
+  g_hidden_rec[i] = {ws, slot, h0, mask};
 }
 const HiddenRec* find_hidden(const void* ws, int slot) {
   for (int i = 0; i < g_n_hidden_rec; ++i)
@@ -320,8 +321,11 @@ int wgrad_split(int64_t rows) {
 // =============================================================================================
 // backbone forward
 // =============================================================================================
+// masks / mask_tokens (NULL, or one entry per group): the uint8 [B,196] patch mask of each group (NULL entry: none) and its
+// fp32 [192] mask token, which replaces each masked patch embedding before the position embeddings are added
 static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_t* outs, int G, int B, int mode,
-                                 void* ws, int64_t ws_bytes, cudaStream_t st) {
+                                 void* ws, int64_t ws_bytes, cudaStream_t st, const uint8_t* const* masks = nullptr,
+                                 const float* const* mask_tokens = nullptr) {
   if (mode < V2S_MODE_FP32 || mode > V2S_MODE_FP16) { set_error("bad compute mode %d", mode); return 1; }
   if (G < 1 || G > MAXG) { set_error("backbone_forward: 1..4 groups"); return 1; }
   if (B < 1) { set_error("backbone_forward: batch must be >= 1"); return 1; }
@@ -345,7 +349,7 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
   auto hid = [&](int g) -> float* const* { return outs && outs[g].hidden[0] ? outs[g].hidden : nullptr; };
   auto want_attn = [&](int g) { return outs && outs[g].attn[0]; };
   for (int g = 0; g < G; ++g)
-    if (gs[g].slot >= 0) record_hidden(ws, gs[g].slot, hid(g) ? hid(g)[0] : nullptr);
+    if (gs[g].slot >= 0) record_hidden(ws, gs[g].slot, hid(g) ? hid(g)[0] : nullptr, masks ? masks[g] : nullptr);
 
   // ---- buffer resolution ----
   auto saved = [&](int g) { return gs[g].slot >= 0; };
@@ -389,8 +393,9 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
       pp[g] = gs[g].params; tok[g] = tmp;
     }
     V2S_TRY(run_gemm(d, at, at, 0, st, prof::C_PATCH));
-    if (two_pass) V2S_TRY(launch_assemble_tokens(pp, tok, x_cur, G, B, st));
-    else V2S_TRY(launch_cls_rows(pp, x_cur, G, B, st));
+    // masked patch rows take mask_token + pos in the kernel that writes the token rows
+    if (two_pass) V2S_TRY(launch_assemble_tokens(pp, tok, x_cur, G, B, st, masks, mask_tokens));
+    else V2S_TRY(launch_cls_rows(pp, x_cur, G, B, st, masks, mask_tokens));
   }
 
   // ---- 12 pre-LN blocks ----
@@ -548,21 +553,32 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
 // dpix_in (whole backward only; NULL or one entry per input group): the groups with dpix_in[g] != NULL also get the fp32
 // image gradient [B,3,224,224] (overwritten).  weight_grads = 0: no parameter gradient at all -- no weight-gradient GEMM,
 // no bias / LayerNorm-parameter / embedding column sum -- and grads may be NULL.
+// masks_in / dmask_in (whole backward only; NULL or one entry per input group): the patch mask the group's forward used,
+// and, with weight gradients, d mask_token fp32 [192] (+=, NULL entry: not wanted).  A masked group's masked patch rows
+// give no gradient to the patch weight, the patch bias or the pixels.
 static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outputs_t* outs_in, int G_in, int B, int mode,
                                   void* ws, int64_t ws_bytes, cudaStream_t st, int layer_hi, int layer_lo,
-                                  float* const* dpix_in, int weight_grads, float* const* dattn_in = nullptr) {
+                                  float* const* dpix_in, int weight_grads, float* const* dattn_in = nullptr,
+                                  const uint8_t* const* masks_in = nullptr, float* const* dmask_in = nullptr) {
   if (layer_lo < 0 || layer_hi > NL || layer_lo >= layer_hi) { set_error("backbone_backward: bad layer range [%d, %d)", layer_lo, layer_hi); return 1; }
+  if (any_mask(masks_in, G_in) && (layer_lo != 0 || layer_hi != NL)) {
+    set_error("backbone_backward: a masked backward covers the whole range [0, %d), not [%d, %d)", NL, layer_lo, layer_hi);
+    return 1;
+  }
   // keep only the groups that saved activations and want gradients
   v2s_group_t gs[MAXG];
   const v2s_group_outputs_t* os[MAXG];
   float* dpix[MAXG];
   float* const* dattn[MAXG];   // per group: NL gradients w.r.t. the attention probabilities (NULL entries skipped), or NULL
+  const uint8_t* mask[MAXG]; float* dmask[MAXG];
   int G = 0;
   for (int i = 0; i < G_in && i < MAXG; ++i)
     if (gs_in[i].slot >= 0 && (gs_in[i].grads || !weight_grads)) {
       os[G] = outs_in ? &outs_in[i] : nullptr;
       dpix[G] = dpix_in ? dpix_in[i] : nullptr;
       dattn[G] = dattn_in ? dattn_in + (int64_t)i * NL : nullptr;
+      mask[G] = masks_in ? masks_in[i] : nullptr;
+      dmask[G] = dmask_in && weight_grads ? dmask_in[i] : nullptr;
       if (dpix[G] && gs_in[i].x_format != 0) {
         set_error("backbone_input_backward: group %d: no image gradient for 16-bit patch-row inputs (x_format 1)", i);
         return 1;
@@ -580,6 +596,12 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     const HiddenRec* rec = find_hidden(ws, gs[g].slot);
     if (rec && rec->h0 != (hid[g] ? hid[g][0] : nullptr)) {
       set_error("backbone_backward: group %d: hidden[] differs from the forward that filled stash slot %d", g, gs[g].slot);
+      return 1;
+    }
+    if (rec && rec->mask != mask[g]) {
+      set_error("backbone_backward: group %d: the patch mask (%s) differs from the forward that filled stash slot %d (%s); "
+                "a masked forward's backward is v2s_backbone_backward_masked, over the whole range", g,
+                mask[g] ? "given" : "none", gs[g].slot, rec->mask ? "masked" : "unmasked");
       return 1;
     }
     const float* dh12 = os[g] ? os[g]->dhidden[NL] : nullptr;
@@ -631,8 +653,9 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
   // bias_goff >= 0: also accumulate the bias gradient (column sums of dY) — inside the tensor-core wgrad
   // kernel (extra N=16 MMA against a ones tile), or with the column-sum kernel on the SIMT path
   const bool tc = at != AT_F32;
+  // remap: dy is a token-row gradient [M, n_out] of which the GEMM reads the patch rows; compact: dy is already [MP, n_out]
   auto wgrad = [&](void* const* dy, int n_out, void* const* x, int k_in, int64_t goff, bool remap,
-                   int64_t bias_goff = -1) -> int {
+                   int64_t bias_goff = -1, bool compact = false) -> int {
     if (!weight_grads) return 0;
     if (bias_goff >= 0 && !tc) {
       const void* src[MAXG]; float* dst[MAXG];
@@ -641,7 +664,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       V2S_TRY(launch_colsum(src, dst, G, (int)M, n_out, at, st, det));
     }
     GemmDesc d = make_gemm_desc();
-    d.M = n_out; d.N = k_in; d.K = remap ? (int)MP : (int)M; d.groups = G;
+    d.M = n_out; d.N = k_in; d.K = (remap || compact) ? (int)MP : (int)M; d.groups = G;
     d.a_rs = 1; d.a_cs = n_out; d.b_rs = k_in; d.b_cs = 1;
     d.a_remap = remap ? 2 : 0;
     d.epi = EPI_ACCUM; d.ldc = k_in; d.split_k = split; d.det = det;
@@ -812,14 +835,14 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       pt[g] = gs[g].x_format == 1 ? const_cast<void*>(gs[g].x) : static_cast<void*>(sb(g, p.s_patches));
       if (dpix[g]) px[npx++] = g;
     }
-    if (weight_grads) V2S_TRY(launch_embed_bwd(cdx, gr, G, B, st, det));
+    if (weight_grads) V2S_TRY(launch_embed_bwd(cdx, gr, G, B, st, det, mask, dmask));
     GemmDesc dp = make_gemm_desc();
     dp.M = (int)MP; dp.N = KPE; dp.K = D; dp.groups = npx;
     dp.a_rs = D; dp.a_cs = 1; dp.b_rs = KPE; dp.b_cs = 1; dp.ldc = KPE;
     if (tc) {          // compact the patch rows, then the ordinary tensor-core wgrad
       const void* src[MAXG];
       for (int g = 0; g < G; ++g) src[g] = dxlp[g];
-      V2S_TRY(launch_gather_patch_rows(src, tmp, G, B, at, st));
+      V2S_TRY(launch_gather_patch_rows(src, tmp, G, B, at, st, mask));
       if (weight_grads) {
         GemmDesc d = make_gemm_desc();
         d.M = D; d.N = KPE; d.K = (int)MP; d.groups = G;
@@ -833,12 +856,20 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
         V2S_TRY(run_gemm(dp, at, at, 0, st, prof::C_PIX));
       }
     } else {
-      V2S_TRY(wgrad(dxlp, D, pt, KPE, OFF_WPE, true));
-      if (npx) {       // fp32 check mode: the patch rows of the token-row gradient into `big`, then col2im
+      // fp32 check mode: the GEMMs read the patch rows of the token-row gradient through the row remap; with a mask they
+      // read them compacted, masked rows zeroed, from `tmp` instead
+      const bool masked = any_mask(mask, G);
+      if (masked) {
+        const void* src[MAXG];
+        for (int g = 0; g < G; ++g) src[g] = dx[g];
+        V2S_TRY(launch_gather_patch_rows(src, tmp, G, B, at, st, mask));
+      }
+      V2S_TRY(wgrad(masked ? tmp : (void* const*)dxlp, D, pt, KPE, OFF_WPE, !masked, -1, masked));
+      if (npx) {       // the patch rows of the image gradient into `big`, then col2im
         const float* rows[MAXG]; float* img[MAXG];
-        dp.epi = EPI_STORE; dp.a_remap = 1;
+        dp.epi = EPI_STORE; dp.a_remap = masked ? 0 : 1;
         for (int i = 0; i < npx; ++i) {
-          dp.A[i] = dx[px[i]]; dp.B[i] = gs[px[i]].params + OFF_WPE; dp.out[i] = big[px[i]];
+          dp.A[i] = masked ? tmp[px[i]] : (void*)dx[px[i]]; dp.B[i] = gs[px[i]].params + OFF_WPE; dp.out[i] = big[px[i]];
           rows[i] = static_cast<const float*>(big[px[i]]); img[i] = dpix[px[i]];
         }
         V2S_TRY(run_gemm(dp, at, at, 0, st, prof::C_PIX));
@@ -1079,6 +1110,45 @@ int v2s_backbone_backward_attn_grads(const v2s_group_t* groups, const v2s_group_
   }
   return backbone_backward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
                                 NL, 0, dpixels, weight_grads ? 1 : 0, dattn);
+}
+
+int v2s_backbone_forward_masked(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, const uint8_t* const* masks,
+                                const float* const* mask_tokens, int n_groups, int batch, int mode, void* workspace,
+                                int64_t workspace_bytes, void* stream) {
+  if (!groups) { set_error("backbone_forward_masked: null groups"); return 1; }
+  for (int g = 0; masks && g < n_groups && g < MAXG; ++g) {
+    if (!masks[g]) continue;
+    if (!mask_tokens || !mask_tokens[g]) { set_error("backbone_forward_masked: group %d has a mask but no mask token", g); return 1; }
+    if (reinterpret_cast<uintptr_t>(mask_tokens[g]) & 15) {
+      set_error("backbone_forward_masked: mask_tokens[%d] is not 16-byte aligned", g);
+      return 1;
+    }
+  }
+  return backbone_forward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
+                               masks, mask_tokens);
+}
+
+int v2s_backbone_backward_masked(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, const uint8_t* const* masks,
+                                 float* const* dmask_tokens, float* const* dattn, float* const* dpixels, int weight_grads,
+                                 int n_groups, int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream) {
+  if (!groups) { set_error("backbone_backward_masked: null groups"); return 1; }
+  for (int g = 0; g < n_groups && g < MAXG; ++g) {
+    for (int l = 0; dattn && l < NL; ++l)
+      if (reinterpret_cast<uintptr_t>(dattn[g * NL + l]) & 3) {
+        set_error("backbone_backward_masked: dattn[%d] (group %d, block %d) is not 4-byte aligned", g * NL + l, g, l);
+        return 1;
+      }
+    if (dpixels && (reinterpret_cast<uintptr_t>(dpixels[g]) & 15)) {
+      set_error("backbone_backward_masked: dpixels[%d] is not 16-byte aligned", g);
+      return 1;
+    }
+    if (dmask_tokens && (reinterpret_cast<uintptr_t>(dmask_tokens[g]) & 3)) {
+      set_error("backbone_backward_masked: dmask_tokens[%d] is not 4-byte aligned", g);
+      return 1;
+    }
+  }
+  return backbone_backward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
+                                NL, 0, dpixels, weight_grads ? 1 : 0, dattn, masks, dmask_tokens);
 }
 
 int v2s_heads_loss_fwd_bwd(const float* head_params, float* head_grads, const float* feat_online,

@@ -41,16 +41,41 @@ __global__ void im2col_kernel(G4<const float*> x, G4<T*> out, int B) {
   }
 }
 
-__global__ void cls_rows_kernel(G4<const float*> params, G4<float*> hidden) {
+// Masked patch tokens (transformers' bool_masked_pos): per group a uint8 [B,196] mask (nonzero = masked; NULL = none)
+// and the fp32 [192] mask token that replaces a masked patch embedding before the position embedding is added.  The
+// kernels below take them as their last argument and read them only in their MASK instantiation.
+struct MaskArgs { const uint8_t* mask[MAXG]; const float* token[MAXG]; };
+MaskArgs pack_masks(const uint8_t* const* mask, const float* const* token, int groups) {
+  MaskArgs m;
+  for (int i = 0; i < MAXG; ++i) {
+    m.mask[i] = (mask && i < groups) ? mask[i] : nullptr;
+    m.token[i] = (token && i < groups) ? token[i] : nullptr;
+  }
+  return m;
+}
+
+// fp32 check mode: the patch GEMM's epilogue wrote hidden[b,1+p,:] = tok + pos[1+p]; this adds the CLS row and, with
+// MASK, overwrites each masked patch row with mask_token + pos[1+p]
+template <bool MASK>
+__global__ void cls_rows_kernel(G4<const float*> params, G4<float*> hidden, MaskArgs mk) {
   const int g = blockIdx.y, b = blockIdx.x, n = threadIdx.x;
   const float* p = params.p[g];
   hidden.p[g][(int64_t)b * NT * D + n] = p[OFF_CLS + n] + p[OFF_POS + n];
+  if constexpr (MASK) {
+    const uint8_t* m = mk.mask[g];
+    if (!m) return;
+    const float t = mk.token[g][n];
+    for (int q = 0; q < NP; ++q)
+      if (m[(int64_t)b * NP + q]) hidden.p[g][((int64_t)b * NT + 1 + q) * D + n] = t + p[OFF_POS + (int64_t)(1 + q) * D + n];
+  }
 }
 
 // hidden[b,0,:] = cls + pos[0];  hidden[b,1+p,:] = tok[b*196+p,:] + pos[1+p]   (HF:117-124)
+// MASK: a masked patch row takes mask_token + pos[1+p] instead (HF:ViTEmbeddings.forward, as a select)
 // one float4 per thread; blockIdx.y = image, blockIdx.z = backbone
+template <bool MASK>
 __global__ void __launch_bounds__(256) assemble_tokens_kernel(G4<const float*> params, G4<const float*> tok,
-                                                              G4<float*> hidden) {
+                                                              G4<float*> hidden, MaskArgs mk) {
   const int g = blockIdx.z, b = blockIdx.y;
   const float* __restrict__ p = params.p[g];
   const float* __restrict__ tk = tok.p[g];
@@ -58,22 +83,33 @@ __global__ void __launch_bounds__(256) assemble_tokens_kernel(G4<const float*> p
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < NT * (D / 4); i += gridDim.x * blockDim.x) {
     const int t = i / (D / 4), c = (i % (D / 4)) * 4;
     const float4 pos = *reinterpret_cast<const float4*>(p + OFF_POS + (int64_t)t * D + c);
-    const float4 v = (t == 0) ? *reinterpret_cast<const float4*>(p + OFF_CLS + c)
-                              : *reinterpret_cast<const float4*>(tk + ((int64_t)b * NP + t - 1) * D + c);
+    float4 v;
+    if constexpr (MASK) {
+      const float* src = (t == 0) ? p + OFF_CLS + c : tk + ((int64_t)b * NP + t - 1) * D + c;
+      if (t > 0 && mk.mask[g] && mk.mask[g][(int64_t)b * NP + t - 1]) src = mk.token[g] + c;
+      v = *reinterpret_cast<const float4*>(src);
+    } else {
+      v = (t == 0) ? *reinterpret_cast<const float4*>(p + OFF_CLS + c)
+                   : *reinterpret_cast<const float4*>(tk + ((int64_t)b * NP + t - 1) * D + c);
+    }
     *reinterpret_cast<float4*>(h + ((int64_t)b * NT + t) * D + c) =
         make_float4(v.x + pos.x, v.y + pos.y, v.z + pos.z, v.w + pos.w);
   }
 }
 
 // compact the patch-token rows of a [B,197,192] tensor into [B*196,192] (drops the CLS rows); 8 bytes per thread
-template <typename T>
-__global__ void __launch_bounds__(256) gather_patch_rows_kernel(G4<const T*> src, G4<T*> dst) {
+// MASK: the rows of masked patches are written as zeros (no gradient reaches W_pe, b_pe or the pixels through them)
+template <typename T, bool MASK>
+__global__ void __launch_bounds__(256) gather_patch_rows_kernel(G4<const T*> src, G4<T*> dst, MaskArgs mk) {
   const int g = blockIdx.z, b = blockIdx.y;
   constexpr int V = 8 / sizeof(T);                 // elements per 8-byte access
   const T* __restrict__ s = src.p[g] + ((int64_t)b * NT + 1) * D;
   T* __restrict__ d = dst.p[g] + (int64_t)b * NP * D;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < NP * D / V; i += gridDim.x * blockDim.x)
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < NP * D / V; i += gridDim.x * blockDim.x) {
+    if constexpr (MASK)
+      if (mk.mask[g] && mk.mask[g][(int64_t)b * NP + i / (D / V)]) { reinterpret_cast<uint2*>(d)[i] = make_uint2(0u, 0u); continue; }
     reinterpret_cast<uint2*>(d)[i] = reinterpret_cast<const uint2*>(s)[i];
+  }
 }
 
 // the inverse permutation of im2col (stride = kernel, no overlap-add): patch rows [B*196, 768] fp32 -> NCHW fp32
@@ -419,22 +455,43 @@ __global__ void __launch_bounds__(256) pool_bwd_kernel(G4<const float*> dfeat, G
 
 // d pos / d cls / d patch-bias from the gradient of the embedding output
 // DET: the patch-bias sum over the 196 patch tokens goes through det_part [group][196][192] in token order
-template <bool DET>
-__global__ void embed_bwd_kernel(G4<const float*> dx, G4<float*> grads, int B, float* det_part, unsigned* det_counters) {
+// MASK (groups with a mask): d patch-bias sums the unmasked (image, patch) rows only; the masked ones are summed into
+// d mask_token (dtok; NULL: not wanted).  DET then carries both sums per token, det_part [group][196][384], through the
+// same fixed-order reduction with twice the shared rows, so that d patch-bias keeps the unmasked kernel's order and bits.
+template <bool DET, bool MASK>
+__global__ void embed_bwd_kernel(G4<const float*> dx, G4<float*> grads, int B, float* det_part, unsigned* det_counters,
+                                 MaskArgs mk, G4<float*> dtok) {
   const int g = blockIdx.y, t = blockIdx.x, n = threadIdx.x;
   const float* d = dx.p[g] + (int64_t)t * D + n;
-  float s = 0.f;
-  for (int b = 0; b < B; ++b) s += d[(int64_t)b * NT * D];
+  float s = 0.f, sm = 0.f;
+  const uint8_t* m = MASK && t > 0 ? mk.mask[g] : nullptr;
+  if (MASK && m) {
+    for (int b = 0; b < B; ++b) {
+      const float v = d[(int64_t)b * NT * D];
+      if (m[(int64_t)b * NP + t - 1]) sm += v; else s += v;
+    }
+  } else {
+    for (int b = 0; b < B; ++b) s += d[(int64_t)b * NT * D];
+  }
   float* gr = grads.p[g];
-  gr[OFF_POS + (int64_t)t * D + n] += s;
+  float* dt = MASK ? dtok.p[g] : nullptr;
+  gr[OFF_POS + (int64_t)t * D + n] += MASK ? s + sm : s;
   if (t == 0) gr[OFF_CLS + n] += s;
-  else if (!DET) atomicAdd(gr + OFF_BPE + n, s);
+  else if (!DET) {
+    atomicAdd(gr + OFF_BPE + n, s);
+    if (MASK && m && dt) atomicAdd(dt + n, sm);
+  }
   if constexpr (DET) {
     if (t == 0) return;
-    __shared__ __align__(16) float red[8 * D];
-    float* part = det_part + (int64_t)g * NP * D;
-    part[(int64_t)(t - 1) * D + n] = s;
-    det_reduce_rows(part, D, NP, det_counters + g, red, 8 * D, [gr](int c, float v) { gr[OFF_BPE + c] += v; });
+    constexpr int W = MASK ? 2 * D : D;          // floats per partial row
+    __shared__ __align__(16) float red[8 * W];
+    float* part = det_part + (int64_t)g * NP * W;
+    part[(int64_t)(t - 1) * W + n] = s;
+    if constexpr (MASK) part[(int64_t)(t - 1) * W + D + n] = sm;
+    det_reduce_rows(part, W, NP, det_counters + g, red, 8 * W, [gr, dt](int c, float v) {
+      if (c < D) gr[OFF_BPE + c] += v;
+      else if (dt) dt[c - D] += v;
+    });
   }
 }
 
@@ -1032,23 +1089,39 @@ int launch_im2col(const float* const* x, void* const* out, int groups, int B, in
   return 0;
 }
 
-int launch_cls_rows(const float* const* params, float* const* hidden, int groups, int B, cudaStream_t s) {
-  cls_rows_kernel<<<dim3(B, groups), D, 0, s>>>(pack4<const float*>(params, groups), pack4<float*>(hidden, groups));
+int launch_cls_rows(const float* const* params, float* const* hidden, int groups, int B, cudaStream_t s,
+                    const uint8_t* const* mask, const float* const* mask_token) {
+  const MaskArgs mk = pack_masks(mask, mask_token, groups);
+  if (any_mask(mask, groups))
+    cls_rows_kernel<true><<<dim3(B, groups), D, 0, s>>>(pack4<const float*>(params, groups), pack4<float*>(hidden, groups), mk);
+  else
+    cls_rows_kernel<false><<<dim3(B, groups), D, 0, s>>>(pack4<const float*>(params, groups), pack4<float*>(hidden, groups), mk);
   V2S_LAUNCH_CHECK();
   return 0;
 }
 
 int launch_assemble_tokens(const float* const* params, const float* const* tok, float* const* hidden, int groups,
-                           int B, cudaStream_t s) {
-  assemble_tokens_kernel<<<dim3(8, B, groups), 256, 0, s>>>(pack4<const float*>(params, groups),
-                                                          pack4<const float*>(tok, groups), pack4<float*>(hidden, groups));
+                           int B, cudaStream_t s, const uint8_t* const* mask, const float* const* mask_token) {
+  const MaskArgs mk = pack_masks(mask, mask_token, groups);
+  if (any_mask(mask, groups))
+    assemble_tokens_kernel<true><<<dim3(8, B, groups), 256, 0, s>>>(pack4<const float*>(params, groups),
+                                                                  pack4<const float*>(tok, groups), pack4<float*>(hidden, groups), mk);
+  else
+    assemble_tokens_kernel<false><<<dim3(8, B, groups), 256, 0, s>>>(pack4<const float*>(params, groups),
+                                                                   pack4<const float*>(tok, groups), pack4<float*>(hidden, groups), mk);
   V2S_LAUNCH_CHECK();
   return 0;
 }
 
-int launch_gather_patch_rows(const void* const* src, void* const* dst, int groups, int B, int at, cudaStream_t s) {
+int launch_gather_patch_rows(const void* const* src, void* const* dst, int groups, int B, int at, cudaStream_t s,
+                             const uint8_t* const* mask) {
   dim3 grid(8, B, groups);
-  V2S_DISPATCH_AT(at, gather_patch_rows_kernel<T><<<grid, 256, 0, s>>>(pack4<const T*>(src, groups), pack4<T*>(dst, groups)));
+  const MaskArgs mk = pack_masks(mask, nullptr, groups);
+  if (any_mask(mask, groups)) {
+    V2S_DISPATCH_AT(at, (gather_patch_rows_kernel<T, true><<<grid, 256, 0, s>>>(pack4<const T*>(src, groups), pack4<T*>(dst, groups), mk)));
+  } else {
+    V2S_DISPATCH_AT(at, (gather_patch_rows_kernel<T, false><<<grid, 256, 0, s>>>(pack4<const T*>(src, groups), pack4<T*>(dst, groups), mk)));
+  }
   V2S_LAUNCH_CHECK();
   return 0;
 }
@@ -1158,14 +1231,20 @@ int launch_pool_bwd(const float* const* dfeat, const int64_t* dfeat_stride, cons
   return 0;
 }
 
-int launch_embed_bwd(const float* const* dx, float* const* grads, int groups, int B, cudaStream_t s, const DetScratch* det) {
+int launch_embed_bwd(const float* const* dx, float* const* grads, int groups, int B, cudaStream_t s, const DetScratch* det,
+                     const uint8_t* const* mask, float* const* dmask_token) {
+  const bool masked = any_mask(mask, groups);
+  const MaskArgs mk = pack_masks(mask, nullptr, groups);
+  const G4<float*> dt = pack4<float*>(dmask_token, groups);
+  const G4<const float*> cdx = pack4<const float*>(dx, groups);
+  const G4<float*> gr = pack4<float*>(grads, groups);
   if (det) {
-    if ((int64_t)groups * NP * D > det->part_floats) { set_error("embed_bwd: deterministic scratch too small"); return 1; }
-    embed_bwd_kernel<true><<<dim3(NT, groups), D, 0, s>>>(pack4<const float*>(dx, groups), pack4<float*>(grads, groups), B,
-                                                          det->part, det->counters);
+    if ((int64_t)groups * NP * D * (masked ? 2 : 1) > det->part_floats) { set_error("embed_bwd: deterministic scratch too small"); return 1; }
+    if (masked) embed_bwd_kernel<true, true><<<dim3(NT, groups), D, 0, s>>>(cdx, gr, B, det->part, det->counters, mk, dt);
+    else embed_bwd_kernel<true, false><<<dim3(NT, groups), D, 0, s>>>(cdx, gr, B, det->part, det->counters, mk, dt);
   } else {
-    embed_bwd_kernel<false><<<dim3(NT, groups), D, 0, s>>>(pack4<const float*>(dx, groups), pack4<float*>(grads, groups), B,
-                                                           nullptr, nullptr);
+    if (masked) embed_bwd_kernel<false, true><<<dim3(NT, groups), D, 0, s>>>(cdx, gr, B, nullptr, nullptr, mk, dt);
+    else embed_bwd_kernel<false, false><<<dim3(NT, groups), D, 0, s>>>(cdx, gr, B, nullptr, nullptr, mk, dt);
   }
   V2S_LAUNCH_CHECK();
   return 0;

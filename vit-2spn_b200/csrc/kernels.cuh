@@ -7,10 +7,20 @@ namespace v2s {
 
 // type tag `at`: 0 = fp32 activations, 1 = bf16, 2 = fp16
 int launch_im2col(const float* const* x, void* const* out, int groups, int B, int at, cudaStream_t s);
-int launch_cls_rows(const float* const* params, float* const* hidden, int groups, int B, cudaStream_t s);
+// mask / mask_token (optional, per group): transformers' bool_masked_pos as uint8 [B,196] (nonzero = masked) and the fp32
+// [192] token a masked patch embedding is replaced by; NULL arrays or entries: no mask, the unmasked kernels run
+inline bool any_mask(const uint8_t* const* mask, int groups) {
+  for (int i = 0; mask && i < groups; ++i) if (mask[i]) return true;
+  return false;
+}
+int launch_cls_rows(const float* const* params, float* const* hidden, int groups, int B, cudaStream_t s,
+                    const uint8_t* const* mask = nullptr, const float* const* mask_token = nullptr);
 int launch_assemble_tokens(const float* const* params, const float* const* tok, float* const* hidden, int groups,
-                           int B, cudaStream_t s);
-int launch_gather_patch_rows(const void* const* src, void* const* dst, int groups, int B, int at, cudaStream_t s);
+                           int B, cudaStream_t s, const uint8_t* const* mask = nullptr,
+                           const float* const* mask_token = nullptr);
+// mask: the rows of masked patches are written as zeros
+int launch_gather_patch_rows(const void* const* src, void* const* dst, int groups, int B, int at, cudaStream_t s,
+                             const uint8_t* const* mask = nullptr);
 // inverse of launch_im2col for fp32: patch rows [B*196, 768] -> NCHW [B,3,224,224] (overwritten)
 int launch_col2im(const float* const* rows, float* const* img, int groups, int B, cudaStream_t s);
 int launch_ln_fwd(const float* const* x, const float* const* gamma, const float* const* beta,
@@ -31,8 +41,11 @@ int launch_pool_fwd(const float* const* hidden, float* const* feat, const int64_
                     int groups, int B, cudaStream_t s);
 int launch_pool_bwd(const float* const* dfeat, const int64_t* dfeat_stride, const float* const* dhidden,
                     float* const* dx, void* const* dx_lp, int groups, int B, int at, cudaStream_t s);
+// mask: d patch-bias from the unmasked patch rows only; dmask_token (optional, per group) += the column sums of the
+// masked ones
 int launch_embed_bwd(const float* const* dx, float* const* grads, int groups, int B, cudaStream_t s,
-                     const DetScratch* det = nullptr);
+                     const DetScratch* det = nullptr, const uint8_t* const* mask = nullptr,
+                     float* const* dmask_token = nullptr);
 // dx (fp32, in/out) += dh; dx_lp (activation type, 16-bit modes only) = updated dx; [B,197,192] per group;
 // dcol (optional, per group) += column sums of dh
 int launch_residual_grad_add(const float* const* dh, float* const* dx, void* const* dx_lp, float* const* dcol, int groups, int B,

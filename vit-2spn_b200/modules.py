@@ -316,6 +316,32 @@ def _run_input_backward(groups, batch, mode, ws, dpixels, weight_grads, outputs=
           "backbone_backward_attn_grads")
 
 
+def _run_forward_masked(groups, batch, mode, ws, masks, mask_tokens, outputs=None):
+    """``_run_forward`` with per-group patch masks (uint8 [B,196] tensors or None) and their fp32 mask tokens."""
+    arr = (Group * len(groups))(*groups)
+    mk = (C.c_void_p * len(groups))(*[t.data_ptr() if t is not None else None for t in masks])
+    tk = (C.c_void_p * len(groups))(*[t.data_ptr() if t is not None else None for t in mask_tokens])
+    base, nbytes = _aligned(ws)
+    check(lib.v2s_backbone_forward_masked(arr, _outputs_array(outputs, len(groups)), mk, tk, len(groups), batch, mode,
+                                          C.c_void_p(base), nbytes, stream_ptr()), "backbone_forward_masked")
+
+
+def _run_masked_backward(groups, batch, mode, ws, masks, dmask_tokens, dpixels, weight_grads, outputs=None,
+                         attn_grads=None):
+    """The whole backward of a masked forward: ``_run_input_backward`` plus the masks the forward used and, per group, an
+    fp32 [192] tensor (or None) that receives d mask_token (+=; only with weight_grads)."""
+    n = len(groups)
+    arr = (Group * n)(*groups)
+
+    def ptrs(ts, k=1):
+        return (C.c_void_p * (k * n))(*[t.data_ptr() if t is not None else None for t in ts]) if ts is not None else None
+    da = ptrs([t for ts in attn_grads for t in ts], 12) if attn_grads is not None else None
+    base, nbytes = _aligned(ws)
+    check(lib.v2s_backbone_backward_masked(arr, _outputs_array(outputs, n), ptrs(masks), ptrs(dmask_tokens), da,
+                                           ptrs(dpixels), int(bool(weight_grads)), n, batch, mode, C.c_void_p(base),
+                                           nbytes, stream_ptr()), "backbone_backward_masked")
+
+
 def _group(store, mode, x, slot, grads=None, hidden=None, feat=None, feat_stride=0, dfeat=None,
            dfeat_stride=0, dhidden=None):
     g = Group()
@@ -436,11 +462,13 @@ class _BackboneFn(torch.autograd.Function):
     grad, to the pixels (v2s_backbone_input_backward; a frozen backbone then computes no weight gradient at all).  The
     attention probabilities are not differentiable: a loss must not use them.  But a returned attention on which
     retain_grad() was called receives d loss / d probabilities in .grad, as in transformers (one extra kernel per such
-    block in the same backward call; blocks at or above the highest layer the loss reaches keep .grad None)."""
+    block in the same backward call; blocks at or above the highest layer the loss reaches keep .grad None).  With `mask`
+    (uint8 [B,196]) the masked patch embeddings are replaced by `mask_token`, an autograd input whose gradient is
+    returned (v2s_backbone_forward_masked / v2s_backbone_backward_masked)."""
 
     @staticmethod
     @_with_device_of(lambda ctx, x, *a, **k: x)
-    def forward(ctx, x, anchor, model, pooled, need_grad, want_hidden=False, want_attn=False):
+    def forward(ctx, x, anchor, model, pooled, need_grad, want_hidden=False, want_attn=False, mask=None, mask_token=None):
         store = model._store
         store.ensure()
         mode = model._mode()
@@ -468,7 +496,14 @@ class _BackboneFn(torch.autograd.Function):
             for i, t in enumerate(attn or ()):
                 o.attn[i] = t.data_ptr()
             outs = [o]
-        _run_forward([g], B, mode, ws, outs)
+        if mask is None:
+            _run_forward([g], B, mode, ws, outs)
+        else:
+            tok = mask_token.detach().reshape(192)
+            if tok.data_ptr() % 16:
+                tok = tok.clone()
+            _run_forward_masked([g], B, mode, ws, [mask], [tok], outs)
+        ctx.mask = mask                 # the backward passes the same array (the library checks it)
         ctx.set_materialize_grads(False)
         ctx.model, ctx.pooled, ctx.mode, ctx.B = model, pooled, mode, B
         ctx.want_hidden, ctx.want_attn = want_hidden, want_attn
@@ -493,12 +528,17 @@ class _BackboneFn(torch.autograd.Function):
                                "detach them before they enter the loss")
         if ctx.ws is None:
             raise RuntimeError("vit2spn: backward through a forward that saved no activations")
-        nones = (None,) * 7
+        nones = (None,) * 9
         if dout is None and all(t is None for t in dhid):
             return nones
         _deterministic()
         want_x, want_w = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        masked = ctx.mask is not None
+        want_t = masked and ctx.needs_input_grad[8]
         grads = store.grads() if want_w else None
+        if want_t and grads is None:
+            # d mask_token comes with the weight gradients: a frozen backbone computes them into a buffer that is dropped
+            grads = torch.zeros(store.numel, dtype=torch.float32, device=ctx.x.device)
         dout = _grad_f32(dout) if dout is not None else None
         outs = None
         keep = []
@@ -521,7 +561,7 @@ class _BackboneFn(torch.autograd.Function):
         start = 12 if dout is not None else max(i for i, t in enumerate(dhid) if t is not None)
         retained = [(l, t) for l, t in enumerate(r() for r in ctx.attn_refs or ())
                     if l < start and t is not None and t.retains_grad]
-        if not want_x and not retained:
+        if not want_x and not retained and not masked:
             _run_backward([g], ctx.B, ctx.mode, ctx.ws, outs)
             ctx.ws = None
             return nones
@@ -529,12 +569,18 @@ class _BackboneFn(torch.autograd.Function):
         attn_grads = [None] * 12
         for l, _ in retained:
             attn_grads[l] = torch.empty(ctx.B, 3, 197, 197, dtype=torch.float32, device=ctx.x.device)
-        _run_input_backward([g], ctx.B, ctx.mode, ctx.ws, [dx] if want_x else None, want_w, outs,
-                            [attn_grads] if retained else None)
+        dtok = None
+        if masked:
+            dtok = torch.zeros(192, dtype=torch.float32, device=ctx.x.device) if want_t else None
+            _run_masked_backward([g], ctx.B, ctx.mode, ctx.ws, [ctx.mask], [dtok], [dx], want_w or want_t, outs,
+                                 [attn_grads] if retained else None)
+        else:
+            _run_input_backward([g], ctx.B, ctx.mode, ctx.ws, [dx] if want_x else None, want_w, outs,
+                                [attn_grads] if retained else None)
         ctx.ws = None
         for l, t in retained:          # as the retain_grad hook: set, or accumulate out of place
             t.grad = attn_grads[l] if t.grad is None else t.grad + attn_grads[l]
-        return (dx,) + nones[1:]
+        return (dx,) + nones[1:8] + (dtok.view(1, 1, 192) if dtok is not None else None,)
 
 
 _warned_random_init = False
@@ -580,9 +626,10 @@ def _load_weight_file(path):
 
 
 class ViTModel(nn.Module):
-    """Drop-in for ``transformers.ViTModel`` as used by the reference (ViT-Tiny/16@224 only)."""
+    """Drop-in for ``transformers.ViTModel`` as used by the reference (ViT-Tiny/16@224 only).  ``use_mask_token=True``
+    adds transformers' ``embeddings.mask_token`` (zeros [1,1,192]) for ``forward(..., bool_masked_pos=...)``."""
 
-    def __init__(self, config=None, add_pooling_layer=True, **kw):
+    def __init__(self, config=None, add_pooling_layer=True, use_mask_token=False, **kw):
         super().__init__()
         config = config or ViTConfig(**kw)
         config._check_supported()
@@ -631,6 +678,13 @@ class ViTModel(nn.Module):
         params = list(self.parameters())
         assert len(params) == 200
         self._store = FlatStore(params, _lib.backbone_layout(), _lib.BACKBONE_NUMEL, _lib.BACKBONE_ACTIVE_NUMEL)
+        if use_mask_token:
+            # outside the flat buffer, whose layout holds exactly the 200 tensors above; registered where transformers'
+            # ViTEmbeddings has it (after cls_token) so that state_dict keys come in the same order
+            emb.mask_token = nn.Parameter(torch.zeros(1, 1, 192))
+            order = ("cls_token", "mask_token", "position_embeddings")
+            assert set(emb._parameters) == set(order), sorted(emb._parameters)
+            emb._parameters = {k: emb._parameters[k] for k in order}
         self.compute_mode = None        # None → package default (set_compute_mode)
 
     @classmethod
@@ -641,9 +695,10 @@ class ViTModel(nn.Module):
         read; missing / unexpected keys are reported.  If no checkpoint can be found this RAISES — training from random
         weights while the script asked for pretrained ones must not happen silently — unless
         ``V2S_ALLOW_RANDOM_INIT=1`` is set (offline boxes, benchmarks, tests: north_star specifies random init
-        there), in which case the HF random initialisation is kept and said so on stderr."""
+        there), in which case the HF random initialisation is kept and said so on stderr.  With ``use_mask_token=True``
+        the checkpoint's ``embeddings.mask_token`` is loaded if it has one; otherwise it stays zeros, as in transformers."""
         cfg_kw = {k: v for k, v in kw.items() if k in ("output_hidden_states", "output_attentions")}
-        model = cls(ViTConfig(**cfg_kw))
+        model = cls(ViTConfig(**cfg_kw), use_mask_token=bool(kw.get("use_mask_token", False)))
         path = _resolve_checkpoint(str(name))
         if path is None:
             if os.environ.get("V2S_ALLOW_RANDOM_INIT", "0") != "1":
@@ -661,7 +716,7 @@ class ViTModel(nn.Module):
         sd = {k[4:] if k.startswith("vit.") else k: v for k, v in sd.items()}
         res = model.load_state_dict(sd, strict=False)
         # a ViTForImageClassification checkpoint has a classifier and no pooler: exactly what transformers tolerates
-        missing = [k for k in res.missing_keys if not k.startswith("pooler.")]
+        missing = [k for k in res.missing_keys if not k.startswith("pooler.") and k != "embeddings.mask_token"]
         unexpected = [k for k in res.unexpected_keys if not k.startswith("classifier.")]
         print(f"vit2spn: loaded {path} ({len(sd) - len(res.unexpected_keys)} tensors; missing {res.missing_keys or 'none'}; "
               f"unexpected {res.unexpected_keys or 'none'})", file=sys.stderr, flush=True)
@@ -685,18 +740,44 @@ class ViTModel(nn.Module):
         a = self.embeddings.cls_token
         return _BackboneFn.apply(x, a, self, True, torch.is_grad_enabled() and (a.requires_grad or x.requires_grad))
 
-    def forward(self, pixel_values, output_hidden_states=None, output_attentions=None, **kw):
+    def _check_mask(self, m, batch):
+        if getattr(self.embeddings, "mask_token", None) is None:
+            raise ValueError("vit2spn: bool_masked_pos needs a mask token: build the model with "
+                             "ViTModel(config, use_mask_token=True)")
+        if not isinstance(m, torch.Tensor) or tuple(m.shape) != (batch, 196):
+            raise ValueError(f"vit2spn: bool_masked_pos must be a [B,196] = [{batch},196] tensor, got "
+                             f"{tuple(m.shape) if isinstance(m, torch.Tensor) else type(m).__name__}")
+        if m.dtype.is_floating_point or m.dtype.is_complex:
+            raise ValueError(f"vit2spn: bool_masked_pos must be bool, uint8 or an integer type, got {m.dtype}")
+
+    @staticmethod
+    def _mask_arg(m, x):
+        """bool_masked_pos as the library reads it: uint8 [B,196] on x's device, 1 = masked."""
+        if m.device != x.device:
+            raise ValueError(f"vit2spn: bool_masked_pos is on {m.device}, pixel_values on {x.device}: pass the mask on "
+                             "the input's device")
+        return (m != 0).to(torch.uint8).contiguous()
+
+    def forward(self, pixel_values, output_hidden_states=None, output_attentions=None, *, bool_masked_pos=None, **kw):
         """As ``transformers.ViTModel``: each flag comes from the keyword, else from the config.  The hidden states
         cost no extra kernel work (the residual stream is written into them) but keep 13 x [B,197,192] fp32 alive; the
-        attention probabilities are fp32 [B,3,197,197] per block, recomputed by one extra kernel per block."""
+        attention probabilities are fp32 [B,3,197,197] per block, recomputed by one extra kernel per block.
+        ``bool_masked_pos`` ([B,196] bool / uint8 / int on the input's device, nonzero = masked; a model built with
+        ``use_mask_token=True``) replaces those patch embeddings by ``embeddings.mask_token``, as transformers does."""
+        if bool_masked_pos is not None:
+            self._check_mask(bool_masked_pos, pixel_values.shape[0])
         x = _check_images(pixel_values)
         a = self.embeddings.cls_token
         want_hidden = bool(self.config.output_hidden_states if output_hidden_states is None else output_hidden_states)
         want_attn = bool(getattr(self.config, "output_attentions", False) if output_attentions is None else output_attentions)
         need_grad = torch.is_grad_enabled() and (a.requires_grad or x.requires_grad)
+        masked = ()
+        if bool_masked_pos is not None:
+            masked = (self._mask_arg(bool_masked_pos, x), self.embeddings.mask_token)
+            need_grad = need_grad or (torch.is_grad_enabled() and masked[1].requires_grad)
         if not (want_hidden or want_attn):
-            return ViTModelOutput(self, _BackboneFn.apply(x, a, self, False, need_grad))
-        res = _BackboneFn.apply(x, a, self, False, need_grad, want_hidden, want_attn)
+            return ViTModelOutput(self, _BackboneFn.apply(x, a, self, False, need_grad, *((False, False) + masked if masked else ())))
+        res = _BackboneFn.apply(x, a, self, False, need_grad, want_hidden, want_attn, *masked)
         last = res[0]
         hidden = tuple(res[1:13]) + (last,) if want_hidden else None
         attentions = tuple(res[13:] if want_hidden else res[1:]) if want_attn else None
