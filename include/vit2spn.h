@@ -26,13 +26,15 @@
 extern "C" {
 #endif
 
-#define V2S_ABI_VERSION 4 /* 4: one entry point per operation: v2s_backbone_forward / _backward take the per-group outputs
-                             and (backward) the layer range, v2s_heads_loss_fwd_bwd the device loss scale, v2s_adam_step
-                             and v2s_ema_update the lp_format; their narrower variants and the bf16-only cast are
-                             removed.  3: v2s_infonce_loss, v2s_preprocess_u8_patches, v2s_group.x_format (was a
-                             reserved zero field); additive to 3: v2s_group_outputs, v2s_test_attention which = 2.  Additive to 4:
-                             v2s_backbone_input_backward, v2s_test_gemm which = 5; v2s_backbone_backward_attn_grads,
-                             v2s_test_attention which = 3; v2s_backbone_forward_masked, v2s_backbone_backward_masked */
+#define V2S_ABI_VERSION 5 /* 5: the backbone calls added to 4 (image, attention-probability and mask-token gradients,
+                             masked forward) are folded into v2s_backbone_forward / _backward: their arguments are
+                             fields of v2s_group_outputs, and v2s_backbone_backward takes weight_grads.  Additive to 4:
+                             v2s_test_gemm which = 5, v2s_test_attention which = 3.  4: one entry point per operation:
+                             v2s_backbone_forward / _backward take the per-group outputs and (backward) the layer range,
+                             v2s_heads_loss_fwd_bwd the device loss scale, v2s_adam_step and v2s_ema_update the
+                             lp_format; their narrower variants and the bf16-only cast are removed.  3: v2s_infonce_loss,
+                             v2s_preprocess_u8_patches, v2s_group.x_format (was a reserved zero field); additive to 3:
+                             v2s_group_outputs, v2s_test_attention which = 2 */
 
 /* compute modes */
 #define V2S_MODE_FP32 0 /* fp32 activations + fp32 SIMT GEMMs: the "fp32 check mode" of north_star */
@@ -107,10 +109,11 @@ typedef struct v2s_group {
   int32_t x_format;       /* 0 or 1, see x (1: bf16 / fp16 modes only) */
 } v2s_group_t;
 
-/* Per-layer outputs of one group (transformers' output_hidden_states / output_attentions).  The two calls below take an
- * array of n_groups of these, or NULL for none.  NULL (or every pointer NULL) requests nothing and costs nothing: the
- * call then launches exactly the kernels of a backbone pass without per-layer outputs.  A saved group's hidden[] must
- * be the same in its forward and its backward call. */
+/* Per-group optional inputs and outputs of the two calls below: transformers' output_hidden_states / output_attentions,
+ * the gradients w.r.t. the pixels and the attention probabilities, and masked patch tokens.  The calls take an array of
+ * n_groups of these, or NULL for none.  NULL (or every pointer NULL) requests nothing and costs nothing: the call then
+ * launches exactly the kernels of a backbone pass without them.  A saved group's hidden[] and mask must be the same in
+ * its forward and its backward call. */
 typedef struct v2s_group_outputs {
   float* hidden[V2S_LAYERS + 1];        /* out: hidden_states[l] fp32 [batch,197,192]; all 13 or none. When set, the
                                            group's residual stream lives here; a saved group's backward reads it back */
@@ -119,6 +122,25 @@ typedef struct v2s_group_outputs {
                                            dhidden[12] is v2s_group.dhidden (set one of the two).  Without dfeat and
                                            dhidden[12] the backward starts at the highest l with a gradient: the
                                            blocks above it are skipped and get no gradient */
+  float* dattn[V2S_LAYERS];             /* backward out: d loss / d attn[l], fp32 [batch,3,197,197], overwritten, 4-byte
+                                           aligned: d ctx V^T, what retain_grad() gives on transformers' attentions.
+                                           NULL entries skipped; blocks at or above the highest layer the loss reaches
+                                           (see dhidden) get nothing written.  Written by the call whose range covers l */
+  float* dpixels;                       /* backward out: d loss / d pixel_values (transformers' input gradient), fp32
+                                           [batch,3,224,224], overwritten, 16-byte aligned, x_format 0 only; written by
+                                           the call whose range ends at layer 0.  The weight gradients are those of the
+                                           call without it (same kernels, same bits) */
+  const uint8_t* mask;                  /* forward and backward in: uint8 [batch,196] patch mask (NULL: none), transformers'
+                                           bool_masked_pos of ViTModel(use_mask_token=True), the input of SimMIM-style
+                                           masked image modelling.  The forward replaces the embedding of every patch p of
+                                           image b with mask[b*196 + p] != 0 by mask_token, after the patch projection and
+                                           its bias and before the position embedding is added.  A saved group's backward
+                                           passes the forward's array; a masked backward runs over [0, 12) only.  The
+                                           patch weight and bias gradients and the image gradient come from the unmasked
+                                           patches only (the image gradient is exactly 0 on masked patches) */
+  const float* mask_token;              /* forward in: fp32 [192], 16-byte aligned, required where mask is set */
+  float* dmask_token;                   /* backward out (+=): fp32 [192], 4-byte aligned: the sum of the residual-stream
+                                           gradient of the masked (image, patch) tokens; only with weight_grads = 1 */
 } v2s_group_outputs_t;
 
 /* ViTBackbone.forward for up to 4 backbones (ref:ssp_vit2spn_tiny.py:114-118; HF
@@ -129,45 +151,12 @@ int v2s_backbone_forward(const v2s_group_t* host_groups, const v2s_group_outputs
  * [layer_lo, layer_hi) only, highest block first: [0, V2S_LAYERS) is the whole backward.  layer_hi == V2S_LAYERS starts
  * from dfeat / dhidden; layer_lo == 0 ends with the embedding gradients; the residual-stream gradient is carried between
  * calls in the workspace.  The flat gradient layout is block-contiguous, so after the call for [lo, hi) the gradients of
- * those blocks are final: a data-parallel host can all-reduce that slice while the next range computes (SURVEY 8e). */
+ * those blocks are final: a data-parallel host can all-reduce that slice while the next range computes (SURVEY 8e).
+ * weight_grads = 1: weight gradients accumulated (+=) into grads; saved groups without grads are skipped.  0: no
+ * parameter gradient is computed and grads may be NULL (frozen backbones; no deterministic scratch is used). */
 int v2s_backbone_backward(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs /* [n_groups] or NULL */,
                           int n_groups, int batch, int mode, void* workspace, int64_t workspace_bytes, int layer_hi,
-                          int layer_lo, void* stream);
-/* d loss / d pixel_values (transformers' input gradient): the backward of v2s_backbone_backward over all blocks that also
- * writes, for each group with host_dpixels[g] != NULL, the fp32 image gradient [batch,3,224,224] (overwritten, 16-byte
- * aligned; not for x_format 1 groups).  host_dpixels has n_groups entries.
- * weight_grads = 1: weight gradients accumulated exactly as v2s_backbone_backward does (same kernels, same bits);
- * 0: no parameter gradient is computed and grads may be NULL (frozen backbones; no deterministic scratch is used). */
-int v2s_backbone_input_backward(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs,
-                                float* const* host_dpixels, int weight_grads, int n_groups, int batch, int mode,
-                                void* workspace, int64_t workspace_bytes, void* stream);
-/* v2s_backbone_input_backward, plus: for every group g and block l with host_dattn[g*12+l] != NULL, the gradient of the
- * loss w.r.t. that block's attention probabilities, fp32 [batch,3,197,197] (overwritten, 4-byte aligned): d ctx V^T,
- * what retain_grad() gives on transformers' attentions.  Blocks at or above the highest layer the loss reaches (see
- * v2s_group_outputs.dhidden) get nothing written.  host_dattn has n_groups*12 entries; host_dpixels may be NULL. */
-int v2s_backbone_backward_attn_grads(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs,
-                                     float* const* host_dattn, float* const* host_dpixels, int weight_grads, int n_groups,
-                                     int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
-/* Masked patch tokens (transformers' ViTModel(use_mask_token=True) with bool_masked_pos, the input of SimMIM-style masked
- * image modelling): v2s_backbone_forward, where each group g with host_masks[g] != NULL replaces the embedding of every
- * patch p of image b with host_masks[g][b*196 + p] != 0 by the mask token, after the patch projection and its bias and
- * before the position embedding is added.  host_masks[g]: uint8 [batch,196] (device); host_mask_tokens[g]: fp32 [192]
- * (device, 16-byte aligned), required where a mask is set.  host_masks may be NULL (no group masked), as may
- * host_mask_tokens when no group is masked.  A saved group's backward must pass the same mask array. */
-int v2s_backbone_forward_masked(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs,
-                                const uint8_t* const* host_masks, const float* const* host_mask_tokens, int n_groups,
-                                int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
-/* The whole backward (blocks [0, 12)) of a forward that may have been masked: v2s_backbone_backward_attn_grads plus, per
- * group, host_masks[g] (the forward's mask array, or NULL) and host_dmask_tokens[g] (fp32 [192], 4-byte aligned, +=;
- * with weight_grads = 1 only: weight_grads = 0 computes no mask-token gradient).  d mask_token sums the residual-stream
- * gradient of the masked (image, patch) tokens; the patch weight and bias gradients and the image gradient come from
- * the unmasked patches only (the image gradient is exactly 0 on masked patches).  Every array may be NULL (n_groups
- * entries each, host_dattn n_groups*12); with all of them NULL this is v2s_backbone_backward_attn_grads.  A masked
- * group's backward over a partial layer range (v2s_backbone_backward) is refused. */
-int v2s_backbone_backward_masked(const v2s_group_t* host_groups, const v2s_group_outputs_t* host_outputs,
-                                 const uint8_t* const* host_masks, float* const* host_dmask_tokens,
-                                 float* const* host_dattn, float* const* host_dpixels, int weight_grads, int n_groups,
-                                 int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
+                          int layer_lo, int weight_grads, void* stream);
 
 /* projection_head + prediction_head on the concatenated online features and projection_head on
  * the target features (ref:ssp_vit2spn_tiny.py:153-158), fused with the loss

@@ -16,7 +16,7 @@ def _declared_symbols():
     return sorted(set(re.findall(r"\b(v2s_[a-z0-9_]+)\s*\(", text)))
 
 
-def test_library_exports_every_declared_symbol_and_abi_versions_agree():
+def test_library_exports_every_declared_symbol_and_abi_version_5_agrees():
     import vit2spn
     lib = ctypes.CDLL(vit2spn.LIB_PATH)
     syms = _declared_symbols()
@@ -24,10 +24,11 @@ def test_library_exports_every_declared_symbol_and_abi_versions_agree():
     for s in syms:
         assert hasattr(lib, s), f"{s} declared in include/vit2spn.h but not exported"
     assert set(vit2spn.EXPORTED) == set(syms), set(vit2spn.EXPORTED) ^ set(syms)
-    # 4: one entry point per operation; 3: InfoNCE, uint8 -> patch-matrix input format; 2: fp16 mode, amp entry points
-    assert lib.v2s_abi_version() == 4
+    # 5: the backbone extras are v2s_group_outputs fields; 4: one entry point per operation; 3: InfoNCE, uint8 ->
+    # patch-matrix input format; 2: fp16 mode, amp entry points
+    assert lib.v2s_abi_version() == 5
     header = open(os.path.join(ROOT, "include", "vit2spn.h")).read()
-    assert int(re.search(r"#define V2S_ABI_VERSION (\d+)", header).group(1)) == vit2spn._lib.ABI_VERSION == 4
+    assert int(re.search(r"#define V2S_ABI_VERSION (\d+)", header).group(1)) == vit2spn._lib.ABI_VERSION == 5
 
 
 def test_layout_matches_hf_parameter_order():

@@ -105,21 +105,21 @@ def test_relevance_matches_published_equations(token):
         explain.attention_relevance(attn, grads, token="first")
 
 
-def test_attn_grads_entry_point_rejects_bad_arguments():
+def test_attn_grad_outputs_reject_bad_arguments():
     from vit2spn import _lib
     B, mode = 2, _lib.MODE_FP32
     nbytes = _lib.lib.v2s_workspace_bytes(B, mode, 1, 1)
     g = _lib.Group()
     g.params, g.x, g.grads, g.slot, g.dfeat = 0x10000, 0x20000, 0x30000, 0, 0x40000
     arr = (_lib.Group * 1)(g)
-    da = (C.c_void_p * 12)()
-    da[3] = 0x100002                                  # not 4-byte aligned
-    rc = _lib.lib.v2s_backbone_backward_attn_grads(arr, None, da, None, 1, 1, B, mode, C.c_void_p(1 << 20), nbytes, None)
+    o = _lib.GroupOutputs()
+    o.dattn[3] = 0x100002                             # not 4-byte aligned
+    outs = (_lib.GroupOutputs * 1)(o)
+    rc = _lib.lib.v2s_backbone_backward(arr, outs, 1, B, mode, C.c_void_p(1 << 20), nbytes, 12, 0, 1, None)
     err = _lib.lib.v2s_last_error().decode()
-    assert rc != 0 and "dattn[3]" in err and "aligned" in err, err
-    rc = _lib.lib.v2s_backbone_backward_attn_grads(arr, None, None, None, 1, 1, B, mode, C.c_void_p(1 << 20), nbytes, None)
-    assert rc != 0 and "null" in _lib.lib.v2s_last_error().decode()
-    da[3] = 0x100004
-    dp = (C.c_void_p * 1)(0x200004)                   # the image gradient keeps its 16-byte rule
-    rc = _lib.lib.v2s_backbone_backward_attn_grads(arr, None, da, dp, 1, 1, B, mode, C.c_void_p(1 << 20), nbytes, None)
-    assert rc != 0 and "dpixels[0]" in _lib.lib.v2s_last_error().decode()
+    assert rc != 0 and "group 0: dattn[3]" in err and "aligned" in err, err
+    outs[0].dattn[3] = 0x100004
+    outs[0].dpixels = 0x200004                        # the image gradient keeps its 16-byte rule
+    rc = _lib.lib.v2s_backbone_backward(arr, outs, 1, B, mode, C.c_void_p(1 << 20), nbytes, 12, 0, 1, None)
+    err = _lib.lib.v2s_last_error().decode()
+    assert rc != 0 and "group 0: dpixels" in err and "aligned" in err, err

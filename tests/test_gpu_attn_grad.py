@@ -1,5 +1,5 @@
 """GPU: gradients w.r.t. the attention probabilities (retain_grad() on ViTModel's attentions,
-v2s_backbone_backward_attn_grads).  The dP = d ctx V^T operator against float64; the retained .grad of all 12 blocks
+v2s_group_outputs.dattn of v2s_backbone_backward).  The dP = d ctx V^T operator against float64; the retained .grad of all 12 blocks
 against the oracle (fp32 check mode; bf16 / fp16 against the fp32 oracle and its rounding model); transformers' None
 pattern; weight gradients and reproducibility; the frozen backbone with pixel gradients; launch counts; the relevance map.
 

@@ -1,7 +1,8 @@
-"""GPU: gradients w.r.t. pixel_values (v2s_backbone_input_backward).  fp32 check mode and bf16 / fp16 against the oracle's
-autograd (16-bit modes against its rounding model), a frozen model computing no parameter gradient, the joint backward
-leaving the weight gradients bit-identical, the launch counts, the other entry points (FineTunedModel, DualStreamNetwork,
-an intermediate hidden state, an integrated-gradients chain) and the image-gradient GEMM operator.
+"""GPU: gradients w.r.t. pixel_values (v2s_group_outputs.dpixels of v2s_backbone_backward).  fp32 check mode and bf16 /
+fp16 against the oracle's autograd (16-bit modes against its rounding model), a frozen model computing no parameter
+gradient, the joint backward leaving the weight gradients bit-identical, a backward split into two layer ranges, the
+launch counts, the other entry points (FineTunedModel, DualStreamNetwork, an intermediate hidden state, an
+integrated-gradients chain) and the image-gradient GEMM operator.
 
 Measured errors go to $V2S_INPUT_GRAD_REPORT (JSON) when set."""
 import json
@@ -148,6 +149,45 @@ def test_joint_backward_keeps_weight_gradients_bit_identical():
             assert not bad, bad[:8]
         assert torch.equal(runs[1][1], runs[2][1])           # the pixel gradient is reproducible too
         assert _rel(runs[1][1], _oracle_dx(p, x.cpu(), up.cpu(), torch.bfloat16)) <= 2e-2
+    finally:
+        torch.use_deterministic_algorithms(prev, warn_only=warn)
+
+
+def test_split_range_backward_with_pixel_and_attention_gradients():
+    """A saved group's backward with dpixels and all 12 dattn[] set, issued as [6, 12) then [0, 6): the image gradient and
+    every attention-probability gradient are those of one [0, 12) call, bit for bit, and so are the weight gradients
+    under torch.use_deterministic_algorithms."""
+    from vit2spn import _lib, modules as M
+    prev, warn = torch.are_deterministic_algorithms_enabled(), torch.is_deterministic_algorithms_warn_only_enabled()
+    torch.use_deterministic_algorithms(True)
+    try:
+        B = 4
+        m = _model(_state(), "bf16")
+        store, mode = m._store, m._mode()
+        store.ensure()
+        x, up = _images(B, 13).to(DEV), _upstream(B, 13).to(DEV)
+        hid = torch.empty(B, 197, 192, device=DEV)
+        ws = M._new_workspace(DEV, B, mode, 1, 1)
+        runs = []
+        for ranges in (((12, 0),), ((12, 6), (6, 0))):
+            M._run_forward([M._group(store, mode, x, 0, hidden=hid)], B, mode, ws)
+            grads = torch.zeros(store.numel, device=DEV)
+            dx = torch.full((B, 3, 224, 224), float("nan"), device=DEV)
+            dattn = [torch.full((B, 3, 197, 197), float("nan"), device=DEV) for _ in range(12)]
+            o = _lib.GroupOutputs()
+            o.dpixels = dx.data_ptr()
+            for l, t in enumerate(dattn):
+                o.dattn[l] = t.data_ptr()
+            gb = M._group(store, mode, x, 0, grads=grads, dhidden=up)
+            for hi, lo in ranges:
+                M._run_backward([gb], B, mode, ws, [o], hi, lo)
+            runs.append((grads, dx, dattn))
+        _flag_clear()
+        (g1, dx1, da1), (g2, dx2, da2) = runs
+        assert not dx1.isnan().any() and not any(t.isnan().any() for t in da1)
+        assert torch.equal(dx1, dx2)
+        assert all(torch.equal(a, b) for a, b in zip(da1, da2))
+        assert torch.count_nonzero(g1) > 0 and torch.equal(g1, g2)
     finally:
         torch.use_deterministic_algorithms(prev, warn_only=warn)
 

@@ -377,8 +377,8 @@ def test_mask_on_cpu_is_refused():
         m(x, bool_masked_pos=torch.zeros(2, 196, dtype=torch.bool))
 
 
-def test_backward_with_another_mask_or_a_partial_range_is_refused():
-    from vit2spn import modules as M
+def test_backward_outputs_with_another_mask_or_a_partial_range_are_refused():
+    from vit2spn import _lib, modules as M
     p, token = _state(), _token()
     B = 2
     m = _model(p, "bf16", token)
@@ -391,16 +391,24 @@ def test_backward_with_another_mask_or_a_partial_range_is_refused():
     hid = torch.empty(B, 197, 192, device=DEV)
     tok = m.embeddings.mask_token.detach().reshape(192)
     g = M._group(store, mode, x, 0, hidden=hid)
-    M._run_forward_masked([g], B, mode, ws, [mask], [tok])
+
+    def outputs(patch_mask, dtok=None):
+        o = _lib.GroupOutputs()
+        o.mask, o.mask_token = patch_mask.data_ptr(), tok.data_ptr()
+        o.dmask_token = dtok.data_ptr() if dtok is not None else None
+        return [o]
+    M._run_forward([g], B, mode, ws, outputs(mask))
     dh = torch.ones(B, 197, 192, device=DEV)
     gb = M._group(store, mode, x, 0, grads=store.grads(), dhidden=dh)
     with pytest.raises(RuntimeError, match="patch mask"):
-        M._run_masked_backward([gb], B, mode, ws, [other], [None], [None], True)
+        M._run_backward([gb], B, mode, ws, outputs(other))
     with pytest.raises(RuntimeError, match="patch mask"):
         M._run_backward([gb], B, mode, ws, None, 12, 6)          # a partial range after a masked forward
     with pytest.raises(RuntimeError, match="patch mask"):
-        M._run_input_backward([gb], B, mode, ws, [None], True)   # the unmasked entry point
+        M._run_backward([gb], B, mode, ws)                       # no mask
+    with pytest.raises(RuntimeError, match="whole range"):
+        M._run_backward([gb], B, mode, ws, outputs(mask), 12, 6)  # the forward's own mask over a partial range
     dtok = torch.zeros(192, device=DEV)
-    M._run_masked_backward([gb], B, mode, ws, [mask], [dtok], [None], True)   # the forward's own mask: accepted
+    M._run_backward([gb], B, mode, ws, outputs(mask, dtok))      # the forward's own mask: accepted
     _flag_clear()
     assert torch.count_nonzero(dtok) > 0

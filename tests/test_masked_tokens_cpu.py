@@ -182,7 +182,7 @@ def test_forward_rejects_bad_masks():
         model(x, bool_masked_pos=torch.zeros(2, 196))
 
 
-def test_masked_entry_points_reject_bad_arguments():
+def test_mask_outputs_reject_bad_arguments():
     from vit2spn import _lib
     B, mode = 2, _lib.MODE_FP32
     nbytes = _lib.lib.v2s_workspace_bytes(B, mode, 1, 1)
@@ -190,32 +190,33 @@ def test_masked_entry_points_reject_bad_arguments():
     g.params, g.x, g.grads, g.slot, g.dfeat = 0x10000, 0x20000, 0x30000, 0, 0x40000
     arr = (_lib.Group * 1)(g)
     ws = C.c_void_p(1 << 20)
-    masks = (C.c_void_p * 1)(0x50000)
-    rc = _lib.lib.v2s_backbone_forward_masked(arr, None, masks, None, 1, B, mode, ws, nbytes, None)
+    o = _lib.GroupOutputs()
+    o.mask = 0x50000
+    outs = (_lib.GroupOutputs * 1)(o)
+    rc = _lib.lib.v2s_backbone_forward(arr, outs, 1, B, mode, ws, nbytes, None)
     err = _lib.lib.v2s_last_error().decode()
-    assert rc != 0 and "no mask token" in err, err
-    toks = (C.c_void_p * 1)(None)
-    rc = _lib.lib.v2s_backbone_forward_masked(arr, None, masks, toks, 1, B, mode, ws, nbytes, None)
-    assert rc != 0 and "no mask token" in _lib.lib.v2s_last_error().decode()
-    toks[0] = 0x60008                                 # fp32 [192] read as float4: 16-byte rule
-    rc = _lib.lib.v2s_backbone_forward_masked(arr, None, masks, toks, 1, B, mode, ws, nbytes, None)
+    assert rc != 0 and "group 0 has a mask but no mask_token" in err, err
+    outs[0].mask_token = 0x60008                      # fp32 [192] read as float4: 16-byte rule
+    rc = _lib.lib.v2s_backbone_forward(arr, outs, 1, B, mode, ws, nbytes, None)
     err = _lib.lib.v2s_last_error().decode()
-    assert rc != 0 and "mask_tokens[0]" in err and "aligned" in err, err
-    rc = _lib.lib.v2s_backbone_forward_masked(None, None, masks, toks, 1, B, mode, ws, nbytes, None)
+    assert rc != 0 and "group 0: mask_token" in err and "aligned" in err, err
+    rc = _lib.lib.v2s_backbone_forward(None, outs, 1, B, mode, ws, nbytes, None)
     assert rc != 0 and "null" in _lib.lib.v2s_last_error().decode()
 
-    dt = (C.c_void_p * 1)(0x70002)
-    rc = _lib.lib.v2s_backbone_backward_masked(arr, None, masks, dt, None, None, 1, 1, B, mode, ws, nbytes, None)
+    o = _lib.GroupOutputs()
+    o.mask, o.dmask_token = 0x50000, 0x70002
+    outs = (_lib.GroupOutputs * 1)(o)
+    rc = _lib.lib.v2s_backbone_backward(arr, outs, 1, B, mode, ws, nbytes, 12, 0, 1, None)
     err = _lib.lib.v2s_last_error().decode()
-    assert rc != 0 and "dmask_tokens[0]" in err and "aligned" in err, err
-    dt[0] = 0x70004
-    dp = (C.c_void_p * 1)(0x200004)
-    rc = _lib.lib.v2s_backbone_backward_masked(arr, None, masks, dt, None, dp, 1, 1, B, mode, ws, nbytes, None)
-    assert rc != 0 and "dpixels[0]" in _lib.lib.v2s_last_error().decode()
-    da = (C.c_void_p * 12)()
-    da[5] = 0x100002
-    rc = _lib.lib.v2s_backbone_backward_masked(arr, None, masks, dt, da, None, 1, 1, B, mode, ws, nbytes, None)
+    assert rc != 0 and "group 0: dmask_token" in err and "aligned" in err, err
+    outs[0].dmask_token = 0x70004
+    outs[0].dpixels = 0x200004
+    rc = _lib.lib.v2s_backbone_backward(arr, outs, 1, B, mode, ws, nbytes, 12, 0, 1, None)
+    assert rc != 0 and "group 0: dpixels" in _lib.lib.v2s_last_error().decode()
+    outs[0].dpixels = None
+    outs[0].dattn[5] = 0x100002
+    rc = _lib.lib.v2s_backbone_backward(arr, outs, 1, B, mode, ws, nbytes, 12, 0, 1, None)
     err = _lib.lib.v2s_last_error().decode()
-    assert rc != 0 and "dattn[5]" in err and "aligned" in err, err
-    rc = _lib.lib.v2s_backbone_backward_masked(None, None, masks, dt, None, None, 1, 1, B, mode, ws, nbytes, None)
+    assert rc != 0 and "group 0: dattn[5]" in err and "aligned" in err, err
+    rc = _lib.lib.v2s_backbone_backward(None, outs, 1, B, mode, ws, nbytes, 12, 0, 1, None)
     assert rc != 0 and "null" in _lib.lib.v2s_last_error().decode()

@@ -67,13 +67,13 @@ def _call(fn, outputs, *, slot=0, dhidden=None, dfeat=None, layer_hi=12, layer_l
     if fn == "forward":
         rc = _lib.lib.v2s_backbone_forward(arr, outs, 1, B, mode, C.c_void_p(1 << 20), nbytes, None)
     else:
-        rc = _lib.lib.v2s_backbone_backward(arr, outs, 1, B, mode, C.c_void_p(1 << 20), nbytes, layer_hi, layer_lo, None)
+        rc = _lib.lib.v2s_backbone_backward(arr, outs, 1, B, mode, C.c_void_p(1 << 20), nbytes, layer_hi, layer_lo, 1, None)
     return rc, _lib.lib.v2s_last_error().decode()
 
 
-def test_backbone_entry_points_reject_malformed_outputs_and_ranges():
+def test_backbone_calls_reject_malformed_outputs_and_ranges():
     from vit2spn import _lib
-    assert C.sizeof(_lib.GroupOutputs) == (13 + 12 + 13) * 8
+    assert C.sizeof(_lib.GroupOutputs) == (13 + 12 + 13 + 12 + 4) * 8
     o = _lib.GroupOutputs()
     for i in range(12):                       # 12 of 13 hidden states
         o.hidden[i] = 0x100000 * (i + 1)

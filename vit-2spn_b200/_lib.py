@@ -17,7 +17,7 @@ MODE_FP16 = 2
 LP_BF16 = 0
 LP_FP16 = 1
 MAX_GROUPS = 4
-ABI_VERSION = 4      # V2S_ABI_VERSION of include/vit2spn.h that the signatures below bind
+ABI_VERSION = 5      # V2S_ABI_VERSION of include/vit2spn.h that the signatures below bind
 
 if not os.path.exists(LIB_PATH):
     raise ImportError(
@@ -43,8 +43,11 @@ class Group(C.Structure):
 
 
 class GroupOutputs(C.Structure):
-    """struct v2s_group_outputs (include/vit2spn.h): per-layer outputs / gradients of one group."""
-    _fields_ = [("hidden", C.c_void_p * 13), ("attn", C.c_void_p * 12), ("dhidden", C.c_void_p * 13)]
+    """struct v2s_group_outputs (include/vit2spn.h): per-layer outputs / gradients, pixel gradient and patch mask of one
+    group."""
+    _fields_ = [("hidden", C.c_void_p * 13), ("attn", C.c_void_p * 12), ("dhidden", C.c_void_p * 13),
+                ("dattn", C.c_void_p * 12), ("dpixels", C.c_void_p), ("mask", C.c_void_p), ("mask_token", C.c_void_p),
+                ("dmask_token", C.c_void_p)]
 
 
 class Range(C.Structure):
@@ -66,16 +69,8 @@ _SIGS = {
     "v2s_workspace_bytes": (_i64, [_i, _i, _i, _i]),
     "v2s_set_deterministic": (C.c_int, [_i]),
     "v2s_backbone_forward": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), _i, _i, _i, _vp, _i64, _vp]),
-    "v2s_backbone_backward": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), _i, _i, _i, _vp, _i64, _i, _i,
+    "v2s_backbone_backward": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), _i, _i, _i, _vp, _i64, _i, _i, _i,
                                         _vp]),
-    "v2s_backbone_input_backward": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), C.POINTER(_vp), _i, _i, _i, _i,
-                                              _vp, _i64, _vp]),
-    "v2s_backbone_backward_attn_grads": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), C.POINTER(_vp),
-                                                   C.POINTER(_vp), _i, _i, _i, _i, _vp, _i64, _vp]),
-    "v2s_backbone_forward_masked": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), C.POINTER(_vp), C.POINTER(_vp),
-                                              _i, _i, _i, _vp, _i64, _vp]),
-    "v2s_backbone_backward_masked": (C.c_int, [C.POINTER(Group), C.POINTER(GroupOutputs), C.POINTER(_vp), C.POINTER(_vp),
-                                               C.POINTER(_vp), C.POINTER(_vp), _i, _i, _i, _i, _vp, _i64, _vp]),
     "v2s_heads_loss_fwd_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _f, _vp, _i,
                                          _vp, _i64, _vp]),
     "v2s_heads_forward": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _vp]),

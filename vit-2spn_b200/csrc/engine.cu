@@ -275,18 +275,34 @@ int add_hidden_grads(int k, const float* const* dh, float* const* dx, void* cons
   return launch_residual_grad_add(a, o, lp, cs, n, B, at, s, det);
 }
 
-// v2s_group_outputs checks shared by forward and backward: hidden / attn all or none, 16-byte aligned hidden states
-int check_outputs(const v2s_group_outputs_t* o, int g, const char* what) {
+// v2s_group_outputs checks shared by forward and backward: hidden / attn all or none, the alignments the kernels read and
+// write with; the forward's mask needs its token, the backward's image gradient an image input
+int check_outputs(const v2s_group_outputs_t* o, const v2s_group_t& gr, int g, bool backward) {
   if (!o) return 0;
+  const char* what = backward ? "backbone_backward" : "backbone_forward";
+  auto misaligned = [](const void* q, uintptr_t bytes) { return (reinterpret_cast<uintptr_t>(q) & (bytes - 1)) != 0; };
   int nh = 0, na = 0;
   for (int l = 0; l <= NL; ++l) {
     if (!o->hidden[l]) continue;
     ++nh;
-    if (reinterpret_cast<uintptr_t>(o->hidden[l]) & 15) { set_error("%s: group %d: hidden[%d] is not 16-byte aligned", what, g, l); return 1; }
+    if (misaligned(o->hidden[l], 16)) { set_error("%s: group %d: hidden[%d] is not 16-byte aligned", what, g, l); return 1; }
   }
   for (int l = 0; l < NL; ++l) na += o->attn[l] ? 1 : 0;
   if (nh != 0 && nh != NL + 1) { set_error("%s: group %d: %d of the 13 hidden[] set (all or none)", what, g, nh); return 1; }
   if (na != 0 && na != NL) { set_error("%s: group %d: %d of the 12 attn[] set (all or none)", what, g, na); return 1; }
+  if (!backward) {
+    if (o->mask && !o->mask_token) { set_error("%s: group %d has a mask but no mask_token", what, g); return 1; }
+    if (o->mask && misaligned(o->mask_token, 16)) { set_error("%s: group %d: mask_token is not 16-byte aligned", what, g); return 1; }
+    return 0;
+  }
+  for (int l = 0; l < NL; ++l)
+    if (misaligned(o->dattn[l], 4)) { set_error("%s: group %d: dattn[%d] is not 4-byte aligned", what, g, l); return 1; }
+  if (misaligned(o->dpixels, 16)) { set_error("%s: group %d: dpixels is not 16-byte aligned", what, g); return 1; }
+  if (o->dpixels && gr.x_format != 0) {
+    set_error("%s: group %d: no image gradient (dpixels) for 16-bit patch-row inputs (x_format 1)", what, g);
+    return 1;
+  }
+  if (misaligned(o->dmask_token, 4)) { set_error("%s: group %d: dmask_token is not 4-byte aligned", what, g); return 1; }
   return 0;
 }
 
@@ -321,11 +337,8 @@ int wgrad_split(int64_t rows) {
 // =============================================================================================
 // backbone forward
 // =============================================================================================
-// masks / mask_tokens (NULL, or one entry per group): the uint8 [B,196] patch mask of each group (NULL entry: none) and its
-// fp32 [192] mask token, which replaces each masked patch embedding before the position embeddings are added
 static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_t* outs, int G, int B, int mode,
-                                 void* ws, int64_t ws_bytes, cudaStream_t st, const uint8_t* const* masks = nullptr,
-                                 const float* const* mask_tokens = nullptr) {
+                                 void* ws, int64_t ws_bytes, cudaStream_t st) {
   if (mode < V2S_MODE_FP32 || mode > V2S_MODE_FP16) { set_error("bad compute mode %d", mode); return 1; }
   if (G < 1 || G > MAXG) { set_error("backbone_forward: 1..4 groups"); return 1; }
   if (B < 1) { set_error("backbone_forward: batch must be >= 1"); return 1; }
@@ -342,14 +355,20 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
       set_error("backbone_forward: group %d: x_format %d (1 = 16-bit patch rows, 16-bit modes only)", g, gs[g].x_format);
       return 1;
     }
-    V2S_TRY(check_outputs(outs ? &outs[g] : nullptr, g, "backbone_forward"));
+    V2S_TRY(check_outputs(outs ? &outs[g] : nullptr, gs[g], g, false));
   }
   const int64_t M = p.M, MP = p.MP;
   // hidden_states[0..12] / attention probabilities requested by group g (NULL / false: none)
   auto hid = [&](int g) -> float* const* { return outs && outs[g].hidden[0] ? outs[g].hidden : nullptr; };
   auto want_attn = [&](int g) { return outs && outs[g].attn[0]; };
-  for (int g = 0; g < G; ++g)
-    if (gs[g].slot >= 0) record_hidden(ws, gs[g].slot, hid(g) ? hid(g)[0] : nullptr, masks ? masks[g] : nullptr);
+  // the uint8 [B,196] patch mask of each group (NULL: none) and its fp32 [192] mask token, which replaces each masked
+  // patch embedding before the position embeddings are added
+  const uint8_t* mask[MAXG]; const float* mask_token[MAXG];
+  for (int g = 0; g < G; ++g) {
+    mask[g] = outs ? outs[g].mask : nullptr;
+    mask_token[g] = outs ? outs[g].mask_token : nullptr;
+    if (gs[g].slot >= 0) record_hidden(ws, gs[g].slot, hid(g) ? hid(g)[0] : nullptr, mask[g]);
+  }
 
   // ---- buffer resolution ----
   auto saved = [&](int g) { return gs[g].slot >= 0; };
@@ -394,8 +413,8 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
     }
     V2S_TRY(run_gemm(d, at, at, 0, st, prof::C_PATCH));
     // masked patch rows take mask_token + pos in the kernel that writes the token rows
-    if (two_pass) V2S_TRY(launch_assemble_tokens(pp, tok, x_cur, G, B, st, masks, mask_tokens));
-    else V2S_TRY(launch_cls_rows(pp, x_cur, G, B, st, masks, mask_tokens));
+    if (two_pass) V2S_TRY(launch_assemble_tokens(pp, tok, x_cur, G, B, st, mask, mask_token));
+    else V2S_TRY(launch_cls_rows(pp, x_cur, G, B, st, mask, mask_token));
   }
 
   // ---- 12 pre-LN blocks ----
@@ -550,39 +569,32 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
 // layers [layer_lo, layer_hi) in descending order; layer_hi == NL starts from the feature / hidden-state gradient,
 // layer_lo == 0 finishes with the embedding gradients.  Between two calls the residual-stream gradient lives in the
 // workspace, so a full backward may be issued in several ranges (gradient all-reduce overlapped per range).
-// dpix_in (whole backward only; NULL or one entry per input group): the groups with dpix_in[g] != NULL also get the fp32
-// image gradient [B,3,224,224] (overwritten).  weight_grads = 0: no parameter gradient at all -- no weight-gradient GEMM,
-// no bias / LayerNorm-parameter / embedding column sum -- and grads may be NULL.
-// masks_in / dmask_in (whole backward only; NULL or one entry per input group): the patch mask the group's forward used,
-// and, with weight gradients, d mask_token fp32 [192] (+=, NULL entry: not wanted).  A masked group's masked patch rows
-// give no gradient to the patch weight, the patch bias or the pixels.
+// weight_grads = 0: no parameter gradient at all -- no weight-gradient GEMM, no bias / LayerNorm-parameter / embedding
+// column sum -- and grads may be NULL.  A masked group's masked patch rows give no gradient to the patch weight, the
+// patch bias or the pixels.
 static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outputs_t* outs_in, int G_in, int B, int mode,
-                                  void* ws, int64_t ws_bytes, cudaStream_t st, int layer_hi, int layer_lo,
-                                  float* const* dpix_in, int weight_grads, float* const* dattn_in = nullptr,
-                                  const uint8_t* const* masks_in = nullptr, float* const* dmask_in = nullptr) {
+                                  void* ws, int64_t ws_bytes, cudaStream_t st, int layer_hi, int layer_lo, int weight_grads) {
   if (layer_lo < 0 || layer_hi > NL || layer_lo >= layer_hi) { set_error("backbone_backward: bad layer range [%d, %d)", layer_lo, layer_hi); return 1; }
-  if (any_mask(masks_in, G_in) && (layer_lo != 0 || layer_hi != NL)) {
+  bool masked_in = false;
+  for (int i = 0; i < G_in && i < MAXG; ++i) {
+    V2S_TRY(check_outputs(outs_in ? &outs_in[i] : nullptr, gs_in[i], i, true));
+    masked_in = masked_in || (outs_in && outs_in[i].mask);
+  }
+  if (masked_in && (layer_lo != 0 || layer_hi != NL)) {
     set_error("backbone_backward: a masked backward covers the whole range [0, %d), not [%d, %d)", NL, layer_lo, layer_hi);
     return 1;
   }
   // keep only the groups that saved activations and want gradients
   v2s_group_t gs[MAXG];
   const v2s_group_outputs_t* os[MAXG];
-  float* dpix[MAXG];
-  float* const* dattn[MAXG];   // per group: NL gradients w.r.t. the attention probabilities (NULL entries skipped), or NULL
-  const uint8_t* mask[MAXG]; float* dmask[MAXG];
+  float* dpix[MAXG]; const uint8_t* mask[MAXG]; float* dmask[MAXG];
   int G = 0;
   for (int i = 0; i < G_in && i < MAXG; ++i)
     if (gs_in[i].slot >= 0 && (gs_in[i].grads || !weight_grads)) {
       os[G] = outs_in ? &outs_in[i] : nullptr;
-      dpix[G] = dpix_in ? dpix_in[i] : nullptr;
-      dattn[G] = dattn_in ? dattn_in + (int64_t)i * NL : nullptr;
-      mask[G] = masks_in ? masks_in[i] : nullptr;
-      dmask[G] = dmask_in && weight_grads ? dmask_in[i] : nullptr;
-      if (dpix[G] && gs_in[i].x_format != 0) {
-        set_error("backbone_input_backward: group %d: no image gradient for 16-bit patch-row inputs (x_format 1)", i);
-        return 1;
-      }
+      dpix[G] = os[G] ? os[G]->dpixels : nullptr;
+      mask[G] = os[G] ? os[G]->mask : nullptr;
+      dmask[G] = os[G] && weight_grads ? os[G]->dmask_token : nullptr;
       gs[G++] = gs_in[i];
     }
   if (G == 0) { set_error("backbone_backward: no group with slot >= 0 and grads"); return 1; }
@@ -591,7 +603,6 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
   float* const* hid[MAXG]; const float* dh_top[MAXG]; int top[MAXG];
   int S = -1;              // where the backward starts: the blocks [S, NL) are skipped
   for (int g = 0; g < G; ++g) {
-    V2S_TRY(check_outputs(os[g], g, "backbone_backward"));
     hid[g] = os[g] && os[g]->hidden[0] ? os[g]->hidden : nullptr;
     const HiddenRec* rec = find_hidden(ws, gs[g].slot);
     if (rec && rec->h0 != (hid[g] ? hid[g][0] : nullptr)) {
@@ -600,7 +611,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     }
     if (rec && rec->mask != mask[g]) {
       set_error("backbone_backward: group %d: the patch mask (%s) differs from the forward that filled stash slot %d (%s); "
-                "a masked forward's backward is v2s_backbone_backward_masked, over the whole range", g,
+                "a masked forward's backward passes the same outputs.mask, over the whole range", g,
                 mask[g] ? "given" : "none", gs[g].slot, rec->mask ? "masked" : "unmasked");
       return 1;
     }
@@ -800,7 +811,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       // d loss / d probabilities = d ctx V^T, while `tmp` still holds d ctx; before the wgrad and its late-wait partner
       const void *aq[MAXG], *ad[MAXG]; float* dp[MAXG]; int n = 0;
       for (int g = 0; g < G; ++g)
-        if (dattn[g] && dattn[g][l]) { aq[n] = qkv[g]; ad[n] = tmp[g]; dp[n] = dattn[g][l]; ++n; }
+        if (os[g] && os[g]->dattn[l]) { aq[n] = qkv[g]; ad[n] = tmp[g]; dp[n] = os[g]->dattn[l]; ++n; }
       if (n) V2S_TRY(launch_attention_dprobs(aq, ad, dp, n, B, at, st));
     }
     if (merged)        // dWo [192,192] (its gradient dxlp is only overwritten by LN1-bwd below) with dWqkv [576,192], d b_qkv
@@ -1074,81 +1085,11 @@ int v2s_backbone_forward(const v2s_group_t* groups, const v2s_group_outputs_t* o
 }
 
 int v2s_backbone_backward(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, int n_groups, int batch,
-                          int mode, void* workspace, int64_t workspace_bytes, int layer_hi, int layer_lo, void* stream) {
+                          int mode, void* workspace, int64_t workspace_bytes, int layer_hi, int layer_lo, int weight_grads,
+                          void* stream) {
   if (!groups) { set_error("null groups"); return 1; }
   return backbone_backward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
-                                layer_hi, layer_lo, nullptr, 1);
-}
-
-int v2s_backbone_input_backward(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, float* const* dpixels,
-                                int weight_grads, int n_groups, int batch, int mode, void* workspace, int64_t workspace_bytes,
-                                void* stream) {
-  if (!groups || !dpixels) { set_error("backbone_input_backward: null groups / dpixels"); return 1; }
-  for (int g = 0; g < n_groups && g < MAXG; ++g)
-    if (dpixels[g] && (reinterpret_cast<uintptr_t>(dpixels[g]) & 15)) {
-      set_error("backbone_input_backward: dpixels[%d] is not 16-byte aligned", g);
-      return 1;
-    }
-  return backbone_backward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
-                                NL, 0, dpixels, weight_grads ? 1 : 0);
-}
-
-int v2s_backbone_backward_attn_grads(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, float* const* dattn,
-                                     float* const* dpixels, int weight_grads, int n_groups, int batch, int mode,
-                                     void* workspace, int64_t workspace_bytes, void* stream) {
-  if (!groups || !dattn) { set_error("backbone_backward_attn_grads: null groups / dattn"); return 1; }
-  for (int g = 0; g < n_groups && g < MAXG; ++g) {
-    for (int l = 0; l < NL; ++l)
-      if (reinterpret_cast<uintptr_t>(dattn[g * NL + l]) & 3) {
-        set_error("backbone_backward_attn_grads: dattn[%d] (group %d, block %d) is not 4-byte aligned", g * NL + l, g, l);
-        return 1;
-      }
-    if (dpixels && (reinterpret_cast<uintptr_t>(dpixels[g]) & 15)) {
-      set_error("backbone_backward_attn_grads: dpixels[%d] is not 16-byte aligned", g);
-      return 1;
-    }
-  }
-  return backbone_backward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
-                                NL, 0, dpixels, weight_grads ? 1 : 0, dattn);
-}
-
-int v2s_backbone_forward_masked(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, const uint8_t* const* masks,
-                                const float* const* mask_tokens, int n_groups, int batch, int mode, void* workspace,
-                                int64_t workspace_bytes, void* stream) {
-  if (!groups) { set_error("backbone_forward_masked: null groups"); return 1; }
-  for (int g = 0; masks && g < n_groups && g < MAXG; ++g) {
-    if (!masks[g]) continue;
-    if (!mask_tokens || !mask_tokens[g]) { set_error("backbone_forward_masked: group %d has a mask but no mask token", g); return 1; }
-    if (reinterpret_cast<uintptr_t>(mask_tokens[g]) & 15) {
-      set_error("backbone_forward_masked: mask_tokens[%d] is not 16-byte aligned", g);
-      return 1;
-    }
-  }
-  return backbone_forward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
-                               masks, mask_tokens);
-}
-
-int v2s_backbone_backward_masked(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, const uint8_t* const* masks,
-                                 float* const* dmask_tokens, float* const* dattn, float* const* dpixels, int weight_grads,
-                                 int n_groups, int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream) {
-  if (!groups) { set_error("backbone_backward_masked: null groups"); return 1; }
-  for (int g = 0; g < n_groups && g < MAXG; ++g) {
-    for (int l = 0; dattn && l < NL; ++l)
-      if (reinterpret_cast<uintptr_t>(dattn[g * NL + l]) & 3) {
-        set_error("backbone_backward_masked: dattn[%d] (group %d, block %d) is not 4-byte aligned", g * NL + l, g, l);
-        return 1;
-      }
-    if (dpixels && (reinterpret_cast<uintptr_t>(dpixels[g]) & 15)) {
-      set_error("backbone_backward_masked: dpixels[%d] is not 16-byte aligned", g);
-      return 1;
-    }
-    if (dmask_tokens && (reinterpret_cast<uintptr_t>(dmask_tokens[g]) & 3)) {
-      set_error("backbone_backward_masked: dmask_tokens[%d] is not 4-byte aligned", g);
-      return 1;
-    }
-  }
-  return backbone_backward_impl(groups, outputs, n_groups, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream,
-                                NL, 0, dpixels, weight_grads ? 1 : 0, dattn, masks, dmask_tokens);
+                                layer_hi, layer_lo, weight_grads ? 1 : 0);
 }
 
 int v2s_heads_loss_fwd_bwd(const float* head_params, float* head_grads, const float* feat_online,

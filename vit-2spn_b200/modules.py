@@ -288,58 +288,14 @@ def _run_forward(groups, batch, mode, ws, outputs=None):
                                    C.c_void_p(base), nbytes, stream_ptr()), "backbone_forward")
 
 
-def _run_backward(groups, batch, mode, ws, outputs=None, layer_hi=12, layer_lo=0):
-    """Backward over blocks [layer_lo, layer_hi), highest first; the default range is the whole backward."""
+def _run_backward(groups, batch, mode, ws, outputs=None, layer_hi=12, layer_lo=0, weight_grads=True):
+    """Backward over blocks [layer_lo, layer_hi), highest first; the default range is the whole backward.
+    weight_grads False computes no parameter gradient at all (the groups' grads may be None)."""
     arr = (Group * len(groups))(*groups)
     base, nbytes = _aligned(ws)
     check(lib.v2s_backbone_backward(arr, _outputs_array(outputs, len(groups)), len(groups), batch, mode,
-                                    C.c_void_p(base), nbytes, int(layer_hi), int(layer_lo), stream_ptr()),
-          "backbone_backward")
-
-
-def _run_input_backward(groups, batch, mode, ws, dpixels, weight_grads, outputs=None, attn_grads=None):
-    """The whole backward, plus the fp32 image gradient of each group whose ``dpixels`` entry is a tensor (None: none);
-    weight_grads False computes no parameter gradient at all (the groups' grads may be None).  ``attn_grads``: per group
-    12 fp32 [B,3,197,197] tensors (or None entries) that receive the gradients w.r.t. the attention probabilities;
-    ``dpixels`` may then be None."""
-    arr = (Group * len(groups))(*groups)
-    dp = (C.c_void_p * len(groups))(*[t.data_ptr() if t is not None else None for t in dpixels]) if dpixels else None
-    base, nbytes = _aligned(ws)
-    if attn_grads is None:
-        check(lib.v2s_backbone_input_backward(arr, _outputs_array(outputs, len(groups)), dp, int(bool(weight_grads)),
-                                              len(groups), batch, mode, C.c_void_p(base), nbytes, stream_ptr()),
-              "backbone_input_backward")
-        return
-    da = (C.c_void_p * (12 * len(groups)))(*[t.data_ptr() if t is not None else None for ts in attn_grads for t in ts])
-    check(lib.v2s_backbone_backward_attn_grads(arr, _outputs_array(outputs, len(groups)), da, dp, int(bool(weight_grads)),
-                                               len(groups), batch, mode, C.c_void_p(base), nbytes, stream_ptr()),
-          "backbone_backward_attn_grads")
-
-
-def _run_forward_masked(groups, batch, mode, ws, masks, mask_tokens, outputs=None):
-    """``_run_forward`` with per-group patch masks (uint8 [B,196] tensors or None) and their fp32 mask tokens."""
-    arr = (Group * len(groups))(*groups)
-    mk = (C.c_void_p * len(groups))(*[t.data_ptr() if t is not None else None for t in masks])
-    tk = (C.c_void_p * len(groups))(*[t.data_ptr() if t is not None else None for t in mask_tokens])
-    base, nbytes = _aligned(ws)
-    check(lib.v2s_backbone_forward_masked(arr, _outputs_array(outputs, len(groups)), mk, tk, len(groups), batch, mode,
-                                          C.c_void_p(base), nbytes, stream_ptr()), "backbone_forward_masked")
-
-
-def _run_masked_backward(groups, batch, mode, ws, masks, dmask_tokens, dpixels, weight_grads, outputs=None,
-                         attn_grads=None):
-    """The whole backward of a masked forward: ``_run_input_backward`` plus the masks the forward used and, per group, an
-    fp32 [192] tensor (or None) that receives d mask_token (+=; only with weight_grads)."""
-    n = len(groups)
-    arr = (Group * n)(*groups)
-
-    def ptrs(ts, k=1):
-        return (C.c_void_p * (k * n))(*[t.data_ptr() if t is not None else None for t in ts]) if ts is not None else None
-    da = ptrs([t for ts in attn_grads for t in ts], 12) if attn_grads is not None else None
-    base, nbytes = _aligned(ws)
-    check(lib.v2s_backbone_backward_masked(arr, _outputs_array(outputs, n), ptrs(masks), ptrs(dmask_tokens), da,
-                                           ptrs(dpixels), int(bool(weight_grads)), n, batch, mode, C.c_void_p(base),
-                                           nbytes, stream_ptr()), "backbone_backward_masked")
+                                    C.c_void_p(base), nbytes, int(layer_hi), int(layer_lo), int(bool(weight_grads)),
+                                    stream_ptr()), "backbone_backward")
 
 
 def _group(store, mode, x, slot, grads=None, hidden=None, feat=None, feat_stride=0, dfeat=None,
@@ -459,12 +415,12 @@ class _BackboneFn(torch.autograd.Function):
     want_attn the outputs are (hidden_states[12], hidden_states[0..11] if want_hidden, attentions[0..11] if
     want_attn): the residual stream is written straight into the 13 hidden-state tensors, the probabilities by one extra
     kernel per block.  Gradients w.r.t. any hidden state flow back, to the parameters that require them and, when x requires
-    grad, to the pixels (v2s_backbone_input_backward; a frozen backbone then computes no weight gradient at all).  The
+    grad, to the pixels (v2s_group_outputs.dpixels; a frozen backbone then computes no weight gradient at all).  The
     attention probabilities are not differentiable: a loss must not use them.  But a returned attention on which
     retain_grad() was called receives d loss / d probabilities in .grad, as in transformers (one extra kernel per such
     block in the same backward call; blocks at or above the highest layer the loss reaches keep .grad None).  With `mask`
     (uint8 [B,196]) the masked patch embeddings are replaced by `mask_token`, an autograd input whose gradient is
-    returned (v2s_backbone_forward_masked / v2s_backbone_backward_masked)."""
+    returned (v2s_group_outputs.mask / mask_token / dmask_token)."""
 
     @staticmethod
     @_with_device_of(lambda ctx, x, *a, **k: x)
@@ -488,21 +444,17 @@ class _BackboneFn(torch.autograd.Function):
             ws = _scratch_workspace(dev, B, mode, 1, 0)
         g = _group(store, mode, x, 0 if need_grad else -1,
                    hidden=None if pooled or want_hidden else out, feat=out if pooled else None, feat_stride=192)
-        outs = None
-        if want_hidden or want_attn:
-            o = GroupOutputs()
-            for i, t in enumerate(hidden or ()):
-                o.hidden[i] = t.data_ptr()
-            for i, t in enumerate(attn or ()):
-                o.attn[i] = t.data_ptr()
-            outs = [o]
-        if mask is None:
-            _run_forward([g], B, mode, ws, outs)
-        else:
+        o = GroupOutputs()
+        for i, t in enumerate(hidden or ()):
+            o.hidden[i] = t.data_ptr()
+        for i, t in enumerate(attn or ()):
+            o.attn[i] = t.data_ptr()
+        if mask is not None:
             tok = mask_token.detach().reshape(192)
             if tok.data_ptr() % 16:
                 tok = tok.clone()
-            _run_forward_masked([g], B, mode, ws, [mask], [tok], outs)
+            o.mask, o.mask_token = mask.data_ptr(), tok.data_ptr()
+        _run_forward([g], B, mode, ws, [o])
         ctx.mask = mask                 # the backward passes the same array (the library checks it)
         ctx.set_materialize_grads(False)
         ctx.model, ctx.pooled, ctx.mode, ctx.B = model, pooled, mode, B
@@ -540,10 +492,9 @@ class _BackboneFn(torch.autograd.Function):
             # d mask_token comes with the weight gradients: a frozen backbone computes them into a buffer that is dropped
             grads = torch.zeros(store.numel, dtype=torch.float32, device=ctx.x.device)
         dout = _grad_f32(dout) if dout is not None else None
-        outs = None
+        o = GroupOutputs()
         keep = []
         if ctx.want_hidden:
-            o = GroupOutputs()
             for i, t in enumerate(ctx.saved_tensors):
                 o.hidden[i] = t.data_ptr()
             for i, t in enumerate(tuple(dhid) + (dout,)):
@@ -551,7 +502,6 @@ class _BackboneFn(torch.autograd.Function):
                     t = _grad_f32(t)
                     keep.append(t)
                     o.dhidden[i] = t.data_ptr()
-            outs = [o]
             g = _group(store, ctx.mode, ctx.x, 0, grads=grads)
         else:
             g = _group(store, ctx.mode, ctx.x, 0, grads=grads,
@@ -561,22 +511,16 @@ class _BackboneFn(torch.autograd.Function):
         start = 12 if dout is not None else max(i for i, t in enumerate(dhid) if t is not None)
         retained = [(l, t) for l, t in enumerate(r() for r in ctx.attn_refs or ())
                     if l < start and t is not None and t.retains_grad]
-        if not want_x and not retained and not masked:
-            _run_backward([g], ctx.B, ctx.mode, ctx.ws, outs)
-            ctx.ws = None
-            return nones
-        dx = torch.empty(ctx.B, 3, 224, 224, dtype=torch.float32, device=ctx.x.device) if want_x else None
-        attn_grads = [None] * 12
+        attn_grads = {}
         for l, _ in retained:
             attn_grads[l] = torch.empty(ctx.B, 3, 197, 197, dtype=torch.float32, device=ctx.x.device)
-        dtok = None
-        if masked:
-            dtok = torch.zeros(192, dtype=torch.float32, device=ctx.x.device) if want_t else None
-            _run_masked_backward([g], ctx.B, ctx.mode, ctx.ws, [ctx.mask], [dtok], [dx], want_w or want_t, outs,
-                                 [attn_grads] if retained else None)
-        else:
-            _run_input_backward([g], ctx.B, ctx.mode, ctx.ws, [dx] if want_x else None, want_w, outs,
-                                [attn_grads] if retained else None)
+            o.dattn[l] = attn_grads[l].data_ptr()
+        dx = torch.empty(ctx.B, 3, 224, 224, dtype=torch.float32, device=ctx.x.device) if want_x else None
+        dtok = torch.zeros(192, dtype=torch.float32, device=ctx.x.device) if want_t else None
+        o.dpixels = dx.data_ptr() if dx is not None else None
+        o.mask = ctx.mask.data_ptr() if masked else None
+        o.dmask_token = dtok.data_ptr() if dtok is not None else None
+        _run_backward([g], ctx.B, ctx.mode, ctx.ws, [o], weight_grads=want_w or want_t)
         ctx.ws = None
         for l, t in retained:          # as the retain_grad hook: set, or accumulate out of place
             t.grad = attn_grads[l] if t.grad is None else t.grad + attn_grads[l]
@@ -857,13 +801,12 @@ class _DualStreamFn(torch.autograd.Function):
             _group(st[0], mode, x1, 0, grads=st[0].grads() if want_w else None, dfeat=dfeat, dfeat_stride=384),
             _group(st[1], mode, x2, 1, grads=st[1].grads() if want_w else None, dfeat=dfeat[:, 192:], dfeat_stride=384),
         ]
-        if not (want_x1 or want_x2):
-            _run_backward(groups, B, mode, ws)
-            dx1 = dx2 = None
-        else:
-            dx1 = torch.empty(B, 3, 224, 224, dtype=torch.float32, device=dpred.device) if want_x1 else None
-            dx2 = torch.empty(B, 3, 224, 224, dtype=torch.float32, device=dpred.device) if want_x2 else None
-            _run_input_backward(groups, B, mode, ws, [dx1, dx2], want_w)
+        dx1 = torch.empty(B, 3, 224, 224, dtype=torch.float32, device=dpred.device) if want_x1 else None
+        dx2 = torch.empty(B, 3, 224, 224, dtype=torch.float32, device=dpred.device) if want_x2 else None
+        outs = [GroupOutputs(), GroupOutputs()]
+        for o, dx in zip(outs, (dx1, dx2)):
+            o.dpixels = dx.data_ptr() if dx is not None else None
+        _run_backward(groups, B, mode, ws, outs, weight_grads=want_w)
         model._release_workspace(ws)
         ctx.ws = None
         return dx1, dx2, None, None, None
