@@ -28,7 +28,8 @@ extern "C" {
 
 #define V2S_ABI_VERSION 5 /* 5: the backbone calls added to 4 (image, attention-probability and mask-token gradients,
                              masked forward) are folded into v2s_backbone_forward / _backward: their arguments are
-                             fields of v2s_group_outputs, and v2s_backbone_backward takes weight_grads.  Additive to 4:
+                             fields of v2s_group_outputs, and v2s_backbone_backward takes weight_grads.  Additive to 5:
+                             v2s_mim_workspace_bytes, v2s_mim_forward, v2s_mim_backward.  Additive to 4:
                              v2s_test_gemm which = 5, v2s_test_attention which = 3.  4: one entry point per operation:
                              v2s_backbone_forward / _backward take the per-group outputs and (backward) the layer range,
                              v2s_heads_loss_fwd_bwd the device loss scale, v2s_adam_step and v2s_ema_update the
@@ -186,6 +187,28 @@ int v2s_heads_forward(const float* head_params, const float* feat_online, const 
 int v2s_heads_backward(const float* head_params, float* head_grads, const float* feat_online,
                        const float* mask_online, const float* dpred, float* dfeat_online, int batch,
                        void* workspace, int64_t workspace_bytes, void* stream);
+/* SimMIM head of transformers' ViTForMaskedImageModeling (encoder_stride 16) on the CUDA path.  Forward: seq = the final
+ * LayerNorm (eps 1e-12) of the 196 patch rows of hidden [batch,197,192] (hidden_states[12]; CLS dropped); reconstruction
+ * [batch,3,224,224] fp32 = PixelShuffle(16)(Conv2d(192, 768, 1)(seq)), always written; with mask (uint8 [batch,196],
+ * nonzero = masked) also loss (1 float) = sum over masked pixels and the 3 channels of |pixels - reconstruction| /
+ * (256 n + 1e-5) / 3, n = masked patches, bit-reproducible (fixed summation order).  pixels: fp32 NCHW [batch,3,224,224],
+ * read only with a mask.  ln_gamma / ln_beta / dec_w [768,192] / dec_b [768] are fp32 (the 16-bit modes cast a copy of
+ * dec_w into the workspace).  with_backward != 0 keeps in the workspace what v2s_mim_backward reads (the normalised rows,
+ * their statistics, the signs sign(r - x) of the masked rows, the W_dec copy, the denominator): pass the same workspace,
+ * batch, mode, mask and hidden to the backward.
+ * Backward of loss: dloss_dev is the loss's upstream gradient, read on the device (GradScaler's scale included).  dhidden
+ * [batch,197,192] is overwritten (CLS rows 0; NULL = not wanted); dpixels (the direct term -c sign, NULL = not wanted),
+ * d_ln_gamma / d_ln_beta, d_dec_w / d_dec_b (NULL = frozen) are accumulated (+=).  Deterministic mode
+ * (v2s_set_deterministic): fixed-order sums; size the workspace while the switch is on. */
+int64_t v2s_mim_workspace_bytes(int batch, int mode);
+int v2s_mim_forward(const float* hidden, const float* ln_gamma, const float* ln_beta, const float* dec_w,
+                    const float* dec_b, const float* pixels, const uint8_t* mask, float* reconstruction, float* loss,
+                    int with_backward, int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
+int v2s_mim_backward(const float* hidden, const float* ln_gamma, const float* dec_w, const uint8_t* mask,
+                     const float* dloss_dev, float* dhidden, float* dpixels, float* d_ln_gamma, float* d_ln_beta,
+                     float* d_dec_w, float* d_dec_b, int batch, int mode, void* workspace, int64_t workspace_bytes,
+                     void* stream);
+
 /* nn.CosineSimilarity(dim=1) loss of ref:174,211 and (optionally, dpred != NULL) its gradient */
 int v2s_cosine_loss(const float* pred, const float* target_proj, float* loss, float* dpred, int batch,
                     int accumulation_steps, float grad_scale, void* stream);

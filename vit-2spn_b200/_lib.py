@@ -75,6 +75,9 @@ _SIGS = {
                                          _vp, _i64, _vp]),
     "v2s_heads_forward": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _vp]),
     "v2s_heads_backward": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _i64, _vp]),
+    "v2s_mim_workspace_bytes": (_i64, [_i, _i]),
+    "v2s_mim_forward": (C.c_int, [_vp] * 9 + [_i, _i, _i, _vp, _i64, _vp]),
+    "v2s_mim_backward": (C.c_int, [_vp] * 11 + [_i, _i, _vp, _i64, _vp]),
     "v2s_cosine_loss": (C.c_int, [_vp, _vp, _vp, _vp, _i, _i, _f, _vp]),
     "v2s_infonce_loss": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i64, _f, _i, _f, _vp, _vp]),
     "v2s_dropout_mask": (C.c_int, [_vp, _i64, _f, C.c_uint64, C.c_uint64, _vp]),

@@ -34,9 +34,9 @@ static int n_recs = 0;
 static int n_events = 0;   // events created so far (recs[i].a/b valid for i < n_events)
 static const char* names[] = {"gemm_patch", "gemm_qkv", "gemm_proj", "gemm_fc1", "gemm_fc2", "gemm_dgrad",
                               "gemm_wgrad", "attn_fwd", "attn_bwd", "ln_fwd", "ln_bwd", "colsum", "misc", "heads", "gemm_mlp_fwd",
-                              "gemm_mlp_bwd", "attn_probs", "gemm_pixels", "attn_dprobs"};
+                              "gemm_mlp_bwd", "attn_probs", "gemm_pixels", "attn_dprobs", "mim_fwd", "mim_bwd"};
 enum { C_PATCH, C_QKV, C_PROJ, C_FC1, C_FC2, C_DGRAD, C_WGRAD, C_ATTN_F, C_ATTN_B, C_LN_F, C_LN_B, C_COLSUM, C_MISC,
-       C_HEADS, C_MLP_F, C_MLP_B, C_ATTN_P, C_PIX, C_ATTN_DP, C_COUNT };
+       C_HEADS, C_MLP_F, C_MLP_B, C_ATTN_P, C_PIX, C_ATTN_DP, C_MIM_F, C_MIM_B, C_COUNT };
 struct Scope {
   int idx = -1;
   cudaStream_t st;
@@ -1012,6 +1012,186 @@ static int heads_backward_impl(const float* hp, float* hg, const float* fo, cons
   return 0;
 }
 
+// =============================================================================================
+// SimMIM head (ViTForMaskedImageModeling): final LayerNorm over the patch rows, the 1x1-conv decoder with PixelShuffle(16)
+// and the masked L1 loss, forward and backward
+// =============================================================================================
+namespace {
+constexpr int64_t MIM_NW = (int64_t)KPE * D;      // decoder weight [768, 192]
+struct MimBufs {
+  char *seq, *wlp, *dsign, *dseq, *acc;
+  float *mean, *rstd, *part, *denom;
+  int n_part;
+  int64_t bytes;                                   // without the deterministic scratch
+};
+// workspace: seq [B*196,192] (activation type) | mean, rstd [B*196] | W_dec 16-bit copy | sign rows [B*196,768] (activation
+// type; fp32 check mode: the decoder rows, then the signs in place) | loss partials | denominator | d seq [B*196,192] fp32 |
+// unscaled decoder gradient [768*192 + 768] fp32 | deterministic scratch (while the switch is on)
+MimBufs mim_plan(int B, int mode, char* base) {
+  const Plan p = make_plan(B, mode);
+  const int64_t MP = p.MP;
+  MimBufs m;
+  int64_t o = 0;
+  auto take = [&](int64_t bytes) { char* r = base + o; o += align_up(bytes); return r; };
+  m.n_part = (int)MP;                              // >= the tensor-core tiles ((MP + 127) / 128 * 4)
+  m.seq = take(MP * D * p.es);
+  m.mean = (float*)take(MP * 4);
+  m.rstd = (float*)take(MP * 4);
+  m.wlp = take(MIM_NW * 2);
+  m.dsign = take(MP * KPE * p.es);
+  m.part = (float*)take((int64_t)m.n_part * 4);
+  m.denom = (float*)take(4);
+  m.dseq = take(MP * D * 4);
+  m.acc = take((MIM_NW + KPE) * 4);
+  m.bytes = o;
+  return m;
+}
+int64_t mim_det_bytes() {
+  int64_t part = gemm_tc_det_part_floats();
+  if (part < (int64_t)296 * DF) part = (int64_t)296 * DF;
+  return align_up(DET_COUNTERS * sizeof(unsigned)) + align_up(part * 4);
+}
+int mim_resolve(int B, int mode, void* ws, int64_t ws_bytes, MimBufs* m) {
+  if (B < 1 || mode < V2S_MODE_FP32 || mode > V2S_MODE_FP16) { set_error("mim: bad batch or mode"); return 1; }
+  if (!ws || (reinterpret_cast<uintptr_t>(ws) & 1023)) { set_error("mim: the workspace must be 1024-byte aligned"); return 1; }
+  *m = mim_plan(B, mode, static_cast<char*>(ws));
+  if (ws_bytes < m->bytes) {
+    set_error("mim: workspace too small: have %lld bytes, need %lld (v2s_mim_workspace_bytes)", (long long)ws_bytes,
+              (long long)m->bytes);
+    return 1;
+  }
+  return 0;
+}
+bool misaligned16(const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) != 0; }
+}  // namespace
+
+static int mim_forward_impl(const float* hidden, const float* ln_gamma, const float* ln_beta, const float* dec_w,
+                            const float* dec_b, const float* pixels, const uint8_t* mask, float* rec, float* loss,
+                            int with_backward, int B, int mode, void* ws, int64_t ws_bytes, cudaStream_t st) {
+  if (!hidden || !ln_gamma || !ln_beta || !dec_w || !dec_b || !rec || (mask && (!pixels || !loss)) || (!mask && loss)) {
+    set_error("mim_forward: null argument (pixels and loss go with a mask, and only with one)");
+    return 1;
+  }
+  if (misaligned16(hidden) || misaligned16(ln_gamma) || misaligned16(ln_beta) || misaligned16(dec_w) || misaligned16(dec_b) ||
+      misaligned16(pixels) || misaligned16(rec)) {
+    set_error("mim_forward: hidden, LayerNorm and decoder parameters, pixels and reconstruction must be 16-byte aligned");
+    return 1;
+  }
+  MimBufs m;
+  V2S_TRY(mim_resolve(B, mode, ws, ws_bytes, &m));
+  const Plan p = make_plan(B, mode);
+  const int at = p.at;
+  const int MP = (int)p.MP;
+  prof::Scope sc(prof::C_MIM_F, 2.0 * MP * KPE * (double)D, st,
+                 (double)B * NT * D * 4 + (double)MP * D * p.es * 2 + (double)MP * KPE * 4 * (mask ? 2 : 1) +
+                     (mask && with_backward ? (double)MP * KPE * p.es : 0.0));
+  {
+    const float* x[1] = {hidden}; const float* g[1] = {ln_gamma}; const float* b[1] = {ln_beta};
+    void* y[1] = {m.seq}; float* mu[1] = {m.mean}; float* rs[1] = {m.rstd};
+    V2S_TRY(launch_ln_fwd(x, g, b, y, mu, rs, 1, MP, at, st, true));
+  }
+  GemmDesc d = make_gemm_desc();
+  d.M = MP; d.N = KPE; d.K = D; d.groups = 1;
+  d.a_rs = D; d.a_cs = 1; d.b_rs = 1; d.b_cs = D; d.ldc = KPE;
+  d.A[0] = m.seq; d.bias[0] = dec_b;
+  if (at) {        // tensor cores: the 16-bit copy of W_dec, then one GEMM whose epilogue writes everything
+    V2S_TRY(launch_cast_lp(dec_w, m.wlp, MIM_NW, st, at == AT_F16));
+    d.B[0] = m.wlp; d.out[0] = rec; d.epi = EPI_MIM;
+    d.mim_x = pixels; d.mim_mask = mask; d.mim_dsign = mask && with_backward ? m.dsign : nullptr; d.mim_loss_part = m.part;
+    int handled = 0;
+    V2S_TRY(launch_gemm_tc(d, at, at, 0, st, &handled));
+    if (!handled) { set_error("mim_forward: the tensor-core decoder GEMM declined the problem"); return 1; }
+  } else {         // fp32 check mode: SIMT GEMM into the decoder rows, then the permutation / loss kernel
+    d.B[0] = dec_w; d.out[0] = m.dsign; d.epi = EPI_STORE;
+    V2S_TRY(launch_gemm_simt(d, AT_F32, AT_F32, AT_F32, st));
+    V2S_TRY(launch_mim_rows((float*)m.dsign, pixels, mask, rec, m.part, B, st));
+  }
+  if (mask) {
+    const int n_part = at ? (MP + 127) / 128 * (KPE / 192) : MP;
+    V2S_TRY(launch_mim_loss_finish(mask, MP, m.part, n_part, loss, m.denom, st));
+  }
+  return 0;
+}
+
+static int mim_backward_impl(const float* hidden, const float* ln_gamma, const float* dec_w, const uint8_t* mask,
+                             const float* dloss, float* dhidden, float* dpixels, float* d_ln_gamma, float* d_ln_beta,
+                             float* d_dec_w, float* d_dec_b, int B, int mode, void* ws, int64_t ws_bytes, cudaStream_t st) {
+  if (!hidden || !ln_gamma || !dec_w || !mask || !dloss) {
+    set_error("mim_backward: null argument (a backward needs the forward's mask and the loss gradient)");
+    return 1;
+  }
+  if ((d_ln_gamma == nullptr) != (d_ln_beta == nullptr)) { set_error("mim_backward: d_ln_gamma and d_ln_beta go together"); return 1; }
+  if (misaligned16(hidden) || misaligned16(ln_gamma) || misaligned16(dhidden) || misaligned16(dpixels)) {
+    set_error("mim_backward: hidden, ln_gamma, dhidden and dpixels must be 16-byte aligned");
+    return 1;
+  }
+  MimBufs m;
+  V2S_TRY(mim_resolve(B, mode, ws, ws_bytes, &m));
+  const Plan p = make_plan(B, mode);
+  const int at = p.at;
+  const int MP = (int)p.MP;
+  DetScratch det_s;
+  const DetScratch* det = nullptr;
+  if (tc_deterministic() && (d_dec_w || d_dec_b || d_ln_gamma)) {
+    const int64_t bytes = mim_det_bytes();
+    if (ws_bytes < m.bytes + bytes) {
+      set_error("mim_backward: deterministic mode: workspace too small (size it with v2s_mim_workspace_bytes while the "
+                "switch is on)");
+      return 1;
+    }
+    char* tail = static_cast<char*>(ws) + m.bytes;
+    det_s.counters = reinterpret_cast<unsigned*>(tail);
+    det_s.part = reinterpret_cast<float*>(tail + align_up(DET_COUNTERS * sizeof(unsigned)));
+    det_s.part_floats = (bytes - align_up(DET_COUNTERS * sizeof(unsigned))) / 4;
+    V2S_CUDA_OK(cudaMemsetAsync(det_s.counters, 0, DET_COUNTERS * sizeof(unsigned), st));
+    det = &det_s;
+  }
+  const bool dec = d_dec_w || d_dec_b, lnb = dhidden || d_ln_gamma;
+  prof::Scope sc(prof::C_MIM_B, 2.0 * MP * KPE * (double)D * ((dec ? 1 : 0) + (lnb ? 1 : 0)), st,
+                 (double)MP * KPE * p.es * ((dec ? 1 : 0) + (lnb ? 1 : 0) + (dpixels ? 1 : 0)) +
+                     (lnb ? (double)MP * D * 4 * 2 + (double)B * NT * D * 4 * 2 : 0.0) +
+                     (dpixels ? (double)MP * KPE * 4 * 2 : 0.0));
+  const void* wop = at ? static_cast<const void*>(m.wlp) : static_cast<const void*>(dec_w);
+  if (dec) {
+    // the unscaled weight gradient sign^T seq and its column sums into zeroed scratch, then c * scratch into dW / db
+    float* acc = (float*)m.acc;
+    V2S_CUDA_OK(cudaMemsetAsync(acc, 0, (MIM_NW + KPE) * 4, st));
+    GemmDesc d = make_gemm_desc();
+    d.M = KPE; d.N = D; d.K = MP; d.groups = 1;
+    d.a_rs = 1; d.a_cs = KPE; d.b_rs = D; d.b_cs = 1; d.ldc = D; d.epi = EPI_ACCUM;
+    d.A[0] = m.dsign; d.B[0] = m.seq; d.out[0] = acc;
+    if (at) {
+      d.split_k = wgrad_split(MP); d.det = det; d.rowsum_out[0] = acc + MIM_NW;
+      int handled = 0;
+      V2S_TRY(launch_gemm_tc(d, at, at, 0, st, &handled));
+      if (!handled) { set_error("mim_backward: the tensor-core decoder wgrad declined the problem"); return 1; }
+    } else {       // one K range per output element: a single atomic add each, so the order is fixed
+      V2S_TRY(launch_gemm_simt(d, AT_F32, AT_F32, AT_F32, st));
+      const void* src[1] = {m.dsign}; float* dst[1] = {acc + MIM_NW};
+      V2S_TRY(launch_colsum(src, dst, 1, MP, KPE, AT_F32, st, det));
+    }
+    V2S_TRY(launch_mim_scale_add(acc, d_dec_w, d_dec_b, (int)MIM_NW, KPE, dloss, m.denom, st));
+  }
+  if (lnb) {
+    // d seq = sign W_dec (unscaled, fp32), then the final LayerNorm's backward with dy = c * d seq
+    GemmDesc d = make_gemm_desc();
+    d.M = MP; d.N = D; d.K = KPE; d.groups = 1;
+    d.a_rs = KPE; d.a_cs = 1; d.b_rs = D; d.b_cs = 1; d.ldc = D; d.epi = EPI_STORE;
+    d.A[0] = m.dsign; d.B[0] = wop; d.out[0] = m.dseq;
+    if (at) {
+      int handled = 0;
+      V2S_TRY(launch_gemm_tc(d, at, at, 0, st, &handled));
+      if (!handled) { set_error("mim_backward: the tensor-core decoder dgrad declined the problem"); return 1; }
+    } else {
+      V2S_TRY(launch_gemm_simt(d, AT_F32, AT_F32, AT_F32, st));
+    }
+    V2S_TRY(launch_mim_ln_bwd((const float*)m.dseq, hidden, m.mean, m.rstd, ln_gamma, dhidden, d_ln_gamma, d_ln_beta, dloss,
+                              m.denom, MP, st, det));
+  }
+  if (dpixels) V2S_TRY(launch_mim_pixel_grad(m.dsign, dpixels, B, at, dloss, m.denom, st));
+  return 0;
+}
+
 }  // namespace v2s
 
 // =============================================================================================
@@ -1076,6 +1256,26 @@ int64_t v2s_workspace_bytes(int batch, int mode, int n_groups, int n_saved) {
   if (batch < 1 || n_groups < 0 || n_groups > MAXG || n_saved < 0 || n_saved > MAXG) return -1;
   const Plan p = make_plan(batch, mode);
   return plan_total(p, n_groups, n_saved) + (tc_deterministic() ? det_scratch_bytes(p, n_saved) : 0);
+}
+
+int64_t v2s_mim_workspace_bytes(int batch, int mode) {
+  if (batch < 1 || mode < V2S_MODE_FP32 || mode > V2S_MODE_FP16) return -1;
+  return mim_plan(batch, mode, nullptr).bytes + (tc_deterministic() ? mim_det_bytes() : 0);
+}
+
+int v2s_mim_forward(const float* hidden, const float* ln_gamma, const float* ln_beta, const float* dec_w, const float* dec_b,
+                    const float* pixels, const uint8_t* mask, float* reconstruction, float* loss, int with_backward, int batch,
+                    int mode, void* workspace, int64_t workspace_bytes, void* stream) {
+  return mim_forward_impl(hidden, ln_gamma, ln_beta, dec_w, dec_b, pixels, mask, reconstruction, loss, with_backward, batch,
+                          mode, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int v2s_mim_backward(const float* hidden, const float* ln_gamma, const float* dec_w, const uint8_t* mask,
+                     const float* dloss_dev, float* dhidden, float* dpixels, float* d_ln_gamma, float* d_ln_beta,
+                     float* d_dec_w, float* d_dec_b, int batch, int mode, void* workspace, int64_t workspace_bytes,
+                     void* stream) {
+  return mim_backward_impl(hidden, ln_gamma, dec_w, mask, dloss_dev, dhidden, dpixels, d_ln_gamma, d_ln_beta, d_dec_w,
+                           d_dec_b, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int v2s_backbone_forward(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, int n_groups, int batch, int mode,

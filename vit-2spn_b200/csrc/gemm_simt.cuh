@@ -17,6 +17,10 @@ enum GemmEpi : int {
   // tensor-core path only (the SIMT kernel refuses it): acc [B*196, 768] of the patch-embedding dgrad is stored fp32
   // straight into the NCHW image gradient out [B,3,224,224]: row (b, py, px), column c*256 + ky*16 + kx
   EPI_PIXELS = 8,
+  // tensor-core path only: SimMIM's 1x1-conv decoder, acc [B*196, 768] + bias stored fp32 into the NCHW reconstruction
+  // out [B,3,224,224] with EPI_PIXELS' permutation (PixelShuffle(16)); with mim_mask also the masked L1 loss partials
+  // (one per output tile) and the sign rows for the backward (see gemm_tc.cu)
+  EPI_MIM = 9,
 };
 
 struct GemmDesc {
@@ -58,6 +62,11 @@ struct GemmDesc {
   // deterministic mode, tensor-core split-K wgrad (EPI_ACCUM) only: scratch for the partial tiles and the per-output-tile
   // arrival counters; the split count then ignores v2s_set_sm_limit and the partials are summed in split order
   const DetScratch* det;
+  // EPI_MIM with a mask: input images (fp32 NCHW), uint8 [M] patch mask, 16-bit sign rows [M, N] (NULL: none), loss partials
+  const float* mim_x;
+  const uint8_t* mim_mask;
+  void* mim_dsign;
+  float* mim_loss_part;
 };
 
 inline GemmDesc make_gemm_desc() {

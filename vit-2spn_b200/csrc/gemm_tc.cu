@@ -50,7 +50,11 @@ enum TcEpi : int {
   T_ACCUM = 4,   // global(fp32) += acc          (TMA reduce-add; split-K)
   T_ACCUM_DET = 5,   // deterministic T_ACCUM: partial tiles to a slab, summed in split order by the last CTA to arrive
   T_PIXELS = 6,  // fp32 image gradient (EPI_PIXELS): the epilogue threads store their rows straight to global memory
+  T_MIM = 7,     // SimMIM decoder (EPI_MIM) without a mask: + bias, the fp32 reconstruction straight to NCHW (as T_PIXELS)
+  T_MIM_LOSS = 8,  // T_MIM + masked L1 partial sums per output tile and the sign(r - x) rows for the backward
 };
+// the epilogues that store from registers straight to global memory (no staging ring, no store warps)
+constexpr bool direct_epi(int e) { return e == T_PIXELS || e == T_MIM || e == T_MIM_LOSS; }
 
 // per-variant epilogue staging: a ring of NSTG buffers of STG bytes per epilogue group.  The residual variant
 // (auxiliary operand prefetched two chunks ahead into the ring) and the plain bf16 store use 3 buffers;
@@ -58,7 +62,7 @@ enum TcEpi : int {
 template <int EPI, bool OUT_BF16> struct Cfg {
   static constexpr int NSTG = (EPI == T_ACCUM || EPI == T_ACCUM_DET || (EPI == T_STORE && !OUT_BF16)) ? 2 : 3;
   static constexpr int STG = OUT_BF16 ? 8192 : 16384;
-  static constexpr int STAGING_BYTES = EPI == T_PIXELS ? 0 : 2 * NSTG * STG;
+  static constexpr int STAGING_BYTES = direct_epi(EPI) ? 0 : 2 * NSTG * STG;
 };
 
 struct alignas(64) TcParams {
@@ -90,7 +94,13 @@ struct alignas(64) TcParams {
   float* det_slab;
   float* det_rowpart;
   unsigned* det_counters;
-  float* pixels[MAXG];   // T_PIXELS: the fp32 image gradients [M / 196, 3, 224, 224] (no tensor map)
+  float* pixels[MAXG];   // T_PIXELS: the fp32 image gradients [M / 196, 3, 224, 224] (no tensor map); T_MIM*: the reconstruction
+  // T_MIM_LOSS (group 0 only): the fp32 NCHW input images, the uint8 [M] patch mask, the 16-bit sign rows [M, 768] (NULL:
+  // forward only) and one loss partial per output tile (m_tile * tiles_n + n_tile)
+  const float* mim_x;
+  const uint8_t* mim_mask;
+  void* mim_dsign;
+  float* mim_loss_part;
 };
 
 
@@ -125,7 +135,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
     for (int g = 0; g < p.groups; ++g) {
       ptx::prefetch_tmap(&p.tmA[g]);
       ptx::prefetch_tmap(&p.tmB[g]);
-      if constexpr (EPI != T_PIXELS) ptx::prefetch_tmap(&p.tmOut[g]);
+      if constexpr (!direct_epi(EPI)) ptx::prefetch_tmap(&p.tmOut[g]);
     }
   }
   if (warp == 1 && lane == 0) {
@@ -311,7 +321,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
     }
     if (DBG && blockIdx.x == 0 && lane == 0) { p.dbg[2] = w_full; p.dbg[3] = w_tempty; p.dbg[4] = clock64() - mma_t0; p.dbg[5] = ntiles; }
-  } else if (EPI != T_PIXELS && (warp == 2 || warp == 3)) {
+  } else if (!direct_epi(EPI) && (warp == 2 || warp == 3)) {
     // ================= store warp of epilogue group ge (whole warp walks the loop; one elected lane issues) ====
     const int ge = warp - 2;
     uint8_t* stg_base = smem + p.stg_off + ge * N_STG * STG_BYTES;
@@ -382,7 +392,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
     }
     if (ptx::elect_one()) ptx::tma_wait_group<0>();
     __syncwarp();
-  } else if (EPI != T_PIXELS && warp >= 4) {
+  } else if (!direct_epi(EPI) && warp >= 4) {
     // ================= epilogue =================
     // 16 warps = 2 groups of 8.  Group ge drains accumulator stage ge.  Inside a group, warps w and w+4 share
     // TMEM lane quarter w%4 and split every 32-column chunk into two 16-column halves (thread = one row x 16 cols).
@@ -582,7 +592,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
       long long* d = p.dbg + 8 + (threadIdx.x == 128 ? 0 : 8);
       d[0] = e_tfull; d[1] = e_aux; d[2] = e_pub; d[3] = e_ld; d[4] = clock64() - epi_t0; d[5] = cnt;
     }
-  } else if (warp >= 4) {
+  } else if (EPI == T_PIXELS && warp >= 4) {
     // ================= image-gradient epilogue (EPI_PIXELS) =================
     // The TMEM drain of the epilogue above (group ge = accumulator stage, warps w and w+4 = lane quarter w%4 and the two
     // 16-column halves of each chunk) without staging: row m = (b, py, px), columns [colh, colh + 16) = (c, ky, kx 0..15)
@@ -616,6 +626,97 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
           for (int j = 0; j < 4; ++j)
             dst[j] = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]),
                                  __uint_as_float(r[4 * j + 3]));
+        }
+      }
+    }
+  } else if (warp >= 4) {
+    // ================= SimMIM decoder epilogue (EPI_MIM) =================
+    // The drain of T_PIXELS (row m = (b, py, px), columns [colh, colh + 16) = 64 contiguous bytes of image row py*16 + ky
+    // of channel colh / 256, which is PixelShuffle(16)'s permutation) plus the decoder bias.  T_MIM_LOSS also reads the
+    // same 64 bytes of the input image: a masked row adds |x - r| to the thread's sum and, with a backward, stores
+    // sign(r - x) (exact in both 16-bit formats) as 16-bit row m of dsign; an unmasked row stores zeros there.  The sums
+    // of a tile's 256 threads are reduced in a fixed order (warp shuffles, then the 8 warps of the group through shared
+    // memory) into the tile's own slot, so the loss does not depend on the grid.
+    constexpr bool LOSS = EPI == T_MIM_LOSS;
+    const int ge = (warp - 4) >> 3, q = warp & 3, hf = ((warp - 4) >> 2) & 1, row = q * 32 + lane;
+    const int wi = (warp - 4) & 7;                   // warp within the group
+    float* red = reinterpret_cast<float*>(ln_part);  // [2 groups][2 tile parities][8 warps]
+    uint32_t acc_phase = 0;
+    int g, m_tile, split, n_tile;
+    for (int i = ge; tile_at(i, g, m_tile, split, n_tile); i += 2) {
+      const int m = m_tile * BM + row;
+      const bool live = m < p.M;
+      const int b = m / NP, t = m - b * NP, py = t / 14, px = t - py * 14;
+      const int64_t pix0 = (int64_t)b * 3 * V2S_IMG * V2S_IMG + py * 16 * V2S_IMG + px * 16;
+      const bool masked = LOSS && live && p.mim_mask[m] != 0;
+      float l1 = 0.f;
+      ptx::mbar_wait(&tfull_bar[ge], acc_phase, p.err_flag, 4);
+      acc_phase ^= 1;
+      ptx::tc_fence_after();
+      const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16) + ge * ACC_STRIDE;
+#pragma unroll 1
+      for (int c = 0; c < N_CHUNKS; ++c) {
+        const int colh = n_tile * BN + c * CHUNK + hf * 16;
+        const float4* b4 = reinterpret_cast<const float4*>(p.bias[0] + colh);
+        float4 bb[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) bb[k] = __ldg(b4 + k);
+        uint32_t r[16];
+        ptx::tmem_ld_32x16(tlane + c * CHUNK + hf * 16, r);
+        ptx::tmem_ld_wait();
+        if (c == N_CHUNKS - 1) {                    // accumulator fully read: hand the stage back to the MMA warp
+          ptx::tc_fence_before();
+          if (lane == 0) ptx::mbar_arrive(&tempty_bar[ge]);
+        }
+        if (!live) continue;
+        const int64_t off = pix0 + (colh >> 8) * V2S_IMG * V2S_IMG + ((colh >> 4) & 15) * V2S_IMG;
+        float v[16];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+          v[4 * k] = __uint_as_float(r[4 * k]) + bb[k].x; v[4 * k + 1] = __uint_as_float(r[4 * k + 1]) + bb[k].y;
+          v[4 * k + 2] = __uint_as_float(r[4 * k + 2]) + bb[k].z; v[4 * k + 3] = __uint_as_float(r[4 * k + 3]) + bb[k].w;
+        }
+        float4* dst = reinterpret_cast<float4*>(p.pixels[0] + off);
+#pragma unroll
+        for (int j = 0; j < 4; ++j) dst[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+        if constexpr (LOSS) {
+          float sg[16];
+          if (masked) {
+            const float4* src = reinterpret_cast<const float4*>(p.mim_x + off);
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+              const float4 x = __ldg(src + j);
+              const float xs[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+              for (int e = 0; e < 4; ++e) {
+                const float d = v[4 * j + e] - xs[e];
+                l1 += fabsf(d);
+                sg[4 * j + e] = d > 0.f ? 1.f : (d < 0.f ? -1.f : 0.f);
+              }
+            }
+          } else {
+#pragma unroll
+            for (int k = 0; k < 16; ++k) sg[k] = 0.f;
+          }
+          if (p.mim_dsign) {
+            uint4* ds = reinterpret_cast<uint4*>(static_cast<uint16_t*>(p.mim_dsign) + (int64_t)m * (4 * BN) + colh);
+#pragma unroll
+            for (int j = 0; j < 2; ++j)
+              ds[j] = make_uint4(LP::pack(sg[8 * j], sg[8 * j + 1]), LP::pack(sg[8 * j + 2], sg[8 * j + 3]),
+                                 LP::pack(sg[8 * j + 4], sg[8 * j + 5]), LP::pack(sg[8 * j + 6], sg[8 * j + 7]));
+          }
+        }
+      }
+      if constexpr (LOSS) {
+        l1 = warp_sum(l1);
+        const int par = (i >> 1) & 1;               // two slots per group: tile i + 2 never overwrites tile i's
+        if (lane == 0) red[(ge * 2 + par) * 8 + wi] = l1;
+        ptx::bar_sync(1 + ge, 256);
+        if (wi == 0 && lane == 0) {
+          float s = 0.f;
+#pragma unroll
+          for (int w = 0; w < 8; ++w) s += red[(ge * 2 + par) * 8 + w];
+          p.mim_loss_part[m_tile * p.tiles_n + n_tile] = s;
         }
       }
     }
@@ -880,12 +981,19 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
     case EPI_BIAS_RESID: epi = T_RESID; break;
     case EPI_ACCUM: epi = T_ACCUM; break;
     case EPI_PIXELS: epi = T_PIXELS; break;
+    case EPI_MIM: epi = d.mim_mask ? T_MIM_LOSS : T_MIM; break;
     default: return 0;
   }
   if (d.alpha != 1.0f) return 0;
   const bool out_bf16 = (to != 0);                        // 16-bit output (bf16 or fp16, as the operands)
   if (epi == T_PIXELS && (out_bf16 || d.M % NP || d.N != KPE || d.ldc != KPE || d.a_remap || d.b_remap)) {
     set_error("gemm_tc: the image-gradient epilogue needs [B*196, 768] fp32 output (M %d N %d)", d.M, d.N);
+    return 1;
+  }
+  if ((epi == T_MIM || epi == T_MIM_LOSS) &&
+      (out_bf16 || d.M % NP || d.N != 4 * BN || d.K != D || d.groups != 1 || !d.bias[0] || (epi == T_MIM_LOSS && !d.mim_x))) {
+    set_error("gemm_tc: the SimMIM decoder epilogue needs one [B*196, 192] x [768, 192]^T problem with a bias and fp32 "
+              "output (M %d N %d K %d)", d.M, d.N, d.K);
     return 1;
   }
   if ((epi == T_RESID || epi == T_ACCUM) && out_bf16) return 0;
@@ -954,9 +1062,17 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
     else V2S_TRY(get_map(&p.tmA[g], d.A[g], d.M, d.K, a_ld, 64, BK, true, CU_TENSOR_MAP_SWIZZLE_128B));
     if (!b_mn) V2S_TRY(get_map(&p.tmB[g], d.B[g], d.K, d.N, b_ld, BK, BN, true, CU_TENSOR_MAP_SWIZZLE_128B));
     else V2S_TRY(get_map(&p.tmB[g], d.B[g], d.N, d.K, b_ld, 64, BK, true, CU_TENSOR_MAP_SWIZZLE_128B));
-    if (epi == T_PIXELS) {
-      if (reinterpret_cast<uintptr_t>(d.out[g]) & 15) { set_error("gemm_tc: image gradient not 16-byte aligned"); return 1; }
+    if (epi == T_PIXELS || epi == T_MIM || epi == T_MIM_LOSS) {
+      if ((reinterpret_cast<uintptr_t>(d.out[g]) | reinterpret_cast<uintptr_t>(d.bias[g]) | reinterpret_cast<uintptr_t>(d.mim_x) |
+           reinterpret_cast<uintptr_t>(d.mim_dsign)) & 15) {
+        set_error("gemm_tc: image, bias and sign rows of a direct-store epilogue must be 16-byte aligned");
+        return 1;
+      }
       p.pixels[g] = static_cast<float*>(d.out[g]);
+      if (epi != T_PIXELS) {
+        p.bias[g] = d.bias[g];
+        p.mim_x = d.mim_x; p.mim_mask = d.mim_mask; p.mim_dsign = d.mim_dsign; p.mim_loss_part = d.mim_loss_part;
+      }
       continue;
     }
     V2S_TRY(get_map(&p.tmOut[g], d.out[g], d.N, d.M, d.ldc, CHUNK, BM, out_bf16, out_swz));
@@ -994,6 +1110,8 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
     case T_RESID: rc = launch_kernel<T_RESID, false>(p, lp_f16, stream); break;
     case T_ACCUM_DET: rc = launch_kernel<T_ACCUM_DET, false>(p, lp_f16, stream); break;
     case T_PIXELS: rc = launch_kernel<T_PIXELS, false>(p, lp_f16, stream); break;
+    case T_MIM: rc = launch_kernel<T_MIM, false>(p, lp_f16, stream); break;
+    case T_MIM_LOSS: rc = launch_kernel<T_MIM_LOSS, false>(p, lp_f16, stream); break;
     default: rc = launch_kernel<T_ACCUM, false>(p, lp_f16, stream); break;
   }
   if (rc) return rc;

@@ -192,7 +192,9 @@ __device__ __forceinline__ uint32_t pack_lp(float a, float b, int f16) {
   return *reinterpret_cast<uint32_t*>(&v);
 }
 
-template <typename T>
+// REMAP (SimMIM's final LayerNorm): output row r = b*196 + p normalises token row b*197 + 1 + p of x (the CLS rows are
+// dropped), so y, mean and rstd are compact patch rows
+template <typename T, bool REMAP = false>
 __global__ void __launch_bounds__(256) ln_fwd_kernel(const __grid_constant__ LnFwdP p) {
   // wait for the predecessor, THEN release the successor: a successor flagged "late wait" (gemm_tc.cu) relies on
   // everything before its predecessor being complete when it starts
@@ -210,7 +212,7 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const __grid_constant__ LnF
     bt[i] = reinterpret_cast<const float4*>(p.beta[g])[l + 16 * i];
   }
   for (int row = blockIdx.x * 16 + hw; row < p.M; row += gridDim.x * 16) {
-    const float4* xr = reinterpret_cast<const float4*>(x + (int64_t)row * D);
+    const float4* xr = reinterpret_cast<const float4*>(x + (int64_t)(REMAP ? row + row / NP + 1 : row) * D);
     float4 v[3];
     float s = 0.f;
 #pragma unroll
@@ -286,9 +288,14 @@ struct LnBwdP {
   int M;
   float* det_part;             // DET: [group][CTA][3 * 192] partial rows
   unsigned* det_counters;      // DET: one per group
+  const float* dloss;          // MIM: the loss's upstream gradient and its denominator 256 n + 1e-5 (device scalars)
+  const float* denom;
 };
 
-template <typename T, bool DET, bool PARAMS>
+// MIM (SimMIM's final LayerNorm, T = float): dy is c * (compact patch-row gradient [M = B*196, 192]) with
+// c = dloss / 3 / denom read on the device; x and dres are token rows [B,197,192] (row r -> b*197 + 1 + p), dres is
+// overwritten (NULL: parameter gradients only) and its CLS rows are set to zero
+template <typename T, bool DET, bool PARAMS, bool MIM = false>
 __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnBwdP p) {
   __shared__ __align__(16) float red[16][3 * D];          // 36 KB; float4 accesses
   // wait for the predecessor, THEN release the successor: a successor flagged "late wait" (gemm_tc.cu) relies on
@@ -308,16 +315,24 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnB
     gm[i] = reinterpret_cast<const float4*>(p.gamma[g])[l + 16 * i];
     ag[i] = ab[i] = ac[i] = make_float4(0.f, 0.f, 0.f, 0.f);
   }
+  float sc = 1.f;
+  if constexpr (MIM) sc = (*p.dloss / 3.f) / *p.denom;
   for (int row = blockIdx.x * 16 + hw; row < p.M; row += gridDim.x * 16) {
     const float mu = p.mean[g][row], rs = p.rstd[g][row];
-    const float4* xr = reinterpret_cast<const float4*>(x + (int64_t)row * D);
+    const int64_t xrow = MIM ? row + row / NP + 1 : row;
+    const float4* xr = reinterpret_cast<const float4*>(x + xrow * D);
     float4 xh[3], gd[3], d[3], o[3];
     float c1 = 0.f, c2 = 0.f;
 #pragma unroll
     for (int i = 0; i < 3; ++i) {
       const float4 xv = xr[l + 16 * i];
       d[i] = load4<T>(dy + (int64_t)row * D + 4 * (l + 16 * i));
-      o[i] = reinterpret_cast<const float4*>(dres + (int64_t)row * D)[l + 16 * i];
+      if constexpr (MIM) {
+        d[i].x *= sc; d[i].y *= sc; d[i].z *= sc; d[i].w *= sc;
+        o[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+      } else {
+        o[i] = reinterpret_cast<const float4*>(dres + (int64_t)row * D)[l + 16 * i];
+      }
       xh[i] = make_float4((xv.x - mu) * rs, (xv.y - mu) * rs, (xv.z - mu) * rs, (xv.w - mu) * rs);
       gd[i] = make_float4(d[i].x * gm[i].x, d[i].y * gm[i].y, d[i].z * gm[i].z, d[i].w * gm[i].w);
       c1 += (gd[i].x + gd[i].y) + (gd[i].z + gd[i].w);
@@ -333,6 +348,13 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnB
     for (int i = 0; i < 3; ++i) {
       o[i].x += rs * (gd[i].x - c1 - xh[i].x * c2); o[i].y += rs * (gd[i].y - c1 - xh[i].y * c2);
       o[i].z += rs * (gd[i].z - c1 - xh[i].z * c2); o[i].w += rs * (gd[i].w - c1 - xh[i].w * c2);
+      if constexpr (MIM) {
+        if (dres) {
+          reinterpret_cast<float4*>(dres + xrow * D)[l + 16 * i] = o[i];
+          if (row % NP == 0) reinterpret_cast<float4*>(dres + (xrow - 1) * D)[l + 16 * i] = make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+        continue;
+      }
       reinterpret_cast<float4*>(dres + (int64_t)row * D)[l + 16 * i] = o[i];
       if (dlp) store4<T>(dlp + (int64_t)row * D + 4 * (l + 16 * i), o[i].x, o[i].y, o[i].z, o[i].w);
       if constexpr (PARAMS) { ac[i].x += o[i].x; ac[i].y += o[i].y; ac[i].z += o[i].z; ac[i].w += o[i].w; }
@@ -1077,6 +1099,104 @@ inline int grid_for(int64_t n, int threads, int max_blocks = 148 * 8) {
   return (int)b;
 }
 
+// ------------------------------------------------------------------------------------------
+// SimMIM head (ViTForMaskedImageModeling): the loss, its scale and the decoder's elementwise passes
+// ------------------------------------------------------------------------------------------
+// c = d loss / d (sum of |x - r| over the masked pixels), read on the device: loss = sum / denom / 3
+__device__ __forceinline__ float mim_scale(const float* dloss, const float* denom) { return (*dloss / 3.f) / *denom; }
+
+// fp32 check mode: rows [B*196, 768] = seq W_dec^T + b (SIMT GEMM) -> the NCHW reconstruction (PixelShuffle(16): row
+// (b, py, px), column ch*256 + ky*16 + kx); MASK: the row's masked L1 sum into part[row] and, in place, the row's
+// sign(r - x) (zeros for an unmasked row).  One block of 192 threads per row, one float4 per thread.
+template <bool MASK>
+__global__ void __launch_bounds__(192) mim_rows_kernel(float* __restrict__ rows, const float* __restrict__ x,
+                                                        const uint8_t* __restrict__ mask, float* __restrict__ rec,
+                                                        float* __restrict__ part) {
+  __shared__ float red[6];
+  const int m = blockIdx.x, j = threadIdx.x, col = 4 * j;
+  const int b = m / NP, t = m - b * NP, py = t / 14, px = t - py * 14;
+  const int64_t off = (int64_t)b * 3 * V2S_IMG * V2S_IMG + (col >> 8) * V2S_IMG * V2S_IMG + (py * 16 + ((col >> 4) & 15)) * V2S_IMG +
+                      px * 16 + (col & 15);
+  float4* rp = reinterpret_cast<float4*>(rows + (int64_t)m * KPE) + j;
+  const float4 r = *rp;
+  *reinterpret_cast<float4*>(rec + off) = r;
+  if constexpr (MASK) {
+    float l1 = 0.f;
+    float4 sg = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (mask[m]) {
+      const float4 xv = *reinterpret_cast<const float4*>(x + off);
+      const float d0 = r.x - xv.x, d1 = r.y - xv.y, d2 = r.z - xv.z, d3 = r.w - xv.w;
+      l1 = (fabsf(d0) + fabsf(d1)) + (fabsf(d2) + fabsf(d3));
+      auto sgn = [](float d) { return d > 0.f ? 1.f : (d < 0.f ? -1.f : 0.f); };
+      sg = make_float4(sgn(d0), sgn(d1), sgn(d2), sgn(d3));
+    }
+    *rp = sg;
+    l1 = warp_sum(l1);
+    if ((j & 31) == 0) red[j >> 5] = l1;
+    __syncthreads();
+    if (j == 0) part[m] = ((red[0] + red[1]) + (red[2] + red[3])) + (red[4] + red[5]);
+  }
+}
+
+// one CTA: the masked patches n of the uint8 [n_mask] mask, the fixed-order sum S of the n_part loss partials;
+// loss = S / denom / 3 with denom = 256 n + 1e-5 (transformers' pixel-mask sum + 1e-5), kept for the backward
+__global__ void __launch_bounds__(1024) mim_loss_finish_kernel(const uint8_t* __restrict__ mask, int n_mask,
+                                                               const float* __restrict__ part, int n_part, float* loss,
+                                                               float* denom) {
+  __shared__ float sred[1024];
+  __shared__ int cred[1024];
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  const int t = threadIdx.x;
+  float s = 0.f;
+  int c = 0;
+  for (int i = t; i < n_part; i += 1024) s += part[i];
+  for (int i = t; i < n_mask; i += 1024) c += mask[i] != 0;
+  sred[t] = s; cred[t] = c;
+  __syncthreads();
+  for (int h = 512; h > 0; h >>= 1) {
+    if (t < h) { sred[t] += sred[t + h]; cred[t] += cred[t + h]; }
+    __syncthreads();
+  }
+  if (t == 0) {
+    const float d = (float)(256 * cred[0]) + 1e-5f;
+    denom[0] = d;
+    loss[0] = sred[0] / d / 3.f;
+  }
+}
+
+// dW[i] += c * acc[i] (i < nw), db[j] += c * acc[nw + j]: the unscaled decoder gradients (sign rows^T seq and their
+// column sums) scaled by the device-side c; dW / db may be NULL (frozen)
+__global__ void __launch_bounds__(256) mim_scale_add_kernel(const float* __restrict__ acc, float* dw, float* db, int nw, int nb,
+                                                            const float* dloss, const float* denom) {
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  const float c = mim_scale(dloss, denom);
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nw + nb; i += gridDim.x * blockDim.x) {
+    if (i < nw) { if (dw) dw[i] += c * acc[i]; }
+    else if (db) db[i - nw] += c * acc[i];
+  }
+}
+
+// d pixels += -c * sign rows, scattered to NCHW (the reconstruction's own permutation); one float4 of the image per thread
+template <typename T>
+__global__ void __launch_bounds__(256) mim_pixel_grad_kernel(const T* __restrict__ sign, float* __restrict__ dx, int B,
+                                                             const float* dloss, const float* denom) {
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  const float c = -mim_scale(dloss, denom);
+  const int64_t total = (int64_t)B * 3 * V2S_IMG * (V2S_IMG / 4);
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int x4 = i % (V2S_IMG / 4), y = (i / (V2S_IMG / 4)) % V2S_IMG;
+    const int ch = (i / (V2S_IMG * V2S_IMG / 4)) % 3;
+    const int64_t b = i / (3 * V2S_IMG * V2S_IMG / 4);
+    const float4 sg = load4<T>(sign + (b * NP + (y / 16) * 14 + x4 / 4) * KPE + ch * 256 + (y % 16) * 16 + (x4 % 4) * 4);
+    float4 v = reinterpret_cast<float4*>(dx)[i];
+    v.x += c * sg.x; v.y += c * sg.y; v.z += c * sg.z; v.w += c * sg.w;
+    reinterpret_cast<float4*>(dx)[i] = v;
+  }
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------
@@ -1134,7 +1254,7 @@ int launch_col2im(const float* const* rows, float* const* img, int groups, int B
 }
 
 int launch_ln_fwd(const float* const* x, const float* const* gamma, const float* const* beta, void* const* y,
-                  float* const* mean, float* const* rstd, int groups, int M, int at, cudaStream_t s) {
+                  float* const* mean, float* const* rstd, int groups, int M, int at, cudaStream_t s, bool patch_rows) {
   LnFwdP p;
   memset(&p, 0, sizeof(p));
   for (int g = 0; g < groups; ++g) {
@@ -1145,7 +1265,8 @@ int launch_ln_fwd(const float* const* x, const float* const* gamma, const float*
   int bx = (M + 15) / 16;
   if (bx > 148 * 6) bx = 148 * 6;
   dim3 grid(bx, groups);
-  V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_fwd_kernel<T>, grid, dim3(256), 0, s, p)));
+  if (patch_rows) { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_fwd_kernel<T, true>, grid, dim3(256), 0, s, p))); }
+  else { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_fwd_kernel<T>, grid, dim3(256), 0, s, p))); }
   V2S_LAUNCH_CHECK();
   return 0;
 }
@@ -1174,6 +1295,58 @@ int launch_ln_bwd(const void* const* dy, const float* const* x, const float* con
   if (!dgamma) { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<T, false, false>, grid, dim3(256), 0, s, p))); }
   else if (det) { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<T, true, true>, grid, dim3(256), 0, s, p))); }
   else { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<T, false, true>, grid, dim3(256), 0, s, p))); }
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_mim_ln_bwd(const float* dseq, const float* hidden, const float* mean, const float* rstd, const float* gamma,
+                      float* dhidden, float* dgamma, float* dbeta, const float* dloss, const float* denom, int M,
+                      cudaStream_t s, const DetScratch* det) {
+  LnBwdP p;
+  memset(&p, 0, sizeof(p));
+  p.dy[0] = dseq; p.x[0] = hidden; p.mean[0] = mean; p.rstd[0] = rstd; p.gamma[0] = gamma; p.dres[0] = dhidden;
+  p.dgamma[0] = dgamma; p.dbeta[0] = dbeta; p.dloss = dloss; p.denom = denom;
+  p.M = M;
+  int bx = (M + 15) / 16;
+  if (bx > 148 * 4) bx = 148 * 4;
+  if (det && dgamma) {
+    if (bx > 148) bx = 148;
+    if ((int64_t)bx * 3 * D > det->part_floats) { set_error("mim ln_bwd: deterministic scratch too small"); return 1; }
+    p.det_part = det->part; p.det_counters = det->counters;
+  }
+  if (!dgamma) V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, false, false, true>, dim3(bx), dim3(256), 0, s, p));
+  else if (det) V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, true, true, true>, dim3(bx), dim3(256), 0, s, p));
+  else V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, false, true, true>, dim3(bx), dim3(256), 0, s, p));
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_mim_rows(float* rows, const float* x, const uint8_t* mask, float* rec, float* part, int B, cudaStream_t s) {
+  if (mask) mim_rows_kernel<true><<<B * NP, 192, 0, s>>>(rows, x, mask, rec, part);
+  else mim_rows_kernel<false><<<B * NP, 192, 0, s>>>(rows, x, mask, rec, part);
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_mim_loss_finish(const uint8_t* mask, int n_mask, const float* part, int n_part, float* loss, float* denom,
+                           cudaStream_t s) {
+  V2S_CUDA_OK(launch_pdl(mim_loss_finish_kernel, dim3(1), dim3(1024), 0, s, mask, n_mask, part, n_part, loss, denom));
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_mim_scale_add(const float* acc, float* dw, float* db, int nw, int nb, const float* dloss, const float* denom,
+                         cudaStream_t s) {
+  V2S_CUDA_OK(launch_pdl(mim_scale_add_kernel, dim3(grid_for(nw + nb, 256, 148 * 2)), dim3(256), 0, s, acc, dw, db, nw, nb,
+                         dloss, denom));
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_mim_pixel_grad(const void* sign, float* dx, int B, int at, const float* dloss, const float* denom, cudaStream_t s) {
+  const dim3 grid(grid_for((int64_t)B * 3 * V2S_IMG * (V2S_IMG / 4), 256, 148 * 16));
+  V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(mim_pixel_grad_kernel<T>, grid, dim3(256), 0, s, static_cast<const T*>(sign), dx, B,
+                                             dloss, denom)));
   V2S_LAUNCH_CHECK();
   return 0;
 }

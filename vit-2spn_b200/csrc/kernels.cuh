@@ -23,9 +23,10 @@ int launch_gather_patch_rows(const void* const* src, void* const* dst, int group
                              const uint8_t* const* mask = nullptr);
 // inverse of launch_im2col for fp32: patch rows [B*196, 768] -> NCHW [B,3,224,224] (overwritten)
 int launch_col2im(const float* const* rows, float* const* img, int groups, int B, cudaStream_t s);
+// patch_rows: y, mean and rstd are the compact patch rows [M = B*196] of the token rows x [B,197,192] (CLS dropped)
 int launch_ln_fwd(const float* const* x, const float* const* gamma, const float* const* beta,
                   void* const* y, float* const* mean, float* const* rstd, int groups, int M, int at,
-                  cudaStream_t s);
+                  cudaStream_t s, bool patch_rows = false);
 // dres (fp32, in/out) += LN-backward(dy); dres_lp (optional, activation type) = updated dres;
 // dcolsum (optional) += column sums of the updated dres (bias gradient of the next linear layer);
 // dgamma == NULL: no parameter gradient at all (dbeta, dcolsum and det ignored)
@@ -33,6 +34,23 @@ int launch_ln_bwd(const void* const* dy, const float* const* x, const float* con
                   const float* const* rstd, const float* const* gamma, float* const* dres,
                   void* const* dres_lp, float* const* dgamma, float* const* dbeta, float* const* dcolsum,
                   int groups, int M, int at, cudaStream_t s, const DetScratch* det = nullptr);
+// SimMIM head (one group).  c = *dloss / 3 / *denom is read on the device by every backward kernel below.
+// Final-LayerNorm backward over the patch rows: dy = c * dseq [M = B*196, 192] fp32, x = hidden [B,197,192]; dhidden (may
+// be NULL) is overwritten, CLS rows zero; dgamma / dbeta (NULL: frozen) +=, in a fixed order with `det`
+int launch_mim_ln_bwd(const float* dseq, const float* hidden, const float* mean, const float* rstd, const float* gamma,
+                      float* dhidden, float* dgamma, float* dbeta, const float* dloss, const float* denom, int M,
+                      cudaStream_t s, const DetScratch* det = nullptr);
+// fp32 check mode: decoder rows [B*196, 768] -> reconstruction; with a mask the loss partials part[B*196] and the sign rows
+// (in place of the decoder rows)
+int launch_mim_rows(float* rows, const float* x, const uint8_t* mask, float* rec, float* part, int B, cudaStream_t s);
+// loss and its denominator from the uint8 mask and the loss partials (one CTA, fixed order)
+int launch_mim_loss_finish(const uint8_t* mask, int n_mask, const float* part, int n_part, float* loss, float* denom,
+                           cudaStream_t s);
+// dw[0, nw) += c * acc[0, nw), db[0, nb) += c * acc[nw, nw + nb) (either may be NULL)
+int launch_mim_scale_add(const float* acc, float* dw, float* db, int nw, int nb, const float* dloss, const float* denom,
+                         cudaStream_t s);
+// dx [B,3,224,224] += -c * sign rows [B*196, 768] (activation type `at`) in NCHW order
+int launch_mim_pixel_grad(const void* sign, float* dx, int B, int at, const float* dloss, const float* denom, cudaStream_t s);
 // db[n] += sum_m dy[m,n]; src type tag `t`.  With `det` (deterministic mode) the sum has a fixed order: partial rows in
 // det->part, or, when det->part is NULL, one CTA per group
 int launch_colsum(const void* const* dy, float* const* db, int groups, int M, int N, int t, cudaStream_t s,

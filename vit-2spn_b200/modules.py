@@ -329,7 +329,8 @@ class ViTConfig:
 
     def __init__(self, hidden_size=192, num_hidden_layers=12, num_attention_heads=3, intermediate_size=768,
                  patch_size=16, image_size=224, output_hidden_states=False, layer_norm_eps=1e-12,
-                 hidden_act="gelu", num_channels=3, qkv_bias=True, initializer_range=0.02, output_attentions=False, **kw):
+                 hidden_act="gelu", num_channels=3, qkv_bias=True, initializer_range=0.02, output_attentions=False,
+                 encoder_stride=16, **kw):
         self.hidden_size = hidden_size
         self.num_hidden_layers = num_hidden_layers
         self.num_attention_heads = num_attention_heads
@@ -343,6 +344,7 @@ class ViTConfig:
         self.num_channels = num_channels
         self.qkv_bias = qkv_bias
         self.initializer_range = initializer_range
+        self.encoder_stride = encoder_stride
         for k, v in kw.items():
             setattr(self, k, v)
 
@@ -400,6 +402,8 @@ class ViTModelOutput:
     @property
     def pooler_output(self):
         m = self._model
+        if m.pooler is None:            # ViTModel(add_pooling_layer=False), as in transformers
+            return None
         return torch.tanh(torch.nn.functional.linear(self.last_hidden_state[:, 0], m.pooler.dense.weight,
                                                      m.pooler.dense.bias))
 
@@ -569,9 +573,25 @@ def _load_weight_file(path):
     return torch.load(path, map_location="cpu", weights_only=True)
 
 
+def _no_checkpoint(cls_name, name):
+    """from_pretrained found no checkpoint: an error unless V2S_ALLOW_RANDOM_INIT=1, then a note on stderr (once)."""
+    if os.environ.get("V2S_ALLOW_RANDOM_INIT", "0") != "1":
+        raise OSError(
+            f"vit2spn.{cls_name}.from_pretrained({name!r}): no local checkpoint, nothing in the HuggingFace cache and "
+            "the hub is not reachable.  The reference starts from these pretrained weights; set "
+            "V2S_ALLOW_RANDOM_INIT=1 to start from HF random initialisation instead.")
+    global _warned_random_init
+    if not _warned_random_init:
+        print(f"vit2spn: from_pretrained({name!r}) found no checkpoint; V2S_ALLOW_RANDOM_INIT=1 -> RANDOM INIT "
+              "(ViT-Tiny/16, HF _init_weights), not the pretrained weights", file=sys.stderr, flush=True)
+        _warned_random_init = True
+
+
 class ViTModel(nn.Module):
     """Drop-in for ``transformers.ViTModel`` as used by the reference (ViT-Tiny/16@224 only).  ``use_mask_token=True``
-    adds transformers' ``embeddings.mask_token`` (zeros [1,1,192]) for ``forward(..., bool_masked_pos=...)``."""
+    adds transformers' ``embeddings.mask_token`` (zeros [1,1,192]) for ``forward(..., bool_masked_pos=...)``.
+    ``add_pooling_layer=False`` drops the pooler from the module (parameters, ``state_dict``; ``pooler_output`` is None),
+    as in transformers; its two tensors stay in the flat store, whose layout always holds 200 tensors."""
 
     def __init__(self, config=None, add_pooling_layer=True, use_mask_token=False, **kw):
         super().__init__()
@@ -606,8 +626,9 @@ class ViTModel(nn.Module):
         enc.layer = nn.ModuleList(layers)
         self.encoder = enc
         self.layernorm = nn.LayerNorm(192, eps=1e-12)
-        self.pooler = _Holder()
-        self.pooler.dense = _linear(192, 192)
+        pooler = _Holder()
+        pooler.dense = _linear(192, 192)
+        self.pooler = pooler if add_pooling_layer else None
         # HF _init_weights (modeling_vit.py:384-398)
         with torch.no_grad():
             for m in self.modules():
@@ -619,7 +640,10 @@ class ViTModel(nn.Module):
                     nn.init.zeros_(m.bias)
             nn.init.trunc_normal_(emb.cls_token, mean=0.0, std=std)
             nn.init.trunc_normal_(emb.position_embeddings, mean=0.0, std=std)
-        params = list(self.parameters())
+            if not add_pooling_layer:
+                nn.init.trunc_normal_(pooler.dense.weight, mean=0.0, std=std)
+                nn.init.zeros_(pooler.dense.bias)
+        params = list(self.parameters()) + ([] if add_pooling_layer else list(pooler.parameters()))
         assert len(params) == 200
         self._store = FlatStore(params, _lib.backbone_layout(), _lib.BACKBONE_NUMEL, _lib.BACKBONE_ACTIVE_NUMEL)
         if use_mask_token:
@@ -645,16 +669,7 @@ class ViTModel(nn.Module):
         model = cls(ViTConfig(**cfg_kw), use_mask_token=bool(kw.get("use_mask_token", False)))
         path = _resolve_checkpoint(str(name))
         if path is None:
-            if os.environ.get("V2S_ALLOW_RANDOM_INIT", "0") != "1":
-                raise OSError(
-                    f"vit2spn.ViTModel.from_pretrained({name!r}): no local checkpoint, nothing in the HuggingFace cache and "
-                    "the hub is not reachable.  The reference starts from these pretrained weights; set "
-                    "V2S_ALLOW_RANDOM_INIT=1 to start from HF random initialisation instead.")
-            global _warned_random_init
-            if not _warned_random_init:
-                print(f"vit2spn: from_pretrained({name!r}) found no checkpoint; V2S_ALLOW_RANDOM_INIT=1 -> RANDOM INIT "
-                      "(ViT-Tiny/16, HF _init_weights), not the pretrained weights", file=sys.stderr, flush=True)
-                _warned_random_init = True
+            _no_checkpoint("ViTModel", name)
             return model
         sd = _load_weight_file(path)
         sd = {k[4:] if k.startswith("vit.") else k: v for k, v in sd.items()}
@@ -726,6 +741,171 @@ class ViTModel(nn.Module):
         hidden = tuple(res[1:13]) + (last,) if want_hidden else None
         attentions = tuple(res[13:] if want_hidden else res[1:]) if want_attn else None
         return ViTModelOutput(self, last, hidden, attentions)
+
+
+# ---------------------------------------------------------------------------------------------
+# ViTForMaskedImageModeling (SimMIM)
+# ---------------------------------------------------------------------------------------------
+def _mim_workspace(device, batch, mode, keep):
+    """Workspace of the SimMIM head: a fresh one when the forward keeps state for its backward, else a cached scratch."""
+    det = _deterministic()                 # the deterministic mode's scratch is part of the size
+    nbytes = lib.v2s_mim_workspace_bytes(batch, mode)
+    if nbytes < 0:
+        raise RuntimeError("v2s_mim_workspace_bytes: bad arguments")
+    if keep:
+        return torch.empty(nbytes + 1024, dtype=torch.uint8, device=device)
+    key = ("mim", device, batch, mode, det)
+    ws = _workspaces.get(key)
+    if ws is None:
+        ws = _workspaces[key] = torch.empty(nbytes + 1024, dtype=torch.uint8, device=device)
+    return ws
+
+
+def _aligned16(t):
+    return t if t is None or t.data_ptr() % 16 == 0 else t.clone()
+
+
+class _MIMHeadFn(torch.autograd.Function):
+    """hidden_states[12] -> (reconstruction, loss) of transformers' ViTForMaskedImageModeling in the CUDA library
+    (v2s_mim_forward / v2s_mim_backward): the final LayerNorm of the patch rows, the 1x1-conv decoder with
+    PixelShuffle(16) and, with a mask, the masked L1 loss.  The backward returns d hidden_states[12] (to the backbone's
+    Function), the LayerNorm and decoder gradients as tensors, and the direct pixel term -c sign(r - x) of the loss (the
+    backbone adds its own).  The reconstruction is not differentiable: a loss must not use it."""
+
+    @staticmethod
+    @_with_device_of(lambda ctx, hidden, *a, **k: hidden)
+    def forward(ctx, hidden, x, ln_w, ln_b, dec_w, dec_b, model, mask, need_grad):
+        mode = model.vit._mode()
+        B, dev = hidden.shape[0], hidden.device
+        keep = need_grad and mask is not None
+        hidden = _aligned16(hidden.detach().contiguous())
+        gam, bet = _aligned16(ln_w.detach()), _aligned16(ln_b.detach())
+        w, b = _aligned16(dec_w.detach().reshape(768, 192).contiguous()), _aligned16(dec_b.detach().contiguous())
+        xs = _aligned16(x.detach()) if mask is not None else None
+        rec = torch.empty(B, 3, 224, 224, dtype=torch.float32, device=dev)
+        loss = torch.empty((), dtype=torch.float32, device=dev) if mask is not None else None
+        ws = _mim_workspace(dev, B, mode, keep)
+        base, nbytes = _aligned(ws)
+        check(lib.v2s_mim_forward(ptr(hidden), ptr(gam), ptr(bet), ptr(w), ptr(b), ptr(xs), ptr(mask), ptr(rec), ptr(loss),
+                                  int(keep), B, mode, C.c_void_p(base), nbytes, stream_ptr()), "mim_forward")
+        ctx.set_materialize_grads(False)
+        ctx.ws = ws if keep else None
+        ctx.mode, ctx.B = mode, B
+        ctx.keep = (hidden, gam, w, mask)
+        return (rec, loss) if mask is not None else rec
+
+    @staticmethod
+    @_with_device_of(lambda ctx, drec, *rest: drec if drec is not None else next((t for t in rest if t is not None), None))
+    def backward(ctx, drec, dloss=None):
+        if drec is not None:
+            raise RuntimeError("vit2spn: ViTForMaskedImageModeling's reconstruction is not differentiable; train through "
+                               "its loss, or detach the reconstruction before it enters a loss")
+        nones = (None,) * 9
+        if dloss is None:
+            return nones
+        if ctx.ws is None:
+            raise RuntimeError("vit2spn: backward through a SimMIM forward that saved nothing (twice, or without grad)")
+        hidden, gam, w, mask = ctx.keep
+        need = ctx.needs_input_grad
+        dev = hidden.device
+        _deterministic()
+        dl = _grad_f32(dloss.reshape(1))
+        dh = torch.empty(ctx.B, 197, 192, dtype=torch.float32, device=dev) if need[0] else None
+        dx = torch.zeros(ctx.B, 3, 224, 224, dtype=torch.float32, device=dev) if need[1] else None
+        want_ln = need[2] or need[3]
+        dg = torch.zeros(192, dtype=torch.float32, device=dev) if want_ln else None
+        db = torch.zeros(192, dtype=torch.float32, device=dev) if want_ln else None
+        dw = torch.zeros(768, 192, dtype=torch.float32, device=dev) if need[4] else None
+        dbd = torch.zeros(768, dtype=torch.float32, device=dev) if need[5] else None
+        base, nbytes = _aligned(ctx.ws)
+        check(lib.v2s_mim_backward(ptr(hidden), ptr(gam), ptr(w), ptr(mask), ptr(dl), ptr(dh), ptr(dx), ptr(dg), ptr(db),
+                                   ptr(dw), ptr(dbd), ctx.B, ctx.mode, C.c_void_p(base), nbytes, stream_ptr()), "mim_backward")
+        ctx.ws = None
+        return (dh, dx, dg if need[2] else None, db if need[3] else None,
+                dw.view(768, 192, 1, 1) if dw is not None else None, dbd, None, None, None)
+
+
+class MaskedImageModelingOutput:
+    """As transformers' ``MaskedImageModelingOutput``: ``loss`` (None without ``bool_masked_pos``), ``reconstruction``
+    [B,3,224,224] fp32, ``hidden_states`` / ``attentions`` (tuples when requested, else None)."""
+
+    def __init__(self, loss, reconstruction, hidden_states=None, attentions=None):
+        self.loss, self.reconstruction = loss, reconstruction
+        self.hidden_states, self.attentions = hidden_states, attentions
+
+
+class ViTForMaskedImageModeling(nn.Module):
+    """Drop-in for ``transformers.ViTForMaskedImageModeling`` (SimMIM; ViT-Tiny/16@224, encoder_stride 16): ``vit`` is a
+    ``ViTModel(config, add_pooling_layer=False, use_mask_token=True)`` and ``decoder`` is ``Conv2d(192, 768, 1)`` +
+    ``PixelShuffle(16)``, so ``state_dict`` keys and strict loads match transformers.  The final LayerNorm, the decoder
+    and the masked L1 loss run as one CUDA head after the CUDA backbone (the Conv2d is only a parameter container)."""
+
+    def __init__(self, config=None, **kw):
+        super().__init__()
+        config = config or ViTConfig(**kw)
+        if getattr(config, "encoder_stride", 16) != 16:
+            raise ValueError(f"vit2spn.ViTForMaskedImageModeling: encoder_stride must be 16 (the patch size), got "
+                             f"{config.encoder_stride}")
+        self.config = config
+        self.vit = ViTModel(config, add_pooling_layer=False, use_mask_token=True)
+        self.decoder = nn.Sequential(nn.Conv2d(192, 16 ** 2 * 3, kernel_size=1), nn.PixelShuffle(16))
+        with torch.no_grad():          # transformers' _init_weights for Conv2d
+            nn.init.trunc_normal_(self.decoder[0].weight, mean=0.0, std=config.initializer_range)
+            nn.init.zeros_(self.decoder[0].bias)
+
+    @property
+    def compute_mode(self):
+        return self.vit.compute_mode
+
+    @compute_mode.setter
+    def compute_mode(self, mode):
+        self.vit.compute_mode = mode
+
+    @classmethod
+    def from_pretrained(cls, name, **kw):
+        """Loads ``vit.*`` and, when present, ``decoder.*`` (a ViTModel checkpoint's keys are taken as ``vit.*``); the
+        same policy as ``ViTModel.from_pretrained`` for missing checkpoints and mismatching keys.  A checkpoint without
+        decoder or mask token keeps their transformers initialisation."""
+        cfg_kw = {k: v for k, v in kw.items() if k in ("output_hidden_states", "output_attentions")}
+        model = cls(ViTConfig(**cfg_kw))
+        path = _resolve_checkpoint(str(name))
+        if path is None:
+            _no_checkpoint("ViTForMaskedImageModeling", name)
+            return model
+        sd = _load_weight_file(path)
+        sd = {k if k.startswith(("vit.", "decoder.")) else "vit." + k: v for k, v in sd.items()}
+        res = model.load_state_dict(sd, strict=False)
+        missing = [k for k in res.missing_keys if not k.startswith("decoder.") and k != "vit.embeddings.mask_token"]
+        unexpected = [k for k in res.unexpected_keys if not k.startswith(("vit.pooler.", "vit.classifier.", "classifier."))]
+        print(f"vit2spn: loaded {path} ({len(sd) - len(res.unexpected_keys)} tensors; missing {res.missing_keys or 'none'}; "
+              f"unexpected {res.unexpected_keys or 'none'})", file=sys.stderr, flush=True)
+        if missing or unexpected:
+            raise RuntimeError(f"vit2spn.ViTForMaskedImageModeling.from_pretrained({name!r}): checkpoint does not match "
+                               f"ViT-Tiny/16: missing {missing}, unexpected {unexpected}")
+        return model
+
+    def forward(self, pixel_values, bool_masked_pos=None, output_hidden_states=None, output_attentions=None, **kw):
+        """As transformers: ``reconstruction`` always, ``loss`` with ``bool_masked_pos`` ([B,196], nonzero = masked).
+        ``loss.backward()`` reaches the decoder, the final LayerNorm, the backbone, the mask token and, when it requires
+        grad, ``pixel_values`` (the loss's own term plus the backbone's)."""
+        if isinstance(pixel_values, torch.Tensor) and pixel_values.dim() == 3:
+            raise ValueError("vit2spn.ViTForMaskedImageModeling: 16-bit patch-row inputs are not accepted: the loss reads "
+                             "the fp32 pixels; pass pixel_values [B,3,224,224]")
+        if kw.get("interpolate_pos_encoding"):
+            raise ValueError("vit2spn.ViTForMaskedImageModeling: interpolate_pos_encoding=True is not supported (224x224 "
+                             "inputs only)")
+        out = self.vit(pixel_values, output_hidden_states=output_hidden_states, output_attentions=output_attentions,
+                       bool_masked_pos=bool_masked_pos)
+        x = _check_images(pixel_values)
+        mask = ViTModel._mask_arg(bool_masked_pos, x) if bool_masked_pos is not None else None
+        hidden = out.hidden_states[-1]
+        ln, conv = self.vit.layernorm, self.decoder[0]
+        tensors = (hidden, x, ln.weight, ln.bias, conv.weight, conv.bias)
+        need_grad = torch.is_grad_enabled() and any(t.requires_grad for t in tensors)
+        res = _MIMHeadFn.apply(*tensors, self, mask, need_grad)
+        rec, loss = res if mask is not None else (res, None)
+        hs = out.hidden_states if isinstance(out.hidden_states, tuple) else None
+        return MaskedImageModelingOutput(loss, rec, hs, out.attentions)
 
 
 class ViTBackbone(nn.Module):

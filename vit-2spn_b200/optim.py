@@ -129,7 +129,9 @@ class FusedAdam(torch.optim.Optimizer):
 
     def zero_grad(self, set_to_none: bool = True):
         """Flat-buffer fast path: ONE memset per store, ``.grad`` views stay attached (they read as zeros
-        instead of None).  Parameters outside vit2spn stores follow torch's semantics."""
+        instead of None).  Parameters outside vit2spn stores, and those of a store whose ``.grad`` is not a view of its
+        flat gradient buffer (the final LayerNorm and the pooler, which autograd gives gradients of their own), follow
+        torch's semantics."""
         handled = set()
         mine = self._all_param_ids()
         for store in list(_STORES):
@@ -137,7 +139,8 @@ class FusedAdam(torch.optim.Optimizer):
             if store.flat_grad is None or not all(id(p) in mine for p in store.params if p.requires_grad):
                 continue
             if store.zero_grads_fast():
-                handled.update(id(p) for p in store.params)
+                handled.update(id(p) for p, v in zip(store.params, store._grad_views)
+                               if p.grad is not None and p.grad.data_ptr() == v.data_ptr())
         for group in self.param_groups:
             for p in group["params"]:
                 if id(p) in handled or p.grad is None:
