@@ -29,7 +29,8 @@ extern "C" {
 #define V2S_ABI_VERSION 5 /* 5: the backbone calls added to 4 (image, attention-probability and mask-token gradients,
                              masked forward) are folded into v2s_backbone_forward / _backward: their arguments are
                              fields of v2s_group_outputs, and v2s_backbone_backward takes weight_grads.  Additive to 5:
-                             v2s_mim_workspace_bytes, v2s_mim_forward, v2s_mim_backward.  Additive to 4:
+                             v2s_mim_workspace_bytes, v2s_mim_forward, v2s_mim_backward, v2s_cls_workspace_bytes, v2s_cls_forward,
+                             v2s_cls_backward.  Additive to 4:
                              v2s_test_gemm which = 5, v2s_test_attention which = 3.  4: one entry point per operation:
                              v2s_backbone_forward / _backward take the per-group outputs and (backward) the layer range,
                              v2s_heads_loss_fwd_bwd the device loss scale, v2s_adam_step and v2s_ema_update the
@@ -208,6 +209,36 @@ int v2s_mim_backward(const float* hidden, const float* ln_gamma, const float* de
                      const float* dloss_dev, float* dhidden, float* dpixels, float* d_ln_gamma, float* d_ln_beta,
                      float* d_dec_w, float* d_dec_b, int batch, int mode, void* workspace, int64_t workspace_bytes,
                      void* stream);
+
+/* Classification head of transformers' ViTForImageClassification on the CUDA path.  Forward: xhat = the final LayerNorm
+ * (eps 1e-12) of the CLS rows of hidden [batch,197,192] (hidden_states[12]); logits [batch, num_labels] fp32 =
+ * xhat cls_w^T + cls_b, always written (cls_w [num_labels,192] and cls_b fp32; the 16-bit modes cast a copy of cls_w,
+ * padded with zero rows to a multiple of 8, into the workspace).  loss_kind (V2S_CLS_LOSS_*) != NONE also writes loss (1
+ * float), the mean of transformers' loss over its labels, bit-reproducible (fixed summation order):
+ *   CE:  labels int64 [batch]; cross-entropy, -100 ignored, mean over the other rows (all ignored: NaN, as torch).  A
+ *        label outside [0, num_labels) other than -100 makes the loss NaN; it is never used as an index.
+ *   MSE: labels fp32 [batch, num_labels]; mean squared error over all elements.
+ *   BCE: labels fp32 [batch, num_labels]; binary cross-entropy with logits, mean over all elements.
+ * with_backward != 0 keeps in the workspace what v2s_cls_backward reads (xhat, its statistics, the unscaled loss
+ * gradient, the label count, the cls_w copy): pass the same workspace, batch, mode, num_labels, loss_kind and hidden.
+ * Backward: G = (*dloss_dev / count) d loss-sum / d logits + dlogits, formed in fp32 and cast to the GEMM operand type.
+ * dloss_dev (the loss's upstream gradient, read on the device: GradScaler's scale included; needs a loss) and dlogits
+ * (fp32 [batch, num_labels]) may each be NULL, not both.  dhidden [batch,197,192] is overwritten (patch rows 0; NULL =
+ * not wanted); d_ln_gamma / d_ln_beta, d_cls_w / d_cls_b (NULL = frozen) are accumulated (+=).  Stages whose outputs are
+ * all NULL are skipped.  Deterministic mode (v2s_set_deterministic): fixed-order sums; size the workspace while the
+ * switch is on. */
+#define V2S_CLS_LOSS_NONE 0
+#define V2S_CLS_LOSS_CE 1
+#define V2S_CLS_LOSS_MSE 2
+#define V2S_CLS_LOSS_BCE 3
+int64_t v2s_cls_workspace_bytes(int batch, int num_labels, int mode);
+int v2s_cls_forward(const float* hidden, const float* ln_gamma, const float* ln_beta, const float* cls_w, const float* cls_b,
+                    int num_labels, int loss_kind, const void* labels, float* logits, float* loss, int with_backward,
+                    int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream);
+int v2s_cls_backward(const float* hidden, const float* ln_gamma, const float* cls_w, int num_labels, int loss_kind,
+                     const void* labels, const float* dlogits, const float* dloss_dev, float* dhidden, float* d_ln_gamma,
+                     float* d_ln_beta, float* d_cls_w, float* d_cls_b, int batch, int mode, void* workspace,
+                     int64_t workspace_bytes, void* stream);
 
 /* nn.CosineSimilarity(dim=1) loss of ref:174,211 and (optionally, dpred != NULL) its gradient */
 int v2s_cosine_loss(const float* pred, const float* target_proj, float* loss, float* dpred, int batch,

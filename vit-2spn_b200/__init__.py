@@ -6,7 +6,8 @@ The directory is named ``vit-2spn_b200`` (not importable by the ``import`` state
 """
 from ._lib import LIB_PATH, EXPORTED, MODE_BF16, MODE_FP32  # noqa: F401  (raises if the .so is missing)
 from .modules import (DualStreamNetwork, FineTunedModel, InfoNCELoss, SingleStreamNetwork, ViTBackbone, ViTConfig, ViTModel,  # noqa: F401
-                      ViTForMaskedImageModeling, get_compute_mode, momentum, preprocess_u8_patches, set_compute_mode)
+                      ViTForImageClassification, ViTForMaskedImageModeling, get_compute_mode, momentum,
+                      preprocess_u8_patches, set_compute_mode)
 from .optim import FusedAdam  # noqa: F401
 from . import augment, explain, parallel  # noqa: F401
 from .train import (accumulation_steps, batch_size, epochs, learning_rate, load_checkpoint,  # noqa: F401

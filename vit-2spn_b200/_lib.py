@@ -16,6 +16,7 @@ MODE_BF16 = 1
 MODE_FP16 = 2
 LP_BF16 = 0
 LP_FP16 = 1
+CLS_LOSS_NONE, CLS_LOSS_CE, CLS_LOSS_MSE, CLS_LOSS_BCE = 0, 1, 2, 3   # V2S_CLS_LOSS_*
 MAX_GROUPS = 4
 ABI_VERSION = 5      # V2S_ABI_VERSION of include/vit2spn.h that the signatures below bind
 
@@ -78,6 +79,9 @@ _SIGS = {
     "v2s_mim_workspace_bytes": (_i64, [_i, _i]),
     "v2s_mim_forward": (C.c_int, [_vp] * 9 + [_i, _i, _i, _vp, _i64, _vp]),
     "v2s_mim_backward": (C.c_int, [_vp] * 11 + [_i, _i, _vp, _i64, _vp]),
+    "v2s_cls_workspace_bytes": (_i64, [_i, _i, _i]),
+    "v2s_cls_forward": (C.c_int, [_vp] * 5 + [_i, _i, _vp, _vp, _vp, _i, _i, _i, _vp, _i64, _vp]),
+    "v2s_cls_backward": (C.c_int, [_vp] * 3 + [_i, _i] + [_vp] * 8 + [_i, _i, _vp, _i64, _vp]),
     "v2s_cosine_loss": (C.c_int, [_vp, _vp, _vp, _vp, _i, _i, _f, _vp]),
     "v2s_infonce_loss": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i64, _f, _i, _f, _vp, _vp]),
     "v2s_dropout_mask": (C.c_int, [_vp, _i64, _f, C.c_uint64, C.c_uint64, _vp]),

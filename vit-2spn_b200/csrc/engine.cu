@@ -34,9 +34,11 @@ static int n_recs = 0;
 static int n_events = 0;   // events created so far (recs[i].a/b valid for i < n_events)
 static const char* names[] = {"gemm_patch", "gemm_qkv", "gemm_proj", "gemm_fc1", "gemm_fc2", "gemm_dgrad",
                               "gemm_wgrad", "attn_fwd", "attn_bwd", "ln_fwd", "ln_bwd", "colsum", "misc", "heads", "gemm_mlp_fwd",
-                              "gemm_mlp_bwd", "attn_probs", "gemm_pixels", "attn_dprobs", "mim_fwd", "mim_bwd"};
+                              "gemm_mlp_bwd", "attn_probs", "gemm_pixels", "attn_dprobs", "mim_fwd", "mim_bwd",
+                              "cls_fwd", "cls_bwd"};
 enum { C_PATCH, C_QKV, C_PROJ, C_FC1, C_FC2, C_DGRAD, C_WGRAD, C_ATTN_F, C_ATTN_B, C_LN_F, C_LN_B, C_COLSUM, C_MISC,
-       C_HEADS, C_MLP_F, C_MLP_B, C_ATTN_P, C_PIX, C_ATTN_DP, C_MIM_F, C_MIM_B, C_COUNT };
+       C_HEADS, C_MLP_F, C_MLP_B, C_ATTN_P, C_PIX, C_ATTN_DP, C_MIM_F, C_MIM_B, C_CLS_F,
+       C_CLS_B, C_COUNT };
 struct Scope {
   int idx = -1;
   cudaStream_t st;
@@ -1046,7 +1048,8 @@ MimBufs mim_plan(int B, int mode, char* base) {
   m.bytes = o;
   return m;
 }
-int64_t mim_det_bytes() {
+// deterministic scratch of a head's backward (SimMIM, classifier): its weight-gradient GEMM and final-LayerNorm backward
+int64_t head_det_bytes() {
   int64_t part = gemm_tc_det_part_floats();
   if (part < (int64_t)296 * DF) part = (int64_t)296 * DF;
   return align_up(DET_COUNTERS * sizeof(unsigned)) + align_up(part * 4);
@@ -1088,7 +1091,7 @@ static int mim_forward_impl(const float* hidden, const float* ln_gamma, const fl
   {
     const float* x[1] = {hidden}; const float* g[1] = {ln_gamma}; const float* b[1] = {ln_beta};
     void* y[1] = {m.seq}; float* mu[1] = {m.mean}; float* rs[1] = {m.rstd};
-    V2S_TRY(launch_ln_fwd(x, g, b, y, mu, rs, 1, MP, at, st, true));
+    V2S_TRY(launch_ln_fwd(x, g, b, y, mu, rs, 1, MP, at, st, LN_PATCH_ROWS));
   }
   GemmDesc d = make_gemm_desc();
   d.M = MP; d.N = KPE; d.K = D; d.groups = 1;
@@ -1133,7 +1136,7 @@ static int mim_backward_impl(const float* hidden, const float* ln_gamma, const f
   DetScratch det_s;
   const DetScratch* det = nullptr;
   if (tc_deterministic() && (d_dec_w || d_dec_b || d_ln_gamma)) {
-    const int64_t bytes = mim_det_bytes();
+    const int64_t bytes = head_det_bytes();
     if (ws_bytes < m.bytes + bytes) {
       set_error("mim_backward: deterministic mode: workspace too small (size it with v2s_mim_workspace_bytes while the "
                 "switch is on)");
@@ -1189,6 +1192,179 @@ static int mim_backward_impl(const float* hidden, const float* ln_gamma, const f
                               m.denom, MP, st, det));
   }
   if (dpixels) V2S_TRY(launch_mim_pixel_grad(m.dsign, dpixels, B, at, dloss, m.denom, st));
+  return 0;
+}
+
+// =============================================================================================
+// Classification head (ViTForImageClassification): final LayerNorm of the CLS rows, the linear classifier and its loss,
+// forward and backward
+// =============================================================================================
+namespace {
+struct ClsBufs {
+  char *xhat, *wlp, *g;
+  float *mean, *rstd, *z, *dz, *part, *cnt, *count, *dxhat;
+  int ldz;                                         // num_labels rounded up to a multiple of 8 (gemm_tc's N and K)
+  int64_t bytes;                                   // without the deterministic scratch
+};
+// workspace: xhat [B,192] (activation type) | mean, rstd [B] | W_cls 16-bit copy [ldz,192] (padding rows zero) | logit
+// GEMM rows z [B,ldz] | unscaled loss gradient dz [B,ldz] | row terms, row counts [B] | label count | G [B,ldz] (activation
+// type) | d xhat [B,192] fp32 | deterministic scratch (while the switch is on)
+ClsBufs cls_plan(int B, int N, int mode, char* base) {
+  const int64_t es = mode == V2S_MODE_FP32 ? 4 : 2;
+  ClsBufs c;
+  int64_t o = 0;
+  auto take = [&](int64_t bytes) { char* r = base + o; o += align_up(bytes); return r; };
+  c.ldz = (N + 7) / 8 * 8;
+  c.xhat = take((int64_t)B * D * es);
+  c.mean = (float*)take((int64_t)B * 4);
+  c.rstd = (float*)take((int64_t)B * 4);
+  c.wlp = take(mode == V2S_MODE_FP32 ? 0 : (int64_t)c.ldz * D * 2);
+  c.z = (float*)take((int64_t)B * c.ldz * 4);
+  c.dz = (float*)take((int64_t)B * c.ldz * 4);
+  c.part = (float*)take((int64_t)B * 4);
+  c.cnt = (float*)take((int64_t)B * 4);
+  c.count = (float*)take(4);
+  c.g = take((int64_t)B * c.ldz * es);
+  c.dxhat = (float*)take((int64_t)B * D * 4);
+  c.bytes = o;
+  return c;
+}
+bool cls_args_ok(int B, int N, int mode) {
+  return B >= 1 && N >= 1 && N <= 65536 && mode >= V2S_MODE_FP32 && mode <= V2S_MODE_FP16;
+}
+int cls_resolve(int B, int N, int mode, int kind, const void* labels, void* ws, int64_t ws_bytes, ClsBufs* c) {
+  if (!cls_args_ok(B, N, mode)) { set_error("cls: bad batch, num_labels (1..65536) or mode"); return 1; }
+  if (kind < V2S_CLS_LOSS_NONE || kind > V2S_CLS_LOSS_BCE) { set_error("cls: bad loss_kind %d", kind); return 1; }
+  if ((kind == V2S_CLS_LOSS_NONE) != (labels == nullptr)) { set_error("cls: labels go with a loss_kind, and only with one"); return 1; }
+  if (misaligned16(labels)) { set_error("cls: labels must be 16-byte aligned"); return 1; }
+  if (!ws || (reinterpret_cast<uintptr_t>(ws) & 1023)) { set_error("cls: the workspace must be 1024-byte aligned"); return 1; }
+  *c = cls_plan(B, N, mode, static_cast<char*>(ws));
+  if (ws_bytes < c->bytes) {
+    set_error("cls: workspace too small: have %lld bytes, need %lld (v2s_cls_workspace_bytes)", (long long)ws_bytes,
+              (long long)c->bytes);
+    return 1;
+  }
+  return 0;
+}
+}  // namespace
+
+static int cls_forward_impl(const float* hidden, const float* ln_gamma, const float* ln_beta, const float* cls_w,
+                            const float* cls_b, int N, int kind, const void* labels, float* logits, float* loss,
+                            int with_backward, int B, int mode, void* ws, int64_t ws_bytes, cudaStream_t st) {
+  if (!hidden || !ln_gamma || !ln_beta || !cls_w || !cls_b || !logits || ((kind != V2S_CLS_LOSS_NONE) != (loss != nullptr))) {
+    set_error("cls_forward: null argument (loss goes with a loss_kind, and only with one)");
+    return 1;
+  }
+  if (misaligned16(hidden) || misaligned16(ln_gamma) || misaligned16(ln_beta) || misaligned16(cls_w) || misaligned16(cls_b) ||
+      misaligned16(logits)) {
+    set_error("cls_forward: hidden, LayerNorm and classifier parameters and logits must be 16-byte aligned");
+    return 1;
+  }
+  ClsBufs c;
+  V2S_TRY(cls_resolve(B, N, mode, kind, labels, ws, ws_bytes, &c));
+  const int at = make_plan(B, mode).at;
+  prof::Scope sc(prof::C_CLS_F, 2.0 * B * c.ldz * (double)D, st,
+                 (double)B * D * 4 * 2 + (double)N * D * 4 + (double)B * c.ldz * 4 * 2 + (double)B * N * 4);
+  {
+    const float* x[1] = {hidden}; const float* g[1] = {ln_gamma}; const float* b[1] = {ln_beta};
+    void* y[1] = {c.xhat}; float* mu[1] = {c.mean}; float* rs[1] = {c.rstd};
+    V2S_TRY(launch_ln_fwd(x, g, b, y, mu, rs, 1, B, at, st, LN_CLS_ROWS));
+  }
+  GemmDesc d = make_gemm_desc();
+  d.M = B; d.K = D; d.groups = 1;
+  d.a_rs = D; d.a_cs = 1; d.b_rs = 1; d.b_cs = D; d.ldc = c.ldz; d.epi = EPI_STORE;
+  d.A[0] = c.xhat; d.out[0] = c.z;
+  if (at) {        // tensor cores: the zero-padded 16-bit copy of W_cls, then logits z = xhat W^T over ldz columns
+    if (c.ldz > N) V2S_CUDA_OK(cudaMemsetAsync(c.wlp + (int64_t)N * D * 2, 0, (int64_t)(c.ldz - N) * D * 2, st));
+    V2S_TRY(launch_cast_lp(cls_w, c.wlp, (int64_t)N * D, st, at == AT_F16));
+    d.N = c.ldz; d.B[0] = c.wlp;
+    int handled = 0;
+    V2S_TRY(launch_gemm_tc(d, at, at, 0, st, &handled));
+    if (!handled) { set_error("cls_forward: the tensor-core logit GEMM declined the problem"); return 1; }
+  } else {
+    d.N = N; d.B[0] = cls_w;
+    V2S_TRY(launch_gemm_simt(d, AT_F32, AT_F32, AT_F32, st));
+  }
+  V2S_TRY(launch_cls_head_rows(c.z, c.ldz, cls_b, N, kind, labels, logits, with_backward ? c.dz : nullptr, c.part, c.cnt, B, st));
+  if (kind != V2S_CLS_LOSS_NONE) V2S_TRY(launch_cls_head_loss_finish(c.part, c.cnt, B, loss, c.count, st));
+  return 0;
+}
+
+static int cls_backward_impl(const float* hidden, const float* ln_gamma, const float* cls_w, int N, int kind,
+                             const void* labels, const float* dlogits, const float* dloss, float* dhidden,
+                             float* d_ln_gamma, float* d_ln_beta, float* d_cls_w, float* d_cls_b, int B, int mode, void* ws,
+                             int64_t ws_bytes, cudaStream_t st) {
+  if (!hidden || !ln_gamma || !cls_w || (!dlogits && !dloss) || (dloss && kind == V2S_CLS_LOSS_NONE)) {
+    set_error("cls_backward: null argument (a backward needs dlogits or dloss_dev, and dloss_dev a loss_kind)");
+    return 1;
+  }
+  if ((d_ln_gamma == nullptr) != (d_ln_beta == nullptr)) { set_error("cls_backward: d_ln_gamma and d_ln_beta go together"); return 1; }
+  if (misaligned16(hidden) || misaligned16(ln_gamma) || misaligned16(cls_w) || misaligned16(dlogits) || misaligned16(dhidden) ||
+      misaligned16(d_cls_w)) {
+    set_error("cls_backward: hidden, ln_gamma, cls_w, dlogits, dhidden and d_cls_w must be 16-byte aligned");
+    return 1;
+  }
+  ClsBufs c;
+  V2S_TRY(cls_resolve(B, N, mode, kind, labels, ws, ws_bytes, &c));
+  const bool wgrad = d_cls_w || d_cls_b, lnb = dhidden || d_ln_gamma;
+  if (!wgrad && !lnb) return 0;
+  const int at = make_plan(B, mode).at;
+  const int64_t es = at ? 2 : 4;
+  DetScratch det_s;
+  const DetScratch* det = nullptr;
+  if (tc_deterministic() && (d_cls_w || d_ln_gamma)) {
+    const int64_t bytes = head_det_bytes();
+    if (ws_bytes < c.bytes + bytes) {
+      set_error("cls_backward: deterministic mode: workspace too small (size it with v2s_cls_workspace_bytes while the "
+                "switch is on)");
+      return 1;
+    }
+    char* tail = static_cast<char*>(ws) + c.bytes;
+    det_s.counters = reinterpret_cast<unsigned*>(tail);
+    det_s.part = reinterpret_cast<float*>(tail + align_up(DET_COUNTERS * sizeof(unsigned)));
+    det_s.part_floats = (bytes - align_up(DET_COUNTERS * sizeof(unsigned))) / 4;
+    V2S_CUDA_OK(cudaMemsetAsync(det_s.counters, 0, DET_COUNTERS * sizeof(unsigned), st));
+    det = &det_s;
+  }
+  prof::Scope sc(prof::C_CLS_B, 2.0 * B * c.ldz * (double)D * ((wgrad ? 1 : 0) + (lnb ? 1 : 0)), st,
+                 (double)B * c.ldz * (4 + es) + (wgrad ? (double)N * D * 4 * 2 : 0.0) +
+                     (lnb ? (double)B * D * 4 * 3 + (dhidden ? (double)B * NT * D * 4 : 0.0) : 0.0));
+  // G = c dz + dlogits in the GEMM operand type
+  V2S_TRY(launch_cls_head_grad(dloss ? c.dz : nullptr, dlogits, dloss, c.count, c.g, B, N, c.ldz, at, st));
+  if (d_cls_w) {
+    // dW += G^T xhat over the num_labels real rows, with d b += the row sums of G^T on the tensor cores
+    GemmDesc d = make_gemm_desc();
+    d.M = N; d.N = D; d.K = B; d.groups = 1;
+    d.a_rs = 1; d.a_cs = c.ldz; d.b_rs = D; d.b_cs = 1; d.ldc = D; d.epi = EPI_ACCUM;
+    d.A[0] = c.g; d.B[0] = c.xhat; d.out[0] = d_cls_w;
+    if (at) {
+      d.det = det; d.rowsum_out[0] = d_cls_b;
+      int handled = 0;
+      V2S_TRY(launch_gemm_tc(d, at, at, 0, st, &handled));
+      if (!handled) { set_error("cls_backward: the tensor-core classifier wgrad declined the problem"); return 1; }
+    } else {       // one K range per output element: a single atomic add each, so the order is fixed
+      V2S_TRY(launch_gemm_simt(d, AT_F32, AT_F32, AT_F32, st));
+    }
+  }
+  if (d_cls_b && !(d_cls_w && at)) V2S_TRY(launch_cls_head_colsum(c.g, c.ldz, B, N, at, d_cls_b, st));
+  if (lnb) {
+    // d xhat = G W_cls (fp32), then the final LayerNorm's backward into the CLS rows
+    GemmDesc d = make_gemm_desc();
+    d.M = B; d.N = D; d.K = at ? c.ldz : N; d.groups = 1;
+    d.a_rs = c.ldz; d.a_cs = 1; d.b_rs = D; d.b_cs = 1; d.ldc = D; d.epi = EPI_STORE;
+    d.A[0] = c.g; d.out[0] = c.dxhat;
+    if (at) {
+      d.B[0] = c.wlp;
+      int handled = 0;
+      V2S_TRY(launch_gemm_tc(d, at, at, 0, st, &handled));
+      if (!handled) { set_error("cls_backward: the tensor-core classifier dgrad declined the problem"); return 1; }
+    } else {
+      d.B[0] = cls_w;
+      V2S_TRY(launch_gemm_simt(d, AT_F32, AT_F32, AT_F32, st));
+    }
+    if (dhidden) V2S_CUDA_OK(cudaMemsetAsync(dhidden, 0, (int64_t)B * NT * D * 4, st));
+    V2S_TRY(launch_cls_head_ln_bwd(c.dxhat, hidden, c.mean, c.rstd, ln_gamma, dhidden, d_ln_gamma, d_ln_beta, B, st, det));
+  }
   return 0;
 }
 
@@ -1260,7 +1436,7 @@ int64_t v2s_workspace_bytes(int batch, int mode, int n_groups, int n_saved) {
 
 int64_t v2s_mim_workspace_bytes(int batch, int mode) {
   if (batch < 1 || mode < V2S_MODE_FP32 || mode > V2S_MODE_FP16) return -1;
-  return mim_plan(batch, mode, nullptr).bytes + (tc_deterministic() ? mim_det_bytes() : 0);
+  return mim_plan(batch, mode, nullptr).bytes + (tc_deterministic() ? head_det_bytes() : 0);
 }
 
 int v2s_mim_forward(const float* hidden, const float* ln_gamma, const float* ln_beta, const float* dec_w, const float* dec_b,
@@ -1276,6 +1452,26 @@ int v2s_mim_backward(const float* hidden, const float* ln_gamma, const float* de
                      void* stream) {
   return mim_backward_impl(hidden, ln_gamma, dec_w, mask, dloss_dev, dhidden, dpixels, d_ln_gamma, d_ln_beta, d_dec_w,
                            d_dec_b, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int64_t v2s_cls_workspace_bytes(int batch, int num_labels, int mode) {
+  if (!cls_args_ok(batch, num_labels, mode)) return -1;
+  return cls_plan(batch, num_labels, mode, nullptr).bytes + (tc_deterministic() ? head_det_bytes() : 0);
+}
+
+int v2s_cls_forward(const float* hidden, const float* ln_gamma, const float* ln_beta, const float* cls_w, const float* cls_b,
+                    int num_labels, int loss_kind, const void* labels, float* logits, float* loss, int with_backward,
+                    int batch, int mode, void* workspace, int64_t workspace_bytes, void* stream) {
+  return cls_forward_impl(hidden, ln_gamma, ln_beta, cls_w, cls_b, num_labels, loss_kind, labels, logits, loss,
+                          with_backward, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+int v2s_cls_backward(const float* hidden, const float* ln_gamma, const float* cls_w, int num_labels, int loss_kind,
+                     const void* labels, const float* dlogits, const float* dloss_dev, float* dhidden, float* d_ln_gamma,
+                     float* d_ln_beta, float* d_cls_w, float* d_cls_b, int batch, int mode, void* workspace,
+                     int64_t workspace_bytes, void* stream) {
+  return cls_backward_impl(hidden, ln_gamma, cls_w, num_labels, loss_kind, labels, dlogits, dloss_dev, dhidden, d_ln_gamma,
+                           d_ln_beta, d_cls_w, d_cls_b, batch, mode, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 int v2s_backbone_forward(const v2s_group_t* groups, const v2s_group_outputs_t* outputs, int n_groups, int batch, int mode,

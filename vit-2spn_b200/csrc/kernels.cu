@@ -192,9 +192,12 @@ __device__ __forceinline__ uint32_t pack_lp(float a, float b, int f16) {
   return *reinterpret_cast<uint32_t*>(&v);
 }
 
-// REMAP (SimMIM's final LayerNorm): output row r = b*196 + p normalises token row b*197 + 1 + p of x (the CLS rows are
-// dropped), so y, mean and rstd are compact patch rows
-template <typename T, bool REMAP = false>
+// token row of x read for compact row `row` of a LayerNorm kernel (LnRows, kernels.cuh)
+__device__ __forceinline__ int64_t ln_token_row(int row, int rows) {
+  return rows == LN_PATCH_ROWS ? row + row / NP + 1 : rows == LN_CLS_ROWS ? (int64_t)row * NT : row;
+}
+
+template <typename T, int ROWS = LN_ALL_ROWS>
 __global__ void __launch_bounds__(256) ln_fwd_kernel(const __grid_constant__ LnFwdP p) {
   // wait for the predecessor, THEN release the successor: a successor flagged "late wait" (gemm_tc.cu) relies on
   // everything before its predecessor being complete when it starts
@@ -212,7 +215,7 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const __grid_constant__ LnF
     bt[i] = reinterpret_cast<const float4*>(p.beta[g])[l + 16 * i];
   }
   for (int row = blockIdx.x * 16 + hw; row < p.M; row += gridDim.x * 16) {
-    const float4* xr = reinterpret_cast<const float4*>(x + (int64_t)(REMAP ? row + row / NP + 1 : row) * D);
+    const float4* xr = reinterpret_cast<const float4*>(x + ln_token_row(row, ROWS) * D);
     float4 v[3];
     float s = 0.f;
 #pragma unroll
@@ -292,10 +295,11 @@ struct LnBwdP {
   const float* denom;
 };
 
-// MIM (SimMIM's final LayerNorm, T = float): dy is c * (compact patch-row gradient [M = B*196, 192]) with
-// c = dloss / 3 / denom read on the device; x and dres are token rows [B,197,192] (row r -> b*197 + 1 + p), dres is
-// overwritten (NULL: parameter gradients only) and its CLS rows are set to zero
-template <typename T, bool DET, bool PARAMS, bool MIM = false>
+// ROWS != LN_ALL_ROWS (a head's final LayerNorm, T = float): dy is the compact row gradient [M, 192] fp32; x and dres
+// are token rows [B,197,192] (ln_token_row), dres is overwritten at those rows (NULL: parameter gradients only).
+// LN_PATCH_ROWS (SimMIM): dy is scaled by c = dloss / 3 / denom, read on the device, and the CLS rows of dres are set to
+// zero.  LN_CLS_ROWS (the classifier): dy is taken as it is, and the caller zeroes the patch rows of dres.
+template <typename T, bool DET, bool PARAMS, int ROWS = LN_ALL_ROWS>
 __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnBwdP p) {
   __shared__ __align__(16) float red[16][3 * D];          // 36 KB; float4 accesses
   // wait for the predecessor, THEN release the successor: a successor flagged "late wait" (gemm_tc.cu) relies on
@@ -315,11 +319,12 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnB
     gm[i] = reinterpret_cast<const float4*>(p.gamma[g])[l + 16 * i];
     ag[i] = ab[i] = ac[i] = make_float4(0.f, 0.f, 0.f, 0.f);
   }
+  constexpr bool HEAD = ROWS != LN_ALL_ROWS;
   float sc = 1.f;
-  if constexpr (MIM) sc = (*p.dloss / 3.f) / *p.denom;
+  if constexpr (ROWS == LN_PATCH_ROWS) sc = (*p.dloss / 3.f) / *p.denom;
   for (int row = blockIdx.x * 16 + hw; row < p.M; row += gridDim.x * 16) {
     const float mu = p.mean[g][row], rs = p.rstd[g][row];
-    const int64_t xrow = MIM ? row + row / NP + 1 : row;
+    const int64_t xrow = ln_token_row(row, ROWS);
     const float4* xr = reinterpret_cast<const float4*>(x + xrow * D);
     float4 xh[3], gd[3], d[3], o[3];
     float c1 = 0.f, c2 = 0.f;
@@ -327,8 +332,8 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnB
     for (int i = 0; i < 3; ++i) {
       const float4 xv = xr[l + 16 * i];
       d[i] = load4<T>(dy + (int64_t)row * D + 4 * (l + 16 * i));
-      if constexpr (MIM) {
-        d[i].x *= sc; d[i].y *= sc; d[i].z *= sc; d[i].w *= sc;
+      if constexpr (HEAD) {
+        if constexpr (ROWS == LN_PATCH_ROWS) { d[i].x *= sc; d[i].y *= sc; d[i].z *= sc; d[i].w *= sc; }
         o[i] = make_float4(0.f, 0.f, 0.f, 0.f);
       } else {
         o[i] = reinterpret_cast<const float4*>(dres + (int64_t)row * D)[l + 16 * i];
@@ -348,10 +353,10 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const __grid_constant__ LnB
     for (int i = 0; i < 3; ++i) {
       o[i].x += rs * (gd[i].x - c1 - xh[i].x * c2); o[i].y += rs * (gd[i].y - c1 - xh[i].y * c2);
       o[i].z += rs * (gd[i].z - c1 - xh[i].z * c2); o[i].w += rs * (gd[i].w - c1 - xh[i].w * c2);
-      if constexpr (MIM) {
+      if constexpr (HEAD) {
         if (dres) {
           reinterpret_cast<float4*>(dres + xrow * D)[l + 16 * i] = o[i];
-          if (row % NP == 0) reinterpret_cast<float4*>(dres + (xrow - 1) * D)[l + 16 * i] = make_float4(0.f, 0.f, 0.f, 0.f);
+          if (ROWS == LN_PATCH_ROWS && row % NP == 0) reinterpret_cast<float4*>(dres + (xrow - 1) * D)[l + 16 * i] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
         continue;
       }
@@ -1197,6 +1202,134 @@ __global__ void __launch_bounds__(256) mim_pixel_grad_kernel(const T* __restrict
   }
 }
 
+// ------------------------------------------------------------------------------------------
+// Classification head (ViTForImageClassification): the loss rows, the fixed-order finish and the logit gradient
+// ------------------------------------------------------------------------------------------
+// sum or max over the 256 threads of the CTA, returned to every thread; `red` holds 8 floats
+template <bool MAX>
+__device__ __forceinline__ float cta_reduce256(float v, float* red) {
+  v = MAX ? warp_max(v) : warp_sum(v);
+  __syncthreads();                       // `red` may still be read by the previous reduction
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  float r = red[0];
+#pragma unroll
+  for (int w = 1; w < 8; ++w) r = MAX ? fmaxf(r, red[w]) : r + red[w];
+  return r;
+}
+
+// One CTA of 256 threads per row b: logits[b, j] = z[b, j] + bias[j] for j < N (z: the logit GEMM's rows, stride ldz).
+// With a loss (kind != V2S_CLS_LOSS_NONE) also the row's loss term part[b], its element count cnt[b] and, when dz is not
+// NULL, the unscaled d term / d logits into dz [B, ldz] (columns N..ldz zero):
+//   cross-entropy (int64 labels [B], -100 ignored): lse - v_y and softmax - onehot, count 1; an ignored row 0 / 0 / 0;
+//     any other label outside [0, N) is never used as an index: NaN term and gradient, count 1;
+//   MSE (fp32 labels [B, N]): sum (v - y)^2 and 2 (v - y), count N;
+//   BCE with logits (fp32 labels [B, N]): sum max(v, 0) - v y + log1p(exp(-|v|)) and sigmoid(v) - y, count N.
+__global__ void __launch_bounds__(256) cls_head_rows_kernel(const float* __restrict__ z, int ldz, const float* __restrict__ bias,
+                                                       int N, int kind, const void* __restrict__ labels,
+                                                       float* __restrict__ logits, float* __restrict__ dz,
+                                                       float* __restrict__ part, float* __restrict__ cnt) {
+  __shared__ float red[8];
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  const int b = blockIdx.x, t = threadIdx.x;
+  const float* zr = z + (int64_t)b * ldz;
+  float* lr = logits + (int64_t)b * N;
+  float* dr = dz ? dz + (int64_t)b * ldz : nullptr;
+  if (kind == V2S_CLS_LOSS_CE) {
+    const int64_t y = static_cast<const int64_t*>(labels)[b];
+    float mx = -INFINITY;
+    for (int j = t; j < N; j += 256) { const float v = zr[j] + bias[j]; lr[j] = v; mx = fmaxf(mx, v); }
+    mx = cta_reduce256<true>(mx, red);
+    float se = 0.f;
+    for (int j = t; j < N; j += 256) se += expf(zr[j] + bias[j] - mx);
+    const float lse = mx + logf(cta_reduce256<false>(se, red));
+    const bool ignored = y == -100, valid = y >= 0 && y < N;
+    if (dr) {
+      for (int j = t; j < ldz; j += 256) {
+        float g = 0.f;
+        if (j < N && !ignored) g = valid ? expf(zr[j] + bias[j] - lse) - (j == y ? 1.f : 0.f) : __int_as_float(0x7fffffff);
+        dr[j] = g;
+      }
+    }
+    if (t == 0) {
+      part[b] = ignored ? 0.f : valid ? lse - (zr[y] + bias[y]) : __int_as_float(0x7fffffff);
+      cnt[b] = ignored ? 0.f : 1.f;
+    }
+    return;
+  }
+  const float* yr = kind == V2S_CLS_LOSS_NONE ? nullptr : static_cast<const float*>(labels) + (int64_t)b * N;
+  float s = 0.f;
+  for (int j = t; j < N; j += 256) {
+    const float v = zr[j] + bias[j];
+    lr[j] = v;
+    if (kind == V2S_CLS_LOSS_MSE) {
+      const float d = v - yr[j];
+      s += d * d;
+      if (dr) dr[j] = 2.f * d;
+    } else if (kind == V2S_CLS_LOSS_BCE) {
+      const float y = yr[j];
+      s += fmaxf(v, 0.f) - v * y + log1pf(expf(-fabsf(v)));
+      if (dr) dr[j] = 1.f / (1.f + expf(-v)) - y;
+    }
+  }
+  if (kind == V2S_CLS_LOSS_NONE) return;
+  if (dr) for (int j = N + t; j < ldz; j += 256) dr[j] = 0.f;
+  s = cta_reduce256<false>(s, red);
+  if (t == 0) { part[b] = s; cnt[b] = (float)N; }
+}
+
+// one CTA: loss = (fixed-order sum of the B row terms) / (sum of the B counts); the count is kept for the backward
+__global__ void __launch_bounds__(1024) cls_head_finish_kernel(const float* __restrict__ part, const float* __restrict__ cnt,
+                                                               int B, float* loss, float* count) {
+  __shared__ float sred[1024], cred[1024];
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  const int t = threadIdx.x;
+  float s = 0.f, c = 0.f;
+  for (int i = t; i < B; i += 1024) { s += part[i]; c += cnt[i]; }
+  sred[t] = s; cred[t] = c;
+  __syncthreads();
+  for (int h = 512; h > 0; h >>= 1) {
+    if (t < h) { sred[t] += sred[t + h]; cred[t] += cred[t + h]; }
+    __syncthreads();
+  }
+  if (t == 0) { count[0] = cred[0]; loss[0] = sred[0] / cred[0]; }
+}
+
+// G [B, ldg] (type T) = c dz + dlogits on columns < N, zero beyond; c = *dloss / *count read on the device (0 when the
+// loss counted nothing: transformers' all-ignored batch has zero gradients); dz / dloss and dlogits [B, N] may be NULL
+template <typename T>
+__global__ void __launch_bounds__(256) cls_head_grad_kernel(const float* __restrict__ dz, const float* __restrict__ dlogits,
+                                                       const float* dloss, const float* count, T* __restrict__ g, int B,
+                                                       int N, int ldg) {
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  const float c = dloss && *count > 0.f ? *dloss / *count : 0.f;
+  for (int b = blockIdx.x; b < B; b += gridDim.x) {          // one row per CTA
+    for (int j = threadIdx.x; j < ldg; j += blockDim.x) {
+      float v = 0.f;
+      if (j < N) {
+        if (dloss) v = c * dz[(int64_t)b * ldg + j];
+        if (dlogits) v += dlogits[(int64_t)b * N + j];
+      }
+      g[(int64_t)b * ldg + j] = from_f<T>(v);
+    }
+  }
+}
+
+// db[j] += sum over the B rows of G[b, j] (G [B, ldg] of type T), one thread per column, rows in order
+template <typename T>
+__global__ void __launch_bounds__(256) cls_head_colsum_kernel(const T* __restrict__ g, int ldg, int B, int N, float* db) {
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= N) return;
+  float s = 0.f;
+  for (int b = 0; b < B; ++b) s += to_f<T>(g[(int64_t)b * ldg + j]);
+  db[j] += s;
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------
@@ -1254,7 +1387,7 @@ int launch_col2im(const float* const* rows, float* const* img, int groups, int B
 }
 
 int launch_ln_fwd(const float* const* x, const float* const* gamma, const float* const* beta, void* const* y,
-                  float* const* mean, float* const* rstd, int groups, int M, int at, cudaStream_t s, bool patch_rows) {
+                  float* const* mean, float* const* rstd, int groups, int M, int at, cudaStream_t s, int rows) {
   LnFwdP p;
   memset(&p, 0, sizeof(p));
   for (int g = 0; g < groups; ++g) {
@@ -1265,7 +1398,8 @@ int launch_ln_fwd(const float* const* x, const float* const* gamma, const float*
   int bx = (M + 15) / 16;
   if (bx > 148 * 6) bx = 148 * 6;
   dim3 grid(bx, groups);
-  if (patch_rows) { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_fwd_kernel<T, true>, grid, dim3(256), 0, s, p))); }
+  if (rows == LN_PATCH_ROWS) { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_fwd_kernel<T, LN_PATCH_ROWS>, grid, dim3(256), 0, s, p))); }
+  else if (rows == LN_CLS_ROWS) { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_fwd_kernel<T, LN_CLS_ROWS>, grid, dim3(256), 0, s, p))); }
   else { V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(ln_fwd_kernel<T>, grid, dim3(256), 0, s, p))); }
   V2S_LAUNCH_CHECK();
   return 0;
@@ -1314,9 +1448,9 @@ int launch_mim_ln_bwd(const float* dseq, const float* hidden, const float* mean,
     if ((int64_t)bx * 3 * D > det->part_floats) { set_error("mim ln_bwd: deterministic scratch too small"); return 1; }
     p.det_part = det->part; p.det_counters = det->counters;
   }
-  if (!dgamma) V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, false, false, true>, dim3(bx), dim3(256), 0, s, p));
-  else if (det) V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, true, true, true>, dim3(bx), dim3(256), 0, s, p));
-  else V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, false, true, true>, dim3(bx), dim3(256), 0, s, p));
+  if (!dgamma) V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, false, false, LN_PATCH_ROWS>, dim3(bx), dim3(256), 0, s, p));
+  else if (det) V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, true, true, LN_PATCH_ROWS>, dim3(bx), dim3(256), 0, s, p));
+  else V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, false, true, LN_PATCH_ROWS>, dim3(bx), dim3(256), 0, s, p));
   V2S_LAUNCH_CHECK();
   return 0;
 }
@@ -1347,6 +1481,56 @@ int launch_mim_pixel_grad(const void* sign, float* dx, int B, int at, const floa
   const dim3 grid(grid_for((int64_t)B * 3 * V2S_IMG * (V2S_IMG / 4), 256, 148 * 16));
   V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(mim_pixel_grad_kernel<T>, grid, dim3(256), 0, s, static_cast<const T*>(sign), dx, B,
                                              dloss, denom)));
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_cls_head_ln_bwd(const float* dxhat, const float* hidden, const float* mean, const float* rstd, const float* gamma,
+                      float* dhidden, float* dgamma, float* dbeta, int B, cudaStream_t s, const DetScratch* det) {
+  LnBwdP p;
+  memset(&p, 0, sizeof(p));
+  p.dy[0] = dxhat; p.x[0] = hidden; p.mean[0] = mean; p.rstd[0] = rstd; p.gamma[0] = gamma; p.dres[0] = dhidden;
+  p.dgamma[0] = dgamma; p.dbeta[0] = dbeta;
+  p.M = B;
+  int bx = (B + 15) / 16;
+  if (bx > 148 * 4) bx = 148 * 4;
+  if (det && dgamma) {
+    if (bx > 148) bx = 148;
+    if ((int64_t)bx * 3 * D > det->part_floats) { set_error("cls ln_bwd: deterministic scratch too small"); return 1; }
+    p.det_part = det->part; p.det_counters = det->counters;
+  }
+  if (!dgamma) V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, false, false, LN_CLS_ROWS>, dim3(bx), dim3(256), 0, s, p));
+  else if (det) V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, true, true, LN_CLS_ROWS>, dim3(bx), dim3(256), 0, s, p));
+  else V2S_CUDA_OK(launch_pdl(ln_bwd_kernel<float, false, true, LN_CLS_ROWS>, dim3(bx), dim3(256), 0, s, p));
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_cls_head_rows(const float* z, int ldz, const float* bias, int N, int kind, const void* labels, float* logits,
+                    float* dz, float* part, float* cnt, int B, cudaStream_t s) {
+  V2S_CUDA_OK(launch_pdl(cls_head_rows_kernel, dim3(B), dim3(256), 0, s, z, ldz, bias, N, kind, labels, logits, dz, part, cnt));
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_cls_head_loss_finish(const float* part, const float* cnt, int B, float* loss, float* count, cudaStream_t s) {
+  V2S_CUDA_OK(launch_pdl(cls_head_finish_kernel, dim3(1), dim3(1024), 0, s, part, cnt, B, loss, count));
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_cls_head_grad(const float* dz, const float* dlogits, const float* dloss, const float* count, void* g, int B, int N,
+                    int ldg, int at, cudaStream_t s) {
+  const dim3 grid(B < 148 * 8 ? B : 148 * 8);
+  V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(cls_head_grad_kernel<T>, grid, dim3(256), 0, s, dz, dlogits, dloss, count,
+                                             static_cast<T*>(g), B, N, ldg)));
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+int launch_cls_head_colsum(const void* g, int ldg, int B, int N, int at, float* db, cudaStream_t s) {
+  V2S_DISPATCH_AT(at, V2S_CUDA_OK(launch_pdl(cls_head_colsum_kernel<T>, dim3((N + 255) / 256), dim3(256), 0, s,
+                                             static_cast<const T*>(g), ldg, B, N, db)));
   V2S_LAUNCH_CHECK();
   return 0;
 }

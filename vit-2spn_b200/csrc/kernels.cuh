@@ -23,10 +23,13 @@ int launch_gather_patch_rows(const void* const* src, void* const* dst, int group
                              const uint8_t* const* mask = nullptr);
 // inverse of launch_im2col for fp32: patch rows [B*196, 768] -> NCHW [B,3,224,224] (overwritten)
 int launch_col2im(const float* const* rows, float* const* img, int groups, int B, cudaStream_t s);
-// patch_rows: y, mean and rstd are the compact patch rows [M = B*196] of the token rows x [B,197,192] (CLS dropped)
+// Which token rows of x [B,197,192] a head's LayerNorm reads; y / dy, mean and rstd are then compact rows.
+// LN_PATCH_ROWS (SimMIM): row r = b*196 + p is token row b*197 + 1 + p (CLS dropped), M = B*196.  LN_CLS_ROWS (the
+// classifier): row b is token row b*197, M = B.
+enum LnRows : int { LN_ALL_ROWS = 0, LN_PATCH_ROWS = 1, LN_CLS_ROWS = 2 };
 int launch_ln_fwd(const float* const* x, const float* const* gamma, const float* const* beta,
                   void* const* y, float* const* mean, float* const* rstd, int groups, int M, int at,
-                  cudaStream_t s, bool patch_rows = false);
+                  cudaStream_t s, int rows = LN_ALL_ROWS);
 // dres (fp32, in/out) += LN-backward(dy); dres_lp (optional, activation type) = updated dres;
 // dcolsum (optional) += column sums of the updated dres (bias gradient of the next linear layer);
 // dgamma == NULL: no parameter gradient at all (dbeta, dcolsum and det ignored)
@@ -51,6 +54,23 @@ int launch_mim_scale_add(const float* acc, float* dw, float* db, int nw, int nb,
                          cudaStream_t s);
 // dx [B,3,224,224] += -c * sign rows [B*196, 768] (activation type `at`) in NCHW order
 int launch_mim_pixel_grad(const void* sign, float* dx, int B, int at, const float* dloss, const float* denom, cudaStream_t s);
+// Classification head (one group; LN_CLS_ROWS).  Final-LayerNorm backward of the CLS rows: dy = dxhat [B, 192] fp32,
+// x = hidden [B,197,192]; dhidden (may be NULL) is written at the CLS rows only; dgamma / dbeta (NULL: frozen) +=, in a
+// fixed order with `det`
+int launch_cls_head_ln_bwd(const float* dxhat, const float* hidden, const float* mean, const float* rstd, const float* gamma,
+                      float* dhidden, float* dgamma, float* dbeta, int B, cudaStream_t s, const DetScratch* det = nullptr);
+// logits [B, N] = z [B, ldz] + bias; with a loss (kind, V2S_CLS_LOSS_*) the row terms part[B], counts cnt[B] and, when dz
+// is not NULL, the unscaled d loss-term / d logits [B, ldz]
+int launch_cls_head_rows(const float* z, int ldz, const float* bias, int N, int kind, const void* labels, float* logits,
+                    float* dz, float* part, float* cnt, int B, cudaStream_t s);
+// loss = sum part / sum cnt (one CTA, fixed order); count = sum cnt
+int launch_cls_head_loss_finish(const float* part, const float* cnt, int B, float* loss, float* count, cudaStream_t s);
+// G [B, ldg] (activation type `at`) = (*dloss / *count) dz + dlogits [B, N], zero padding columns; dz / dloss (together)
+// and dlogits may be NULL
+int launch_cls_head_grad(const float* dz, const float* dlogits, const float* dloss, const float* count, void* g, int B, int N,
+                    int ldg, int at, cudaStream_t s);
+// db[0, N) += column sums of G [B, ldg] (type `at`), rows in order
+int launch_cls_head_colsum(const void* g, int ldg, int B, int N, int at, float* db, cudaStream_t s);
 // db[n] += sum_m dy[m,n]; src type tag `t`.  With `det` (deterministic mode) the sum has a fixed order: partial rows in
 // det->part, or, when det->part is NULL, one CTA per group
 int launch_colsum(const void* const* dy, float* const* db, int groups, int M, int N, int t, cudaStream_t s,

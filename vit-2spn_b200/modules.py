@@ -330,7 +330,7 @@ class ViTConfig:
     def __init__(self, hidden_size=192, num_hidden_layers=12, num_attention_heads=3, intermediate_size=768,
                  patch_size=16, image_size=224, output_hidden_states=False, layer_norm_eps=1e-12,
                  hidden_act="gelu", num_channels=3, qkv_bias=True, initializer_range=0.02, output_attentions=False,
-                 encoder_stride=16, **kw):
+                 encoder_stride=16, num_labels=2, problem_type=None, **kw):
         self.hidden_size = hidden_size
         self.num_hidden_layers = num_hidden_layers
         self.num_attention_heads = num_attention_heads
@@ -345,6 +345,8 @@ class ViTConfig:
         self.qkv_bias = qkv_bias
         self.initializer_range = initializer_range
         self.encoder_stride = encoder_stride
+        self.num_labels = num_labels            # ViTForImageClassification's head; the backbone ignores both
+        self.problem_type = problem_type
         for k, v in kw.items():
             setattr(self, k, v)
 
@@ -906,6 +908,236 @@ class ViTForMaskedImageModeling(nn.Module):
         rec, loss = res if mask is not None else (res, None)
         hs = out.hidden_states if isinstance(out.hidden_states, tuple) else None
         return MaskedImageModelingOutput(loss, rec, hs, out.attentions)
+
+
+# ---------------------------------------------------------------------------------------------
+# ViTForImageClassification
+# ---------------------------------------------------------------------------------------------
+_LOSS_KINDS = {"single_label_classification": _lib.CLS_LOSS_CE, "regression": _lib.CLS_LOSS_MSE,
+               "multi_label_classification": _lib.CLS_LOSS_BCE}
+
+
+def _cls_workspace(device, batch, num_labels, mode, keep):
+    """Workspace of the classification head: a fresh one when the forward keeps state for its backward, else a cached
+    scratch."""
+    det = _deterministic()                 # the deterministic mode's scratch is part of the size
+    nbytes = lib.v2s_cls_workspace_bytes(batch, num_labels, mode)
+    if nbytes < 0:
+        raise RuntimeError("v2s_cls_workspace_bytes: bad arguments")
+    if keep:
+        return torch.empty(nbytes + 1024, dtype=torch.uint8, device=device)
+    key = ("cls", device, batch, num_labels, mode, det)
+    ws = _workspaces.get(key)
+    if ws is None:
+        ws = _workspaces[key] = torch.empty(nbytes + 1024, dtype=torch.uint8, device=device)
+    return ws
+
+
+class _ClsHeadFn(torch.autograd.Function):
+    """hidden_states[12] -> (logits, loss) of transformers' ViTForImageClassification in the CUDA library
+    (v2s_cls_forward / v2s_cls_backward): the final LayerNorm of the CLS rows, the linear classifier and, with labels,
+    the loss of ``kind`` (V2S_CLS_LOSS_*).  Both outputs are differentiable: one backward call takes the gradient of the
+    logits, of the loss or of both, and returns d hidden_states[12] (CLS rows only) to the backbone's Function and the
+    LayerNorm and classifier gradients as tensors."""
+
+    @staticmethod
+    @_with_device_of(lambda ctx, hidden, *a, **k: hidden)
+    def forward(ctx, hidden, ln_w, ln_b, cls_w, cls_b, model, kind, labels, need_grad):
+        mode = model.vit._mode()
+        B, dev = hidden.shape[0], hidden.device
+        N = cls_w.shape[0]
+        hidden = _aligned16(hidden.detach().contiguous())
+        gam, bet = _aligned16(ln_w.detach()), _aligned16(ln_b.detach())
+        w, b = _aligned16(cls_w.detach().contiguous()), _aligned16(cls_b.detach().contiguous())
+        logits = torch.empty(B, N, dtype=torch.float32, device=dev)
+        loss = torch.empty((), dtype=torch.float32, device=dev) if labels is not None else None
+        ws = _cls_workspace(dev, B, N, mode, need_grad)
+        base, nbytes = _aligned(ws)
+        check(lib.v2s_cls_forward(ptr(hidden), ptr(gam), ptr(bet), ptr(w), ptr(b), N, kind, ptr(labels), ptr(logits),
+                                  ptr(loss), int(need_grad), B, mode, C.c_void_p(base), nbytes, stream_ptr()), "cls_forward")
+        ctx.set_materialize_grads(False)
+        ctx.ws = ws if need_grad else None
+        ctx.mode, ctx.B, ctx.N, ctx.kind = mode, B, N, kind
+        ctx.keep = (hidden, gam, w, labels)
+        return (logits, loss) if labels is not None else logits
+
+    @staticmethod
+    @_with_device_of(lambda ctx, dlogits, *rest: dlogits if dlogits is not None else next((t for t in rest if t is not None), None))
+    def backward(ctx, dlogits, dloss=None):
+        nones = (None,) * 9
+        if dlogits is None and dloss is None:
+            return nones
+        if ctx.ws is None:
+            raise RuntimeError("vit2spn: backward through a classification forward that saved nothing (twice, or without "
+                               "grad)")
+        hidden, gam, w, labels = ctx.keep
+        need = ctx.needs_input_grad
+        dev, B, N = hidden.device, ctx.B, ctx.N
+        _deterministic()
+        dl = _grad_f32(dloss.reshape(1)) if dloss is not None else None
+        dz = _grad_f32(dlogits) if dlogits is not None else None
+        dh = torch.empty(B, 197, 192, dtype=torch.float32, device=dev) if need[0] else None
+        want_ln = need[1] or need[2]
+        dg = torch.zeros(192, dtype=torch.float32, device=dev) if want_ln else None
+        db = torch.zeros(192, dtype=torch.float32, device=dev) if want_ln else None
+        dw = torch.zeros(N, 192, dtype=torch.float32, device=dev) if need[3] else None
+        dbc = torch.zeros(N, dtype=torch.float32, device=dev) if need[4] else None
+        base, nbytes = _aligned(ctx.ws)
+        check(lib.v2s_cls_backward(ptr(hidden), ptr(gam), ptr(w), N, ctx.kind, ptr(labels), ptr(dz), ptr(dl), ptr(dh),
+                                   ptr(dg), ptr(db), ptr(dw), ptr(dbc), B, ctx.mode, C.c_void_p(base), nbytes,
+                                   stream_ptr()), "cls_backward")
+        ctx.ws = None
+        return (dh, dg if need[1] else None, db if need[2] else None, dw, dbc, None, None, None, None)
+
+
+class ImageClassifierOutput:
+    """As transformers' ``ImageClassifierOutput``: ``loss`` (None without ``labels``), ``logits`` [B, num_labels] fp32,
+    ``hidden_states`` / ``attentions`` (tuples when requested, else None)."""
+
+    def __init__(self, loss, logits, hidden_states=None, attentions=None):
+        self.loss, self.logits = loss, logits
+        self.hidden_states, self.attentions = hidden_states, attentions
+
+
+def _meta(t):
+    return t.detach().to("meta")
+
+
+_CHECKED_LABELS = set()         # (loss kind, batch, num_labels, label shape, label dtype) that torch's checks accepted
+
+
+class ViTForImageClassification(nn.Module):
+    """Drop-in for ``transformers.ViTForImageClassification`` (ViT-Tiny/16@224): ``vit`` is a
+    ``ViTModel(config, add_pooling_layer=False)`` and ``classifier`` is ``nn.Linear(192, config.num_labels)``, so
+    ``state_dict`` keys and strict loads match transformers.  The final LayerNorm of the CLS token, the classifier and
+    its loss run as one CUDA head after the CUDA backbone."""
+
+    def __init__(self, config=None, **kw):
+        super().__init__()
+        config = config or ViTConfig(**kw)
+        if config.num_labels < 1:
+            raise ValueError(f"vit2spn.ViTForImageClassification: num_labels must be >= 1, got {config.num_labels} "
+                             "(transformers' Identity classifier is not supported)")
+        self.config = config
+        self.num_labels = config.num_labels
+        self.vit = ViTModel(config, add_pooling_layer=False)
+        self.classifier = nn.Linear(192, config.num_labels)
+        with torch.no_grad():          # transformers' _init_weights for nn.Linear
+            nn.init.trunc_normal_(self.classifier.weight, mean=0.0, std=config.initializer_range)
+            nn.init.zeros_(self.classifier.bias)
+
+    @property
+    def compute_mode(self):
+        return self.vit.compute_mode
+
+    @compute_mode.setter
+    def compute_mode(self, mode):
+        self.vit.compute_mode = mode
+
+    @classmethod
+    def from_pretrained(cls, name, num_labels=None, ignore_mismatched_sizes=False, **kw):
+        """Loads a classification checkpoint (with or without the ``vit.`` prefix; ``num_labels`` defaults to its
+        classifier's rows), a ViTModel or ViT-2SPN backbone checkpoint (pooler ignored; the classifier keeps its
+        initialisation) or a SimMIM checkpoint (decoder and mask token ignored); the same policy as
+        ``ViTModel.from_pretrained`` for missing checkpoints and mismatching keys.  A classifier of another size is an
+        error unless ``ignore_mismatched_sizes=True``, which re-initialises it and says so on stderr, as transformers
+        does."""
+        cfg_kw = {k: v for k, v in kw.items() if k in ("output_hidden_states", "output_attentions")}
+        path = _resolve_checkpoint(str(name))
+        if path is None:
+            _no_checkpoint("ViTForImageClassification", name)
+            return cls(ViTConfig(num_labels=2 if num_labels is None else num_labels, **cfg_kw))
+        sd = _load_weight_file(path)
+        sd = {k if k.startswith(("vit.", "classifier.", "decoder.")) else "vit." + k: v for k, v in sd.items()}
+        sd = {k: v for k, v in sd.items()
+              if not k.startswith(("vit.pooler.", "decoder.")) and k != "vit.embeddings.mask_token"}
+        if num_labels is None:
+            num_labels = sd["classifier.weight"].shape[0] if "classifier.weight" in sd else 2
+        model = cls(ViTConfig(num_labels=num_labels, **cfg_kw))
+        own = model.classifier.weight.shape
+        if "classifier.weight" in sd and tuple(sd["classifier.weight"].shape) != tuple(own):
+            found = tuple(sd["classifier.weight"].shape)
+            if not ignore_mismatched_sizes:
+                raise RuntimeError(f"vit2spn.ViTForImageClassification.from_pretrained({name!r}): the checkpoint's "
+                                   f"classifier.weight has shape {found}, the model's {tuple(own)} (num_labels "
+                                   f"{num_labels}); pass ignore_mismatched_sizes=True to re-initialise the classifier")
+            sd = {k: v for k, v in sd.items() if not k.startswith("classifier.")}
+            print(f"vit2spn: some weights of ViTForImageClassification were not initialized from the checkpoint at "
+                  f"{path} and are newly initialized because the shapes did not match: classifier.weight: found shape "
+                  f"{found} in the checkpoint and {tuple(own)} in the model; classifier.bias likewise.  You should "
+                  "probably train this model on a down-stream task.", file=sys.stderr, flush=True)
+        res = model.load_state_dict(sd, strict=False)
+        missing = [k for k in res.missing_keys if not k.startswith("classifier.")]
+        unexpected = list(res.unexpected_keys)
+        print(f"vit2spn: loaded {path} ({len(sd) - len(res.unexpected_keys)} tensors; missing {res.missing_keys or 'none'}; "
+              f"unexpected {res.unexpected_keys or 'none'})", file=sys.stderr, flush=True)
+        if missing or unexpected:
+            raise RuntimeError(f"vit2spn.ViTForImageClassification.from_pretrained({name!r}): checkpoint does not match "
+                               f"ViT-Tiny/16: missing {missing}, unexpected {unexpected}")
+        return model
+
+    def _labels(self, labels, x):
+        """(loss kind, labels as the library reads them) with transformers' ForSequenceClassificationLoss semantics,
+        including its problem_type inference on the config; shape and dtype errors are torch's own."""
+        if labels.device != x.device:
+            raise ValueError(f"vit2spn: labels are on {labels.device}, pixel_values on {x.device}: pass the labels on the "
+                             "input's device")
+        cfg, N, B = self.config, self.num_labels, x.shape[0]
+        if cfg.problem_type is None:
+            if N == 1:
+                cfg.problem_type = "regression"
+            elif N > 1 and labels.dtype in (torch.long, torch.int):
+                cfg.problem_type = "single_label_classification"
+            else:
+                cfg.problem_type = "multi_label_classification"
+        if cfg.problem_type not in _LOSS_KINDS:
+            raise RuntimeError(f"Invalid problem type: {cfg.problem_type}")
+        kind = _LOSS_KINDS[cfg.problem_type]
+        y = labels.view(-1) if kind == _lib.CLS_LOSS_CE else labels
+        key = (kind, B, N, tuple(labels.shape), labels.dtype)
+        if key not in _CHECKED_LABELS:
+            # torch's own shape / dtype checks, on meta tensors; they cost about a millisecond of host time, so each
+            # label signature is checked once
+            z = torch.empty(B, N, device="meta")
+            if kind == _lib.CLS_LOSS_CE:
+                torch.nn.functional.cross_entropy(z.view(-1, N), _meta(y), ignore_index=-100)
+            elif kind == _lib.CLS_LOSS_MSE:
+                zz, yy = (z.squeeze(), labels.squeeze()) if N == 1 else (z, labels)
+                torch.nn.functional.mse_loss(zz, _meta(yy))
+                if tuple(yy.shape) != tuple(zz.shape):
+                    raise ValueError(f"vit2spn: regression labels must have the logits' shape {tuple(zz.shape)} (got "
+                                     f"{tuple(yy.shape)}); broadcasting them is not supported")
+            else:
+                torch.nn.functional.binary_cross_entropy_with_logits(z, _meta(labels))
+            _CHECKED_LABELS.add(key)
+        if kind == _lib.CLS_LOSS_CE:
+            return kind, _aligned16(y.to(torch.int64).contiguous())
+        return kind, _aligned16(labels.detach().to(torch.float32).reshape(B, N).contiguous())
+
+    def forward(self, pixel_values, labels=None, output_hidden_states=None, output_attentions=None, **kw):
+        """As transformers: ``logits`` always, ``loss`` with ``labels``.  Both are differentiable: ``loss.backward()``,
+        a loss of the user's own on the logits, or both, reach the classifier, the final LayerNorm, the backbone and,
+        when it requires grad, ``pixel_values``.  A frozen ``vit`` (linear probe) runs no backbone backward."""
+        for k in ("head_mask", "bool_masked_pos", "num_items_in_batch"):
+            if kw.get(k) is not None:
+                raise ValueError(f"vit2spn.ViTForImageClassification: {k} is not supported")
+        if kw.get("interpolate_pos_encoding"):
+            raise ValueError("vit2spn.ViTForImageClassification: interpolate_pos_encoding=True is not supported (224x224 "
+                             "inputs only)")
+        if isinstance(pixel_values, torch.Tensor) and pixel_values.dim() == 3:
+            raise ValueError("vit2spn.ViTForImageClassification: 16-bit patch-row inputs are not accepted; pass "
+                             "pixel_values [B,3,224,224]")
+        x = _check_images(pixel_values)
+        kind, lab = (_lib.CLS_LOSS_NONE, None) if labels is None else self._labels(labels, x)
+        out = self.vit(pixel_values, output_hidden_states=output_hidden_states, output_attentions=output_attentions)
+        hidden = out.hidden_states[-1]
+        ln, fc = self.vit.layernorm, self.classifier
+        tensors = (hidden, ln.weight, ln.bias, fc.weight, fc.bias)
+        need_grad = torch.is_grad_enabled() and any(t.requires_grad for t in tensors)
+        res = _ClsHeadFn.apply(*tensors, self, kind, lab, need_grad)
+        logits, loss = res if lab is not None else (res, None)
+        hs = out.hidden_states if isinstance(out.hidden_states, tuple) else None
+        return ImageClassifierOutput(loss, logits, hs, out.attentions)
 
 
 class ViTBackbone(nn.Module):
