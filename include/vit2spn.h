@@ -30,7 +30,7 @@ extern "C" {
                              masked forward) are folded into v2s_backbone_forward / _backward: their arguments are
                              fields of v2s_group_outputs, and v2s_backbone_backward takes weight_grads.  Additive to 5:
                              v2s_mim_workspace_bytes, v2s_mim_forward, v2s_mim_backward, v2s_cls_workspace_bytes, v2s_cls_forward,
-                             v2s_cls_backward.  Additive to 4:
+                             v2s_cls_backward, v2s_set_image_size.  Additive to 4:
                              v2s_test_gemm which = 5, v2s_test_attention which = 3.  4: one entry point per operation:
                              v2s_backbone_forward / _backward take the per-group outputs and (backward) the layer range,
                              v2s_heads_loss_fwd_bwd the device loss scale, v2s_adam_step and v2s_ema_update the
@@ -329,6 +329,18 @@ int v2s_set_sm_limit(int n_sms);
  * read, so size the workspace while the switch is on.  With the
  * switch off nothing changes, v2s_workspace_bytes included.  Python sets it from torch.are_deterministic_algorithms_enabled(). */
 int v2s_set_deterministic(int on);
+
+/* Input image size of the backbone calls (default 224 x 224): height and width multiples of 16, at most 196 patches
+ * (197 tokens).  Process-wide, read when work is enqueued, like v2s_set_deterministic.  With gh = height / 16 and
+ * gw = width / 16 a sequence has N = 1 + gh * gw tokens: v2s_workspace_bytes sizes for N tokens (at 224 x 224 exactly as
+ * without the call); v2s_backbone_forward / _backward read x as fp32 [batch,3,height,width], and hidden, attn, dattn,
+ * dpixels and mask follow N ([batch,N,192], [batch,3,N,N], [batch,3,height,width], [batch,N-1]); v2s_test_attention runs
+ * at N tokens and v2s_test_gemm which = 5 at the image size.  At any size other than 224 x 224 the position table is
+ * interpolated as transformers' ViTModel(interpolate_pos_encoding=True) does it (bicubic, align_corners false, from the
+ * 14 x 14 grid to gh x gw: one more kernel in a forward, and one in a backward that reaches the embeddings with
+ * weight_grads), and x_format 1, feat / dfeat, v2s_mim_* and v2s_cls_* are refused.  A saved group's backward must run
+ * at the size of its forward. */
+int v2s_set_image_size(int height, int width);
 
 /* test hooks: individual operators, used by tests/ to localise a parity failure */
 /* GEMM, 16-bit operands: which 0 NT (a [m,k], b [n,k] -> c [m,n] 16-bit), 1 NN (b [k,n]), 2 TN (a [k,m], b [k,n],

@@ -65,9 +65,15 @@ struct alignas(64) AttnFwdPParams {
   int B, total_jobs;
   int* err_flag;
   long long* dbg;   // optional cycle counters of CTA 0 (V2S_GEMM_DEBUG): [0..3] UMMA warp waits, [8..15] softmax thread phases
+  int N, ntiles;    // VAR: tokens (2..197) and query tiles (1 or 2) per image
+  int KP;           // VAR: keys padded to round_up(N, 16): the N of the S UMMA, KP / 16 K-steps of P V
 };
 
-template <bool DBG, typename LP>   // DBG: instrumented build (phase cycle counters), launched only when V2S_GEMM_DEBUG is set
+// DBG: instrumented build (phase cycle counters), launched only when V2S_GEMM_DEBUG is set.  VAR: p.N tokens instead of 197
+// (v2s_set_image_size): S = Q K^T is a 128 x KP tile (KP = round_up(N, 16); TMA zero-fills the keys past N per image) and
+// P V takes KP / 16 K-steps; 32-key chunks past N are skipped and the one chunk that holds key N is bounds-checked
+// (keys >= N get p = 0); with N <= 128 a job is one query tile
+template <bool DBG, typename LP, bool VAR = false>
 __global__ void __launch_bounds__(PF_THREADS, 1) attn_fwd_persist_kernel(const __grid_constant__ AttnFwdPParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -103,10 +109,12 @@ __global__ void __launch_bounds__(PF_THREADS, 1) attn_fwd_persist_kernel(const _
   ptx::pdl_launch_dependents();     // after the wait: see the dependent-launch note in gemm_tc.cu
 
   const int njobs = ((int)blockIdx.x < p.total_jobs) ? (p.total_jobs - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
+  const int nt = VAR ? p.N : NT;
+  const bool two_tiles = !VAR || p.ntiles == 2;
   auto decode = [&](int n, int& t, int& h, int& b, int& g) {
     const int J = blockIdx.x + n * gridDim.x;
-    t = J & 1;
-    int r = J >> 1;
+    t = two_tiles ? (J & 1) : 0;
+    int r = two_tiles ? (J >> 1) : J;
     h = r % NH; r /= NH;
     b = r % p.B; g = r / p.B;
   };
@@ -129,7 +137,8 @@ __global__ void __launch_bounds__(PF_THREADS, 1) attn_fwd_persist_kernel(const _
     }
   } else if (warp == 1) {
     // ---- UMMA issuer: S(n) as soon as its stage and slot are ready, then P V of job n-1 ----
-    const uint32_t idesc_s = make_idesc_lp(LP::kIdescFmt, QT, KPAD, 0, 0);
+    const int kp = VAR ? p.KP : KPAD;
+    const uint32_t idesc_s = make_idesc_lp(LP::kIdescFmt, QT, kp, 0, 0);
     const uint32_t idesc_o = make_idesc_lp(LP::kIdescFmt, QT, DH, 0, 1);
     const uint32_t sbase = ptx::smem_u32(smem);
     long long w_load = 0, w_tfree = 0, w_p = 0; const long long t_mma0 = clock64();
@@ -160,7 +169,7 @@ __global__ void __launch_bounds__(PF_THREADS, 1) attn_fwd_persist_kernel(const _
         const uint32_t tslot = tmem_base + sl * 256;
         if (ptx::elect_one()) {
 #pragma unroll
-          for (int j = 0; j < KPAD / 16; ++j) {
+          for (int j = 0; j < kp / 16; ++j) {
             const uint32_t a = tslot + (j < PF_KSPLIT / 16 ? 8 * j : PF_TM_PB + 8 * (j - PF_KSPLIT / 16));
             ptx::umma_bf16_ts(tslot + PF_TM_O, a, ptx::desc_lo(sv + j * 2048, 8192), ptx::DESC_HI_SW128_SBO1024, idesc_o,
                               j > 0 ? 1u : 0u);
@@ -219,7 +228,18 @@ __global__ void __launch_bounds__(PF_THREADS, 1) attn_fwd_persist_kernel(const _
       float mx = -INFINITY;
       // only the last chunk of the second key half (keys 176..207) contains padding keys (>= 197): every other
       // chunk runs the unmasked variant, so the per-element bound checks stay out of the hot loop
-      auto max32 = [&](const uint32_t* v) {
+      // VAR: the scores of keys >= N become -inf in the registers of a chunk that reaches past N (they then add nothing
+      // to the maximum and give p = 0); a chunk wholly below N is left alone.  It runs right after the chunk's load
+      // has landed and before the next load is issued, while only one register buffer is live.
+      auto mask32 = [&](uint32_t* v, int kb, int n) {   // keys kb + i, i < n
+        if (VAR && kb + n > nt) {
+          const int lim = nt - kb;
+#pragma unroll
+          for (int i = 0; i < n; ++i) v[i] = i < lim ? v[i] : 0xff800000u;
+        }
+      };
+      auto max32 = [&](const uint32_t* v, int kb) {   // VAR: a chunk wholly past N is skipped
+        if (VAR && kb >= nt) return;
 #pragma unroll
         for (int i = 0; i < 32; ++i) mx = fmaxf(mx, __uint_as_float(v[i]));
       };
@@ -229,16 +249,21 @@ __global__ void __launch_bounds__(PF_THREADS, 1) attn_fwd_persist_kernel(const _
       };
       ptx::tmem_ld_32x32(taddr + key0, r);
       ptx::tmem_ld_wait();
+      mask32(r, key0, 32);
       ptx::tmem_ld_32x32(taddr + key0 + 32, r2);
-      max32(r);
+      max32(r, key0);
       ptx::tmem_ld_wait();
+      mask32(r2, key0 + 32, 32);
       ptx::tmem_ld_32x32(taddr + key0 + 64, r);
-      max32(r2);
+      max32(r2, key0 + 32);
       ptx::tmem_ld_wait();
+      mask32(r, key0 + 64, 32);
       if (hf == 0) ptx::tmem_ld_32x16(taddr + 96, r2);
-      if (hf == 0) max32(r); else max32_tail(r);
+      if (hf == 0 || VAR) max32(r, key0 + 64);
+      else max32_tail(r);
       if (hf == 0) {
         ptx::tmem_ld_wait();
+        mask32(r2, 96, 16);
 #pragma unroll
         for (int i = 0; i < 16; ++i) mx = fmaxf(mx, __uint_as_float(r2[i]));
       }
@@ -251,7 +276,9 @@ __global__ void __launch_bounds__(PF_THREADS, 1) attn_fwd_persist_kernel(const _
       // pass 2: p = exp2((s - max) * scale * log2e); bf16 pairs back into tensor memory
       const float moff = mx * SCALE_LOG2E;
       float sum = 0.f;
-      auto exp32 = [&](const uint32_t* v, int pcol) {
+      // VAR: masked keys give exp2(-inf) = 0; a chunk wholly past N holds keys >= KP, which P V does not read: skipped
+      auto exp32 = [&](const uint32_t* v, int pcol, int kb) {
+        if (VAR && kb >= nt) return;
         uint32_t pw[16];
 #pragma unroll
         for (int i = 0; i < 16; ++i) {
@@ -274,25 +301,32 @@ __global__ void __launch_bounds__(PF_THREADS, 1) attn_fwd_persist_kernel(const _
         ptx::tmem_st_32x16(taddr + pcol, pw);
       };
       ptx::tmem_ld_wait();
+      mask32(r, key0, 32);
       ptx::tmem_ld_32x32(taddr + key0 + 32, r2);
-      exp32(r, pcol0);
+      exp32(r, pcol0, key0);
       ptx::tmem_ld_wait();
+      mask32(r2, key0 + 32, 32);
       ptx::tmem_ld_32x32(taddr + key0 + 64, r);
-      exp32(r2, pcol0 + 16);
+      exp32(r2, pcol0 + 16, key0 + 32);
       ptx::tmem_ld_wait();
+      mask32(r, key0 + 64, 32);
       if (hf == 0) ptx::tmem_ld_32x16(taddr + 96, r2);
-      if (hf == 0) exp32(r, pcol0 + 32); else exp32_tail(r, pcol0 + 32);
+      if (hf == 0 || VAR) exp32(r, pcol0 + 32, key0 + 64);
+      else exp32_tail(r, pcol0 + 32);
       if (hf == 0) {
         ptx::tmem_ld_wait();
-        uint32_t pw[8];
+        mask32(r2, 96, 16);
+        if (!VAR || 96 < nt) {
+          uint32_t pw[8];
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const float e0 = ptx::ex2_approx(fmaf(__uint_as_float(r2[2 * i]), SCALE_LOG2E, -moff));
-          const float e1 = ptx::ex2_approx(fmaf(__uint_as_float(r2[2 * i + 1]), SCALE_LOG2E, -moff));
-          sum += e0 + e1;
-          pw[i] = LP::pack(e0, e1);
+          for (int i = 0; i < 8; ++i) {
+            const float e0 = ptx::ex2_approx(fmaf(__uint_as_float(r2[2 * i]), SCALE_LOG2E, -moff));
+            const float e1 = ptx::ex2_approx(fmaf(__uint_as_float(r2[2 * i + 1]), SCALE_LOG2E, -moff));
+            sum += e0 + e1;
+            pw[i] = LP::pack(e0, e1);
+          }
+          ptx::tmem_st_32x8(taddr + 48, pw);
         }
-        ptx::tmem_st_32x8(taddr + 48, pw);
       }
       ptx::tmem_st_wait();
       ptx::tc_fence_before();
@@ -302,7 +336,7 @@ __global__ void __launch_bounds__(PF_THREADS, 1) attn_fwd_persist_kernel(const _
       ptx::bar_sync(bar_id, 256);
       V2S_TICK(4)
       sum += xsum[(hf ^ 1) * 128 + row];
-      if (hf == 0 && qrow < NT && p.lse[g]) p.lse[g][((int64_t)b * NH + h) * NT + qrow] = mx * SCALE + __logf(sum);
+      if (hf == 0 && qrow < nt && p.lse[g]) p.lse[g][((int64_t)b * NH + h) * nt + qrow] = mx * SCALE + __logf(sum);
       const float inv = 1.0f / sum;
       // epilogue: this thread's 32 output columns -> bf16 -> staging tile -> TMA store
       ptx::mbar_wait(&bar_o[sl], j & 1, p.err_flag, 36);
@@ -375,6 +409,8 @@ struct alignas(64) AttnBwdParams {
   int B, total_jobs;
   int* err_flag;
   long long* dbg;   // optional phase cycle counters of CTA 0 (V2S_GEMM_DEBUG): [16..27]
+  int N;            // VAR: tokens per image (2..197)
+  int ntiles, KP;   // VAR: query tiles per job (1 or 2) and keys padded to round_up(N, 16)
 };
 
 // the same accesses through 32-bit shared addresses with the per-row part precomputed (rowbase = tile + r * 128,
@@ -390,7 +426,11 @@ __device__ __forceinline__ uint4 load_p_chunk(const uint8_t* tile, int r, int c8
   return *reinterpret_cast<const uint4*>(tile + block * (QT * 128) + r * 128 + ((chunk ^ (r & 7)) << 4));
 }
 
-template <bool DBG, typename LP>
+// VAR: p.N tokens instead of 197 (v2s_set_image_size): S and dP are 128 x KP tiles (KP = round_up(N, 16)), dQ takes KP / 16
+// K-steps and dK / dV cover one 128-key tile when KP <= 128; 32-key chunks past N are skipped and the P chunks that hold
+// key N are bounds-checked, so keys >= N get P = 0 and dS = 0; query rows >= N are masked through their lse as the rows
+// >= 197 are; with N <= 128 a job is one query tile (dK / dV then accumulate over that one tile)
+template <bool DBG, typename LP, bool VAR = false>
 __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_constant__ AttnBwdParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -414,6 +454,9 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
     b = r % p.B; g = r / p.B;
   };
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;   // warp-uniform for the compiler
+  const int tl = VAR ? p.ntiles - 1 : 1;        // the job's last query tile
+  const int kp = VAR ? p.KP : KPAD;
+  const int nmt = VAR && kp <= QT ? 1 : 2;      // 128-key tiles of dK / dV
 
   if (warp == 0) {
     if (lane == 0) {
@@ -452,7 +495,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
     const uint32_t sbase = ptx::smem_u32(smem);
     const uint32_t sq = sbase + B_OFF_Q, sdo = sbase + B_OFF_DO, sk = sbase + B_OFF_K, sv = sbase + B_OFF_V;
     const uint32_t sp = sbase + B_OFF_P, sds = sbase + B_OFF_DS;
-    const uint32_t idesc_s = make_idesc_lp(LP::kIdescFmt, QT, KPAD, 0, 0);
+    const uint32_t idesc_s = make_idesc_lp(LP::kIdescFmt, QT, kp, 0, 0);
     const uint32_t idesc_dq = make_idesc_lp(LP::kIdescFmt, QT, DH, 0, 1);
     const uint32_t idesc_kv = make_idesc_lp(LP::kIdescFmt, QT, DH, 1, 1);
     constexpr uint32_t LOAD0_BYTES = Q_TILE_BYTES + 2 * KV_TILE_BYTES;
@@ -486,7 +529,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
       }
       __syncwarp();
 #pragma unroll 1
-      for (int t = 0; t < 2; ++t) {
+      for (int t = 0; t <= tl; ++t) {
         if (t == 1) {
           ptx::mbar_wait(&bar_kv[0], ph, p.err_flag, 21);     // tile-0 MMAs no longer read Q/dO/P/dS
           ptx::mbar_wait(bar_free, ph, p.err_flag, 22);       // dQ_0 drained, staging store done
@@ -515,7 +558,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
           for (int k = 0; k < DH / 16; ++k) mma(tmem_base, sdo + k * 32, 16, sv + k * 32, 16, idesc_s, k > 0);
           ptx::umma_commit(&bar_dp[t]);
 #pragma unroll
-          for (int mt = 0; mt < 2; ++mt)
+          for (int mt = 0; mt < nmt; ++mt)
 #pragma unroll
             for (int k = 0; k < QT / 16; ++k)
               mma(tmem_base + TM_DV + mt * DH, sp + 2 * mt * (QT * 128) + k * 2048, QT * 128, sdo + k * 2048, 8192,
@@ -527,11 +570,11 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
         ptx::tc_fence_after();
         if (ptx::elect_one()) {
 #pragma unroll
-          for (int j = 0; j < KPAD / 16; ++j)
+          for (int j = 0; j < kp / 16; ++j)
             mma(tmem_base, sds + (j >> 2) * (QT * 128) + (j & 3) * 32, 16, sk + j * 2048, 8192, idesc_dq, j > 0);
           ptx::umma_commit(&bar_dq[t]);
 #pragma unroll
-          for (int mt = 0; mt < 2; ++mt)
+          for (int mt = 0; mt < nmt; ++mt)
 #pragma unroll
             for (int k = 0; k < QT / 16; ++k)
               mma(tmem_base + TM_DK + mt * DH, sds + 2 * mt * (QT * 128) + k * 2048, QT * 128, sq + k * 2048, 8192,
@@ -542,17 +585,17 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
       }
       if (has_next) {
         // the next job's operands, each as soon as the chain has released its buffer (one barrier phase for all four)
-        ptx::mbar_wait(&bar_dq[1], ph, p.err_flag, 19);       // S_1, dP_1, dV, dQ_1 retired: K and V are dead
+        ptx::mbar_wait(&bar_dq[tl], ph, p.err_flag, 19);      // the last tile's S, dP, dV, dQ retired: K and V are dead
         if (ptx::elect_one()) {
           ptx::mbar_arrive_expect_tx(&bar_load[0], LOAD0_BYTES);
           ptx::tma_load_3d(smem + B_OFF_K, &p.tmKV[g2], &bar_load[0], D + h2 * DH, 0, b2);
           ptx::tma_load_3d(smem + B_OFF_V, &p.tmKV[g2], &bar_load[0], 2 * D + h2 * DH, 0, b2);
         }
         __syncwarp();
-        ptx::mbar_wait(&bar_kv[1], ph, p.err_flag, 20);       // dK retired: Q is dead
+        ptx::mbar_wait(&bar_kv[tl], ph, p.err_flag, 20);      // dK retired: Q is dead
         if (ptx::elect_one()) ptx::tma_load_3d(smem + B_OFF_Q, &p.tmQ[g2], &bar_load[0], h2 * DH, 0, b2);
         __syncwarp();
-        ptx::mbar_wait(bar_done, ph, p.err_flag, 18);         // the dQ_1 store has read its staging tile (the dO buffer)
+        ptx::mbar_wait(bar_done, ph, p.err_flag, 18);         // the last dQ store has read its staging tile (the dO buffer)
         if (ptx::elect_one()) {
           ptx::mbar_arrive_expect_tx(&bar_do[0], Q_TILE_BYTES);
           ptx::tma_load_3d(smem + B_OFF_DO, &p.tmDO[g2], &bar_do[0], h2 * DH, 0, b2);
@@ -577,17 +620,18 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
 #define V2S_TICK(k) if (DBG) { c1 = clock64(); tk[k] += c1 - c0; c0 = c1; }
     // The O row (for D = rowsum(dO * O)) and the row's log-sum-exp come from global memory.  Their loads are issued one
     // tile ahead into registers (this warp role has 200+ registers to spare), so the DRAM latency is never on the chain.
+    const int nt = VAR ? p.N : NT;
     uint4 ov[8];
     float lse_nxt = 0.f;
     auto fetch_row = [&](int n2, int t2) {
       int h2, b2, g2;
       decode(n2, h2, b2, g2);
       const int qr = t2 * QT + row;
-      if (qr < NT) {
-        const uint4* orow = reinterpret_cast<const uint4*>(p.ctx[g2] + ((int64_t)b2 * NT + qr) * D + h2 * DH);
+      if (qr < nt) {
+        const uint4* orow = reinterpret_cast<const uint4*>(p.ctx[g2] + ((int64_t)b2 * nt + qr) * D + h2 * DH);
 #pragma unroll
         for (int c = 0; c < 8; ++c) ov[c] = __ldg(orow + c);
-        lse_nxt = __ldg(p.lse[g2] + ((int64_t)b2 * NH + h2) * NT + qr);
+        lse_nxt = __ldg(p.lse[g2] + ((int64_t)b2 * NH + h2) * nt + qr);
       }
     };
     if (njobs > 0) fetch_row(0, 0);
@@ -596,9 +640,9 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
     const uint32_t ph = n & 1;
     int h, b, g;
     decode(n, h, b, g);
-    for (int t = 0; t < 2; ++t) {
+    for (int t = 0; t <= tl; ++t) {
       const int qrow = t * QT + row;
-      const bool valid = qrow < NT;
+      const bool valid = qrow < nt;
       // padding query rows (>= 197): lse2 = +huge makes every p underflow to exactly 0, no per-element row mask needed
       const float lse2 = valid ? lse_nxt * LOG2E : 3.0e38f;
       // ---- P = exp(S/8 - lse) ----
@@ -607,6 +651,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
       ptx::tc_fence_after();
 #pragma unroll 1
       for (int c = 0; c < 3; ++c) {
+        if (VAR && col0 + c * 32 >= nt) break;      // keys >= KP: read by neither dQ nor the kept rows of dK / dV
         ptx::tmem_ld_32x32(tlane + col0 + c * 32, r);
         ptx::tmem_ld_wait();
         // only keys 176..207 (second half, last chunk) contain padding keys: the bound check stays out of the other chunks
@@ -614,7 +659,12 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           float e[8];
-          if (!tail) {
+          if (VAR) {
+            const int kb = col0 + c * 32 + j * 8;
+#pragma unroll
+            for (int i = 0; i < 8; ++i)
+              e[i] = (kb + i < nt) ? ptx::ex2_approx(fmaf(__uint_as_float(r[8 * j + i]), SCALE_LOG2E, -lse2)) : 0.f;
+          } else if (!tail) {
 #pragma unroll
             for (int i = 0; i < 8; ++i) e[i] = ptx::ex2_approx(fmaf(__uint_as_float(r[8 * j + i]), SCALE_LOG2E, -lse2));
           } else {
@@ -627,7 +677,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
           store_p_chunk_s(prow_s, rx, (col0 + c * 32) / 8 + j, v);
         }
       }
-      if (half == 0) {      // keys 96..111
+      if (half == 0 && (!VAR || 96 < nt)) {      // keys 96..111
         ptx::tmem_ld_32x16(tlane + 96, r);
         ptx::tmem_ld_wait();
 #pragma unroll
@@ -635,7 +685,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
           float e[8];
 #pragma unroll
           for (int i = 0; i < 8; ++i)
-            e[i] = ptx::ex2_approx(fmaf(__uint_as_float(r[8 * j + i]), SCALE_LOG2E, -lse2));
+            e[i] = (!VAR || 96 + 8 * j + i < nt) ? ptx::ex2_approx(fmaf(__uint_as_float(r[8 * j + i]), SCALE_LOG2E, -lse2)) : 0.f;
           uint4 v;
           v.x = LP::pack(e[0], e[1]); v.y = LP::pack(e[2], e[3]); v.z = LP::pack(e[4], e[5]); v.w = LP::pack(e[6], e[7]);
           store_p_chunk_s(prow_s, rx, 12 + j, v);
@@ -663,7 +713,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
           }
         }
       }
-      if (t == 0) fetch_row(n, 1);
+      if (t == 0 && tl != 0) fetch_row(n, 1);
       else if (n + 1 < njobs) fetch_row(n + 1, 0);
       V2S_TICK(9)
       // ---- dS = P * (dP - D) / 8 ----
@@ -673,6 +723,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
       ptx::tc_fence_after();
 #pragma unroll 1
       for (int c = 0; c < 3; ++c) {
+        if (VAR && col0 + c * 32 >= nt) break;
         ptx::tmem_ld_32x32(tlane + col0 + c * 32, r);
         ptx::tmem_ld_wait();
 #pragma unroll
@@ -691,7 +742,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
           store_p_chunk_s(dsrow_s, rx, c8, v);
         }
       }
-      if (half == 0) {
+      if (half == 0 && (!VAR || 96 < nt)) {
         ptx::tmem_ld_32x16(tlane + 96, r);
         ptx::tmem_ld_wait();
 #pragma unroll
@@ -739,17 +790,17 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
         ptx::tma_commit_group();
         ptx::tma_wait_group_read<0>();
       }
-      ptx::mbar_arrive(t == 0 ? bar_free : bar_done);     // (thread 32: after its store has read the staging tile)
+      ptx::mbar_arrive(t == 0 && tl != 0 ? bar_free : bar_done);     // (thread 32: after its store has read the staging tile)
       V2S_TICK(6)
     }
     // ---- dK, dV: TMEM → bf16 → staged in the P buffer → TMA store (rows = keys) ----
-    ptx::mbar_wait(&bar_kv[1], ph, p.err_flag, 29);      // every MMA of the job has retired
+    ptx::mbar_wait(&bar_kv[tl], ph, p.err_flag, 29);      // every MMA of the job has retired
     V2S_TICK(7)
     ptx::tc_fence_after();
 #pragma unroll 1
     for (int which = 0; which < 2; ++which) {          // 0: dK, 1: dV
 #pragma unroll 1
-      for (int mt = 0; mt < 2; ++mt) {
+      for (int mt = 0; mt < nmt; ++mt) {
         ptx::tmem_ld_32x32(tlane + (which ? TM_DV : TM_DK) + mt * DH + half * 32, r);
         ptx::tmem_ld_wait();
         uint8_t* stg = smem + B_OFF_P + (which * 2 + mt) * Q_TILE_BYTES;
@@ -768,7 +819,7 @@ __global__ void __launch_bounds__(B_THREADS, 1) attn_bwd_tc_kernel(const __grid_
     ptx::bar_sync(1, 256);
     if (threadIdx.x == 32) {
       for (int which = 0; which < 2; ++which)
-        for (int mt = 0; mt < 2; ++mt)
+        for (int mt = 0; mt < nmt; ++mt)
           ptx::tma_store_3d(&p.tmDQKV[g], smem + B_OFF_P + (which * 2 + mt) * Q_TILE_BYTES,
                             (1 + which) * D + h * DH, mt * QT, b);
       ptx::tma_commit_group();
@@ -819,9 +870,12 @@ struct alignas(64) AttnProbsParams {
   const float* lse[MAXG];              // unused by DP
   float* probs[MAXG];
   int* err_flag;
+  int N, ntiles;                       // VAR: tokens per image and query tiles (grid.x = 3 * ntiles)
+  int KP;                              // VAR: keys padded to round_up(N, 16), the N of the S UMMA
 };
 
-template <typename LP, bool DP>
+// VAR: p.N tokens instead of 197 (v2s_set_image_size): a 128 x KP score tile (KP = round_up(N, 16)), output rows of stride N
+template <typename LP, bool DP, bool VAR = false>
 __global__ void __launch_bounds__(PR_THREADS, 2) attn_probs_tc_kernel(const __grid_constant__ AttnProbsParams p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -829,9 +883,11 @@ __global__ void __launch_bounds__(PR_THREADS, 2) attn_probs_tc_kernel(const __gr
   uint64_t* bar_s = bar_load + 1;
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bar_s + 1);
   float* stg = reinterpret_cast<float*>(smem);
-  const int t = blockIdx.x & 1, h = blockIdx.x >> 1, b = blockIdx.y, g = blockIdx.z;
+  const int nt = VAR ? p.N : NT;
+  const bool two_tiles = !VAR || p.ntiles == 2;
+  const int t = two_tiles ? blockIdx.x & 1 : 0, h = two_tiles ? blockIdx.x >> 1 : blockIdx.x, b = blockIdx.y, g = blockIdx.z;
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;
-  const int nrows = NT - t * QT < QT ? NT - t * QT : QT;
+  const int nrows = nt - t * QT < QT ? nt - t * QT : QT;
 
   if (warp == 0) {
     if (lane == 0) {
@@ -858,7 +914,7 @@ __global__ void __launch_bounds__(PR_THREADS, 2) attn_probs_tc_kernel(const __gr
     __syncwarp();
     ptx::mbar_wait(bar_load, 0, p.err_flag, 61);
     ptx::tc_fence_after();
-    const uint32_t idesc_s = make_idesc_lp(LP::kIdescFmt, QT, KPAD, 0, 0);
+    const uint32_t idesc_s = make_idesc_lp(LP::kIdescFmt, QT, VAR ? p.KP : KPAD, 0, 0);
     const uint32_t sq = ptx::smem_u32(smem) + PR_OFF_Q, sk = ptx::smem_u32(smem) + PR_OFF_K;
     if (ptx::elect_one()) {
 #pragma unroll
@@ -872,33 +928,36 @@ __global__ void __launch_bounds__(PR_THREADS, 2) attn_probs_tc_kernel(const __gr
     const int qrow = t * QT + row;
     const bool valid = row < nrows;
     const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16);
-    const float lse2 = !DP && valid ? __ldg(p.lse[g] + ((int64_t)b * NH + h) * NT + qrow) * LOG2E : 0.f;
+    const float lse2 = !DP && valid ? __ldg(p.lse[g] + ((int64_t)b * NH + h) * nt + qrow) * LOG2E : 0.f;
     auto epi = [&](uint32_t v) { return DP ? __uint_as_float(v) : ptx::ex2_approx(fmaf(__uint_as_float(v), SCALE_LOG2E, -lse2)); };
-    float* srow = stg + row * NT;
+    float* srow = stg + row * nt;
     uint32_t r[32];
     ptx::mbar_wait(bar_s, 0, p.err_flag, 62);     // S complete: the Q / K tiles are dead, staging may overwrite them
     ptx::tc_fence_after();
 #pragma unroll 1
     for (int c = 0; c < 6; ++c) {
+      if (VAR && c * 32 >= nt) break;
       ptx::tmem_ld_32x32(taddr + c * 32, r);
       ptx::tmem_ld_wait();
       if (valid) {
 #pragma unroll
-        for (int i = 0; i < 32; ++i) srow[c * 32 + i] = epi(r[i]);
+        for (int i = 0; i < 32; ++i)
+          if (!VAR || c * 32 + i < nt) srow[c * 32 + i] = epi(r[i]);
       }
     }
-    ptx::tmem_ld_32x16(taddr + 192, r);
+    if (!VAR || 192 < nt) ptx::tmem_ld_32x16(taddr + 192, r);
     ptx::tmem_ld_wait();
-    if (valid) {
+    if (valid && (!VAR || 192 < nt)) {
 #pragma unroll
-      for (int i = 0; i < NT - 192; ++i) srow[192 + i] = epi(r[i]);
+      for (int i = 0; i < NT - 192; ++i)
+        if (!VAR || 192 + i < nt) srow[192 + i] = epi(r[i]);
     }
   }
   ptx::tc_fence_before();
   __syncthreads();
   {
-    float* dst = p.probs[g] + (((int64_t)b * NH + h) * NT + t * QT) * NT;
-    const int n = nrows * NT;
+    float* dst = p.probs[g] + (((int64_t)b * NH + h) * nt + t * QT) * nt;
+    const int n = nrows * nt;
     for (int i = threadIdx.x; i < n; i += PR_THREADS) dst[i] = stg[i];
   }
   if (warp == 0) {
@@ -907,33 +966,41 @@ __global__ void __launch_bounds__(PR_THREADS, 2) attn_probs_tc_kernel(const __gr
   }
 }
 
-// launches attn_probs_tc_kernel<LP, DP> over (2 query tiles x 3 heads, B images, groups)
-template <bool DP>
-int launch_probs_kernel(const AttnProbsParams& p, int groups, int B, cudaStream_t s, int lp_f16) {
+// launches attn_probs_tc_kernel<LP, DP, VAR> over (query tiles x 3 heads, B images, groups)
+template <bool DP, bool VAR>
+int launch_probs_kernel_t(const AttnProbsParams& p, int groups, int B, cudaStream_t s, int lp_f16) {
   static bool attr[MAX_DEVICES] = {false};
   if (!attr[cur_device()]) {
-    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_tc_kernel<LpBf16, DP>, cudaFuncAttributeMaxDynamicSharedMemorySize, PR_SMEM));
-    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_tc_kernel<LpF16, DP>, cudaFuncAttributeMaxDynamicSharedMemorySize, PR_SMEM));
+    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_tc_kernel<LpBf16, DP, VAR>, cudaFuncAttributeMaxDynamicSharedMemorySize, PR_SMEM));
+    V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_tc_kernel<LpF16, DP, VAR>, cudaFuncAttributeMaxDynamicSharedMemorySize, PR_SMEM));
     attr[cur_device()] = true;
   }
-  const dim3 grid(NH * 2, B, groups);
-  if (lp_f16) V2S_CUDA_OK(launch_pdl(attn_probs_tc_kernel<LpF16, DP>, grid, dim3(PR_THREADS), (size_t)PR_SMEM, s, p));
-  else V2S_CUDA_OK(launch_pdl(attn_probs_tc_kernel<LpBf16, DP>, grid, dim3(PR_THREADS), (size_t)PR_SMEM, s, p));
+  const dim3 grid(NH * (VAR ? p.ntiles : 2), B, groups);
+  if (lp_f16) V2S_CUDA_OK(launch_pdl(attn_probs_tc_kernel<LpF16, DP, VAR>, grid, dim3(PR_THREADS), (size_t)PR_SMEM, s, p));
+  else V2S_CUDA_OK(launch_pdl(attn_probs_tc_kernel<LpBf16, DP, VAR>, grid, dim3(PR_THREADS), (size_t)PR_SMEM, s, p));
   V2S_LAUNCH_CHECK();
   return 0;
+}
+template <bool DP>
+int launch_probs_kernel(AttnProbsParams& p, int groups, int B, cudaStream_t s, int lp_f16) {
+  const int nt = image_geom().nt;
+  if (nt == NT) return launch_probs_kernel_t<DP, false>(p, groups, B, s, lp_f16);
+  p.N = nt; p.ntiles = (nt + QT - 1) / QT; p.KP = (nt + 15) / 16 * 16;
+  return launch_probs_kernel_t<DP, true>(p, groups, B, s, lp_f16);
 }
 
 }  // namespace
 
 int launch_attn_probs_tc(const void* const* qkv, const float* const* lse, float* const* probs, int groups, int B,
                          cudaStream_t s, int lp_f16) {
+  const int nt = image_geom().nt;   // tokens per image: the token dimension of the tensor maps
   AttnProbsParams p;
   memset(&p, 0, sizeof(p));
   p.err_flag = tc_err_flag();
   for (int g = 0; g < groups; ++g) {
     if (!lse[g] || !probs[g]) { set_error("attention probabilities: group %d has no lse / output", g); return 1; }
-    V2S_TRY(tmap_get_3d(&p.tmQ[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, QT, true, 128));
-    V2S_TRY(tmap_get_3d(&p.tmKV[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, KPAD, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmQ[g], qkv[g], 3 * D, nt, B, 3 * D * 2, (uint64_t)nt * 3 * D * 2, DH, QT, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmKV[g], qkv[g], 3 * D, nt, B, 3 * D * 2, (uint64_t)nt * 3 * D * 2, DH, KPAD, true, 128));
     p.lse[g] = lse[g];
     p.probs[g] = probs[g];
   }
@@ -942,13 +1009,14 @@ int launch_attn_probs_tc(const void* const* qkv, const float* const* lse, float*
 
 int launch_attn_dprobs_tc(const void* const* qkv, const void* const* dctx, float* const* dprobs, int groups, int B,
                           cudaStream_t s, int lp_f16) {
+  const int nt = image_geom().nt;   // tokens per image: the token dimension of the tensor maps
   AttnProbsParams p;
   memset(&p, 0, sizeof(p));
   p.err_flag = tc_err_flag();
   for (int g = 0; g < groups; ++g) {
     if (!dctx[g] || !dprobs[g]) { set_error("attention-probability gradient: group %d has no d ctx / output", g); return 1; }
-    V2S_TRY(tmap_get_3d(&p.tmQ[g], dctx[g], D, NT, B, D * 2, (uint64_t)NT * D * 2, DH, QT, true, 128));
-    V2S_TRY(tmap_get_3d(&p.tmKV[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, KPAD, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmQ[g], dctx[g], D, nt, B, D * 2, (uint64_t)nt * D * 2, DH, QT, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmKV[g], qkv[g], 3 * D, nt, B, 3 * D * 2, (uint64_t)nt * 3 * D * 2, DH, KPAD, true, 128));
     p.probs[g] = dprobs[g];
   }
   return launch_probs_kernel<true>(p, groups, B, s, lp_f16);
@@ -956,15 +1024,32 @@ int launch_attn_dprobs_tc(const void* const* qkv, const void* const* dctx, float
 
 int launch_attn_fwd_tc(const void* const* qkv, void* const* ctx, float* const* lse, int groups, int B,
                        cudaStream_t s, int lp_f16) {
+  const int nt = image_geom().nt;   // tokens per image: the token dimension of the tensor maps
   AttnFwdPParams p;
   memset(&p, 0, sizeof(p));
   for (int g = 0; g < groups; ++g) {
-    V2S_TRY(tmap_get_3d(&p.tmQ[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, QT, true, 128));
-    V2S_TRY(tmap_get_3d(&p.tmKV[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, KPAD, true, 128));
-    V2S_TRY(tmap_get_3d(&p.tmCtx[g], ctx[g], D, NT, B, D * 2, (uint64_t)NT * D * 2, DH, QT, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmQ[g], qkv[g], 3 * D, nt, B, 3 * D * 2, (uint64_t)nt * 3 * D * 2, DH, QT, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmKV[g], qkv[g], 3 * D, nt, B, 3 * D * 2, (uint64_t)nt * 3 * D * 2, DH, KPAD, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmCtx[g], ctx[g], D, nt, B, D * 2, (uint64_t)nt * D * 2, DH, QT, true, 128));
     p.lse[g] = lse ? lse[g] : nullptr;
   }
   p.B = B; p.total_jobs = 2 * NH * B * groups; p.err_flag = tc_err_flag(); p.dbg = tc_dbg_counters();
+  if (nt != NT) {       // the variable-length instantiation: ceil(N / 128) query tiles per (head, image)
+    p.N = nt; p.ntiles = (nt + QT - 1) / QT; p.KP = (nt + 15) / 16 * 16;
+    p.total_jobs = p.ntiles * NH * B * groups;
+    static bool vattr[MAX_DEVICES] = {false};
+    if (!vattr[cur_device()]) {
+      V2S_CUDA_OK(cudaFuncSetAttribute(attn_fwd_persist_kernel<false, LpBf16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PF_SMEM));
+      V2S_CUDA_OK(cudaFuncSetAttribute(attn_fwd_persist_kernel<false, LpF16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, PF_SMEM));
+      vattr[cur_device()] = true;
+    }
+    const int grid = p.total_jobs < tc_num_sms() ? p.total_jobs : tc_num_sms();
+    p.dbg = nullptr;
+    if (lp_f16) V2S_CUDA_OK(launch_pdl(attn_fwd_persist_kernel<false, LpF16, true>, dim3(grid), dim3(PF_THREADS), (size_t)PF_SMEM, s, p));
+    else V2S_CUDA_OK(launch_pdl(attn_fwd_persist_kernel<false, LpBf16, true>, dim3(grid), dim3(PF_THREADS), (size_t)PF_SMEM, s, p));
+    V2S_LAUNCH_CHECK();
+    return 0;
+  }
   static bool pattr[MAX_DEVICES] = {false};
   if (!pattr[cur_device()]) {
     V2S_CUDA_OK(cudaFuncSetAttribute(attn_fwd_persist_kernel<false, LpBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PF_SMEM));
@@ -992,20 +1077,36 @@ namespace v2s {
 
 int launch_attn_bwd_tc(const void* const* qkv, const void* const* ctx, const float* const* lse,
                        const void* const* dctx, void* const* dqkv, int groups, int B, cudaStream_t s, int lp_f16) {
+  const int nt = image_geom().nt;   // tokens per image: the token dimension of the tensor maps
   AttnBwdParams p;
   memset(&p, 0, sizeof(p));
   p.err_flag = tc_err_flag();
   for (int g = 0; g < groups; ++g) {
-    V2S_TRY(tmap_get_3d(&p.tmQ[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, QT, true, 128));
-    V2S_TRY(tmap_get_3d(&p.tmKV[g], qkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, KPAD, true, 128));
-    V2S_TRY(tmap_get_3d(&p.tmDO[g], dctx[g], D, NT, B, D * 2, (uint64_t)NT * D * 2, DH, QT, true, 128));
-    V2S_TRY(tmap_get_3d(&p.tmDQKV[g], dqkv[g], 3 * D, NT, B, 3 * D * 2, (uint64_t)NT * 3 * D * 2, DH, QT, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmQ[g], qkv[g], 3 * D, nt, B, 3 * D * 2, (uint64_t)nt * 3 * D * 2, DH, QT, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmKV[g], qkv[g], 3 * D, nt, B, 3 * D * 2, (uint64_t)nt * 3 * D * 2, DH, KPAD, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmDO[g], dctx[g], D, nt, B, D * 2, (uint64_t)nt * D * 2, DH, QT, true, 128));
+    V2S_TRY(tmap_get_3d(&p.tmDQKV[g], dqkv[g], 3 * D, nt, B, 3 * D * 2, (uint64_t)nt * 3 * D * 2, DH, QT, true, 128));
     p.ctx[g] = static_cast<const bf16*>(ctx[g]);
     p.lse[g] = lse[g];
   }
   p.dbg = tc_dbg_counters();
   p.B = B;
   p.total_jobs = NH * B * groups;
+  if (nt != NT) {       // the variable-length instantiation: ceil(N / 128) query tiles per job
+    p.N = nt; p.ntiles = (nt + QT - 1) / QT; p.KP = (nt + 15) / 16 * 16;
+    p.dbg = nullptr;
+    static bool vattr[MAX_DEVICES] = {false};
+    if (!vattr[cur_device()]) {
+      V2S_CUDA_OK(cudaFuncSetAttribute(attn_bwd_tc_kernel<false, LpBf16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, B_SMEM));
+      V2S_CUDA_OK(cudaFuncSetAttribute(attn_bwd_tc_kernel<false, LpF16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, B_SMEM));
+      vattr[cur_device()] = true;
+    }
+    const dim3 grid(p.total_jobs < tc_num_sms() ? p.total_jobs : tc_num_sms());
+    if (lp_f16) V2S_CUDA_OK(launch_pdl(attn_bwd_tc_kernel<false, LpF16, true>, grid, dim3(B_THREADS), (size_t)B_SMEM, s, p));
+    else V2S_CUDA_OK(launch_pdl(attn_bwd_tc_kernel<false, LpBf16, true>, grid, dim3(B_THREADS), (size_t)B_SMEM, s, p));
+    V2S_LAUNCH_CHECK();
+    return 0;
+  }
   static bool attr[MAX_DEVICES] = {false};
   if (!attr[cur_device()]) {
     V2S_CUDA_OK(cudaFuncSetAttribute(attn_bwd_tc_kernel<false, LpBf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, B_SMEM));

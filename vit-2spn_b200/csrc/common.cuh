@@ -163,6 +163,12 @@ __device__ __forceinline__ float gelu_grad_f(float x) {
   return cdf + x * pdf;
 }
 
+// ---- input image size of the backbone calls (v2s_set_image_size; default 224 x 224) ----------------
+// H, W: pixels (multiples of 16); gh x gw: the patch grid; np = gh * gw patches, nt = np + 1 tokens (at most 197)
+struct ImageGeom { int H, W, gh, gw, np, nt; };
+const ImageGeom& image_geom();
+inline bool geom_is_default(const ImageGeom& g) { return g.H == V2S_IMG && g.W == V2S_IMG; }
+
 // per-group pointer bundles passed by value to grouped kernels (blockIdx.z = group)
 template <typename T> struct GPtr {
   T* p[MAXG];

@@ -17,6 +17,10 @@ namespace v2s {
 static thread_local char g_err[1024] = "";
 int64_t g_launch_count = 0;
 
+// v2s_set_image_size: process-wide, read when work is enqueued
+static ImageGeom g_geom = {V2S_IMG, V2S_IMG, V2S_IMG / 16, V2S_IMG / 16, NP, NT};
+const ImageGeom& image_geom() { return g_geom; }
+
 void set_error(const char* fmt, ...) {
   va_list ap;
   va_start(ap, fmt);
@@ -64,16 +68,17 @@ struct LayerStash {   // byte offsets relative to the slot base
 struct Plan {
   int B, at;
   int64_t es;          // activation element size
-  int64_t M, MP;
+  int64_t M, MP;       // token rows B * nt and patch rows B * np at the image size of image_geom()
+  bool interp;         // the position table is interpolated (image size other than 224 x 224)
   int64_t heads_bytes;
   // per-group forward scratch (groups that do not save activations)
-  int64_t f_patches, f_xa, f_xb, f_xn, f_qkv, f_ctx, f_h, f_bytes;
+  int64_t f_patches, f_xa, f_xb, f_xn, f_qkv, f_ctx, f_h, f_pos, f_bytes;
   // per-slot stash
   int64_t s_patches, s_x[NL + 1];
   LayerStash s_layer[NL];
-  int64_t s_bytes;
+  int64_t s_pos, s_bytes;
   // per-slot backward scratch
-  int64_t b_dx, b_dxlp, b_big, b_tmp, b_bytes;
+  int64_t b_dx, b_dxlp, b_big, b_tmp, b_dpos, b_bytes;
 };
 
 Plan make_plan(int B, int mode) {
@@ -82,8 +87,11 @@ Plan make_plan(int B, int mode) {
   p.B = B;
   p.at = mode == V2S_MODE_BF16 ? AT_BF16 : mode == V2S_MODE_FP16 ? AT_F16 : AT_F32;   // activation type tag
   p.es = p.at ? 2 : 4;
-  p.M = (int64_t)B * NT;
-  p.MP = (int64_t)B * NP;
+  const ImageGeom& geo = image_geom();
+  p.M = (int64_t)B * geo.nt;
+  p.MP = (int64_t)B * geo.np;
+  p.interp = !geom_is_default(geo);
+  const int64_t pos_bytes = p.interp ? (int64_t)geo.nt * D * 4 : 0;   // pos' / d pos' [nt,192] fp32
   p.heads_bytes = align_up((int64_t)B * 8192 * 4 + 4096);
   int64_t o = 0;
   auto take = [&](int64_t bytes) { int64_t r = o; o += align_up(bytes); return r; };
@@ -94,6 +102,7 @@ Plan make_plan(int B, int mode) {
   p.f_qkv = take(p.M * 3 * D * p.es);
   p.f_ctx = take(p.M * D * p.es);
   p.f_h = take(p.M * DF * p.es);
+  p.f_pos = take(pos_bytes);
   p.f_bytes = o;
   o = 0;
   p.s_patches = take(p.MP * KPE * p.es);
@@ -104,19 +113,21 @@ Plan make_plan(int B, int mode) {
     s.xn1 = take(p.M * D * p.es);
     s.qkv = take(p.M * 3 * D * p.es);
     s.ctx = take(p.M * D * p.es);
-    s.lse = take((int64_t)B * NH * NT * 4);
+    s.lse = take((int64_t)B * NH * geo.nt * 4);
     s.x_mid = take(p.M * D * 4);
     s.mean2 = take(p.M * 4); s.rstd2 = take(p.M * 4);
     s.xn2 = take(p.M * D * p.es);
     s.u = take(p.M * DF * p.es);
     s.h = take(p.M * DF * p.es);
   }
+  p.s_pos = take(pos_bytes);
   p.s_bytes = o;
   o = 0;
   p.b_dx = take(p.M * D * 4);
   p.b_dxlp = take(p.M * D * p.es);
   p.b_big = take(p.M * DF * p.es);
   p.b_tmp = take(p.M * D * p.es);
+  p.b_dpos = take(pos_bytes);
   p.b_bytes = o;
   return p;
 }
@@ -230,13 +241,15 @@ inline const void* weight_ptr(const v2s_group_t& g, int at, int64_t off) {
 
 int launch_attention_fwd(const void* const* qkv, void* const* ctx, float* const* lse, int groups, int B, int at,
                          cudaStream_t s) {
-  prof::Scope scope(prof::C_ATTN_F, 4.0 * B * NH * (double)NT * NT * DH * groups, s, (double)B * NT * 4 * D * 2.0 * groups);
+  const double nt = image_geom().nt;
+  prof::Scope scope(prof::C_ATTN_F, 4.0 * B * NH * nt * nt * DH * groups, s, (double)B * nt * 4 * D * 2.0 * groups);
   if (at != AT_F32) return launch_attn_fwd_tc(qkv, ctx, lse, groups, B, s, at == AT_F16);
   return launch_attn_fwd_simt(qkv, ctx, lse, groups, B, at, s);
 }
 int launch_attention_bwd(const void* const* qkv, const void* const* ctx, const float* const* lse,
                          const void* const* dctx, void* const* dqkv, int groups, int B, int at, cudaStream_t s) {
-  prof::Scope scope(prof::C_ATTN_B, 10.0 * B * NH * (double)NT * NT * DH * groups, s, (double)B * NT * 8 * D * 2.0 * groups);
+  const double nt = image_geom().nt;
+  prof::Scope scope(prof::C_ATTN_B, 10.0 * B * NH * nt * nt * DH * groups, s, (double)B * nt * 8 * D * 2.0 * groups);
   if (at != AT_F32) return launch_attn_bwd_tc(qkv, ctx, lse, dctx, dqkv, groups, B, s, at == AT_F16);
   return launch_attn_bwd_simt(qkv, ctx, lse, dctx, dqkv, groups, B, at, s);
 }
@@ -245,8 +258,9 @@ int launch_attention_bwd(const void* const* qkv, const void* const* ctx, const f
 int launch_attention_probs(const void* const* qkv, const float* const* lse, float* const* probs, int groups, int B, int at,
                            cudaStream_t s) {
   // algorithmic bytes: Q and K read once, lse, the fp32 probabilities written once
-  prof::Scope scope(prof::C_ATTN_P, 2.0 * B * NH * (double)NT * NT * DH * groups, s,
-                    ((double)B * NT * 2 * D * (at ? 2.0 : 4.0) + (double)B * NH * NT * 4 + (double)B * NH * NT * NT * 4) * groups);
+  const double nt = image_geom().nt;
+  prof::Scope scope(prof::C_ATTN_P, 2.0 * B * NH * nt * nt * DH * groups, s,
+                    ((double)B * nt * 2 * D * (at ? 2.0 : 4.0) + (double)B * NH * nt * 4 + (double)B * NH * nt * nt * 4) * groups);
   if (at != AT_F32) return launch_attn_probs_tc(qkv, lse, probs, groups, B, s, at == AT_F16);
   return launch_attn_probs_simt(qkv, lse, probs, groups, B, at, s);
 }
@@ -255,8 +269,9 @@ int launch_attention_probs(const void* const* qkv, const float* const* lse, floa
 int launch_attention_dprobs(const void* const* qkv, const void* const* dctx, float* const* dprobs, int groups, int B, int at,
                             cudaStream_t s) {
   // algorithmic bytes: d ctx and V read once, the fp32 gradient written once
-  prof::Scope scope(prof::C_ATTN_DP, 2.0 * B * NH * (double)NT * NT * DH * groups, s,
-                    ((double)B * NT * 2 * D * (at ? 2.0 : 4.0) + (double)B * NH * NT * NT * 4) * groups);
+  const double nt = image_geom().nt;
+  prof::Scope scope(prof::C_ATTN_DP, 2.0 * B * NH * nt * nt * DH * groups, s,
+                    ((double)B * nt * 2 * D * (at ? 2.0 : 4.0) + (double)B * NH * nt * nt * 4) * groups);
   if (at != AT_F32) return launch_attn_dprobs_tc(qkv, dctx, dprobs, groups, B, s, at == AT_F16);
   return launch_attn_dprobs_simt(qkv, dctx, dprobs, groups, B, at, s);
 }
@@ -312,19 +327,41 @@ int check_outputs(const v2s_group_outputs_t* o, const v2s_group_t& gr, int g, bo
 // them back: remember per (workspace, stash slot) which hidden[0] the forward used, so that a backward given other
 // tensors (or none, or some where the forward had none) is an error rather than a silent wrong gradient.  The same
 // holds for the patch mask: the backward must be given the mask array its forward used (or none for none).
-struct HiddenRec { const void* ws; int slot; const float* h0; const uint8_t* mask; };
+// The image size is recorded the same way: the stash layout and every token row follow it.
+struct HiddenRec { const void* ws; int slot; const float* h0; const uint8_t* mask; int img_h, img_w; };
 static HiddenRec g_hidden_rec[64];
 static int g_n_hidden_rec = 0;
 void record_hidden(const void* ws, int slot, const float* h0, const uint8_t* mask) {
+  const ImageGeom& geo = image_geom();
   for (int i = 0; i < g_n_hidden_rec; ++i)
-    if (g_hidden_rec[i].ws == ws && g_hidden_rec[i].slot == slot) { g_hidden_rec[i].h0 = h0; g_hidden_rec[i].mask = mask; return; }
+    if (g_hidden_rec[i].ws == ws && g_hidden_rec[i].slot == slot) {
+      g_hidden_rec[i].h0 = h0; g_hidden_rec[i].mask = mask; g_hidden_rec[i].img_h = geo.H; g_hidden_rec[i].img_w = geo.W;
+      return;
+    }
   const int i = g_n_hidden_rec < 64 ? g_n_hidden_rec++ : (int)((reinterpret_cast<uintptr_t>(ws) / 1024 + (uintptr_t)slot) % 64);
-  g_hidden_rec[i] = {ws, slot, h0, mask};
+  g_hidden_rec[i] = {ws, slot, h0, mask, geo.H, geo.W};
 }
 const HiddenRec* find_hidden(const void* ws, int slot) {
   for (int i = 0; i < g_n_hidden_rec; ++i)
     if (g_hidden_rec[i].ws == ws && g_hidden_rec[i].slot == slot) return &g_hidden_rec[i];
   return nullptr;
+}
+
+// a GemmDesc carrying the token geometry of image_geom() (patch-row remaps, EPI_PATCH, EPI_PIXELS)
+GemmDesc geo_gemm_desc() {
+  GemmDesc d = make_gemm_desc();
+  const ImageGeom& geo = image_geom();
+  d.np = geo.np; d.nt = geo.nt; d.img_h = geo.H; d.img_w = geo.W; d.img_gw = geo.gw;
+  return d;
+}
+
+// the calls that exist at 224 x 224 only refuse another image size
+int refuse_image_size(const char* what) {
+  const ImageGeom& geo = image_geom();
+  if (geom_is_default(geo)) return 0;
+  set_error("%s: supported for 224 x 224 inputs only (the image size is %d x %d; v2s_set_image_size(224, 224))", what, geo.H,
+            geo.W);
+  return 1;
 }
 
 int wgrad_split(int64_t rows) {
@@ -357,6 +394,8 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
       set_error("backbone_forward: group %d: x_format %d (1 = 16-bit patch rows, 16-bit modes only)", g, gs[g].x_format);
       return 1;
     }
+    if (gs[g].x_format == 1) V2S_TRY(refuse_image_size("backbone_forward: patch-row inputs (x_format 1)"));
+    if (gs[g].feat) V2S_TRY(refuse_image_size("backbone_forward: the pooled feature (feat)"));
     V2S_TRY(check_outputs(outs ? &outs[g] : nullptr, gs[g], g, false));
   }
   const int64_t M = p.M, MP = p.MP;
@@ -393,9 +432,20 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
     }
     if (nu > 0) V2S_TRY(launch_im2col(ux, uo, nu, B, at, st));
   }
+  // another image size than 224 x 224: the position table interpolated to the patch grid, pos' [nt,192] per group
+  const float* pos[MAXG] = {nullptr, nullptr, nullptr, nullptr};
+  if (p.interp) {
+    const float* pp[MAXG]; float* po[MAXG];
+    for (int g = 0; g < G; ++g) {
+      po[g] = reinterpret_cast<float*>(saved(g) ? sb(g, p.s_pos) : fb(g, p.f_pos));
+      pp[g] = gs[g].params; pos[g] = po[g];
+    }
+    prof::Scope sc(prof::C_MISC, (double)image_geom().nt * D * 4 * 17 * G, st);
+    V2S_TRY(launch_pos_interp_fwd(pp, po, G, st));
+  }
   float* x_cur[MAXG];
   {
-    GemmDesc d = make_gemm_desc();
+    GemmDesc d = geo_gemm_desc();
     d.M = (int)MP; d.N = D; d.K = KPE; d.groups = G;
     d.a_rs = KPE; d.a_cs = 1; d.b_rs = 1; d.b_cs = KPE;
     d.ldc = D;
@@ -409,14 +459,14 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
       d.A[g] = patches[g];
       d.B[g] = weight_ptr(gs[g], at, OFF_WPE);
       d.bias[g] = gs[g].params + OFF_BPE;
-      d.aux[g] = gs[g].params + OFF_POS;
+      d.aux[g] = pos[g] ? pos[g] : gs[g].params + OFF_POS;
       d.out[g] = two_pass ? tmp : x_cur[g];
       pp[g] = gs[g].params; tok[g] = tmp;
     }
     V2S_TRY(run_gemm(d, at, at, 0, st, prof::C_PATCH));
     // masked patch rows take mask_token + pos in the kernel that writes the token rows
-    if (two_pass) V2S_TRY(launch_assemble_tokens(pp, tok, x_cur, G, B, st, mask, mask_token));
-    else V2S_TRY(launch_cls_rows(pp, x_cur, G, B, st, mask, mask_token));
+    if (two_pass) V2S_TRY(launch_assemble_tokens(pp, tok, x_cur, G, B, st, mask, mask_token, pos));
+    else V2S_TRY(launch_cls_rows(pp, x_cur, G, B, st, mask, mask_token, pos));
   }
 
   // ---- 12 pre-LN blocks ----
@@ -456,7 +506,7 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
       V2S_TRY(launch_ln_fwd(xin, gam, bet, xn, mean, rstd, G, (int)M, at, st));
     }
     {  // fused QKV projection
-      GemmDesc d = make_gemm_desc();
+      GemmDesc d = geo_gemm_desc();
       d.M = (int)M; d.N = 3 * D; d.K = D; d.groups = G;
       d.a_rs = D; d.a_cs = 1; d.b_rs = 1; d.b_cs = D; d.epi = EPI_STORE; d.ldc = 3 * D;
       for (int g = 0; g < G; ++g) {
@@ -475,7 +525,7 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
       if (na) V2S_TRY(launch_attention_probs(cq, al, ap, na, B, at, st));
     }
     {  // attention output projection + residual
-      GemmDesc d = make_gemm_desc();
+      GemmDesc d = geo_gemm_desc();
       d.M = (int)M; d.N = D; d.K = D; d.groups = G;
       d.a_rs = D; d.a_cs = 1; d.b_rs = 1; d.b_cs = D; d.epi = EPI_BIAS_RESID; d.ldc = D;
       for (int g = 0; g < G; ++g) {
@@ -530,7 +580,7 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
         prof::Scope sc(prof::C_LN_F, (double)M * D * (4 + p.es) * G, st);
         V2S_TRY(launch_ln_fwd(xm, gam, bet, xn2, m2, r2, G, (int)M, at, st));
       }
-      GemmDesc d = make_gemm_desc();   // fc1 + GELU
+      GemmDesc d = geo_gemm_desc();   // fc1 + GELU
       d.M = (int)M; d.N = DF; d.K = D; d.groups = G;
       d.a_rs = D; d.a_cs = 1; d.b_rs = 1; d.b_cs = D; d.epi = EPI_BIAS_GELU; d.ldc = DF;
       for (int g = 0; g < G; ++g) {
@@ -540,7 +590,7 @@ static int backbone_forward_impl(const v2s_group_t* gs, const v2s_group_outputs_
       V2S_TRY(run_gemm(d, at, at, at, st, prof::C_FC1));
     }
     {  // fc2 + residual
-      GemmDesc d = make_gemm_desc();
+      GemmDesc d = geo_gemm_desc();
       d.M = (int)M; d.N = D; d.K = DF; d.groups = G;
       d.a_rs = DF; d.a_cs = 1; d.b_rs = 1; d.b_cs = DF; d.epi = EPI_BIAS_RESID; d.ldc = D;
       for (int g = 0; g < G; ++g) {
@@ -580,6 +630,8 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
   bool masked_in = false;
   for (int i = 0; i < G_in && i < MAXG; ++i) {
     V2S_TRY(check_outputs(outs_in ? &outs_in[i] : nullptr, gs_in[i], i, true));
+    if (gs_in[i].slot >= 0 && gs_in[i].dfeat) V2S_TRY(refuse_image_size("backbone_backward: the pooled-feature gradient (dfeat)"));
+    if (gs_in[i].slot >= 0 && gs_in[i].x_format == 1) V2S_TRY(refuse_image_size("backbone_backward: patch-row inputs (x_format 1)"));
     masked_in = masked_in || (outs_in && outs_in[i].mask);
   }
   if (masked_in && (layer_lo != 0 || layer_hi != NL)) {
@@ -609,6 +661,18 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
     const HiddenRec* rec = find_hidden(ws, gs[g].slot);
     if (rec && rec->h0 != (hid[g] ? hid[g][0] : nullptr)) {
       set_error("backbone_backward: group %d: hidden[] differs from the forward that filled stash slot %d", g, gs[g].slot);
+      return 1;
+    }
+    if (!rec && !geom_is_default(image_geom())) {
+      // the record of its forward is gone (more than 64 workspace slots since): at another size than 224 x 224 the stash
+      // layout cannot be confirmed, so the backward is refused rather than read at a token count it may not have
+      set_error("backbone_backward: group %d: no record of the forward that filled stash slot %d; a backward at %d x %d "
+                "needs one (re-run the forward)", g, gs[g].slot, image_geom().H, image_geom().W);
+      return 1;
+    }
+    if (rec && (rec->img_h != image_geom().H || rec->img_w != image_geom().W)) {
+      set_error("backbone_backward: group %d: the image size (%d x %d) differs from the forward that filled stash slot %d "
+                "(%d x %d)", g, image_geom().H, image_geom().W, gs[g].slot, rec->img_h, rec->img_w);
       return 1;
     }
     if (rec && rec->mask != mask[g]) {
@@ -676,7 +740,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       prof::Scope sc(prof::C_COLSUM, (double)M * n_out * p.es * G, st);
       V2S_TRY(launch_colsum(src, dst, G, (int)M, n_out, at, st, det));
     }
-    GemmDesc d = make_gemm_desc();
+    GemmDesc d = geo_gemm_desc();
     d.M = n_out; d.N = k_in; d.K = (remap || compact) ? (int)MP : (int)M; d.groups = G;
     d.a_rs = 1; d.a_cs = n_out; d.b_rs = k_in; d.b_cs = 1;
     d.a_remap = remap ? 2 : 0;
@@ -705,7 +769,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
   auto wgrad2 = [&](void* const* dy1, int n_out1, void* const* x1, int k_in1, int64_t goff1, int64_t bias1,
                     void* const* dy2, int n_out2, void* const* x2, int k_in2, int64_t goff2, int64_t bias2) -> int {
     if (!weight_grads) return 0;
-    GemmDesc d = make_gemm_desc();
+    GemmDesc d = geo_gemm_desc();
     d.M = n_out1; d.N = k_in1; d.K = (int)M; d.groups = 2 * G;
     d.a_rs = 1; d.a_cs = n_out1; d.b_rs = k_in1; d.b_cs = 1;
     d.M2 = n_out2; d.N2 = k_in2;
@@ -724,7 +788,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
   // every launch waits.
   auto dgrad = [&](void* const* dy, int n_out, int64_t woff, int k_in, void* const* out, int epi,
                    void* const* aux, bool late = false) -> int {
-    GemmDesc d = make_gemm_desc();
+    GemmDesc d = geo_gemm_desc();
     d.M = (int)M; d.N = k_in; d.K = n_out; d.groups = G;
     d.a_rs = n_out; d.a_cs = 1; d.b_rs = k_in; d.b_cs = 1;
     d.epi = epi; d.ldc = k_in; d.late_wait = (late && weight_grads) ? 1 : 0;
@@ -848,8 +912,19 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       pt[g] = gs[g].x_format == 1 ? const_cast<void*>(gs[g].x) : static_cast<void*>(sb(g, p.s_patches));
       if (dpix[g]) px[npx++] = g;
     }
-    if (weight_grads) V2S_TRY(launch_embed_bwd(cdx, gr, G, B, st, det, mask, dmask));
-    GemmDesc dp = make_gemm_desc();
+    if (weight_grads) {
+      // an interpolated table: d pos' rows into the backward scratch, then the interpolation's transpose into d pos
+      float* dpos[MAXG];
+      for (int g = 0; g < G; ++g) dpos[g] = reinterpret_cast<float*>(bb(g, p.b_dpos));
+      V2S_TRY(launch_embed_bwd(cdx, gr, G, B, st, det, mask, dmask, p.interp ? dpos : nullptr));
+      if (p.interp) {
+        const float* cd[MAXG];
+        for (int g = 0; g < G; ++g) cd[g] = dpos[g];
+        prof::Scope sc(prof::C_MISC, (double)image_geom().nt * D * 4 * 17 * G, st);
+        V2S_TRY(launch_pos_interp_bwd(cd, gr, G, st));
+      }
+    }
+    GemmDesc dp = geo_gemm_desc();
     dp.M = (int)MP; dp.N = KPE; dp.K = D; dp.groups = npx;
     dp.a_rs = D; dp.a_cs = 1; dp.b_rs = KPE; dp.b_cs = 1; dp.ldc = KPE;
     if (tc) {          // compact the patch rows, then the ordinary tensor-core wgrad
@@ -857,7 +932,7 @@ static int backbone_backward_impl(const v2s_group_t* gs_in, const v2s_group_outp
       for (int g = 0; g < G; ++g) src[g] = dxlp[g];
       V2S_TRY(launch_gather_patch_rows(src, tmp, G, B, at, st, mask));
       if (weight_grads) {
-        GemmDesc d = make_gemm_desc();
+        GemmDesc d = geo_gemm_desc();
         d.M = D; d.N = KPE; d.K = (int)MP; d.groups = G;
         d.a_rs = 1; d.a_cs = D; d.b_rs = KPE; d.b_cs = 1; d.epi = EPI_ACCUM; d.ldc = KPE; d.split_k = split; d.det = det;
         for (int g = 0; g < G; ++g) { d.A[g] = tmp[g]; d.B[g] = pt[g]; d.out[g] = gs[g].grads + OFF_WPE; }
@@ -1080,6 +1155,7 @@ static int mim_forward_impl(const float* hidden, const float* ln_gamma, const fl
     set_error("mim_forward: hidden, LayerNorm and decoder parameters, pixels and reconstruction must be 16-byte aligned");
     return 1;
   }
+  V2S_TRY(refuse_image_size("mim_forward"));
   MimBufs m;
   V2S_TRY(mim_resolve(B, mode, ws, ws_bytes, &m));
   const Plan p = make_plan(B, mode);
@@ -1128,6 +1204,7 @@ static int mim_backward_impl(const float* hidden, const float* ln_gamma, const f
     set_error("mim_backward: hidden, ln_gamma, dhidden and dpixels must be 16-byte aligned");
     return 1;
   }
+  V2S_TRY(refuse_image_size("mim_backward"));
   MimBufs m;
   V2S_TRY(mim_resolve(B, mode, ws, ws_bytes, &m));
   const Plan p = make_plan(B, mode);
@@ -1260,6 +1337,7 @@ static int cls_forward_impl(const float* hidden, const float* ln_gamma, const fl
     set_error("cls_forward: hidden, LayerNorm and classifier parameters and logits must be 16-byte aligned");
     return 1;
   }
+  V2S_TRY(refuse_image_size("cls_forward"));
   ClsBufs c;
   V2S_TRY(cls_resolve(B, N, mode, kind, labels, ws, ws_bytes, &c));
   const int at = make_plan(B, mode).at;
@@ -1304,6 +1382,7 @@ static int cls_backward_impl(const float* hidden, const float* ln_gamma, const f
     set_error("cls_backward: hidden, ln_gamma, cls_w, dlogits, dhidden and d_cls_w must be 16-byte aligned");
     return 1;
   }
+  V2S_TRY(refuse_image_size("cls_backward"));
   ClsBufs c;
   V2S_TRY(cls_resolve(B, N, mode, kind, labels, ws, ws_bytes, &c));
   const bool wgrad = d_cls_w || d_cls_b, lnb = dhidden || d_ln_gamma;
@@ -1607,6 +1686,21 @@ int v2s_set_sm_limit(int n_sms) {
   return 0;
 }
 
+int v2s_set_image_size(int height, int width) {
+  if (height < 16 || width < 16 || height % 16 || width % 16) {
+    set_error("set_image_size: %d x %d: height and width must be positive multiples of 16", height, width);
+    return 1;
+  }
+  const int64_t np = (int64_t)(height / 16) * (width / 16);
+  if (np > NP) {
+    set_error("set_image_size: %d x %d has %lld patches; at most %d (%d tokens with CLS), e.g. 224 x 224, 208 x 208 or "
+              "128 x 384", height, width, (long long)np, NP, NT);
+    return 1;
+  }
+  g_geom = {height, width, height / 16, width / 16, (int)np, (int)np + 1};
+  return 0;
+}
+
 int v2s_set_deterministic(int on) {
   tc_set_deterministic(on);
   return 0;
@@ -1644,7 +1738,8 @@ int v2s_prof_report(char* host_buf, int64_t buf_bytes) {
 }
 
 // test hook: which = 0 forward (qkv -> ctx, lse), 1 backward (qkv, ctx, lse, dctx -> dqkv), 2 probabilities (qkv, lse ->
-// fp32 [batch,3,197,197] in ctx), 3 their gradient (qkv, dctx -> fp32 [batch,3,197,197] in ctx);
+// fp32 [batch,3,N,N] in ctx), 3 their gradient (qkv, dctx -> fp32 [batch,3,N,N] in ctx), N = the token count of the image
+// size v2s_set_image_size set (197 by default);
 // variant 0 = tensor-core kernels, 1 = SIMT reference kernels; bf16 tensors, one backbone
 int v2s_test_attention(int which, const void* qkv, void* ctx, float* lse, const void* dctx, void* dqkv, int batch,
                        int variant, void* stream) {

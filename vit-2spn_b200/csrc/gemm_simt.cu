@@ -9,7 +9,7 @@ namespace {
 
 constexpr int BK = 16, PAD = 4;   // tile = (16*TM) x (16*TM) x 16, 256 threads, TM x TM outputs per thread
 
-__device__ __forceinline__ int64_t remap_row(int64_t r) { return r + r / NP + 1; }
+__device__ __forceinline__ int64_t remap_row(int64_t r, int np) { return r + r / np + 1; }
 
 template <typename TA, typename TB, typename TO, int TM>
 __global__ void __launch_bounds__(256) gemm_simt_kernel(const GemmDesc d) {
@@ -50,8 +50,8 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(const GemmDesc d) {
       const int m = m0 + mm, k = k0 + kk;
       float v = 0.f;
       if (m < d.M && k < k_end) {
-        const int64_t row = d.a_remap == 1 ? remap_row(m) : (int64_t)m;
-        const int64_t col = d.a_remap == 2 ? remap_row(k) : (int64_t)k;
+        const int64_t row = d.a_remap == 1 ? remap_row(m, d.np) : (int64_t)m;
+        const int64_t col = d.a_remap == 2 ? remap_row(k, d.np) : (int64_t)k;
         v = to_f<TA>(A[row * d.a_rs + col * d.a_cs]);
       }
       ra[i] = v;
@@ -64,7 +64,7 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(const GemmDesc d) {
       const int n = n0 + nn, k = k0 + kk;
       float v = 0.f;
       if (n < d.N && k < k_end) {
-        const int64_t krow = d.b_remap ? remap_row(k) : (int64_t)k;
+        const int64_t krow = d.b_remap ? remap_row(k, d.np) : (int64_t)k;
         v = to_f<TB>(B[krow * d.b_rs + (int64_t)n * d.b_cs]);
       }
       rb[i] = v;
@@ -129,10 +129,10 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(const GemmDesc d) {
           out2[idx] = from_f<TO>(gelu_f(v));
           break;
         case EPI_PATCH: {
-          const int b = m / NP, p = m % NP;
+          const int b = m / d.np, p = m % d.np;
           const float* pos = static_cast<const float*>(d.aux[g]);
           v += bias[n] + pos[(int64_t)(1 + p) * D + n];
-          out[((int64_t)b * NT + 1 + p) * d.ldc + n] = from_f<TO>(v);
+          out[((int64_t)b * d.nt + 1 + p) * d.ldc + n] = from_f<TO>(v);
         } break;
         case EPI_DGELU: {
           const TO* u = static_cast<const TO*>(d.aux[g]);

@@ -27,7 +27,7 @@ struct GemmDesc {
   int M, N, K;
   int64_t a_rs, a_cs;  // A(m,k) = A[m*a_rs + k*a_cs]
   int64_t b_rs, b_cs;  // B(k,n) = B[k*b_rs + n*b_cs]
-  int a_remap;         // patch index b*196+p -> token row b*197+1+p: 1 = on A's m index, 2 = on A's k index
+  int a_remap;         // patch index b*np+p -> token row b*nt+1+p: 1 = on A's m index, 2 = on A's k index
   int b_remap;         // same for the K index of B (wgrad of the patch embedding)
   int split_k;         // number of K splits: EPI_ACCUM (atomic adds), or EPI_STORE with split_stride > 0
   int64_t split_stride; // EPI_STORE + split_k: split s writes its partial result at out + s * split_stride (no bias)
@@ -67,6 +67,9 @@ struct GemmDesc {
   const uint8_t* mim_mask;
   void* mim_dsign;
   float* mim_loss_part;
+  // the token geometry of EPI_PATCH and the row remaps (patch index b*np+p -> token row b*nt+1+p) and of EPI_PIXELS (image
+  // img_h x img_w, patch grid img_gw wide): 196 / 197 / 224 x 224 / 14 unless the image size is set otherwise
+  int np, nt, img_h, img_w, img_gw;
 };
 
 inline GemmDesc make_gemm_desc() {
@@ -75,6 +78,7 @@ inline GemmDesc make_gemm_desc() {
   d.alpha = 1.0f;
   d.split_k = 1;
   d.groups = 1;
+  d.np = NP; d.nt = NT; d.img_h = V2S_IMG; d.img_w = V2S_IMG; d.img_gw = V2S_IMG / 16;
   return d;
 }
 

@@ -52,9 +52,10 @@ enum TcEpi : int {
   T_PIXELS = 6,  // fp32 image gradient (EPI_PIXELS): the epilogue threads store their rows straight to global memory
   T_MIM = 7,     // SimMIM decoder (EPI_MIM) without a mask: + bias, the fp32 reconstruction straight to NCHW (as T_PIXELS)
   T_MIM_LOSS = 8,  // T_MIM + masked L1 partial sums per output tile and the sign(r - x) rows for the backward
+  T_PIXELS_VAR = 9,  // T_PIXELS at another image size (v2s_set_image_size): the patch grid and image from TcParams
 };
 // the epilogues that store from registers straight to global memory (no staging ring, no store warps)
-constexpr bool direct_epi(int e) { return e == T_PIXELS || e == T_MIM || e == T_MIM_LOSS; }
+constexpr bool direct_epi(int e) { return e == T_PIXELS || e == T_MIM || e == T_MIM_LOSS || e == T_PIXELS_VAR; }
 
 // per-variant epilogue staging: a ring of NSTG buffers of STG bytes per epilogue group.  The residual variant
 // (auxiliary operand prefetched two chunks ahead into the ring) and the plain bf16 store use 3 buffers;
@@ -101,6 +102,8 @@ struct alignas(64) TcParams {
   const uint8_t* mim_mask;
   void* mim_dsign;
   float* mim_loss_part;
+  // T_PIXELS_VAR: image height and width, patch-grid width, patches per image
+  int img_h, img_w, img_gw, img_np;
 };
 
 
@@ -592,20 +595,24 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
       long long* d = p.dbg + 8 + (threadIdx.x == 128 ? 0 : 8);
       d[0] = e_tfull; d[1] = e_aux; d[2] = e_pub; d[3] = e_ld; d[4] = clock64() - epi_t0; d[5] = cnt;
     }
-  } else if (EPI == T_PIXELS && warp >= 4) {
+  } else if ((EPI == T_PIXELS || EPI == T_PIXELS_VAR) && warp >= 4) {
     // ================= image-gradient epilogue (EPI_PIXELS) =================
     // The TMEM drain of the epilogue above (group ge = accumulator stage, warps w and w+4 = lane quarter w%4 and the two
     // 16-column halves of each chunk) without staging: row m = (b, py, px), columns [colh, colh + 16) = (c, ky, kx 0..15)
     // are 64 contiguous bytes of image row py*16 + ky, stored straight from registers.  The 32 lanes of a warp are
     // consecutive rows, i.e. mostly consecutive px, so the warp's four 16-byte stores fill one 2 KB run of 64-byte
     // segments (the stride-16 patch convolution's col2im is a pure permutation).
+    // T_PIXELS_VAR: the same at the image size in TcParams (W a multiple of 16 keeps every 64-byte run 16-byte aligned)
+    constexpr bool VARG = EPI == T_PIXELS_VAR;
+    const int g_np = VARG ? p.img_np : NP, g_gw = VARG ? p.img_gw : 14;
+    const int IH = VARG ? p.img_h : V2S_IMG, IW = VARG ? p.img_w : V2S_IMG;
     const int ge = (warp - 4) >> 3, q = warp & 3, hf = ((warp - 4) >> 2) & 1, row = q * 32 + lane;
     uint32_t acc_phase = 0;
     int g, m_tile, split, n_tile;
     for (int i = ge; tile_at(i, g, m_tile, split, n_tile); i += 2) {
       const int m = m_tile * BM + row;
-      const int b = m / NP, t = m - b * NP, py = t / 14, px = t - py * 14;
-      float* img = p.pixels[g] + (int64_t)b * 3 * V2S_IMG * V2S_IMG + py * 16 * V2S_IMG + px * 16;
+      const int b = m / g_np, t = m - b * g_np, py = t / g_gw, px = t - py * g_gw;
+      float* img = p.pixels[g] + (int64_t)b * 3 * IH * IW + py * 16 * IW + px * 16;
       ptx::mbar_wait(&tfull_bar[ge], acc_phase, p.err_flag, 4);
       acc_phase ^= 1;
       ptx::tc_fence_after();
@@ -621,7 +628,7 @@ __global__ void __launch_bounds__(N_THREADS, 1) gemm_tc_kernel(const __grid_cons
           if (lane == 0) ptx::mbar_arrive(&tempty_bar[ge]);
         }
         if (m < p.M) {
-          float4* dst = reinterpret_cast<float4*>(img + (colh >> 8) * V2S_IMG * V2S_IMG + ((colh >> 4) & 15) * V2S_IMG);
+          float4* dst = reinterpret_cast<float4*>(img + (colh >> 8) * IH * IW + ((colh >> 4) & 15) * IW);
 #pragma unroll
           for (int j = 0; j < 4; ++j)
             dst[j] = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]),
@@ -980,14 +987,16 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
     case EPI_STORE: epi = T_STORE; break;
     case EPI_BIAS_RESID: epi = T_RESID; break;
     case EPI_ACCUM: epi = T_ACCUM; break;
-    case EPI_PIXELS: epi = T_PIXELS; break;
+    case EPI_PIXELS: epi = (d.img_h == V2S_IMG && d.img_w == V2S_IMG) ? T_PIXELS : T_PIXELS_VAR; break;
     case EPI_MIM: epi = d.mim_mask ? T_MIM_LOSS : T_MIM; break;
     default: return 0;
   }
   if (d.alpha != 1.0f) return 0;
   const bool out_bf16 = (to != 0);                        // 16-bit output (bf16 or fp16, as the operands)
-  if (epi == T_PIXELS && (out_bf16 || d.M % NP || d.N != KPE || d.ldc != KPE || d.a_remap || d.b_remap)) {
-    set_error("gemm_tc: the image-gradient epilogue needs [B*196, 768] fp32 output (M %d N %d)", d.M, d.N);
+  if ((epi == T_PIXELS || epi == T_PIXELS_VAR) &&
+      (out_bf16 || d.M % d.np || d.N != KPE || d.ldc != KPE || d.a_remap || d.b_remap || d.img_w % 16 || d.img_h % 16 ||
+       d.np != (d.img_h / 16) * (d.img_w / 16) || d.img_gw != d.img_w / 16)) {
+    set_error("gemm_tc: the image-gradient epilogue needs [B*np, 768] fp32 output (M %d N %d, np %d)", d.M, d.N, d.np);
     return 1;
   }
   if ((epi == T_MIM || epi == T_MIM_LOSS) &&
@@ -1062,14 +1071,14 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
     else V2S_TRY(get_map(&p.tmA[g], d.A[g], d.M, d.K, a_ld, 64, BK, true, CU_TENSOR_MAP_SWIZZLE_128B));
     if (!b_mn) V2S_TRY(get_map(&p.tmB[g], d.B[g], d.K, d.N, b_ld, BK, BN, true, CU_TENSOR_MAP_SWIZZLE_128B));
     else V2S_TRY(get_map(&p.tmB[g], d.B[g], d.N, d.K, b_ld, 64, BK, true, CU_TENSOR_MAP_SWIZZLE_128B));
-    if (epi == T_PIXELS || epi == T_MIM || epi == T_MIM_LOSS) {
+    if (direct_epi(epi)) {
       if ((reinterpret_cast<uintptr_t>(d.out[g]) | reinterpret_cast<uintptr_t>(d.bias[g]) | reinterpret_cast<uintptr_t>(d.mim_x) |
            reinterpret_cast<uintptr_t>(d.mim_dsign)) & 15) {
         set_error("gemm_tc: image, bias and sign rows of a direct-store epilogue must be 16-byte aligned");
         return 1;
       }
       p.pixels[g] = static_cast<float*>(d.out[g]);
-      if (epi != T_PIXELS) {
+      if (epi == T_MIM || epi == T_MIM_LOSS) {
         p.bias[g] = d.bias[g];
         p.mim_x = d.mim_x; p.mim_mask = d.mim_mask; p.mim_dsign = d.mim_dsign; p.mim_loss_part = d.mim_loss_part;
       }
@@ -1110,6 +1119,10 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
     case T_RESID: rc = launch_kernel<T_RESID, false>(p, lp_f16, stream); break;
     case T_ACCUM_DET: rc = launch_kernel<T_ACCUM_DET, false>(p, lp_f16, stream); break;
     case T_PIXELS: rc = launch_kernel<T_PIXELS, false>(p, lp_f16, stream); break;
+    case T_PIXELS_VAR:
+      p.img_h = d.img_h; p.img_w = d.img_w; p.img_gw = d.img_gw; p.img_np = d.np;
+      rc = launch_kernel<T_PIXELS_VAR, false>(p, lp_f16, stream);
+      break;
     case T_MIM: rc = launch_kernel<T_MIM, false>(p, lp_f16, stream); break;
     case T_MIM_LOSS: rc = launch_kernel<T_MIM_LOSS, false>(p, lp_f16, stream); break;
     default: rc = launch_kernel<T_ACCUM, false>(p, lp_f16, stream); break;
@@ -1121,7 +1134,8 @@ int launch_gemm_tc(const GemmDesc& d, int ta, int tb, int to, cudaStream_t strea
 
 // test hook (v2s_test_gemm): which = 0 NT (A[M,K], B[N,K]), 1 NN/dgrad (A[M,K], B[K,N]),
 // 2 TN/wgrad (A[K,M], B[K,N], out fp32 +=), 3 NT with fp32 out, 4 = 2 plus the bias row sums (+=) at c + M*N,
-// 5 the image gradient (A = patch-row gradient [M = B*196, 192], B = W_pe [192, 768], c fp32 [B,3,224,224] written;
+// 5 the image gradient (A = patch-row gradient [M = B*np, 192], B = W_pe [192, 768], c fp32 [B,3,H,W] written at the
+// image size of v2s_set_image_size;
 // tensor-core path only); variant: 0 = tensor-core path, 1 = SIMT reference.  bf16 operands; out bf16 for which 0/1, fp32 accumulate-into for
 // which 2/4.  Deterministic mode, which 2/4: the caller's c buffer continues with the scratch a backward call takes
 // from its workspace (DetScratch: DET_COUNTERS counters, then gemm_tc_det_part_floats() floats)
@@ -1141,6 +1155,8 @@ int gemm_tc_test(int which, const void* a, const void* b, void* c, int m, int n,
   else if (which == 5) {
     if (n != KPE || k != D || (variant & 1)) { set_error("gemm_tc_test: which 5 is n = 768, k = 192, tensor-core path"); return 1; }
     d.a_rs = k; d.a_cs = 1; d.b_rs = n; d.b_cs = 1; d.epi = EPI_PIXELS; to = 0;
+    const ImageGeom& geo = image_geom();      // images of the size v2s_set_image_size set
+    d.np = geo.np; d.nt = geo.nt; d.img_h = geo.H; d.img_w = geo.W; d.img_gw = geo.gw;
   }
   else { set_error("gemm_tc_test: which must be 0..5"); return 1; }
   // variant: bit 0 = SIMT reference instead of the tensor-core path, bit 1 = fp16 instead of bf16 tensors

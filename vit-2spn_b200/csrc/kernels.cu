@@ -18,12 +18,12 @@ template <typename T, typename S> G4<T> pack4(S const* src, int groups) {
 }
 
 // ------------------------------------------------------------------------------------------
-// im2col: NCHW fp32 image → patch matrix [B*196, 768], k = c*256 + ky*16 + kx
+// im2col: NCHW fp32 image [B,3,H,W] → patch matrix [B*np, 768], k = c*256 + ky*16 + kx
 // ------------------------------------------------------------------------------------------
 template <typename T>
-__global__ void im2col_kernel(G4<const float*> x, G4<T*> out, int B) {
+__global__ void im2col_kernel(G4<const float*> x, G4<T*> out, int B, ImageGeom geo) {
   const int g = blockIdx.y;
-  const int64_t total = (int64_t)B * NP * (KPE / 4);
+  const int64_t total = (int64_t)B * geo.np * (KPE / 4);
   const float* __restrict__ xin = x.p[g];
   T* __restrict__ o = out.p[g];
   for (int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
@@ -31,12 +31,12 @@ __global__ void im2col_kernel(G4<const float*> x, G4<T*> out, int B) {
     const int kx4 = idx % 4;
     const int ky = (idx / 4) % 16;
     const int c = (idx / 64) % 3;
-    const int p = (idx / 192) % NP;
-    const int b = idx / (192 * NP);
-    const int py = p / 14, px = p % 14;
+    const int p = (idx / 192) % geo.np;
+    const int b = idx / (192 * geo.np);
+    const int py = p / geo.gw, px = p % geo.gw;
     const float4 v = *reinterpret_cast<const float4*>(
-        xin + (((int64_t)b * 3 + c) * V2S_IMG + py * 16 + ky) * V2S_IMG + px * 16 + kx4 * 4);
-    T* dst = o + ((int64_t)b * NP + p) * KPE + c * 256 + ky * 16 + kx4 * 4;
+        xin + (((int64_t)b * 3 + c) * geo.H + py * 16 + ky) * geo.W + px * 16 + kx4 * 4);
+    T* dst = o + ((int64_t)b * geo.np + p) * KPE + c * 256 + ky * 16 + kx4 * 4;
     dst[0] = from_f<T>(v.x); dst[1] = from_f<T>(v.y); dst[2] = from_f<T>(v.z); dst[3] = from_f<T>(v.w);
   }
 }
@@ -55,44 +55,49 @@ MaskArgs pack_masks(const uint8_t* const* mask, const float* const* token, int g
 }
 
 // fp32 check mode: the patch GEMM's epilogue wrote hidden[b,1+p,:] = tok + pos[1+p]; this adds the CLS row and, with
-// MASK, overwrites each masked patch row with mask_token + pos[1+p]
+// MASK, overwrites each masked patch row with mask_token + pos[1+p].  pos: the position table [nt,192] (params + OFF_POS,
+// or its interpolation)
 template <bool MASK>
-__global__ void cls_rows_kernel(G4<const float*> params, G4<float*> hidden, MaskArgs mk) {
+__global__ void cls_rows_kernel(G4<const float*> params, G4<const float*> pos, G4<float*> hidden, MaskArgs mk, ImageGeom geo) {
   const int g = blockIdx.y, b = blockIdx.x, n = threadIdx.x;
   const float* p = params.p[g];
-  hidden.p[g][(int64_t)b * NT * D + n] = p[OFF_CLS + n] + p[OFF_POS + n];
+  const float* ps = pos.p[g];
+  hidden.p[g][(int64_t)b * geo.nt * D + n] = p[OFF_CLS + n] + ps[n];
   if constexpr (MASK) {
     const uint8_t* m = mk.mask[g];
     if (!m) return;
     const float t = mk.token[g][n];
-    for (int q = 0; q < NP; ++q)
-      if (m[(int64_t)b * NP + q]) hidden.p[g][((int64_t)b * NT + 1 + q) * D + n] = t + p[OFF_POS + (int64_t)(1 + q) * D + n];
+    for (int q = 0; q < geo.np; ++q)
+      if (m[(int64_t)b * geo.np + q]) hidden.p[g][((int64_t)b * geo.nt + 1 + q) * D + n] = t + ps[(int64_t)(1 + q) * D + n];
   }
 }
 
 // hidden[b,0,:] = cls + pos[0];  hidden[b,1+p,:] = tok[b*196+p,:] + pos[1+p]   (HF:117-124)
 // MASK: a masked patch row takes mask_token + pos[1+p] instead (HF:ViTEmbeddings.forward, as a select)
 // one float4 per thread; blockIdx.y = image, blockIdx.z = backbone
+// pos: the position table [nt,192] (params + OFF_POS, or its interpolation)
 template <bool MASK>
-__global__ void __launch_bounds__(256) assemble_tokens_kernel(G4<const float*> params, G4<const float*> tok,
-                                                              G4<float*> hidden, MaskArgs mk) {
+__global__ void __launch_bounds__(256) assemble_tokens_kernel(G4<const float*> params, G4<const float*> postab,
+                                                              G4<const float*> tok, G4<float*> hidden, MaskArgs mk,
+                                                              ImageGeom geo) {
   const int g = blockIdx.z, b = blockIdx.y;
   const float* __restrict__ p = params.p[g];
+  const float* __restrict__ ps = postab.p[g];
   const float* __restrict__ tk = tok.p[g];
   float* __restrict__ h = hidden.p[g];
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < NT * (D / 4); i += gridDim.x * blockDim.x) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < geo.nt * (D / 4); i += gridDim.x * blockDim.x) {
     const int t = i / (D / 4), c = (i % (D / 4)) * 4;
-    const float4 pos = *reinterpret_cast<const float4*>(p + OFF_POS + (int64_t)t * D + c);
+    const float4 pos = *reinterpret_cast<const float4*>(ps + (int64_t)t * D + c);
     float4 v;
     if constexpr (MASK) {
-      const float* src = (t == 0) ? p + OFF_CLS + c : tk + ((int64_t)b * NP + t - 1) * D + c;
-      if (t > 0 && mk.mask[g] && mk.mask[g][(int64_t)b * NP + t - 1]) src = mk.token[g] + c;
+      const float* src = (t == 0) ? p + OFF_CLS + c : tk + ((int64_t)b * geo.np + t - 1) * D + c;
+      if (t > 0 && mk.mask[g] && mk.mask[g][(int64_t)b * geo.np + t - 1]) src = mk.token[g] + c;
       v = *reinterpret_cast<const float4*>(src);
     } else {
       v = (t == 0) ? *reinterpret_cast<const float4*>(p + OFF_CLS + c)
-                   : *reinterpret_cast<const float4*>(tk + ((int64_t)b * NP + t - 1) * D + c);
+                   : *reinterpret_cast<const float4*>(tk + ((int64_t)b * geo.np + t - 1) * D + c);
     }
-    *reinterpret_cast<float4*>(h + ((int64_t)b * NT + t) * D + c) =
+    *reinterpret_cast<float4*>(h + ((int64_t)b * geo.nt + t) * D + c) =
         make_float4(v.x + pos.x, v.y + pos.y, v.z + pos.z, v.w + pos.w);
   }
 }
@@ -100,32 +105,33 @@ __global__ void __launch_bounds__(256) assemble_tokens_kernel(G4<const float*> p
 // compact the patch-token rows of a [B,197,192] tensor into [B*196,192] (drops the CLS rows); 8 bytes per thread
 // MASK: the rows of masked patches are written as zeros (no gradient reaches W_pe, b_pe or the pixels through them)
 template <typename T, bool MASK>
-__global__ void __launch_bounds__(256) gather_patch_rows_kernel(G4<const T*> src, G4<T*> dst, MaskArgs mk) {
+__global__ void __launch_bounds__(256) gather_patch_rows_kernel(G4<const T*> src, G4<T*> dst, MaskArgs mk, ImageGeom geo) {
   const int g = blockIdx.z, b = blockIdx.y;
   constexpr int V = 8 / sizeof(T);                 // elements per 8-byte access
-  const T* __restrict__ s = src.p[g] + ((int64_t)b * NT + 1) * D;
-  T* __restrict__ d = dst.p[g] + (int64_t)b * NP * D;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < NP * D / V; i += gridDim.x * blockDim.x) {
+  const T* __restrict__ s = src.p[g] + ((int64_t)b * geo.nt + 1) * D;
+  T* __restrict__ d = dst.p[g] + (int64_t)b * geo.np * D;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < geo.np * D / V; i += gridDim.x * blockDim.x) {
     if constexpr (MASK)
-      if (mk.mask[g] && mk.mask[g][(int64_t)b * NP + i / (D / V)]) { reinterpret_cast<uint2*>(d)[i] = make_uint2(0u, 0u); continue; }
+      if (mk.mask[g] && mk.mask[g][(int64_t)b * geo.np + i / (D / V)]) { reinterpret_cast<uint2*>(d)[i] = make_uint2(0u, 0u); continue; }
     reinterpret_cast<uint2*>(d)[i] = reinterpret_cast<const uint2*>(s)[i];
   }
 }
 
-// the inverse permutation of im2col (stride = kernel, no overlap-add): patch rows [B*196, 768] fp32 -> NCHW fp32
-// [B,3,224,224]; one float4 of the image per thread, so the stores are contiguous (fp32 check mode's image gradient)
-__global__ void __launch_bounds__(256) col2im_kernel(G4<const float*> rows, G4<float*> img, int B) {
+// the inverse permutation of im2col (stride = kernel, no overlap-add): patch rows [B*np, 768] fp32 -> NCHW fp32
+// [B,3,H,W]; one float4 of the image per thread, so the stores are contiguous (fp32 check mode's image gradient)
+__global__ void __launch_bounds__(256) col2im_kernel(G4<const float*> rows, G4<float*> img, int B, ImageGeom geo) {
   const int g = blockIdx.y;
   const float* __restrict__ src = rows.p[g];
   float* __restrict__ dst = img.p[g];
-  const int64_t total = (int64_t)B * 3 * V2S_IMG * (V2S_IMG / 4);
+  const int W4 = geo.W / 4;
+  const int64_t total = (int64_t)B * 3 * geo.H * W4;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-    const int x4 = i % (V2S_IMG / 4), y = (i / (V2S_IMG / 4)) % V2S_IMG;
-    const int c = (i / (V2S_IMG * V2S_IMG / 4)) % 3;
-    const int64_t b = i / (3 * V2S_IMG * V2S_IMG / 4);
+    const int x4 = i % W4, y = (i / W4) % geo.H;
+    const int c = (i / ((int64_t)geo.H * W4)) % 3;
+    const int64_t b = i / (3 * (int64_t)geo.H * W4);
     const int px = x4 / 4, py = y / 16;
     reinterpret_cast<float4*>(dst)[i] = *reinterpret_cast<const float4*>(
-        src + (b * NP + py * 14 + px) * KPE + c * 256 + (y % 16) * 16 + (x4 % 4) * 4);
+        src + (b * geo.np + py * geo.gw + px) * KPE + c * 256 + (y % 16) * 16 + (x4 % 4) * 4);
   }
 }
 
@@ -454,18 +460,20 @@ __global__ void pool_fwd_kernel(G4<const float*> hidden, G4<float*> feat, G4<int
   feat.p[g][(int64_t)b * stride.p[g] + n] = s * (1.0f / NT);
 }
 
-// dx[b,t,:] = dfeat[b,:] / 197 (+ dhidden[b,t,:]); also the activation-type copy.  float4 per thread.
+// dx[b,t,:] = dfeat[b,:] / 197 (+ dhidden[b,t,:]) over the nt tokens of the image size; also the activation-type copy.
+// float4 per thread.  dfeat (the pooled feature) exists at 224 x 224 only, hence the constant 1/197; at other sizes this
+// kernel starts the backward from d hidden_states[12] alone.
 template <typename T>
 __global__ void __launch_bounds__(256) pool_bwd_kernel(G4<const float*> dfeat, G4<int64_t> stride, G4<const float*> dhidden,
-                                                       G4<float*> dx, G4<T*> dx_lp) {
+                                                       G4<float*> dx, G4<T*> dx_lp, int nt) {
   const int g = blockIdx.z, b = blockIdx.y;
   const float* __restrict__ df = dfeat.p[g];
   const float* __restrict__ dh = dhidden.p[g];
   float* __restrict__ o = dx.p[g];
   T* __restrict__ ol = dx_lp.p[g];
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < NT * (D / 4); i += gridDim.x * blockDim.x) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nt * (D / 4); i += gridDim.x * blockDim.x) {
     const int c = (i % (D / 4)) * 4;
-    const int64_t idx = (int64_t)b * NT * D + (int64_t)i * 4;
+    const int64_t idx = (int64_t)b * nt * D + (int64_t)i * 4;
     float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
     if (df) {
       const float4 f = *reinterpret_cast<const float4*>(df + (int64_t)b * stride.p[g] + c);
@@ -480,29 +488,32 @@ __global__ void __launch_bounds__(256) pool_bwd_kernel(G4<const float*> dfeat, G
   }
 }
 
-// d pos / d cls / d patch-bias from the gradient of the embedding output
+// d pos / d cls / d patch-bias from the gradient of the embedding output.  dpos (per group): where the position-table
+// gradient goes -- grads + OFF_POS (+=), or with pos_set the rows of d pos' [nt,192] of an interpolated table (=)
 // DET: the patch-bias sum over the 196 patch tokens goes through det_part [group][196][192] in token order
 // MASK (groups with a mask): d patch-bias sums the unmasked (image, patch) rows only; the masked ones are summed into
 // d mask_token (dtok; NULL: not wanted).  DET then carries both sums per token, det_part [group][196][384], through the
 // same fixed-order reduction with twice the shared rows, so that d patch-bias keeps the unmasked kernel's order and bits.
 template <bool DET, bool MASK>
 __global__ void embed_bwd_kernel(G4<const float*> dx, G4<float*> grads, int B, float* det_part, unsigned* det_counters,
-                                 MaskArgs mk, G4<float*> dtok) {
+                                 MaskArgs mk, G4<float*> dtok, G4<float*> dpos, int pos_set, ImageGeom geo) {
   const int g = blockIdx.y, t = blockIdx.x, n = threadIdx.x;
   const float* d = dx.p[g] + (int64_t)t * D + n;
   float s = 0.f, sm = 0.f;
   const uint8_t* m = MASK && t > 0 ? mk.mask[g] : nullptr;
   if (MASK && m) {
     for (int b = 0; b < B; ++b) {
-      const float v = d[(int64_t)b * NT * D];
-      if (m[(int64_t)b * NP + t - 1]) sm += v; else s += v;
+      const float v = d[(int64_t)b * geo.nt * D];
+      if (m[(int64_t)b * geo.np + t - 1]) sm += v; else s += v;
     }
   } else {
-    for (int b = 0; b < B; ++b) s += d[(int64_t)b * NT * D];
+    for (int b = 0; b < B; ++b) s += d[(int64_t)b * geo.nt * D];
   }
   float* gr = grads.p[g];
   float* dt = MASK ? dtok.p[g] : nullptr;
-  gr[OFF_POS + (int64_t)t * D + n] += MASK ? s + sm : s;
+  float* dp = dpos.p[g] + (int64_t)t * D + n;
+  if (pos_set) *dp = MASK ? s + sm : s;
+  else *dp += MASK ? s + sm : s;
   if (t == 0) gr[OFF_CLS + n] += s;
   else if (!DET) {
     atomicAdd(gr + OFF_BPE + n, s);
@@ -512,10 +523,10 @@ __global__ void embed_bwd_kernel(G4<const float*> dx, G4<float*> grads, int B, f
     if (t == 0) return;
     constexpr int W = MASK ? 2 * D : D;          // floats per partial row
     __shared__ __align__(16) float red[8 * W];
-    float* part = det_part + (int64_t)g * NP * W;
+    float* part = det_part + (int64_t)g * geo.np * W;
     part[(int64_t)(t - 1) * W + n] = s;
     if constexpr (MASK) part[(int64_t)(t - 1) * W + D + n] = sm;
-    det_reduce_rows(part, W, NP, det_counters + g, red, 8 * W, [gr, dt](int c, float v) {
+    det_reduce_rows(part, W, geo.np, det_counters + g, red, 8 * W, [gr, dt](int c, float v) {
       if (c < D) gr[OFF_BPE + c] += v;
       else if (dt) dt[c - D] += v;
     });
@@ -528,15 +539,15 @@ __global__ void embed_bwd_kernel(G4<const float*> dx, G4<float*> grads, int B, f
 constexpr int ASTR = DH + 1;  // odd row stride: conflict-free when lanes walk rows
 
 template <typename T>
-__global__ void __launch_bounds__(256) attn_fwd_simt_kernel(G4<const T*> qkv, G4<T*> ctx, G4<float*> lse) {
+__global__ void __launch_bounds__(256) attn_fwd_simt_kernel(G4<const T*> qkv, G4<T*> ctx, G4<float*> lse, int nt) {
   extern __shared__ float sm[];
   float* Ks = sm;                    // [197][65]
   float* Vs = Ks + NT * ASTR;        // [197][65]
   float* Ps = Vs + NT * ASTR;        // [8][200]
   float* Qs = Ps + 8 * 200;          // [8][64]
   const int h = blockIdx.x, b = blockIdx.y, g = blockIdx.z;
-  const T* base = qkv.p[g] + (int64_t)b * NT * 3 * D;
-  for (int i = threadIdx.x; i < NT * DH; i += blockDim.x) {
+  const T* base = qkv.p[g] + (int64_t)b * nt * 3 * D;
+  for (int i = threadIdx.x; i < nt * DH; i += blockDim.x) {
     const int t = i / DH, d = i % DH;
     Ks[t * ASTR + d] = to_f<T>(base[(int64_t)t * 3 * D + D + h * DH + d]);
     Vs[t * ASTR + d] = to_f<T>(base[(int64_t)t * 3 * D + 2 * D + h * DH + d]);
@@ -546,12 +557,12 @@ __global__ void __launch_bounds__(256) attn_fwd_simt_kernel(G4<const T*> qkv, G4
   float* P = Ps + warp * 200;
   float* Q = Qs + warp * DH;
   const float scale = 0.125f;  // 64^-0.5
-  for (int i = warp; i < NT; i += 8) {
+  for (int i = warp; i < nt; i += 8) {
     Q[lane] = to_f<T>(base[(int64_t)i * 3 * D + h * DH + lane]);
     Q[lane + 32] = to_f<T>(base[(int64_t)i * 3 * D + h * DH + lane + 32]);
     __syncwarp();
     float mx = -INFINITY;
-    for (int j = lane; j < NT; j += 32) {
+    for (int j = lane; j < nt; j += 32) {
       float s = 0.f;
 #pragma unroll 16
       for (int d = 0; d < DH; ++d) s = fmaf(Q[d], Ks[j * ASTR + d], s);
@@ -561,20 +572,20 @@ __global__ void __launch_bounds__(256) attn_fwd_simt_kernel(G4<const T*> qkv, G4
     }
     mx = warp_max(mx);
     float sum = 0.f;
-    for (int j = lane; j < NT; j += 32) { const float e = expf(P[j] - mx); P[j] = e; sum += e; }
+    for (int j = lane; j < nt; j += 32) { const float e = expf(P[j] - mx); P[j] = e; sum += e; }
     sum = warp_sum(sum);
     __syncwarp();
     const float inv = 1.0f / sum;
     float o0 = 0.f, o1 = 0.f;
-    for (int j = 0; j < NT; ++j) {
+    for (int j = 0; j < nt; ++j) {
       const float p = P[j];
       o0 = fmaf(p, Vs[j * ASTR + lane], o0);
       o1 = fmaf(p, Vs[j * ASTR + lane + 32], o1);
     }
-    T* out = ctx.p[g] + ((int64_t)b * NT + i) * D + h * DH;
+    T* out = ctx.p[g] + ((int64_t)b * nt + i) * D + h * DH;
     out[lane] = from_f<T>(o0 * inv);
     out[lane + 32] = from_f<T>(o1 * inv);
-    if (lane == 0 && lse.p[g]) lse.p[g][((int64_t)b * NH + h) * NT + i] = mx + logf(sum);
+    if (lane == 0 && lse.p[g]) lse.p[g][((int64_t)b * NH + h) * nt + i] = mx + logf(sum);
     __syncwarp();
   }
 }
@@ -582,7 +593,7 @@ __global__ void __launch_bounds__(256) attn_fwd_simt_kernel(G4<const T*> qkv, G4
 template <typename T>
 __global__ void __launch_bounds__(256) attn_bwd_simt_kernel(G4<const T*> qkv, G4<const T*> ctx,
                                                             G4<const float*> lse, G4<const T*> dctx,
-                                                            G4<T*> dqkv) {
+                                                            G4<T*> dqkv, int nt) {
   extern __shared__ float sm[];
   float* Qs = sm;                     // [197][65]
   float* Ks = Qs + NT * ASTR;
@@ -593,10 +604,10 @@ __global__ void __launch_bounds__(256) attn_bwd_simt_kernel(G4<const T*> qkv, G4
   float* Ps = Ds + NT;                // [8][200]
   float* dSs = Ps + 8 * 200;          // [8][200]
   const int h = blockIdx.x, b = blockIdx.y, g = blockIdx.z;
-  const T* base = qkv.p[g] + (int64_t)b * NT * 3 * D;
-  const T* ob = ctx.p[g] + (int64_t)b * NT * D + h * DH;
-  const T* dob = dctx.p[g] + (int64_t)b * NT * D + h * DH;
-  for (int i = threadIdx.x; i < NT * DH; i += blockDim.x) {
+  const T* base = qkv.p[g] + (int64_t)b * nt * 3 * D;
+  const T* ob = ctx.p[g] + (int64_t)b * nt * D + h * DH;
+  const T* dob = dctx.p[g] + (int64_t)b * nt * D + h * DH;
+  for (int i = threadIdx.x; i < nt * DH; i += blockDim.x) {
     const int t = i / DH, d = i % DH;
     Qs[t * ASTR + d] = to_f<T>(base[(int64_t)t * 3 * D + h * DH + d]);
     Ks[t * ASTR + d] = to_f<T>(base[(int64_t)t * 3 * D + D + h * DH + d]);
@@ -604,21 +615,21 @@ __global__ void __launch_bounds__(256) attn_bwd_simt_kernel(G4<const T*> qkv, G4
     dOs[t * ASTR + d] = to_f<T>(dob[(int64_t)t * D + d]);
   }
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  for (int t = warp; t < NT; t += 8) {
+  for (int t = warp; t < nt; t += 8) {
     float s = 0.f;
     for (int d = lane; d < DH; d += 32) s += to_f<T>(ob[(int64_t)t * D + d]) * to_f<T>(dob[(int64_t)t * D + d]);
     s = warp_sum(s);
-    if (lane == 0) { Ds[t] = s; Ls[t] = lse.p[g][((int64_t)b * NH + h) * NT + t]; }
+    if (lane == 0) { Ds[t] = s; Ls[t] = lse.p[g][((int64_t)b * NH + h) * nt + t]; }
   }
   __syncthreads();
   float* P = Ps + warp * 200;
   float* dS = dSs + warp * 200;
   const float scale = 0.125f;
-  T* dq_base = dqkv.p[g] + (int64_t)b * NT * 3 * D;
+  T* dq_base = dqkv.p[g] + (int64_t)b * nt * 3 * D;
   // phase A: dQ_i = scale * sum_j dS_ij K_j
-  for (int i = warp; i < NT; i += 8) {
+  for (int i = warp; i < nt; i += 8) {
     const float li = Ls[i], di = Ds[i];
-    for (int j = lane; j < NT; j += 32) {
+    for (int j = lane; j < nt; j += 32) {
       float s = 0.f, dp = 0.f;
 #pragma unroll 16
       for (int d = 0; d < DH; ++d) {
@@ -630,7 +641,7 @@ __global__ void __launch_bounds__(256) attn_bwd_simt_kernel(G4<const T*> qkv, G4
     }
     __syncwarp();
     float a0 = 0.f, a1 = 0.f;
-    for (int j = 0; j < NT; ++j) {
+    for (int j = 0; j < nt; ++j) {
       const float w = dS[j];
       a0 = fmaf(w, Ks[j * ASTR + lane], a0);
       a1 = fmaf(w, Ks[j * ASTR + lane + 32], a1);
@@ -641,8 +652,8 @@ __global__ void __launch_bounds__(256) attn_bwd_simt_kernel(G4<const T*> qkv, G4
     __syncwarp();
   }
   // phase B: dV_j = sum_i P_ij dO_i ; dK_j = scale * sum_i dS_ij Q_i
-  for (int j = warp; j < NT; j += 8) {
-    for (int i = lane; i < NT; i += 32) {
+  for (int j = warp; j < nt; j += 8) {
+    for (int i = lane; i < nt; i += 32) {
       float s = 0.f, dp = 0.f;
 #pragma unroll 16
       for (int d = 0; d < DH; ++d) {
@@ -655,7 +666,7 @@ __global__ void __launch_bounds__(256) attn_bwd_simt_kernel(G4<const T*> qkv, G4
     }
     __syncwarp();
     float v0 = 0.f, v1 = 0.f, k0 = 0.f, k1 = 0.f;
-    for (int i = 0; i < NT; ++i) {
+    for (int i = 0; i < nt; ++i) {
       const float p = P[i], w = dS[i];
       v0 = fmaf(p, dOs[i * ASTR + lane], v0);
       v1 = fmaf(p, dOs[i * ASTR + lane + 32], v1);
@@ -675,15 +686,15 @@ __global__ void __launch_bounds__(256) attn_bwd_simt_kernel(G4<const T*> qkv, G4
 // DP = true: dP = dO V^T, the gradient w.r.t. the probabilities, with a = d ctx [B,197,192] (else a = qkv).
 template <typename T, bool DP>
 __global__ void __launch_bounds__(256) attn_probs_simt_kernel(G4<const T*> qkv, G4<const T*> a, G4<const float*> lse,
-                                                              G4<float*> probs) {
+                                                              G4<float*> probs, int nt) {
   extern __shared__ float sm[];
   float* Ks = sm;                    // [197][65]: K, or V (DP)
   float* Qs = Ks + NT * ASTR;        // [8][64]: rows of Q, or of d ctx (DP)
   const int h = blockIdx.x, b = blockIdx.y, g = blockIdx.z;
   constexpr int A_LD = DP ? D : 3 * D;
-  const T* base = qkv.p[g] + (int64_t)b * NT * 3 * D;
-  const T* abase = a.p[g] + (int64_t)b * NT * A_LD;
-  for (int i = threadIdx.x; i < NT * DH; i += blockDim.x) {
+  const T* base = qkv.p[g] + (int64_t)b * nt * 3 * D;
+  const T* abase = a.p[g] + (int64_t)b * nt * A_LD;
+  for (int i = threadIdx.x; i < nt * DH; i += blockDim.x) {
     const int t = i / DH, d = i % DH;
     Ks[t * ASTR + d] = to_f<T>(base[(int64_t)t * 3 * D + (DP ? 2 * D : D) + h * DH + d]);
   }
@@ -691,13 +702,13 @@ __global__ void __launch_bounds__(256) attn_probs_simt_kernel(G4<const T*> qkv, 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* Q = Qs + warp * DH;
   const float scale = 0.125f;
-  for (int i = warp; i < NT; i += 8) {
+  for (int i = warp; i < nt; i += 8) {
     Q[lane] = to_f<T>(abase[(int64_t)i * A_LD + h * DH + lane]);
     Q[lane + 32] = to_f<T>(abase[(int64_t)i * A_LD + h * DH + lane + 32]);
     __syncwarp();
-    const float li = DP ? 0.f : lse.p[g][((int64_t)b * NH + h) * NT + i];
-    float* out = probs.p[g] + (((int64_t)b * NH + h) * NT + i) * NT;
-    for (int j = lane; j < NT; j += 32) {
+    const float li = DP ? 0.f : lse.p[g][((int64_t)b * NH + h) * nt + i];
+    float* out = probs.p[g] + (((int64_t)b * NH + h) * nt + i) * nt;
+    for (int j = lane; j < nt; j += 32) {
       float s = 0.f;
 #pragma unroll 16
       for (int d = 0; d < DH; ++d) s = fmaf(Q[d], Ks[j * ASTR + d], s);
@@ -1330,38 +1341,138 @@ __global__ void __launch_bounds__(256) cls_head_colsum_kernel(const T* __restric
   db[j] += s;
 }
 
+// ------------------------------------------------------------------------------------------
+// Position-table interpolation (transformers' ViTEmbeddings.interpolate_pos_encoding): row 0 (CLS) is copied, the 14 x 14
+// grid of rows 1..196 is resized to gh x gw as F.interpolate(mode="bicubic", align_corners=False) does it: source
+// coordinate (dst + 0.5) * 14 / out - 0.5, cubic-convolution weights with A = -0.75, taps clamped to [0, 13].
+// ------------------------------------------------------------------------------------------
+constexpr int PG = 14;   // side of the stored grid
+__device__ __forceinline__ void cubic_taps(int dst, int out, int* idx, float* w) {
+  const float scale = (float)PG / (float)out;
+  const float real = scale * ((float)dst + 0.5f) - 0.5f;
+  const float fl = floorf(real);
+  const float t = real - fl;
+  const int i0 = (int)fl;
+  constexpr float A = -0.75f;
+  const float x1 = t + 1.0f, x2 = 1.0f - t, x3 = 2.0f - t;
+  w[0] = ((A * x1 - 5.0f * A) * x1 + 8.0f * A) * x1 - 4.0f * A;
+  w[1] = ((A + 2.0f) * t - (A + 3.0f)) * t * t + 1.0f;
+  w[2] = ((A + 2.0f) * x2 - (A + 3.0f)) * x2 * x2 + 1.0f;
+  w[3] = ((A * x3 - 5.0f * A) * x3 + 8.0f * A) * x3 - 4.0f * A;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) idx[k] = min(max(i0 - 1 + k, 0), PG - 1);
+}
+// the weight of source cell `src` in output `dst` (sum over the taps that clamp onto it)
+__device__ __forceinline__ float cubic_weight(int dst, int out, int src) {
+  int idx[4]; float w[4];
+  cubic_taps(dst, out, idx, w);
+  float r = 0.f;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) r += idx[k] == src ? w[k] : 0.f;
+  return r;
+}
+
+// pos' [nt,192] (fp32) from the flat parameters; one CTA of 192 threads per output row
+__global__ void pos_interp_fwd_kernel(G4<const float*> params, G4<float*> out, ImageGeom geo) {
+  const int g = blockIdx.y, r = blockIdx.x, n = threadIdx.x;
+  const float* pos = params.p[g] + OFF_POS;
+  float* o = out.p[g] + (int64_t)r * D + n;
+  if (r == 0) { *o = pos[n]; return; }
+  const int oy = (r - 1) / geo.gw, ox = (r - 1) % geo.gw;
+  int iy[4], ix[4]; float wy[4], wx[4];
+  cubic_taps(oy, geo.gh, iy, wy);
+  cubic_taps(ox, geo.gw, ix, wx);
+  float acc = 0.f;
+#pragma unroll
+  for (int a = 0; a < 4; ++a) {
+    const float* row = pos + (int64_t)(1 + iy[a] * PG) * D + n;
+    const float v = row[(int64_t)ix[0] * D] * wx[0] + row[(int64_t)ix[1] * D] * wx[1] + row[(int64_t)ix[2] * D] * wx[2] +
+                    row[(int64_t)ix[3] * D] * wx[3];
+    acc += v * wy[a];
+  }
+  *o = acc;
+}
+
+// grads[OFF_POS ...] += the transpose of the interpolation applied to d pos' [nt,192].  A gather: each source cell sums the
+// contributions of every output cell in a fixed order (no atomics, deterministic); one CTA per source row
+__global__ void pos_interp_bwd_kernel(G4<const float*> dpos, G4<float*> grads, ImageGeom geo) {
+  const int g = blockIdx.y, r = blockIdx.x, n = threadIdx.x;
+  const float* dp = dpos.p[g] + n;
+  float* o = grads.p[g] + OFF_POS + (int64_t)r * D + n;
+  if (r == 0) { *o += dp[0]; return; }
+  const int sy = (r - 1) / PG, sx = (r - 1) % PG;
+  float acc = 0.f;
+  for (int oy = 0; oy < geo.gh; ++oy) {
+    const float wy = cubic_weight(oy, geo.gh, sy);
+    if (wy == 0.f) continue;
+    float rs = 0.f;
+    for (int ox = 0; ox < geo.gw; ++ox) {
+      const float wx = cubic_weight(ox, geo.gw, sx);
+      if (wx != 0.f) rs += wx * dp[(int64_t)(1 + oy * geo.gw + ox) * D];
+    }
+    acc += wy * rs;
+  }
+  *o += acc;
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------
 // launchers
 // ------------------------------------------------------------------------------------------
-int launch_im2col(const float* const* x, void* const* out, int groups, int B, int at, cudaStream_t s) {
-  dim3 grid(grid_for((int64_t)B * NP * (KPE / 4), 256, 148 * 16), groups);
-  V2S_DISPATCH_AT(at, im2col_kernel<T><<<grid, 256, 0, s>>>(pack4<const float*>(x, groups), pack4<T*>(out, groups), B));
+int launch_pos_interp_fwd(const float* const* params, float* const* out, int groups, cudaStream_t s) {
+  const ImageGeom& geo = image_geom();
+  pos_interp_fwd_kernel<<<dim3(geo.nt, groups), D, 0, s>>>(pack4<const float*>(params, groups), pack4<float*>(out, groups), geo);
   V2S_LAUNCH_CHECK();
   return 0;
 }
 
+int launch_pos_interp_bwd(const float* const* dpos, float* const* grads, int groups, cudaStream_t s) {
+  pos_interp_bwd_kernel<<<dim3(NT, groups), D, 0, s>>>(pack4<const float*>(dpos, groups), pack4<float*>(grads, groups),
+                                                        image_geom());
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+int launch_im2col(const float* const* x, void* const* out, int groups, int B, int at, cudaStream_t s) {
+  const ImageGeom& geo = image_geom();
+  dim3 grid(grid_for((int64_t)B * geo.np * (KPE / 4), 256, 148 * 16), groups);
+  V2S_DISPATCH_AT(at, im2col_kernel<T><<<grid, 256, 0, s>>>(pack4<const float*>(x, groups), pack4<T*>(out, groups), B, geo));
+  V2S_LAUNCH_CHECK();
+  return 0;
+}
+
+// the position table of each group: pos[g] (an interpolated table), or params[g] + OFF_POS
+static G4<const float*> pos_tables(const float* const* params, const float* const* pos, int groups) {
+  G4<const float*> r = pack4<const float*>(params, groups);
+  for (int g = 0; g < groups; ++g) r.p[g] = pos && pos[g] ? pos[g] : params[g] + OFF_POS;
+  return r;
+}
+
 int launch_cls_rows(const float* const* params, float* const* hidden, int groups, int B, cudaStream_t s,
-                    const uint8_t* const* mask, const float* const* mask_token) {
+                    const uint8_t* const* mask, const float* const* mask_token, const float* const* pos) {
   const MaskArgs mk = pack_masks(mask, mask_token, groups);
+  const G4<const float*> pt = pos_tables(params, pos, groups);
+  const ImageGeom& geo = image_geom();
   if (any_mask(mask, groups))
-    cls_rows_kernel<true><<<dim3(B, groups), D, 0, s>>>(pack4<const float*>(params, groups), pack4<float*>(hidden, groups), mk);
+    cls_rows_kernel<true><<<dim3(B, groups), D, 0, s>>>(pack4<const float*>(params, groups), pt, pack4<float*>(hidden, groups), mk, geo);
   else
-    cls_rows_kernel<false><<<dim3(B, groups), D, 0, s>>>(pack4<const float*>(params, groups), pack4<float*>(hidden, groups), mk);
+    cls_rows_kernel<false><<<dim3(B, groups), D, 0, s>>>(pack4<const float*>(params, groups), pt, pack4<float*>(hidden, groups), mk, geo);
   V2S_LAUNCH_CHECK();
   return 0;
 }
 
 int launch_assemble_tokens(const float* const* params, const float* const* tok, float* const* hidden, int groups,
-                           int B, cudaStream_t s, const uint8_t* const* mask, const float* const* mask_token) {
+                           int B, cudaStream_t s, const uint8_t* const* mask, const float* const* mask_token,
+                           const float* const* pos) {
   const MaskArgs mk = pack_masks(mask, mask_token, groups);
+  const G4<const float*> pt = pos_tables(params, pos, groups);
+  const ImageGeom& geo = image_geom();
   if (any_mask(mask, groups))
-    assemble_tokens_kernel<true><<<dim3(8, B, groups), 256, 0, s>>>(pack4<const float*>(params, groups),
-                                                                  pack4<const float*>(tok, groups), pack4<float*>(hidden, groups), mk);
+    assemble_tokens_kernel<true><<<dim3(8, B, groups), 256, 0, s>>>(pack4<const float*>(params, groups), pt,
+                                                                  pack4<const float*>(tok, groups), pack4<float*>(hidden, groups), mk, geo);
   else
-    assemble_tokens_kernel<false><<<dim3(8, B, groups), 256, 0, s>>>(pack4<const float*>(params, groups),
-                                                                   pack4<const float*>(tok, groups), pack4<float*>(hidden, groups), mk);
+    assemble_tokens_kernel<false><<<dim3(8, B, groups), 256, 0, s>>>(pack4<const float*>(params, groups), pt,
+                                                                   pack4<const float*>(tok, groups), pack4<float*>(hidden, groups), mk, geo);
   V2S_LAUNCH_CHECK();
   return 0;
 }
@@ -1371,17 +1482,18 @@ int launch_gather_patch_rows(const void* const* src, void* const* dst, int group
   dim3 grid(8, B, groups);
   const MaskArgs mk = pack_masks(mask, nullptr, groups);
   if (any_mask(mask, groups)) {
-    V2S_DISPATCH_AT(at, (gather_patch_rows_kernel<T, true><<<grid, 256, 0, s>>>(pack4<const T*>(src, groups), pack4<T*>(dst, groups), mk)));
+    V2S_DISPATCH_AT(at, (gather_patch_rows_kernel<T, true><<<grid, 256, 0, s>>>(pack4<const T*>(src, groups), pack4<T*>(dst, groups), mk, image_geom())));
   } else {
-    V2S_DISPATCH_AT(at, (gather_patch_rows_kernel<T, false><<<grid, 256, 0, s>>>(pack4<const T*>(src, groups), pack4<T*>(dst, groups), mk)));
+    V2S_DISPATCH_AT(at, (gather_patch_rows_kernel<T, false><<<grid, 256, 0, s>>>(pack4<const T*>(src, groups), pack4<T*>(dst, groups), mk, image_geom())));
   }
   V2S_LAUNCH_CHECK();
   return 0;
 }
 
 int launch_col2im(const float* const* rows, float* const* img, int groups, int B, cudaStream_t s) {
-  dim3 grid(grid_for((int64_t)B * 3 * V2S_IMG * (V2S_IMG / 4), 256, 148 * 16), groups);
-  col2im_kernel<<<grid, 256, 0, s>>>(pack4<const float*>(rows, groups), pack4<float*>(img, groups), B);
+  const ImageGeom& geo = image_geom();
+  dim3 grid(grid_for((int64_t)B * 3 * geo.H * (geo.W / 4), 256, 148 * 16), groups);
+  col2im_kernel<<<grid, 256, 0, s>>>(pack4<const float*>(rows, groups), pack4<float*>(img, groups), B, geo);
   V2S_LAUNCH_CHECK();
   return 0;
 }
@@ -1583,25 +1695,30 @@ int launch_pool_bwd(const float* const* dfeat, const int64_t* dfeat_stride, cons
   dim3 grid(8, B, groups);
   V2S_DISPATCH_AT(at, pool_bwd_kernel<T><<<grid, 256, 0, s>>>(pack4<const float*>(dfeat, groups), st,
                                                              pack4<const float*>(dhidden, groups), pack4<float*>(dx, groups),
-                                                             pack4<T*>(dx_lp, groups)));
+                                                             pack4<T*>(dx_lp, groups), image_geom().nt));
   V2S_LAUNCH_CHECK();
   return 0;
 }
 
 int launch_embed_bwd(const float* const* dx, float* const* grads, int groups, int B, cudaStream_t s, const DetScratch* det,
-                     const uint8_t* const* mask, float* const* dmask_token) {
+                     const uint8_t* const* mask, float* const* dmask_token, float* const* dpos) {
   const bool masked = any_mask(mask, groups);
   const MaskArgs mk = pack_masks(mask, nullptr, groups);
   const G4<float*> dt = pack4<float*>(dmask_token, groups);
   const G4<const float*> cdx = pack4<const float*>(dx, groups);
   const G4<float*> gr = pack4<float*>(grads, groups);
+  G4<float*> dp = gr;
+  for (int g = 0; g < groups; ++g) dp.p[g] = dpos ? dpos[g] : grads[g] + OFF_POS;
+  const int pos_set = dpos ? 1 : 0;
+  const ImageGeom& geo = image_geom();
+  const dim3 grid(geo.nt, groups);
   if (det) {
-    if ((int64_t)groups * NP * D * (masked ? 2 : 1) > det->part_floats) { set_error("embed_bwd: deterministic scratch too small"); return 1; }
-    if (masked) embed_bwd_kernel<true, true><<<dim3(NT, groups), D, 0, s>>>(cdx, gr, B, det->part, det->counters, mk, dt);
-    else embed_bwd_kernel<true, false><<<dim3(NT, groups), D, 0, s>>>(cdx, gr, B, det->part, det->counters, mk, dt);
+    if ((int64_t)groups * geo.np * D * (masked ? 2 : 1) > det->part_floats) { set_error("embed_bwd: deterministic scratch too small"); return 1; }
+    if (masked) embed_bwd_kernel<true, true><<<grid, D, 0, s>>>(cdx, gr, B, det->part, det->counters, mk, dt, dp, pos_set, geo);
+    else embed_bwd_kernel<true, false><<<grid, D, 0, s>>>(cdx, gr, B, det->part, det->counters, mk, dt, dp, pos_set, geo);
   } else {
-    if (masked) embed_bwd_kernel<false, true><<<dim3(NT, groups), D, 0, s>>>(cdx, gr, B, nullptr, nullptr, mk, dt);
-    else embed_bwd_kernel<false, false><<<dim3(NT, groups), D, 0, s>>>(cdx, gr, B, nullptr, nullptr, mk, dt);
+    if (masked) embed_bwd_kernel<false, true><<<grid, D, 0, s>>>(cdx, gr, B, nullptr, nullptr, mk, dt, dp, pos_set, geo);
+    else embed_bwd_kernel<false, false><<<grid, D, 0, s>>>(cdx, gr, B, nullptr, nullptr, mk, dt, dp, pos_set, geo);
   }
   V2S_LAUNCH_CHECK();
   return 0;
@@ -1613,7 +1730,7 @@ int launch_attn_fwd_simt(const void* const* qkv, void* const* ctx, float* const*
   dim3 grid(NH, B, groups);
   V2S_DISPATCH_AT(at, {
     V2S_CUDA_OK(cudaFuncSetAttribute(attn_fwd_simt_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attn_fwd_simt_kernel<T><<<grid, 256, smem, s>>>(pack4<const T*>(qkv, groups), pack4<T*>(ctx, groups), pack4<float*>(lse, groups));
+    attn_fwd_simt_kernel<T><<<grid, 256, smem, s>>>(pack4<const T*>(qkv, groups), pack4<T*>(ctx, groups), pack4<float*>(lse, groups), image_geom().nt);
   });
   V2S_LAUNCH_CHECK();
   return 0;
@@ -1627,7 +1744,7 @@ int launch_attn_bwd_simt(const void* const* qkv, const void* const* ctx, const f
     V2S_CUDA_OK(cudaFuncSetAttribute(attn_bwd_simt_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attn_bwd_simt_kernel<T><<<grid, 256, smem, s>>>(pack4<const T*>(qkv, groups), pack4<const T*>(ctx, groups),
                                                    pack4<const float*>(lse, groups), pack4<const T*>(dctx, groups),
-                                                   pack4<T*>(dqkv, groups));
+                                                   pack4<T*>(dqkv, groups), image_geom().nt);
   });
   V2S_LAUNCH_CHECK();
   return 0;
@@ -1640,7 +1757,7 @@ int launch_attn_probs_simt(const void* const* qkv, const float* const* lse, floa
   V2S_DISPATCH_AT(at, {
     V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_simt_kernel<T, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attn_probs_simt_kernel<T, false><<<grid, 256, smem, s>>>(pack4<const T*>(qkv, groups), pack4<const T*>(qkv, groups),
-                                                             pack4<const float*>(lse, groups), pack4<float*>(probs, groups));
+                                                             pack4<const float*>(lse, groups), pack4<float*>(probs, groups), image_geom().nt);
   });
   V2S_LAUNCH_CHECK();
   return 0;
@@ -1653,7 +1770,7 @@ int launch_attn_dprobs_simt(const void* const* qkv, const void* const* dctx, flo
   V2S_DISPATCH_AT(at, {
     V2S_CUDA_OK(cudaFuncSetAttribute(attn_probs_simt_kernel<T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attn_probs_simt_kernel<T, true><<<grid, 256, smem, s>>>(pack4<const T*>(qkv, groups), pack4<const T*>(dctx, groups),
-                                                            G4<const float*>{}, pack4<float*>(dprobs, groups));
+                                                            G4<const float*>{}, pack4<float*>(dprobs, groups), image_geom().nt);
   });
   V2S_LAUNCH_CHECK();
   return 0;
@@ -1663,7 +1780,7 @@ int launch_residual_grad_add(const float* const* dh, float* const* dx, void* con
                              int at, cudaStream_t s, const DetScratch* det) {
   for (int i = 0; i < groups; ++i)
     if (reinterpret_cast<uintptr_t>(dh[i]) & 15) { set_error("hidden-state gradients must be 16-byte aligned"); return 1; }
-  const int rows = B * NT;
+  const int rows = B * image_geom().nt;
   dim3 grid(grid_for(rows, RGA_RL, 148 * 2), groups);
   if (det && (int64_t)groups * grid.x * D > det->part_floats) { set_error("residual_grad_add: deterministic scratch too small"); return 1; }
   if (det) {

@@ -13,11 +13,19 @@ inline bool any_mask(const uint8_t* const* mask, int groups) {
   for (int i = 0; mask && i < groups; ++i) if (mask[i]) return true;
   return false;
 }
+// The kernels that lay out tokens and patches (im2col, cls_rows, assemble_tokens, gather_patch_rows, col2im, embed_bwd,
+// pool_bwd, residual_grad_add and the SIMT attention) work at the image size of image_geom().  pos (optional, per group):
+// an interpolated position table [nt,192] read instead of params + OFF_POS
 int launch_cls_rows(const float* const* params, float* const* hidden, int groups, int B, cudaStream_t s,
-                    const uint8_t* const* mask = nullptr, const float* const* mask_token = nullptr);
+                    const uint8_t* const* mask = nullptr, const float* const* mask_token = nullptr,
+                    const float* const* pos = nullptr);
 int launch_assemble_tokens(const float* const* params, const float* const* tok, float* const* hidden, int groups,
                            int B, cudaStream_t s, const uint8_t* const* mask = nullptr,
-                           const float* const* mask_token = nullptr);
+                           const float* const* mask_token = nullptr, const float* const* pos = nullptr);
+// position-table interpolation to the patch grid of image_geom(): pos' [nt,192] fp32 from params + OFF_POS, and its
+// backward, grads + OFF_POS += the transpose applied to d pos' (fixed order, no atomics)
+int launch_pos_interp_fwd(const float* const* params, float* const* out, int groups, cudaStream_t s);
+int launch_pos_interp_bwd(const float* const* dpos, float* const* grads, int groups, cudaStream_t s);
 // mask: the rows of masked patches are written as zeros
 int launch_gather_patch_rows(const void* const* src, void* const* dst, int groups, int B, int at, cudaStream_t s,
                              const uint8_t* const* mask = nullptr);
@@ -80,10 +88,11 @@ int launch_pool_fwd(const float* const* hidden, float* const* feat, const int64_
 int launch_pool_bwd(const float* const* dfeat, const int64_t* dfeat_stride, const float* const* dhidden,
                     float* const* dx, void* const* dx_lp, int groups, int B, int at, cudaStream_t s);
 // mask: d patch-bias from the unmasked patch rows only; dmask_token (optional, per group) += the column sums of the
-// masked ones
+// masked ones; dpos (optional, per group): the position-table gradient is written (=) to these [nt,192] rows instead of
+// added to grads + OFF_POS
 int launch_embed_bwd(const float* const* dx, float* const* grads, int groups, int B, cudaStream_t s,
                      const DetScratch* det = nullptr, const uint8_t* const* mask = nullptr,
-                     float* const* dmask_token = nullptr);
+                     float* const* dmask_token = nullptr, float* const* dpos = nullptr);
 // dx (fp32, in/out) += dh; dx_lp (activation type, 16-bit modes only) = updated dx; [B,197,192] per group;
 // dcol (optional, per group) += column sums of dh
 int launch_residual_grad_add(const float* const* dh, float* const* dx, void* const* dx_lp, float* const* dcol, int groups, int B,

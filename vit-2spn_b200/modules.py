@@ -219,9 +219,19 @@ def _deterministic():
     return on
 
 
-def _scratch_workspace(device, batch, mode, n_groups, n_saved):
+_DEFAULT_SIZE = (224, 224)
+
+
+def _image_size(size=_DEFAULT_SIZE):
+    """Pass the input image size (H, W) on to the library (``v2s_set_image_size``): called before every call that sizes a
+    workspace or enqueues backbone work, 224 x 224 included, so that the size of one call never reaches another."""
+    check(_lib.lib.v2s_set_image_size(int(size[0]), int(size[1])), "set_image_size")
+
+
+def _scratch_workspace(device, batch, mode, n_groups, n_saved, size=_DEFAULT_SIZE):
     """Persistent scratch for calls that keep nothing across calls (no-grad forwards)."""
-    key = (device, batch, mode, n_groups, n_saved, _deterministic())
+    key = (device, batch, mode, n_groups, n_saved, tuple(size), _deterministic())
+    _image_size(size)
     ws = _workspaces.get(key)
     if ws is None:
         nbytes = lib.v2s_workspace_bytes(batch, mode, n_groups, n_saved)
@@ -237,22 +247,25 @@ def _aligned(ws):
     return ws.data_ptr() + off, ws.numel() - off
 
 
-def _new_workspace(device, batch, mode, n_groups, n_saved):
+def _new_workspace(device, batch, mode, n_groups, n_saved, size=_DEFAULT_SIZE):
     _deterministic()                # the deterministic mode's scratch is part of the size
+    _image_size(size)
     nbytes = lib.v2s_workspace_bytes(batch, mode, n_groups, n_saved)
     if nbytes < 0:
         raise RuntimeError("v2s_workspace_bytes: bad arguments")
     return torch.empty(nbytes + 1024, dtype=torch.uint8, device=device)
 
 
-def _check_images(x, allow_patches=False):
+def _check_images(x, allow_patches=False, size=None):
     if allow_patches and x.dim() == 3 and tuple(x.shape[1:]) == (196, 768) and x.dtype in (torch.bfloat16, torch.float16):
         _require_cuda(x, "patch rows")          # the 16-bit patch matrix of preprocess_u8_patches (v2s_group.x_format 1)
         if x.requires_grad and torch.is_grad_enabled():
             raise ValueError("vit2spn: no gradient w.r.t. 16-bit patch rows; pass fp32 pixel_values [B,3,224,224] to get "
                              "d loss / d pixel_values")
         return x.contiguous()
-    if x.dim() != 4 or tuple(x.shape[1:]) != (3, 224, 224):
+    if size is not None and x.dim() == 4 and tuple(x.shape[1:]) == (3,) + tuple(size):
+        pass                                    # another image size, already checked by ViTModel._check_size
+    elif x.dim() != 4 or tuple(x.shape[1:]) != (3, 224, 224):
         raise ValueError(f"expected pixel_values of shape [B,3,224,224], got {tuple(x.shape)}")
     _require_cuda(x, "pixel_values")
     return x.contiguous().to(torch.float32)
@@ -281,16 +294,19 @@ def _outputs_array(outputs, n):
     return (GroupOutputs * n)(*[o if o is not None else GroupOutputs() for o in outputs])
 
 
-def _run_forward(groups, batch, mode, ws, outputs=None):
+def _run_forward(groups, batch, mode, ws, outputs=None, size=_DEFAULT_SIZE):
+    _image_size(size)
     arr = (Group * len(groups))(*groups)
     base, nbytes = _aligned(ws)
     check(lib.v2s_backbone_forward(arr, _outputs_array(outputs, len(groups)), len(groups), batch, mode,
                                    C.c_void_p(base), nbytes, stream_ptr()), "backbone_forward")
 
 
-def _run_backward(groups, batch, mode, ws, outputs=None, layer_hi=12, layer_lo=0, weight_grads=True):
+def _run_backward(groups, batch, mode, ws, outputs=None, layer_hi=12, layer_lo=0, weight_grads=True, size=_DEFAULT_SIZE):
     """Backward over blocks [layer_lo, layer_hi), highest first; the default range is the whole backward.
-    weight_grads False computes no parameter gradient at all (the groups' grads may be None)."""
+    weight_grads False computes no parameter gradient at all (the groups' grads may be None).  `size`: the image size
+    of the forward."""
+    _image_size(size)
     arr = (Group * len(groups))(*groups)
     base, nbytes = _aligned(ws)
     check(lib.v2s_backbone_backward(arr, _outputs_array(outputs, len(groups)), len(groups), batch, mode,
@@ -426,7 +442,9 @@ class _BackboneFn(torch.autograd.Function):
     retain_grad() was called receives d loss / d probabilities in .grad, as in transformers (one extra kernel per such
     block in the same backward call; blocks at or above the highest layer the loss reaches keep .grad None).  With `mask`
     (uint8 [B,196]) the masked patch embeddings are replaced by `mask_token`, an autograd input whose gradient is
-    returned (v2s_group_outputs.mask / mask_token / dmask_token)."""
+    returned (v2s_group_outputs.mask / mask_token / dmask_token).  An x of another size than 224 x 224 (the
+    interpolate_pos_encoding path, never pooled) runs at N = 1 + (H/16)(W/16) tokens with the interpolated position
+    table (v2s_set_image_size): hidden states [B,N,192], attentions [B,3,N,N], the mask [B,N-1]."""
 
     @staticmethod
     @_with_device_of(lambda ctx, x, *a, **k: x)
@@ -436,18 +454,20 @@ class _BackboneFn(torch.autograd.Function):
         mode = model._mode()
         B = x.shape[0]
         dev = x.device
-        hidden = [torch.empty(B, 197, 192, dtype=torch.float32, device=dev) for _ in range(13)] if want_hidden else None
-        attn = [torch.empty(B, 3, 197, 197, dtype=torch.float32, device=dev) for _ in range(12)] if want_attn else None
+        size = tuple(x.shape[2:]) if x.dim() == 4 else _DEFAULT_SIZE
+        N = 1 + (size[0] // 16) * (size[1] // 16)
+        hidden = [torch.empty(B, N, 192, dtype=torch.float32, device=dev) for _ in range(13)] if want_hidden else None
+        attn = [torch.empty(B, 3, N, N, dtype=torch.float32, device=dev) for _ in range(12)] if want_attn else None
         if pooled:
             out = torch.empty(B, 192, dtype=torch.float32, device=dev)
         elif want_hidden:
             out = hidden[12]
         else:
-            out = torch.empty(B, 197, 192, dtype=torch.float32, device=dev)
+            out = torch.empty(B, N, 192, dtype=torch.float32, device=dev)
         if need_grad:
-            ws = _new_workspace(dev, B, mode, 1, 1)
+            ws = _new_workspace(dev, B, mode, 1, 1, size)
         else:
-            ws = _scratch_workspace(dev, B, mode, 1, 0)
+            ws = _scratch_workspace(dev, B, mode, 1, 0, size)
         g = _group(store, mode, x, 0 if need_grad else -1,
                    hidden=None if pooled or want_hidden else out, feat=out if pooled else None, feat_stride=192)
         o = GroupOutputs()
@@ -460,7 +480,8 @@ class _BackboneFn(torch.autograd.Function):
             if tok.data_ptr() % 16:
                 tok = tok.clone()
             o.mask, o.mask_token = mask.data_ptr(), tok.data_ptr()
-        _run_forward([g], B, mode, ws, [o])
+        _run_forward([g], B, mode, ws, [o], size=size)
+        ctx.size, ctx.N = size, N
         ctx.mask = mask                 # the backward passes the same array (the library checks it)
         ctx.set_materialize_grads(False)
         ctx.model, ctx.pooled, ctx.mode, ctx.B = model, pooled, mode, B
@@ -519,14 +540,14 @@ class _BackboneFn(torch.autograd.Function):
                     if l < start and t is not None and t.retains_grad]
         attn_grads = {}
         for l, _ in retained:
-            attn_grads[l] = torch.empty(ctx.B, 3, 197, 197, dtype=torch.float32, device=ctx.x.device)
+            attn_grads[l] = torch.empty(ctx.B, 3, ctx.N, ctx.N, dtype=torch.float32, device=ctx.x.device)
             o.dattn[l] = attn_grads[l].data_ptr()
-        dx = torch.empty(ctx.B, 3, 224, 224, dtype=torch.float32, device=ctx.x.device) if want_x else None
+        dx = torch.empty(ctx.B, 3, *ctx.size, dtype=torch.float32, device=ctx.x.device) if want_x else None
         dtok = torch.zeros(192, dtype=torch.float32, device=ctx.x.device) if want_t else None
         o.dpixels = dx.data_ptr() if dx is not None else None
         o.mask = ctx.mask.data_ptr() if masked else None
         o.dmask_token = dtok.data_ptr() if dtok is not None else None
-        _run_backward([g], ctx.B, ctx.mode, ctx.ws, [o], weight_grads=want_w or want_t)
+        _run_backward([g], ctx.B, ctx.mode, ctx.ws, [o], weight_grads=want_w or want_t, size=ctx.size)
         ctx.ws = None
         for l, t in retained:          # as the retain_grad hook: set, or accumulate out of place
             t.grad = attn_grads[l] if t.grad is None else t.grad + attn_grads[l]
@@ -701,12 +722,12 @@ class ViTModel(nn.Module):
         a = self.embeddings.cls_token
         return _BackboneFn.apply(x, a, self, True, torch.is_grad_enabled() and (a.requires_grad or x.requires_grad))
 
-    def _check_mask(self, m, batch):
+    def _check_mask(self, m, batch, n_patches=196):
         if getattr(self.embeddings, "mask_token", None) is None:
             raise ValueError("vit2spn: bool_masked_pos needs a mask token: build the model with "
                              "ViTModel(config, use_mask_token=True)")
-        if not isinstance(m, torch.Tensor) or tuple(m.shape) != (batch, 196):
-            raise ValueError(f"vit2spn: bool_masked_pos must be a [B,196] = [{batch},196] tensor, got "
+        if not isinstance(m, torch.Tensor) or tuple(m.shape) != (batch, n_patches):
+            raise ValueError(f"vit2spn: bool_masked_pos must be a [B,{n_patches}] = [{batch},{n_patches}] tensor, got "
                              f"{tuple(m.shape) if isinstance(m, torch.Tensor) else type(m).__name__}")
         if m.dtype.is_floating_point or m.dtype.is_complex:
             raise ValueError(f"vit2spn: bool_masked_pos must be bool, uint8 or an integer type, got {m.dtype}")
@@ -719,15 +740,43 @@ class ViTModel(nn.Module):
                              "the input's device")
         return (m != 0).to(torch.uint8).contiguous()
 
-    def forward(self, pixel_values, output_hidden_states=None, output_attentions=None, *, bool_masked_pos=None, **kw):
+    @staticmethod
+    def _check_size(x, interpolate):
+        """The input-size rules of ``forward``: 224 x 224 without ``interpolate_pos_encoding``; with it H and W multiples
+        of 16 and at most 196 patches (197 tokens).  Returns the number of patches."""
+        if not isinstance(x, torch.Tensor) or x.dim() != 4 or x.shape[1] != 3:
+            return 196                      # _check_images words the error
+        H, W = int(x.shape[2]), int(x.shape[3])
+        if not interpolate:
+            if (H, W) != (224, 224):
+                raise ValueError(f"Input image size ({H}*{W}) doesn't match model (224*224).  Pass "
+                                 "interpolate_pos_encoding=True for other sizes (up to 197 tokens).")
+            return 196
+        if H % 16 or W % 16 or H < 16 or W < 16:
+            raise ValueError(f"vit2spn: with interpolate_pos_encoding the image height and width must be multiples of 16, "
+                             f"got {H}*{W}.  transformers' stride-16 patch convolution ignores the last H mod 16 rows and "
+                             f"W mod 16 columns, so x[..., :{16 * (H // 16)}, :{16 * (W // 16)}] gives the same outputs.")
+        n = (H // 16) * (W // 16)
+        if n > 196:
+            raise ValueError(f"vit2spn: a {H}*{W} input has {n} patches ({n + 1} tokens); the CUDA path runs at most 197 "
+                             "tokens (196 patches), e.g. 224*224, 208*208 or 128*384")
+        return n
+
+    def forward(self, pixel_values, output_hidden_states=None, output_attentions=None, *, bool_masked_pos=None,
+                interpolate_pos_encoding=None, **kw):
         """As ``transformers.ViTModel``: each flag comes from the keyword, else from the config.  The hidden states
         cost no extra kernel work (the residual stream is written into them) but keep 13 x [B,197,192] fp32 alive; the
         attention probabilities are fp32 [B,3,197,197] per block, recomputed by one extra kernel per block.
         ``bool_masked_pos`` ([B,196] bool / uint8 / int on the input's device, nonzero = masked; a model built with
-        ``use_mask_token=True``) replaces those patch embeddings by ``embeddings.mask_token``, as transformers does."""
+        ``use_mask_token=True``) replaces those patch embeddings by ``embeddings.mask_token``, as transformers does.
+        ``interpolate_pos_encoding=True`` accepts fp32 [B,3,H,W] with H and W multiples of 16 and at most 196 patches:
+        the sequence then has N = 1 + (H/16)(W/16) tokens (hidden states [B,N,192], attentions [B,3,N,N], the mask
+        [B,N-1]) and the 14 x 14 position table is resized bicubically to the patch grid, as transformers does (at 224 x
+        224 it is used unchanged)."""
+        n_patches = self._check_size(pixel_values, bool(interpolate_pos_encoding))
         if bool_masked_pos is not None:
-            self._check_mask(bool_masked_pos, pixel_values.shape[0])
-        x = _check_images(pixel_values)
+            self._check_mask(bool_masked_pos, pixel_values.shape[0], n_patches)
+        x = _check_images(pixel_values, size=tuple(pixel_values.shape[2:]) if interpolate_pos_encoding else None)
         a = self.embeddings.cls_token
         want_hidden = bool(self.config.output_hidden_states if output_hidden_states is None else output_hidden_states)
         want_attn = bool(getattr(self.config, "output_attentions", False) if output_attentions is None else output_attentions)
@@ -751,6 +800,7 @@ class ViTModel(nn.Module):
 def _mim_workspace(device, batch, mode, keep):
     """Workspace of the SimMIM head: a fresh one when the forward keeps state for its backward, else a cached scratch."""
     det = _deterministic()                 # the deterministic mode's scratch is part of the size
+    _image_size()
     nbytes = lib.v2s_mim_workspace_bytes(batch, mode)
     if nbytes < 0:
         raise RuntimeError("v2s_mim_workspace_bytes: bad arguments")
@@ -788,6 +838,7 @@ class _MIMHeadFn(torch.autograd.Function):
         loss = torch.empty((), dtype=torch.float32, device=dev) if mask is not None else None
         ws = _mim_workspace(dev, B, mode, keep)
         base, nbytes = _aligned(ws)
+        _image_size()                   # the heads run at 224 x 224 only
         check(lib.v2s_mim_forward(ptr(hidden), ptr(gam), ptr(bet), ptr(w), ptr(b), ptr(xs), ptr(mask), ptr(rec), ptr(loss),
                                   int(keep), B, mode, C.c_void_p(base), nbytes, stream_ptr()), "mim_forward")
         ctx.set_materialize_grads(False)
@@ -820,6 +871,7 @@ class _MIMHeadFn(torch.autograd.Function):
         dw = torch.zeros(768, 192, dtype=torch.float32, device=dev) if need[4] else None
         dbd = torch.zeros(768, dtype=torch.float32, device=dev) if need[5] else None
         base, nbytes = _aligned(ctx.ws)
+        _image_size()                   # the heads run at 224 x 224 only
         check(lib.v2s_mim_backward(ptr(hidden), ptr(gam), ptr(w), ptr(mask), ptr(dl), ptr(dh), ptr(dx), ptr(dg), ptr(db),
                                    ptr(dw), ptr(dbd), ctx.B, ctx.mode, C.c_void_p(base), nbytes, stream_ptr()), "mim_backward")
         ctx.ws = None
@@ -921,6 +973,7 @@ def _cls_workspace(device, batch, num_labels, mode, keep):
     """Workspace of the classification head: a fresh one when the forward keeps state for its backward, else a cached
     scratch."""
     det = _deterministic()                 # the deterministic mode's scratch is part of the size
+    _image_size()
     nbytes = lib.v2s_cls_workspace_bytes(batch, num_labels, mode)
     if nbytes < 0:
         raise RuntimeError("v2s_cls_workspace_bytes: bad arguments")
@@ -953,6 +1006,7 @@ class _ClsHeadFn(torch.autograd.Function):
         loss = torch.empty((), dtype=torch.float32, device=dev) if labels is not None else None
         ws = _cls_workspace(dev, B, N, mode, need_grad)
         base, nbytes = _aligned(ws)
+        _image_size()                   # the heads run at 224 x 224 only
         check(lib.v2s_cls_forward(ptr(hidden), ptr(gam), ptr(bet), ptr(w), ptr(b), N, kind, ptr(labels), ptr(logits),
                                   ptr(loss), int(need_grad), B, mode, C.c_void_p(base), nbytes, stream_ptr()), "cls_forward")
         ctx.set_materialize_grads(False)
@@ -983,6 +1037,7 @@ class _ClsHeadFn(torch.autograd.Function):
         dw = torch.zeros(N, 192, dtype=torch.float32, device=dev) if need[3] else None
         dbc = torch.zeros(N, dtype=torch.float32, device=dev) if need[4] else None
         base, nbytes = _aligned(ctx.ws)
+        _image_size()                   # the heads run at 224 x 224 only
         check(lib.v2s_cls_backward(ptr(hidden), ptr(gam), ptr(w), N, ctx.kind, ptr(labels), ptr(dz), ptr(dl), ptr(dh),
                                    ptr(dg), ptr(db), ptr(dw), ptr(dbc), B, ctx.mode, C.c_void_p(base), nbytes,
                                    stream_ptr()), "cls_backward")
